@@ -5,11 +5,14 @@ GPU generator, ``marl_demandresponse_b200/montecarlo.py``) against the reference
 ``eval_parameters_bangbang_average_consumption`` (:152-230) is taken -- parsed out of the file and executed
 with the real legacy env, controller and config as its globals -- and evaluated on a handful of random
 grid points.  Authoring container only (needs ``/root/reference``); the GPU generator is compared with the
-same restatement in ``test_monte_carlo_table_generator_matches_oracle``.
+same restatement in ``test_monte_carlo_table_generator_matches_oracle``.  Without the reference checkout the
+restatement is compared with the evaluator's values on the same points, stored in
+``tests/golden/host_vs_reference/values.json`` (``tests/golden/make_golden_host.py``).
 """
 import ast
 import copy
 import datetime
+import json
 import os
 import random
 import sys
@@ -20,9 +23,15 @@ import pytest
 
 from oracle import refenv
 
-pytestmark = pytest.mark.skipif(not refenv.available(), reason="needs the reference checkout (/root/reference)")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+sys.path.insert(0, GOLDEN)
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+
+def grid_indices():
+    """24 seeded grid points plus the corners: first / last entry, a midnight and an end-of-year point."""
+    rng = np.random.default_rng(5)
+    idx = np.sort(rng.choice(4_199_040, size=24, replace=False))
+    return np.unique(np.concatenate([idx, [0, 4_199_039, 5, 71]]))
 
 
 def reference_point_evaluator():
@@ -66,12 +75,18 @@ def test_table_restatement_matches_reference_point_evaluator():
     from marl_demandresponse_b200 import montecarlo as mc
     from oracle.montecarlo import table_entries
 
-    evaluate, config_dict = reference_point_evaluator()
-    rng = np.random.default_rng(5)
-    idx = np.sort(rng.choice(4_199_040, size=24, replace=False))
-    # corners of the grid as well: first / last entry, a midnight and an end-of-year point
-    idx = np.unique(np.concatenate([idx, [0, 4_199_039, 5, 71]]))
+    idx = grid_indices()
     pts = mc.grid_points(idx)
+    if not refenv.available():
+        with open(os.path.join(GOLDEN, "host_vs_reference", "values.json")) as f:
+            g = json.load(f)["montecarlo"]
+        assert g["indices"] == idx.tolist()
+        prop = mc.env_prop_for_table(g["house"])
+        got = table_entries(prop, mc.initial_state(pts, prop), pts["OD_temp"])
+        np.testing.assert_allclose(got, np.asarray(g["values"], dtype=np.float64), rtol=1e-9, atol=1e-6)
+        assert np.ptp(got) > 100.0
+        return
+    evaluate, config_dict = reference_point_evaluator()
     house = {k: config_dict["default_house_prop"][k] for k in ("Ua", "Ca", "Cm", "Hm", "target_temp", "deadband", "window_area",
                                                                "shading_coeff", "solar_gain_bool") if k in config_dict["default_house_prop"]}
     if "solar_gain_bool" in house:
