@@ -1282,44 +1282,22 @@ extern "C" int drsim_run_tape(drsim_t *h, const drsim_step_args *args, int n_ste
     return fail(DRSIM_E_ARG, "drsim_run: injected noise / sampled ids are per-step inputs (n_steps must be 1)");
   CU_TRY(cudaSetDevice(h->device));
   const uint8_t *tape = a.actions;
-  // On-device policy on the staged fused kernel with at most one tile per CTA: the step loop runs INSIDE
-  // the kernel (k_fused_tma<0>, StepIn::n_steps), one launch per block of scheduled records -- a small
-  // cluster then costs the in-kernel step latency instead of one dependent launch per step.
+  // Action tape, or an on-device policy, on k_small / k_fused_tma / k_fused_rows: the step loop runs INSIDE the kernel
+  // (StepIn::stream_steps), one launch per block of scheduled records.  Nothing a CTA reads of step k + 1 comes from
+  // another CTA, so the steps of a block have no boundary between them (no launch ramp / tail, no grid-wide wait).
+  // k_small keeps the state in registers and k_fused_tma runs a tile through all the steps before its next tile,
+  // both on any number of tiles.  k_fused_rows takes the steps in turn over all its tiles, so a CTA needs at least two
+  // (its next step's first tile must not be the tile it is still updating): it runs on min(resident CTAs, tiles / 2)
+  // CTAs, and only when that costs at most a tenth of the resident grid.
   const SimParams &p = h->p;
-  const bool small = small_handle(h);   // k_small: steps in registers, any number of replicas per launch
-  const bool episode = !tape && h->fused_ok && h->real_bytes == 4 &&
-                       (small || (h->fused_direct && h->geom.use_tma && !h->geom.use_rows && h->geom.n_tiles <= h->fused_grid)) &&
-                       p.policy != DRSIM_POLICY_EXTERNAL && p.policy != DRSIM_POLICY_GREEDY_MYOPIC &&
-                       p.base_mode == DRSIM_BASE_CONSTANT && !getenv("DRSIM_NO_EPISODE");
-  if (episode) {
-    int left = n_steps;
-    while (left > 0) {
-      StepIn in = make_in(h, &a, 1, 0, (cudaStream_t)stream);   // (re)generates the schedule block when the step leaves it
-      if (!in.sched_rec) break;                                  // no scheduled records (should not happen): per-step loop
-      const int k = (int)std::min<int64_t>(left, h->sched_base + drsim_handle::kSched - h->step);
-      in.n_steps = k;
-      const int rc = launch_fused<float>(h, in, (cudaStream_t)stream);
-      if (rc) return rc;
-      h->step += k;
-      left -= k;
-    }
-    if (left == 0) return 0;
-    n_steps = left;
-  }
-  // Action tape (or an on-device bang-bang policy) on a staged fused kernel with at least two tiles per CTA: the step
-  // loop runs INSIDE the kernel (StepIn::stream_steps), one launch per block of scheduled records.  Nothing a CTA
-  // reads of step k + 1 comes from another CTA, so the steps of a block have no boundary between them (no launch
-  // ramp / tail, no grid-wide wait).
-  // every CTA needs at least two tiles (its next step's first tile must not be the tile it is still updating): the
-  // stream runs on min(resident CTAs, tiles / 2) CTAs, and only when that costs at most a tenth of the resident grid
+  const bool small = small_handle(h);
   const int sgrid = h->fused_ok ? std::min(h->fused_grid, h->geom.n_tiles / 2) : 0;
   const bool tma_path = h->fused_direct && h->geom.use_tma && !h->geom.use_rows;
-  const bool rows_path = h->geom.use_rows && h->geom.in_stride && p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
+  const bool rows_path = tape && h->geom.use_rows && h->geom.in_stride && p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2 &&
+                         sgrid * 10 >= h->fused_grid * 9;
   const bool policy_ok = tape ? p.policy == DRSIM_POLICY_EXTERNAL
-                              : (tma_path && p.policy != DRSIM_POLICY_EXTERNAL && p.policy != DRSIM_POLICY_GREEDY_MYOPIC);
-  const bool taped = n_steps > 1 && h->fused_ok && h->real_bytes == 4 &&
-                     (small ? (tape && p.policy == DRSIM_POLICY_EXTERNAL)
-                            : ((tma_path || rows_path) && policy_ok && sgrid * 10 >= h->fused_grid * 9)) &&
+                              : (p.policy != DRSIM_POLICY_EXTERNAL && p.policy != DRSIM_POLICY_GREEDY_MYOPIC);
+  const bool taped = n_steps > 1 && h->fused_ok && h->real_bytes == 4 && (small || tma_path || rows_path) && policy_ok &&
                      p.base_mode == DRSIM_BASE_CONSTANT && !h->mirror_next &&
                      !h->act_poll_next && !h->obs_override && !h->reward_override && !h->broken && !getenv("DRSIM_NO_STREAM");
   int first = 0;
@@ -1335,7 +1313,7 @@ extern "C" int drsim_run_tape(drsim_t *h, const drsim_step_args *args, int n_ste
       in.tape_first = first;
       in.tape_stride = action_stride;
       if (k == 1 && tape) in.actions = tape + (size_t)(tape_planes > 0 ? first % tape_planes : first) * action_stride;
-      h->launch_grid = small ? 0 : sgrid;
+      h->launch_grid = (small || tma_path) ? 0 : sgrid;
       const int rc = launch_fused<float>(h, in, (cudaStream_t)stream);
       h->launch_grid = 0;
       if (rc) return rc;

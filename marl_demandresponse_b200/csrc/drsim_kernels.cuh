@@ -99,15 +99,13 @@ struct StepIn {
   int64_t xseq;
   int do_interp;
   int advance;  // 1 = real step, 0 = refresh (recompute signal / obs without advancing time)
-  // in-kernel episode (drsim_run under an on-device policy, k_fused_tma<0> only): this launch advances
-  // n_steps consecutive steps; step k uses the schedule records sched_rec + k * R.  0 / 1 = one step.
-  int n_steps;
-  // in-kernel step loop over an action tape (drsim_run_tape on k_fused_tma, every CTA owning at least two tiles):
-  // this launch advances stream_steps consecutive steps, a CTA taking (step 0: its tiles), (step 1: its tiles) ...
-  // Every byte a CTA reads of step k + 1 was written by the same thread of the same CTA in step k (state planes,
-  // running metrics) or is an input of the call (tape, schedule records), so no step boundary exists between CTAs:
-  // no launch ramp and tail, no grid-wide dependency.  Step k reads the records sched_rec + k * R and the action
-  // plane `actions + ((tape_first + k) % tape_planes) * tape_stride` (tape_planes 0: no rotation).  0 / 1 = one step.
+  // in-kernel step loop (drsim_run_tape: an action tape or an on-device policy on k_fused_tma, k_fused_rows, k_small):
+  // this launch advances stream_steps consecutive steps.  Every byte a CTA reads of step k + 1 was written by the
+  // same thread of the same CTA in step k (state planes, running metrics) or is an input of the call (tape, schedule
+  // records), so no step boundary exists between CTAs: no launch ramp and tail, no grid-wide dependency.  k_fused_tma
+  // runs each of its tiles through all the steps before the next tile (tile-major), k_fused_rows takes (step 0: its
+  // tiles), (step 1: its tiles) ...  Step k reads the records sched_rec + k * R and the action plane
+  // `actions + ((tape_first + k) % tape_planes) * tape_stride` (tape_planes 0: no rotation).  0 / 1 = one step.
   int stream_steps, tape_planes, tape_first;
   size_t tape_stride;
 };
@@ -1473,6 +1471,12 @@ DRSIM_D void bulk_store_wait_read() {
   asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 #endif
 }
+// ... and for the global writes of those stores too: two bulk stores to the same address are not ordered
+DRSIM_D void bulk_store_wait_all() {
+#if defined(__CUDA_ARCH__)
+  asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+#endif
+}
 DRSIM_D void fence_proxy_async_smem() {
 #if defined(__CUDA_ARCH__)
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -2129,14 +2133,16 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   // slots, so completion is one cp.async.wait_all of the thread itself -- no barrier, no mbarrier, and
   // none of the per-copy issue latency of 512-byte TMA bulk loads (measured: 20 % of the stall samples)
   float nx_od = 0.f, nx_solar = 0.f;
-  // `part`: 1 = launch-invariant static planes only (may run before pdl_wait), 2 = the rest, 3 = both
-  const int n_stream = in.stream_steps > 1 ? in.stream_steps : 1;   // in-kernel step loop over an action tape
+  const int n_steps = in.stream_steps > 1 ? in.stream_steps : 1;   // in-kernel step loop (StepIn::stream_steps)
   auto step_actions = [&](int st) -> const uint8_t * {
-    if (n_stream == 1 || !in.actions) return actions;
+    if (n_steps == 1 || !in.actions) return actions;
     const int j = in.tape_first + st;
     return in.actions + (size_t)(in.tape_planes > 0 ? j % in.tape_planes : j) * in.tape_stride;
   };
-  auto prefetch = [&](int t, int st, int part) {
+  // every tile starts at step 0 of the launch.  `part`: 1 = launch-invariant static planes only (may run
+  // before pdl_wait), 2 = the rest, 3 = both
+  auto prefetch = [&](int t, int part) {
+    constexpr int st = 0;
     const int tr0 = t * g.envs_per_tile;
     const int tslots = min(g.envs_per_tile, p.R - tr0) * Ns;
     const size_t tbase = (size_t)tr0 * Ns;
@@ -2164,33 +2170,29 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
       }
     }
   };
-  // schedule record + running metrics of tile t's clusters -> shared memory (threads e < E, cp.async)
-  auto fetch_env = [&](int t, int st, int par) {
+  // schedule record + running metrics of tile t's clusters at step 0 -> shared memory (threads e < E, cp.async)
+  auto fetch_env = [&](int t, int par) {
     const int tr0 = t * g.envs_per_tile;
     if ((int)threadIdx.x < min(g.envs_per_tile, p.R - tr0))
-      env_stage_fetch(s_stage_base + (size_t)par * g.envs_per_tile + threadIdx.x, in.sched_rec + (size_t)st * p.R, pl.metrics,
-                      tr0 + threadIdx.x);
+      env_stage_fetch(s_stage_base + (size_t)par * g.envs_per_tile + threadIdx.x, in.sched_rec, pl.metrics, tr0 + threadIdx.x);
   };
   pdl_trigger();
-  if ((int)blockIdx.x < g.n_tiles) prefetch(blockIdx.x, 0, 1);
+  if ((int)blockIdx.x < g.n_tiles) prefetch(blockIdx.x, 1);
   pdl_wait();
   if ((int)blockIdx.x < g.n_tiles) {
-    prefetch(blockIdx.x, 0, 2);
-    if (fast) fetch_env(blockIdx.x, 0, 0);
+    prefetch(blockIdx.x, 2);
+    if (fast) fetch_env(blockIdx.x, 0);
   }
 
-  // In-kernel episode (MODE 0, host guarantees at most one tile per CTA and scheduled records for all
-  // n_steps): the step loop runs inside the tile loop; between steps the thread's updated state goes back
-  // into its own staging slots, the next step's (static) record is fetched while this one computes, and the
-  // running metrics travel through the staged record -- nothing is re-read from global memory.
-  const int n_epi = (MODE == 0 && in.n_steps > 1) ? in.n_steps : 1;
-  for (int st = 0; st < n_stream; ++st)
+  // Tile-major step loop: a tile runs through all n_steps steps before the CTA moves to its next tile.
+  // Between two steps of a tile the thread's updated state goes back into its own staging slots, the static
+  // planes stay there, the next step's action word, (od, solar) pair and schedule record are fetched while
+  // this step computes, and the running metrics travel through the staged record: the tile's planes come
+  // from global memory once per launch.  Every step still stores everything a single step stores.
   for (int tile = blockIdx.x; tile < g.n_tiles; tile += gridDim.x)
-  for (int epi = 0; epi < n_epi; ++epi, parity ^= 1) {
-    const bool epi_more = MODE == 0 && epi + 1 < n_epi;
-    // the item after this one: the CTA's next tile of this step, or its first tile of the next step of the stream
-    int nt = tile + gridDim.x, nst = st;
-    if (nt >= g.n_tiles && st + 1 < n_stream) { nt = blockIdx.x; nst = st + 1; }
+  for (int st = 0; st < n_steps; ++st, parity ^= 1) {
+    const bool more = st + 1 < n_steps;   // the item after this one is this tile's next step
+    const int nt = tile + gridDim.x;      // ... otherwise the CTA's next tile, from step 0
     const int r0 = tile * g.envs_per_tile;
     const int E = min(g.envs_per_tile, p.R - r0);
     const int slots = E * Ns;
@@ -2236,22 +2238,18 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
       if (fast) { const float2 v = s_os[threadIdx.x]; w.od = v.x; w.solar = v.y; }
       else { w.od = nx_od; w.solar = nx_solar; }
     }
-    // the thread holds its inputs in registers: its staging slots are free, the next tile's copies are
-    // issued now and have the whole tile to land
-    if (nt < g.n_tiles) prefetch(nt, nst, 3);
-    if constexpr (MODE == 0) {
-      if (epi_more && active && fast)   // house-update inputs of the next step of the episode (static record)
-        cp_async8(s_os + threadIdx.x, &in.sched_rec[(size_t)(epi + 1) * p.R + r0 + e_loc].od_prev_f);
-    }
+    // the thread holds its inputs in registers: on the tile's last step its staging slots are free, the next
+    // tile's copies are issued now and have the whole tile to land
+    if (!more && nt < g.n_tiles) prefetch(nt, 3);
     if (active) house4_compute_f32<MODE != 0>(pl, p, w, base + s0, min(4, p.N - n0), h, red, pol_keep);
-    if constexpr (MODE == 0) {
-      if (epi_more && active) {   // the next step reads its state from the thread's own staging slots
-        float4 *o4 = reinterpret_cast<float4 *>(s_in) + threadIdx.x;
-        o4[0] = make_float4(h.ta[0], h.ta[1], h.ta[2], h.ta[3]);
-        o4[kTileSlots / 4] = make_float4(h.tm[0], h.tm[1], h.tm[2], h.tm[3]);
-        reinterpret_cast<int4 *>(s_in)[(size_t)2 * (kTileSlots / 4) + threadIdx.x] = make_int4(h.sso[0], h.sso[1], h.sso[2], h.sso[3]);
-        s_flags[threadIdx.x] = h.flags;
-      }
+    if (more && active) {   // the next step reads its state from the thread's own staging slots, its small inputs come now
+      if (ext) cp_async4(s_act + threadIdx.x, step_actions(st + 1) + base + s0);
+      if (fast) cp_async8(s_os + threadIdx.x, &in.sched_rec[(size_t)(st + 1) * p.R + r0 + e_loc].od_prev_f);
+      float4 *o4 = reinterpret_cast<float4 *>(s_in) + threadIdx.x;
+      o4[0] = make_float4(h.ta[0], h.ta[1], h.ta[2], h.ta[3]);
+      o4[kTileSlots / 4] = make_float4(h.tm[0], h.tm[1], h.tm[2], h.tm[3]);
+      reinterpret_cast<int4 *>(s_in)[(size_t)2 * (kTileSlots / 4) + threadIdx.x] = make_int4(h.sso[0], h.sso[1], h.sso[2], h.sso[3]);
+      s_flags[threadIdx.x] = h.flags;
     }
     // the previous tile's row store must have drained the warp's staging rows before they are rewritten
     // (waited for here, after the house update, not at the top of the tile)
@@ -2335,14 +2333,15 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
     __syncthreads();
     // every warp is past the previous tile's phase 3: the other parity of s_stage is free again
     if (fast) {
-      if (nt < g.n_tiles) fetch_env(nt, nst, parity ^ 1);
-      if constexpr (MODE == 0) {
-        if (epi_more && (int)threadIdx.x < E) {   // record of the next step; its metrics part is filled by env_stage_store
-          const char *src = reinterpret_cast<const char *>(in.sched_rec + (size_t)(epi + 1) * p.R + r0 + threadIdx.x);
+      if (more) {
+        if ((int)threadIdx.x < E) {   // record of the next step; its metrics part is filled by env_stage_store
+          const char *src = reinterpret_cast<const char *>(in.sched_rec + (size_t)(st + 1) * p.R + r0 + threadIdx.x);
           char *d = reinterpret_cast<char *>(s_stage_base + (size_t)(parity ^ 1) * g.envs_per_tile + threadIdx.x);
 #pragma unroll
           for (int q = 0; q < 5; ++q) cp_async16(d + 16 * q, src + 16 * q);
         }
+      } else if (nt < g.n_tiles) {
+        fetch_env(nt, parity ^ 1);
       }
     }
 
@@ -2453,6 +2452,9 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
       __syncwarp();
       if (lane == 0 && w0 < slots) {
         const int nrows = min(128, slots - w0);
+        // the tile's previous step stored the same rows: its global writes must have landed, or they could
+        // overwrite this step's (waited for here, a whole step after that store was issued)
+        if (st > 0) bulk_store_wait_all();
         bulk_store_s2g_hint(pl.obs + (base + w0) * D, s_tile + (size_t)w0 * D, (uint32_t)((size_t)nrows * D * sizeof(real)),
                             pol_stream);
         store_pending = true;
@@ -2462,10 +2464,7 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
     if (threadIdx.x < E && fast) {
       double a[kRed] = {0, 0, 0, 0, 0};
       combine(threadIdx.x, a, true);
-      double *m_next = nullptr;
-      if constexpr (MODE == 0) {
-        if (epi_more) m_next = (s_stage_base + (size_t)(parity ^ 1) * g.envs_per_tile + threadIdx.x)->m;
-      }
+      double *m_next = more ? (s_stage_base + (size_t)(parity ^ 1) * g.envs_per_tile + threadIdx.x)->m : nullptr;
       env_stage_store<real>(pl, p, r0 + threadIdx.x, s_stage[threadIdx.x], a, in.host_env, m_next);
     }
   }
@@ -2759,8 +2758,8 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
 // one house per lane: the lock-out state machine and the thermal update of house4_compute_f32 per
 // lane, the five cluster sums by shuffle butterflies, the power fold-in / reward / row of every
 // house by its own lane, neighbour messages by shuffles instead of shared memory.  The state lives
-// in registers across the steps of one launch (StepIn::n_steps: on-device policy; StepIn::
-// stream_steps: action tape) and goes back to the planes after every step like everything else the
+// in registers across the steps of one launch (StepIn::stream_steps: on-device policy or action
+// tape) and goes back to the planes after every step like everything else the
 // step produces.  Conditions (checked by the host): fp32, scheduled env path, plain columns.
 // ------------------------------------------------------------------------------------------
 constexpr int kSmallWarps = 4;   // clusters per CTA
@@ -2797,7 +2796,7 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small(Planes<float> pl, Si
   double m[DRSIM_N_METRICS];
 #pragma unroll
   for (int q = 0; q < DRSIM_N_METRICS; ++q) m[q] = pl.metrics[(size_t)r * DRSIM_N_METRICS + q];
-  const int n_steps = max(1, max(in.n_steps, in.stream_steps));
+  const int n_steps = max(1, in.stream_steps);
   const float pmax_n = cap * p.hf.inv_cop * p.hf.inv_nrs;
   const float tg20 = tg - 20.f;
 
