@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define DRSIM_ABI_VERSION 3
+#define DRSIM_ABI_VERSION 4
 #define DRSIM_MAX_SIGNAL_TERMS 8
 #define DRSIM_INTERP_SUBTABLES 162      /* 3*3*3*3*2 nearest-neighbour cells            */
 #define DRSIM_INTERP_SUBTABLE_LEN 25920 /* 9*5*8*12*6 values of the 5-D multilinear part */
@@ -48,6 +48,9 @@ enum { DRSIM_SIG_FLAT = 0, DRSIM_SIG_SINUSOIDALS = 1, DRSIM_SIG_REGULAR_STEPS = 
 /* observation layouts: none, utils/norm.py:178-218 (hand-engineered, with neighbour messages),
  * "TarMAC" = own-state features only + static neighbour index tensor (SURVEY 8a-12) */
 enum { DRSIM_OBS_NONE = 0, DRSIM_OBS_HAND_ENGINEERED = 1, DRSIM_OBS_TARMAC = 2 };
+/* element type of the observation rows: the build's `real`, or bfloat16 (fp32 build only).  A bf16 row element is
+ * the fp32 element the kernels compute, rounded to nearest-even where it is stored; nothing else changes. */
+enum { DRSIM_OBS_F32 = 0, DRSIM_OBS_BF16 = 1 };
 /* neighbour source: arithmetic ring (agent_communication_builder.py:63-85) or explicit table */
 enum { DRSIM_COMM_RING = 0, DRSIM_COMM_TABLE = 1 };
 /* where per-step noise comes from when the matching pointer of drsim_step_args is NULL */
@@ -97,7 +100,7 @@ typedef struct drsim_config {
   /* RewardProperties (environment_properties.py:221-258) */
   double alpha_temp, alpha_sig, norm_reg_sig;
   int32_t penalty_mode;
-  int32_t pad0_;
+  int32_t obs_dtype; /* DRSIM_OBS_F32 | DRSIM_OBS_BF16 (needs precision DRSIM_F32 and an observation layout) */
   double alpha_ind_l2, alpha_common_l2, alpha_common_max;
 
   /* PowerGridProperties (power_grid_properties.py:6-70) */
@@ -157,19 +160,20 @@ typedef struct drsim_host_state {
 } drsim_host_state;
 
 /* Device pointers of a handle (zero-copy views for torch / cupy).  `real` planes are float
- * (DRSIM_F32) or double (DRSIM_F64). */
+ * (DRSIM_F32) or double (DRSIM_F64); `row` elements are obs_bytes wide: real, or bfloat16 (DRSIM_OBS_BF16). */
 typedef struct drsim_ptrs {
   int32_t n_rep, n_house, house_stride, obs_dim, real_bytes, nb_comm;
   /* 1 (DRSIM_F32): the t_air / t_mass planes hold the DEVIATION from the house set-point,
    * Ta - target and Tm - target (what reward, messages, controllers and the interpolator consume;
    * it also keeps fp32 rounding at the 1e-7 degC level); 0 (DRSIM_F64): absolute degC. */
-  int32_t temp_is_deviation, pad_;
+  int32_t temp_is_deviation;
+  int32_t obs_bytes;           /* size of one observation-row element: 8, 4 or 2 (bfloat16) */
   void *t_air, *t_mass;        /* real  [R][stride] */
   int32_t *sso;                /* i32   [R][stride] */
   uint8_t *flags;              /* u8    [R][stride]  bit0 = turned_on, bit1 = lockout */
   void *target, *cap;          /* real  [R][stride] */
   void *reward;                /* real  [R][stride] */
-  void *obs;                   /* real  [R][stride][obs_dim] */
+  void *obs;                   /* row   [R][stride][obs_dim] */
   uint8_t *actions;            /* u8    [R][stride]  internal action plane (policies / host API) */
   int64_t *epoch;              /* i64   [R] */
   double *od_temp, *signal, *base_power, *power, *solar, *pen_sum, *pen_max; /* f64 [R] */
@@ -323,8 +327,9 @@ int drsim_step_host(drsim_t *h, const uint8_t *actions, const double *od_noise, 
                     const int32_t *interp_ids, double *env_out, void *stream);
 
 /* Environment.step with HOST buffers and the reference's full return value (environment.py:108: per-agent
- * observations and rewards): drsim_step_host, then reward_out[R][N] and obs_out[R][N][obs_dim] (`real` = float or
- * double as the handle was built; row-major, no padding; either may be NULL) are copied back behind the kernel,
+ * observations and rewards): drsim_step_host, then reward_out[R][N] (`real` = float or double as the handle was built)
+ * and obs_out[R][N][obs_dim] (float, double or bfloat16 as drsim_ptrs.obs_bytes says; row-major, no padding; either may
+ * be NULL) are copied back behind the kernel,
  * ahead of the call's one stream synchronisation.  On BASELINE config 4 that is 90 MB per step: PCIe-bound. */
 int drsim_step_host_full(drsim_t *h, const uint8_t *actions, const double *od_noise, const double *perlin,
                          const int32_t *interp_ids, double *env_out, void *reward_out, void *obs_out, void *stream);
@@ -341,7 +346,7 @@ typedef struct drsim_snapshot_view {
   const int32_t *sso;                    /* [R][N] */
   const uint8_t *on, *lockout;           /* [R][N] */
   const double *env;                     /* [R][8] */
-  const void *obs;                       /* [R][N][obs_dim] float | double as the handle was built, or NULL */
+  const void *obs;                       /* [R][N][obs_dim] float | double | bfloat16 as the handle was built, or NULL */
 } drsim_snapshot_view;
 int drsim_snapshot(drsim_t *h, drsim_snapshot_view *out, void *stream);
 /* Environment.step for the dict API: drsim_step_host (host action / noise buffers in) followed by the snapshot,
@@ -358,7 +363,9 @@ typedef struct drsim_actor_net {
   const float *w3, *b3; /* [2][h2], [2] */
   int32_t h1, h2;       /* 1 .. 111 each */
   /* 0 = one TF32 pass per product (|dp| <= 5e-3 against an fp32 forward), 1 = "3xTF32": every operand split into
-   * hi + lo TF32 halves, three tensor-core passes per product, fp32-grade probabilities (|dp| ~ 1e-6) */
+   * hi + lo TF32 halves, three tensor-core passes per product, fp32-grade probabilities (|dp| ~ 1e-6).
+   * On a handle with bfloat16 rows (DRSIM_OBS_BF16) only 1 is accepted: the 3xTF32 actor widens the rows as it loads
+   * them, with results bit-identical to the same actor on the widened fp32 rows; 0 fails with DRSIM_E_ARG. */
   int32_t precision;
   int32_t pad_;
 } drsim_actor_net;
@@ -377,11 +384,12 @@ int drsim_policy_step(drsim_t *h, const drsim_actor_net *net, uint64_t seed, flo
  * MAPPO.store_transition (mappo.py:105-127; training_manager.py:224-240) in one call.  All DEVICE pointers, plane
  * layout of the handle (row stride = house_stride); obs / reward / next_obs 16-byte aligned, actions / prob 4-byte
  * aligned; the step kernels write the slot directly:
- *   obs      [R][stride][obs_dim] f32  state_t the actor reads (NULL: the handle's own rows = the last step's result)
+ *   obs      [R][stride][obs_dim] row  state_t the actor reads (NULL: the handle's own rows = the last step's result)
  *   actions  [R][stride] u8            a_t drawn by the actor, consumed by the step            (Transition.action)
  *   prob     [R][stride] f32           probability of a_t under the actor (mappo.py:95)        (Transition.a_log_prob)
  *   reward   [R][stride] f32           r_t                                                       (Transition.reward)
- *   next_obs [R][stride][obs_dim] f32  state_{t+1}: pass it as `obs` of the next transition     (Transition.next_state)
+ *   next_obs [R][stride][obs_dim] row  state_{t+1}: pass it as `obs` of the next transition     (Transition.next_state)
+ * (`row` = f32, or bf16 on a handle built with DRSIM_OBS_BF16)
  * Transition.others_actions is the `actions` plane without the agent's own entry; `done` is the caller's
  * (training_manager.py:233: end of the episode).  The reference does not evaluate its critic during the rollout
  * (mappo.py:99-103 is commented out): Critic(cat(state, others_actions)) runs in update() on these buffers. */

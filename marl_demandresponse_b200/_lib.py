@@ -9,7 +9,7 @@ import os
 
 from . import _build
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_SIGNAL_TERMS = 8
 INTERP_SUBTABLES = 162
 INTERP_SUBTABLE_LEN = 25920
@@ -24,6 +24,7 @@ PEN = {"individual_L2": 0, "common_L2": 1, "common_max_error": 2, "mixture": 3}
 BASE = {"constant": 0, "interpolation": 1}
 SIG = {"flat": 0, "sinusoidals": 1, "regular_steps": 2, "perlin": 3}
 OBS = {"none": 0, "hand_engineered": 1, "tarmac": 2}
+OBS_DTYPE = {"float32": 0, "bfloat16": 1}
 COMM_RING, COMM_TABLE = 0, 1
 NOISE = {"zero": 0, "philox": 1}
 POLICY = {"external": 0, "deadband_bangbang": 1, "bangbang": 2, "always_on": 3, "greedy_myopic": 4}
@@ -45,7 +46,7 @@ class Config(C.Structure):
         ("default_cooling_capacity", _d),
         ("day_temp", _d), ("night_temp", _d), ("temp_std", _d), ("phase", _d),
         ("alpha_temp", _d), ("alpha_sig", _d), ("norm_reg_sig", _d),
-        ("penalty_mode", _i32), ("pad0_", _i32),
+        ("penalty_mode", _i32), ("obs_dtype", _i32),
         ("alpha_ind_l2", _d), ("alpha_common_l2", _d), ("alpha_common_max", _d),
         ("base_power_mode", _i32), ("interp_update_period", _i32), ("interp_nb_agents", _i32), ("signal_mode", _i32),
         ("avg_power_per_hvac", _d),
@@ -99,7 +100,7 @@ class ActorNet(C.Structure):
 class Ptrs(C.Structure):
     _fields_ = [
         ("n_rep", _i32), ("n_house", _i32), ("house_stride", _i32), ("obs_dim", _i32), ("real_bytes", _i32),
-        ("nb_comm", _i32), ("temp_is_deviation", _i32), ("pad_", _i32),
+        ("nb_comm", _i32), ("temp_is_deviation", _i32), ("obs_bytes", _i32),
         ("t_air", C.c_void_p), ("t_mass", C.c_void_p), ("sso", C.c_void_p), ("flags", C.c_void_p),
         ("target", C.c_void_p), ("cap", C.c_void_p), ("reward", C.c_void_p), ("obs", C.c_void_p),
         ("actions", C.c_void_p), ("epoch", C.c_void_p),

@@ -79,12 +79,15 @@ class BatchedEnv:
     Parameters mirror ``Environment`` plus: ``n_replicas``; ``obs_layout`` in
     {"hand_engineered", "tarmac", "none"}; ``policy`` ("external" actions or an on-device
     controller); ``noise`` ("philox": counter-based streams keyed by (replica, step); "zero");
-    ``rep_offset`` = global index of the first local replica (sharding across GPUs).
+    ``rep_offset`` = global index of the first local replica (sharding across GPUs); ``obs_dtype`` =
+    "float32" or "bfloat16" (fp32 build: the rows are written, stored and handed out in bf16, each element the
+    fp32 value rounded to nearest-even).
     """
 
     def __init__(self, env_props: Any = None, n_replicas: int = 1, device: int = 0, precision: str = "f32",
                  obs_layout: str = "hand_engineered", policy: str = "external", noise: str = "philox",
-                 seed: int = 0, path: str = "auto", rep_offset: int = 0, interp_table: Optional[np.ndarray] = None):
+                 seed: int = 0, path: str = "auto", rep_offset: int = 0, interp_table: Optional[np.ndarray] = None,
+                 obs_dtype: str = "float32"):
         self.props: EnvironmentProperties = as_props(env_props)
         self.init_props = self.props
         self.n_replicas = int(n_replicas)
@@ -92,7 +95,7 @@ class BatchedEnv:
         self.rep_offset = int(rep_offset)
         self.seed = int(seed)
         cfg = flatten_config(self.props, n_replicas, precision, obs_layout, policy, noise, seed, path,
-                             rep_offset=rep_offset)
+                             rep_offset=rep_offset, obs_dtype=obs_dtype)
         self.sim = DrSim(cfg, device)
         self.device = device
         mode = self.props.cluster_prop.agents_comm_prop.mode

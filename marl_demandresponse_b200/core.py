@@ -51,8 +51,12 @@ def comm_width(props: EnvironmentProperties) -> int:
 def flatten_config(props: Any, n_rep: int = 1, precision: str = "f32", obs_layout: str = "hand_engineered",
                    policy: str = "external", noise: str = "zero", seed: int = 0, path: str = "auto",
                    comm_table: bool | None = None, house_offset: int = 0, n_house_local: int | None = None,
-                   rep_offset: int = 0) -> _lib.Config:
-    """``EnvironmentProperties`` -> ``drsim_config`` (include/drsim.h)."""
+                   rep_offset: int = 0, obs_dtype: str = "float32") -> _lib.Config:
+    """``EnvironmentProperties`` -> ``drsim_config`` (include/drsim.h).  ``obs_dtype``: element type of the
+    observation rows, "float32" (the build's precision) or "bfloat16" (fp32 build only: every row element is the
+    fp32 value rounded to nearest-even)."""
+    if obs_dtype not in _lib.OBS_DTYPE:
+        raise ValueError(f"obs_dtype must be one of {sorted(_lib.OBS_DTYPE)}, got {obs_dtype!r}")
     p = as_props(props)
     hp, hv = p.cluster_prop.house_prop, p.cluster_prop.house_prop.hvac_prop
     gp, rp = p.power_grid_prop, p.reward_prop
@@ -104,6 +108,7 @@ def flatten_config(props: Any, n_rep: int = 1, precision: str = "f32", obs_layou
     c.amplitude_per_hvac = float(sp.amplitude_per_hvac)
     c.nb_octaves, c.octaves_step, c.period = sp.nb_octaves, sp.octaves_step, sp.period
     c.obs_layout = _lib.OBS[obs_layout]
+    c.obs_dtype = _lib.OBS_DTYPE[obs_dtype]
     c.nb_comm = comm_width(p)
     mode = p.cluster_prop.agents_comm_prop.mode
     if comm_table is None:
@@ -183,6 +188,7 @@ class DrSim:
         self.ptrs = ptrs
         self.R, self.N, self.Ns, self.D = ptrs.n_rep, ptrs.n_house, ptrs.house_stride, ptrs.obs_dim
         self.real = np.float64 if ptrs.real_bytes == 8 else np.float32
+        self.obs_bf16 = ptrs.obs_bytes == 2   # rows of bfloat16: raw uint16 bits on the numpy side
         self._views: Optional[Dict[str, Any]] = None
 
     # ---- lifetime -------------------------------------------------------------------------
@@ -406,7 +412,7 @@ class DrSim:
             import torch
 
             want = {np.uint8: (torch.uint8, torch.bool), np.float64: (torch.float64,), np.float32: (torch.float32,),
-                    np.int32: (torch.int32,)}[dtype]
+                    np.int32: (torch.int32,), np.uint16: (torch.bfloat16,)}[dtype]
             if x.is_cuda or x.dtype not in want or not x.is_contiguous() or tuple(x.shape) != tuple(shape):
                 raise ValueError(f"{what}: expected a contiguous CPU tensor of dtype {want[0]} and shape {tuple(shape)}, "
                                  f"got {x.dtype} {tuple(x.shape)} (cuda={x.is_cuda}, contiguous={x.is_contiguous()})")
@@ -429,7 +435,8 @@ class DrSim:
                   env_out: Optional[np.ndarray] = None, reward_out=None, obs_out=None, stream=None) -> Optional[np.ndarray]:
         """Host-buffer step (``drsim_step_host``): numpy (or pinned torch CPU) buffers in and out.
         ``actions`` uint8 / bool ``[R, N]`` with values 0 / 1; ``env_out`` fp64 ``[R, 4]``.  With ``reward_out``
-        ``[R, N]`` and / or ``obs_out`` ``[R, N, D]`` (dtype of the build) the call is ``drsim_step_host_full``:
+        ``[R, N]`` and / or ``obs_out`` ``[R, N, D]`` (dtype of the build; with bfloat16 rows a pinned CPU
+        ``torch.bfloat16`` tensor or a numpy ``uint16`` array of the raw bits) the call is ``drsim_step_host_full``:
         the reference's full ``step`` result comes back to the host."""
         keep: list = []
         R, N = self.R, self.N
@@ -445,7 +452,8 @@ class DrSim:
             _lib.check(self._L.drsim_step_host(self._h, *args, self._stream(stream)))
         else:
             args += [self._host_buf(reward_out, self.real, (R, N), keep, "reward_out", writable=True),
-                     self._host_buf(obs_out, self.real, (R, N, self.D), keep, "obs_out", writable=True)]
+                     self._host_buf(obs_out, np.uint16 if self.obs_bf16 else self.real, (R, N, self.D), keep, "obs_out",
+                                    writable=True)]
             _lib.check(self._L.drsim_step_host_full(self._h, *args, self._stream(stream)))
         return env_out
 
@@ -460,7 +468,7 @@ class DrSim:
                "sso": as_arr(v.sso, (R, N)), "on": as_arr(v.on, (R, N)), "lockout": as_arr(v.lockout, (R, N)),
                "env": as_arr(v.env, (R, 8)), "obs": None}
         if D and v.obs:
-            ct = C.c_double if self.ptrs.real_bytes == 8 else C.c_float
+            ct = C.c_uint16 if self.obs_bf16 else (C.c_double if self.ptrs.real_bytes == 8 else C.c_float)
             out["obs"] = as_arr(C.cast(v.obs, C.POINTER(ct)), (R, N, D))
         self._snap_key, self._snap_arrays = key, out
         return out
@@ -534,7 +542,8 @@ class DrSim:
     # ---- zero-copy torch views ------------------------------------------------------------
     def views(self) -> Dict[str, Any]:
         """Torch CUDA tensors aliasing the library's buffers (no copies).  House planes are
-        ``[R, N]`` views of ``[R, Ns]`` storage; ``obs`` is ``[R, N, D]``."""
+        ``[R, N]`` views of ``[R, Ns]`` storage; ``obs`` is ``[R, N, D]`` (``torch.bfloat16`` on a handle with
+        bfloat16 rows)."""
         if self._views is not None:
             return self._views
         import torch
@@ -564,7 +573,13 @@ class DrSim:
         v["flags"] = t(p.flags, (R, Ns), "|u1")[:, :N]
         v["actions"] = t(p.actions, (R, Ns), "|u1")[:, :N]
         v["actions_padded"] = t(p.actions, (R, Ns), "|u1")
-        v["obs_padded"] = t(p.obs, (R, Ns, D), rt) if D else None
+        if not D:
+            v["obs_padded"] = None
+        elif self.obs_bf16:   # __cuda_array_interface__ has no bfloat16 typestr: alias the bits as int16
+            v["obs_padded"] = t(p.obs, (R, Ns, D), "<i2").view(torch.bfloat16)
+            v["obs_padded"]._drsim_owner = self
+        else:
+            v["obs_padded"] = t(p.obs, (R, Ns, D), rt)
         v["obs"] = v["obs_padded"][:, :N, :] if D else None
         v["epoch"] = t(p.epoch, (R,), "<i8")
         for k in ("od_temp", "signal", "base_power", "power", "solar", "pen_sum", "pen_max", "rew_sig"):

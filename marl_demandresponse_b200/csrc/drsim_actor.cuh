@@ -29,7 +29,7 @@ constexpr int kActTmemCols = 256;   // power of two >= N1 + N2
 constexpr uint32_t PURPOSE_POLICY = 6;
 
 struct ActorArgs {
-  const float *obs;        // [rows][D]
+  const void *obs;         // [rows][D] float, or __nv_bfloat16 (k_actor3x<PRE, __nv_bfloat16>)
   const unsigned char *image;   // k_actor2: packed weight operands (k_actor_pack)
   const float *w1, *b1;    // [h1][D], [h1]
   const float *w2, *b2;    // [h2][h1], [h2]
@@ -285,7 +285,7 @@ __global__ void __launch_bounds__(kAct2Threads, 1) k_actor2(ActorArgs a) {
       const int n_valid = (int)min((long long)kActRows, a.rows - row0);
       const uint32_t bytes = (uint32_t)(n_valid * a.D * 4);     // rows % 4 == 0: a multiple of 16
       mbar_expect_tx(ldbar, bytes);
-      bulk_load_g2s(s_stage, a.obs + (size_t)row0 * a.D, bytes, ldbar);
+      bulk_load_g2s(s_stage, static_cast<const float *>(a.obs) + (size_t)row0 * a.D, bytes, ldbar);
     }
   };
   uint32_t ld_phase = 0;
@@ -488,7 +488,9 @@ DRSIM_D void tmem_wait_ld_dep(uint32_t r[16]) {
       a.dbg[(it * 3 + role) * 16 + (slot)] = (unsigned long long)clock64();                       \
   } while (0)
 
-template <int PRE>   // 16-byte K chunks per thread in the observation operand (>= K1 / 8)
+// O = element type of the observation rows.  bf16 rows are widened in the producers' load: a bf16 value is exact in
+// TF32, so its hi half is the value itself, its lo half zero, and the products equal those on the widened fp32 rows.
+template <int PRE, typename O = float>   // PRE: 16-byte K chunks per thread in the observation operand (>= K1 / 8)
 __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3x(ActorArgs a) {
   extern __shared__ __align__(1024) unsigned char smem[];
   // mbarriers: 0 a1_ready (256) | 1 GEMM1 done | 2..6 a2_ready[chunk] (256) | 7, 8 GEMM2 done [slot] |
@@ -544,13 +546,16 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3x(ActorArgs a) {
     auto fetch = [&](int tile) {
       const long long row = (long long)tile * kActRows + t;
       const bool live = row < a.rows;
-      const float *g = a.obs + (size_t)(live ? row : 0) * a.D;
+      const O *g = static_cast<const O *>(a.obs) + (size_t)(live ? row : 0) * a.D;
       if ((a.D & 1) == 0) {
 #pragma unroll
         for (int j = 0; j < PRE * 2; ++j) {
           const int k = c_lo * 4 + 2 * j;
           float2 v = make_float2(0.f, 0.f);
-          if (live && k < c_hi * 4 && k < a.D) v = __ldg(reinterpret_cast<const float2 *>(g + k));
+          if (live && k < c_hi * 4 && k < a.D) {
+            if constexpr (sizeof(O) == 2) v = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162 *>(g + k)));
+            else v = __ldg(reinterpret_cast<const float2 *>(g + k));
+          }
           pre[2 * j] = v.x;
           pre[2 * j + 1] = v.y;
         }
@@ -558,7 +563,7 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3x(ActorArgs a) {
 #pragma unroll
         for (int j = 0; j < PRE * 4; ++j) {
           const int k = c_lo * 4 + j;
-          pre[j] = (live && k < c_hi * 4 && k < a.D) ? __ldg(g + k) : 0.f;
+          pre[j] = (live && k < c_hi * 4 && k < a.D) ? (float)__ldg(g + k) : 0.f;
         }
       }
     };

@@ -7,6 +7,7 @@
 #include <cstring>
 #include <cstdlib>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "drsim_kernels.cuh"
@@ -50,6 +51,7 @@ struct drsim_handle {
   int device = 0;
   int sm_count = 148;
   int real_bytes = 4;
+  int obs_bytes = 4;   // observation-row element: real_bytes, or 2 (DRSIM_OBS_BF16)
   unsigned char *slab = nullptr;
   size_t slab_bytes = 0;
   // offsets inside the slab
@@ -134,7 +136,7 @@ static Planes<real> make_planes(const drsim_handle *h) {
   pl.interp_sub = h->has_interp ? h->at<uint8_t>(h->o_sub) : nullptr;
   pl.dur = h->has_dur ? h->at<int32_t>(h->o_dur) : nullptr;
   pl.reward = h->reward_override ? static_cast<real *>(h->reward_override) : h->at<real>(h->o_reward);
-  pl.obs = !h->p.obs_dim ? nullptr : (h->obs_override ? static_cast<real *>(h->obs_override) : h->at<real>(h->o_obs));
+  pl.obs = !h->p.obs_dim ? nullptr : (h->obs_override ? h->obs_override : static_cast<void *>(h->slab + h->o_obs));
   pl.actions = h->at<uint8_t>(h->o_actions);
   pl.epoch = h->at<int64_t>(h->o_epoch);
   pl.od_temp = h->at<double>(h->o_od);
@@ -208,6 +210,15 @@ static int fill_params(const drsim_config &c, SimParams &p, std::string &why) {
   else if (p.obs_layout == DRSIM_OBS_TARMAC) p.obs_dim = p.own_dim;
   else if (p.obs_layout == DRSIM_OBS_HAND_ENGINEERED) p.obs_dim = p.own_dim + p.nb_comm * p.msg_dim;
   else { why = "obs_layout"; return -1; }
+  if (c.obs_dtype != DRSIM_OBS_F32 && c.obs_dtype != DRSIM_OBS_BF16) { why = "obs_dtype"; return -1; }
+  if (c.obs_dtype == DRSIM_OBS_BF16 && c.precision != DRSIM_F32) {
+    why = "obs_dtype = DRSIM_OBS_BF16 needs precision = DRSIM_F32 (the fp64 build keeps fp64 rows)";
+    return -1;
+  }
+  if (c.obs_dtype == DRSIM_OBS_BF16 && p.obs_layout == DRSIM_OBS_NONE) {
+    why = "obs_dtype = DRSIM_OBS_BF16 needs an observation layout (obs_layout = none writes no rows)";
+    return -1;
+  }
   if (p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0 && p.N != p.n_global &&
       (p.comm_mode != DRSIM_COMM_RING || p.N < p.nb_comm)) {
     why = "house-sharded cluster with neighbour messages: only the ring (`neighbours`) mode is exchanged as a halo, and every "
@@ -236,9 +247,13 @@ static void plan_fused(drsim_handle *h, int e_cap = 1 << 30) {
   g.envs_per_tile = std::max(1, std::min(std::min(p.R, kTileSlots / p.Ns), e_cap));
   g.n_tiles = (p.R + g.envs_per_tile - 1) / g.envs_per_tile;
   g.max_segs = p.Ns >= 128 ? 2 : (128 + p.Ns - 1) / p.Ns + 1;
+  // bf16 rows of odd width: a 4-row group is 8 D bytes, not a multiple of the 16 a bulk store moves -- general path
+  if (h->obs_bytes == 2 && (p.obs_dim & 1)) return;
   g.need_msg = (p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0) ? 1 : 0;
   const int rb = h->real_bytes;
   const int slots = g.envs_per_tile * p.Ns;
+  // staging is planned for rows of `real` whatever the row dtype: a bf16 handle then takes the kernel variant and tile
+  // of the fp32 handle (its rows fill half of each staging slot), so its rows are the fp32 handle's rows, rounded
   const size_t row = (size_t)p.obs_dim * rb;
   auto layout = [&](bool direct, int chunk, bool allow_tma = true) {
     size_t off = 0;
@@ -307,42 +322,57 @@ static void plan_fused(drsim_handle *h, int e_cap = 1 << 30) {
 template <typename real>
 static int plan_shard(drsim_handle *h);
 
+// O = observation-row element type (real, or __nv_bfloat16 on an fp32 handle with DRSIM_OBS_BF16)
+template <typename real, typename O>
+static int configure_fused(drsim_handle *h, bool direct, int &per_sm) {
+  using Of = std::conditional_t<sizeof(O) == 8, float, O>;   // row type of the fp32-only kernels (never run on fp64)
+  const bool f = h->fused_ok;
+  if (f && h->geom.use_rows) {
+    if (sizeof(real) == 4) {
+      auto kern = h->geom.in_stride ? k_fused_rows<true, false, Of> : k_fused_rows<false, false, Of>;
+      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+      if (h->geom.in_stride)
+        CU_TRY(cudaFuncSetAttribute(k_fused_rows<true, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, h->geom.smem_bytes));
+    }
+    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  } else if (f && direct && h->geom.use_tma) {
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_tma<0, false, Of>, kThreads, h->geom.smem_bytes));
+  } else if (f && direct) {
+    CU_TRY(cudaFuncSetAttribute(k_fused_direct<real, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_direct<real, O>, kThreads, h->geom.smem_bytes));
+  } else if (f) {
+    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused<real, false, O>, kThreads, h->geom.smem_bytes));
+  }
+  const size_t obs_smem = (size_t)kObsChunk * h->p.obs_dim * sizeof(O);
+  if (obs_smem > 48 * 1024)
+    CU_TRY(cudaFuncSetAttribute(k_obs<real, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem));
+  return 0;
+}
+
 template <typename real>
 static int configure_kernels(drsim_handle *h) {
+  const bool direct = h->geom.chunk_rows == h->geom.envs_per_tile * h->p.Ns || h->p.obs_dim == 0;
+  int per_sm = 0;
+  int rc;
+  if constexpr (sizeof(real) == 4) {
+    rc = h->obs_bytes == 2 ? configure_fused<float, __nv_bfloat16>(h, direct, per_sm) : configure_fused<float, float>(h, direct, per_sm);
+  } else {
+    rc = configure_fused<real, real>(h, direct, per_sm);
+  }
+  if (rc) return rc;
   if (h->fused_ok) {
-    const bool direct = h->geom.chunk_rows == h->geom.envs_per_tile * h->p.Ns || h->p.obs_dim == 0;
     h->fused_direct = direct;
-    int per_sm = 0;
-    if (h->geom.use_rows) {
-      if (sizeof(real) == 4) {
-        auto kern = h->geom.in_stride ? k_fused_rows<true> : k_fused_rows<false>;
-        CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-        if (h->geom.in_stride)
-          CU_TRY(cudaFuncSetAttribute(k_fused_rows<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, h->geom.smem_bytes));
-      }
-      CU_TRY(cudaFuncSetAttribute(k_fused<real, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    } else if (direct && h->geom.use_tma) {
-      CU_TRY(cudaFuncSetAttribute(k_fused_tma<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaFuncSetAttribute(k_fused_tma<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaFuncSetAttribute(k_fused_tma<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_tma<0>, kThreads, h->geom.smem_bytes));
-    } else if (direct) {
-      CU_TRY(cudaFuncSetAttribute(k_fused_direct<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_direct<real>, kThreads, h->geom.smem_bytes));
-    } else {
-      CU_TRY(cudaFuncSetAttribute(k_fused<real, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused<real, false>, kThreads, h->geom.smem_bytes));
-    }
     if (per_sm < 1) { h->fused_ok = false; }
     else { h->fused_grid = std::min(h->geom.n_tiles, per_sm * h->sm_count); h->fused_per_sm = per_sm; }
   }
-  const size_t obs_smem = (size_t)kObsChunk * h->p.obs_dim * sizeof(real);
-  if (obs_smem > 48 * 1024)
-    CU_TRY(cudaFuncSetAttribute(k_obs<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem));
   if (h->p.policy == DRSIM_POLICY_GREEDY_MYOPIC) {
     int n2 = 1;
     while (n2 < h->p.N) n2 <<= 1;
@@ -372,6 +402,7 @@ extern "C" int drsim_create(const drsim_config *cfg, int device, drsim_t **out) 
   h->device = device;
   h->sm_count = prop.multiProcessorCount;
   h->real_bytes = cfg->precision == DRSIM_F64 ? 8 : 4;
+  h->obs_bytes = cfg->obs_dtype == DRSIM_OBS_BF16 ? 2 : h->real_bytes;
   const int rb = h->real_bytes;
   h->has_ratio = p.st_thermal || p.msg_thermal;
   h->has_interp = p.base_mode == DRSIM_BASE_INTERPOLATION;
@@ -391,7 +422,7 @@ extern "C" int drsim_create(const drsim_config *cfg, int device, drsim_t **out) 
   if (h->has_interp) { h->o_sub = cv.take(HP); h->o_interp = cv.take((size_t)DRSIM_INTERP_SUBTABLES * DRSIM_INTERP_SUBTABLE_LEN * rb); }
   h->o_reward = cv.take(HP * rb);
   h->o_dur = cv.take(HP * 4);
-  h->o_obs = cv.take(HP * p.obs_dim * rb + 16);
+  h->o_obs = cv.take(HP * p.obs_dim * h->obs_bytes + 16);
   h->o_actions = cv.take(HP);
   h->o_act_stage = cv.take(HP);
   const size_t E8 = (size_t)p.R * 8;
@@ -543,6 +574,7 @@ extern "C" int drsim_buffers(drsim_t *h, drsim_ptrs *o) {
   o->n_rep = h->p.R; o->n_house = h->p.N; o->house_stride = h->p.Ns; o->obs_dim = h->p.obs_dim;
   o->real_bytes = h->real_bytes; o->nb_comm = h->p.nb_comm;
   o->temp_is_deviation = h->real_bytes == 4 ? 1 : 0;
+  o->obs_bytes = h->obs_bytes;
   o->t_air = h->slab + h->o_t_air; o->t_mass = h->slab + h->o_t_mass;
   o->sso = h->at<int32_t>(h->o_sso); o->flags = h->at<uint8_t>(h->o_flags);
   o->target = h->slab + h->o_target; o->cap = h->slab + h->o_cap;
@@ -921,7 +953,11 @@ static int launch_env_phase(drsim_handle *h, const StepIn &in, const double *acc
   PeerCtx pc = make_peer(h);
   if (acc || n_parts >= 0) pc.world = 1;  // explicit partials (or the handle's own): no peer wait
   launch_pdl(k_env<real>, (p.R + 127) / 128, 128, 0, s, pl, p, in, (const double *)(acc ? acc : pl.acc), acc ? n_parts : 1, pc);
-  launch_pdl(k_obs<real>, p.R * h->obs_chunks, kObsChunk, (size_t)kObsChunk * p.obs_dim * sizeof(real), s, pl, p, in, h->obs_chunks);
+  auto kobs = k_obs<real, real>;
+  if constexpr (sizeof(real) == 4) {
+    if (h->obs_bytes == 2) kobs = k_obs<float, __nv_bfloat16>;
+  }
+  launch_pdl(kobs, p.R * h->obs_chunks, kObsChunk, (size_t)kObsChunk * p.obs_dim * h->obs_bytes, s, pl, p, in, h->obs_chunks);
   h->launches += 2;
   CU_TRY(cudaGetLastError());
   return 0;
@@ -940,12 +976,13 @@ static int plan_shard(drsim_handle *h) {
   h->shard_ok = false;
   if (getenv("DRSIM_NO_SHARD_KERNEL")) return 0;
   const int rb = (int)sizeof(real);
+  if (h->obs_bytes == 2 && (p.obs_dim & 1)) return 0;   // bf16 rows of odd width: four-kernel path (see plan_fused)
   const bool plain = shard_plain(h);
   g.chunks = h->chunks;
   g.n_tiles = p.R * h->chunks;
   const int min_ctas = FusedOcc<real>::min_ctas;
   const size_t budget = min_ctas >= 2 ? 110 * 1024 : 200 * 1024;
-  const size_t group = (size_t)kShardGroup * p.obs_dim * rb;
+  const size_t group = (size_t)kShardGroup * p.obs_dim * h->obs_bytes;
   g.nbuf = (size_t)(kThreads / 32) * 2 * group <= 48 * 1024 ? 2 : 1;
   // (also where the reducer parks the tile partials it collects: room for at least kReduceThreads of them)
   const size_t rows = plain ? (size_t)kTileSlots * 10 * 4
@@ -966,11 +1003,12 @@ static int plan_shard(drsim_handle *h) {
     g.smem_bytes = g.off_saved + g.t_smem * g.tile_bytes;
     bool done = false;
     if constexpr (sizeof(real) == 4) {
-      if (plain) {
-        CU_TRY(cudaFuncSetAttribute(k_shard<float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shard<float, true>, kThreads, g.smem_bytes));
-        done = true;
-      }
+      const bool bf = h->obs_bytes == 2;
+      auto kern = plain ? (bf ? k_shard<float, true, __nv_bfloat16> : k_shard<float, true>)
+                        : (bf ? k_shard<float, false, __nv_bfloat16> : k_shard<float, false>);
+      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
+      done = true;
     }
     if (!done) {
       CU_TRY(cudaFuncSetAttribute(k_shard<real, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
@@ -1023,15 +1061,13 @@ static int launch_shard(drsim_handle *h, StepIn in, cudaStream_t s) {
   sc.dbg = h->shard_dbg;
   PeerCtx pc = make_peer(h);
   if (!needs_halo(p)) pc.rowll = reinterpret_cast<unsigned long long *const *>(h->slab + h->o_peer_tab + 64 * 8);
-  bool plain = false;
+  auto kern = k_shard<real, false>;
   if constexpr (sizeof(real) == 4) {
-    if (shard_plain(h)) {
-      launch_pdl(k_shard<float, true>, h->shard_grid, kThreads, (size_t)h->shard.smem_bytes, s, pl, p, in, h->shard, sc, pc);
-      plain = true;
-    }
+    const bool bf = h->obs_bytes == 2;
+    if (shard_plain(h)) kern = bf ? k_shard<float, true, __nv_bfloat16> : k_shard<float, true>;
+    else if (bf) kern = k_shard<float, false, __nv_bfloat16>;
   }
-  if (!plain)
-    launch_pdl(k_shard<real, false>, h->shard_grid, kThreads, (size_t)h->shard.smem_bytes, s, pl, p, in, h->shard, sc, pc);
+  launch_pdl(kern, h->shard_grid, kThreads, (size_t)h->shard.smem_bytes, s, pl, p, in, h->shard, sc, pc);
   h->launches++;
   CU_TRY(cudaGetLastError());
   return 0;
@@ -1044,7 +1080,8 @@ static int exchange_error(const drsim_handle *h) {
   return 0;
 }
 
-// picks the compile-time specialisation of the production kernel (see k_fused_tma)
+// picks the compile-time specialisation of the production kernel (see k_fused_tma); O = row element type
+template <typename O>
 static void launch_tma(drsim_handle *h, const StepIn &in, cudaStream_t s) {
   const Planes<float> pl = make_planes<float>(h);
   const SimParams &p = h->p;
@@ -1055,24 +1092,25 @@ static void launch_tma(drsim_handle *h, const StepIn &in, cudaStream_t s) {
                       p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
   const bool poll = in.act_poll_err != nullptr;   // copy-engine mode of drsim_step_host
   if (common && !g.need_msg && g.envs_per_tile == 1) {
-    if (poll) launch_pdl(k_fused_tma<1, true>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<1>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    if (poll) launch_pdl(k_fused_tma<1, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    else launch_pdl(k_fused_tma<1, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
   } else if (common && g.need_msg && g.envs_per_tile > 1) {
-    if (poll) launch_pdl(k_fused_tma<2, true>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<2>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    if (poll) launch_pdl(k_fused_tma<2, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    else launch_pdl(k_fused_tma<2, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
   } else {
-    if (poll) launch_pdl(k_fused_tma<0, true>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<0>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    if (poll) launch_pdl(k_fused_tma<0, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    else launch_pdl(k_fused_tma<0, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
   }
 }
 
+template <typename O>
 static void launch_rows(drsim_handle *h, const StepIn &in, cudaStream_t s) {
   const Planes<float> pl = make_planes<float>(h);
   const int grid = h->launch_grid ? h->launch_grid : h->fused_grid;
   if (h->geom.in_stride && in.act_poll_err)
-    launch_pdl(k_fused_rows<true, true>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-  else if (h->geom.in_stride) launch_pdl(k_fused_rows<true>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-  else launch_pdl(k_fused_rows<false>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
+    launch_pdl(k_fused_rows<true, true, O>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
+  else if (h->geom.in_stride) launch_pdl(k_fused_rows<true, false, O>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
+  else launch_pdl(k_fused_rows<false, false, O>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
 }
 
 // steps the wide-row kernel cannot take (injected noise, on-device policies, common penalty modes)
@@ -1105,6 +1143,18 @@ static int snap_targets(drsim_handle *h, SnapPtrs &o, unsigned char **obs_dev);
 static bool small64_handle(const drsim_handle *h) {
   const SimParams &p = h->p;
   return !getenv("DRSIM_NO_SMALL") && h->real_bytes == 8 && h->fused_ok && p.Ns <= 32 && p.N == p.n_global && p.R <= 256;
+}
+
+// one launch of the tile kernel chosen for this handle, rows of element type O
+template <typename real, typename O>
+static void launch_tile(drsim_handle *h, const StepIn &in, bool rows_ok, cudaStream_t s) {
+  const Planes<real> pl = make_planes<real>(h);
+  if constexpr (sizeof(real) == 4) {
+    if (rows_ok) { launch_rows<O>(h, in, s); return; }
+    if (h->fused_direct && h->geom.use_tma) { launch_tma<O>(h, in, s); return; }
+  }
+  if (h->fused_direct) k_fused_direct<real, O><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
+  else k_fused<real, false, O><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
 }
 
 template <typename real>
@@ -1140,7 +1190,8 @@ static int launch_fused(drsim_handle *h, const StepIn &in, cudaStream_t s) {
         launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
         h->launches++;
       }
-      launch_pdl(k_small, (p.R + kSmallWarps - 1) / kSmallWarps, kSmallWarps * 32, 0, s, pl, p, in);
+      launch_pdl(h->obs_bytes == 2 ? k_small<__nv_bfloat16> : k_small<float>, (p.R + kSmallWarps - 1) / kSmallWarps,
+                 kSmallWarps * 32, 0, s, pl, p, in);
       h->launches++;
       CU_TRY(cudaGetLastError());
       return 0;
@@ -1157,10 +1208,15 @@ static int launch_fused(drsim_handle *h, const StepIn &in, cudaStream_t s) {
                        (p.policy == DRSIM_POLICY_EXTERNAL || p.policy == DRSIM_POLICY_GREEDY_MYOPIC) &&
                        p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
   if (h->geom.use_rows && !rows_ok) return launch_chunked_fallback<real>(h, in, s);
-  if (rows_ok) launch_rows(h, in, s);
-  else if (h->fused_direct && h->geom.use_tma) launch_tma(h, in, s);
-  else if (h->fused_direct) k_fused_direct<real><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, p, in, h->geom);
-  else k_fused<real, false><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, p, in, h->geom);
+  if constexpr (sizeof(real) == 4) {
+    if (h->obs_bytes == 2) {
+      launch_tile<float, __nv_bfloat16>(h, in, rows_ok, s);
+      h->launches++;
+      CU_TRY(cudaGetLastError());
+      return 0;
+    }
+  }
+  launch_tile<real, real>(h, in, rows_ok, s);
   h->launches++;
   CU_TRY(cudaGetLastError());
   return 0;
@@ -1445,7 +1501,7 @@ static size_t snap_layout(const drsim_handle *h, size_t off[8]) {
   size_t o = 0;
   auto take = [&](size_t b) { const size_t r = o; o += (b + 255) / 256 * 256; return r; };
   off[0] = take(HN * 8); off[1] = take(HN * 8); off[2] = take(HN * 8); off[3] = take(HN * 4); off[4] = take(HN);
-  off[5] = take(HN); off[6] = take((size_t)h->p.R * kSnapEnv * 8); off[7] = take(HN * h->p.obs_dim * h->real_bytes);
+  off[5] = take(HN); off[6] = take((size_t)h->p.R * kSnapEnv * 8); off[7] = take(HN * h->p.obs_dim * h->obs_bytes);
   return o;
 }
 
@@ -1479,7 +1535,7 @@ static int enqueue_snapshot(drsim_handle *h, cudaStream_t s) {
   else k_snapshot<float><<<(unsigned)((n + 255) / 256), 256, 0, s>>>(make_planes<float>(h), p, o);
   h->launches++;
   if (p.obs_dim) {
-    const size_t row = (size_t)p.obs_dim * h->real_bytes;
+    const size_t row = (size_t)p.obs_dim * h->obs_bytes;
     if (p.Ns == p.N) CU_TRY(cudaMemcpyAsync(h->h_snap + off[7], h->slab + h->o_obs, (size_t)p.R * p.N * row, cudaMemcpyDeviceToHost, s));
     else CU_TRY(cudaMemcpy2DAsync(h->h_snap + off[7], (size_t)p.N * row, h->slab + h->o_obs, (size_t)p.Ns * row, (size_t)p.N * row, p.R,
                                   cudaMemcpyDeviceToHost, s));
@@ -1628,7 +1684,7 @@ static int step_host_impl(drsim_t *h, const uint8_t *actions, const double *od_n
                                   (size_t)p.N * h->real_bytes, p.R, cudaMemcpyDeviceToHost, s));
   }
   if (obs_out) {
-    const size_t row = (size_t)p.obs_dim * h->real_bytes;
+    const size_t row = (size_t)p.obs_dim * h->obs_bytes;
     if (p.Ns == p.N) CU_TRY(cudaMemcpyAsync(obs_out, h->slab + h->o_obs, (size_t)p.R * p.N * row, cudaMemcpyDeviceToHost, s));
     else CU_TRY(cudaMemcpy2DAsync(obs_out, (size_t)p.N * row, h->slab + h->o_obs, (size_t)p.Ns * row, (size_t)p.N * row, p.R,
                                   cudaMemcpyDeviceToHost, s));
@@ -1839,7 +1895,7 @@ extern "C" int drsim_peer_status(drsim_t *h, void *stream) {
   return 0;
 }
 
-static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const float *obs_in, uint8_t *actions_out,
+static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const void *obs_in, uint8_t *actions_out,
                             float *prob_drawn, float *prob_on, void *stream);
 
 extern "C" int drsim_policy_step(drsim_t *h, const drsim_actor_net *net, uint64_t seed, float *prob_drawn, float *prob_on,
@@ -1861,7 +1917,7 @@ extern "C" int drsim_rollout_transition(drsim_t *h, const drsim_actor_net *net, 
   if (misaligned(slot->obs, 16) || misaligned(slot->reward, 16) || misaligned(slot->next_obs, 16) || misaligned(slot->actions, 4) ||
       misaligned(slot->prob, 4))
     return fail(DRSIM_E_ARG, "drsim_rollout_transition: obs / reward / next_obs must be 16-byte aligned, actions / prob 4-byte aligned");
-  int rc = policy_step_impl(h, net, seed, static_cast<const float *>(slot->obs), slot->actions, slot->prob, nullptr, stream);
+  int rc = policy_step_impl(h, net, seed, slot->obs, slot->actions, slot->prob, nullptr, stream);
   if (rc) return rc;
   drsim_step_args a{};
   a.actions = slot->actions;
@@ -1873,7 +1929,7 @@ extern "C" int drsim_rollout_transition(drsim_t *h, const drsim_actor_net *net, 
   return rc;
 }
 
-static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const float *obs_in, uint8_t *actions_out,
+static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const void *obs_in, uint8_t *actions_out,
                             float *prob_drawn, float *prob_on, void *stream) {
   if (!h || !net) return fail(DRSIM_E_ARG, "null argument");
   const SimParams &p = h->p;
@@ -1881,9 +1937,13 @@ static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t see
   if (p.obs_dim < 1 || p.obs_dim > 64) return fail(DRSIM_E_ARG, "drsim_policy_step: obs_dim must be in [1, 64]");
   if (net->h1 < 1 || net->h1 > 128 || net->h2 < 1 || net->h2 > 128) return fail(DRSIM_E_ARG, "drsim_policy_step: h1, h2 in [1, 128]");
   if (!net->w1 || !net->b1 || !net->w2 || !net->b2 || !net->w3 || !net->b3) return fail(DRSIM_E_ARG, "drsim_policy_step: null weight pointer");
+  const bool bf16 = h->obs_bytes == 2;
+  if (bf16 && net->precision != 1)
+    return fail(DRSIM_E_ARG, "drsim_policy_step: bfloat16 observation rows need precision = 1 (3xTF32); the single-pass actor "
+                             "stages fp32 rows");
   CU_TRY(cudaSetDevice(h->device));
   ActorArgs a{};
-  a.obs = obs_in ? obs_in : h->at<float>(h->o_obs);
+  a.obs = obs_in ? obs_in : static_cast<const void *>(h->slab + h->o_obs);
   a.w1 = net->w1; a.b1 = net->b1; a.w2 = net->w2; a.b2 = net->b2; a.w3 = net->w3; a.b3 = net->b3;
   a.actions = actions_out ? actions_out : h->at<uint8_t>(h->o_actions);
   a.prob = prob_drawn; a.prob_on = prob_on;
@@ -1922,7 +1982,11 @@ static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t see
     a.dbg = h->actor_dbg;
     k_actor_pack3x<<<40, 512, 0, (cudaStream_t)stream>>>(a, h->actor_image);
     const int pre = a.K1 / 8;                     // 16-byte K chunks per producer thread
-    auto kern = pre <= 2 ? k_actor3x<2> : pre <= 4 ? k_actor3x<4> : pre <= 7 ? k_actor3x<7> : k_actor3x<kAct3PreChunks>;
+    auto kern = bf16 ? (pre <= 2   ? k_actor3x<2, __nv_bfloat16>
+                        : pre <= 4 ? k_actor3x<4, __nv_bfloat16>
+                        : pre <= 7 ? k_actor3x<7, __nv_bfloat16>
+                                   : k_actor3x<kAct3PreChunks, __nv_bfloat16>)
+                     : (pre <= 2 ? k_actor3x<2> : pre <= 4 ? k_actor3x<4> : pre <= 7 ? k_actor3x<7> : k_actor3x<kAct3PreChunks>);
     CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
     launch_pdl(kern, std::min(tiles, h->sm_count), kAct3Threads, (size_t)a.smem_bytes, (cudaStream_t)stream, a);
     h->launches++;

@@ -17,6 +17,7 @@
 // Reference citations are relative to /root/reference/server/app.
 #pragma once
 
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
 #include "drsim_device.cuh"
@@ -44,7 +45,7 @@ struct Planes {
   const int32_t *dur;        // per-HVAC lock-out duration [R][Ns], or NULL: SimParams::lockout_duration for all
   // per-house outputs
   real *reward;
-  real *obs;
+  void *obs;                 // [R][Ns][D] rows of element type `real`, or __nv_bfloat16 (drsim_config.obs_dtype)
   uint8_t *actions;
   // per-env [R]
   int64_t *epoch;
@@ -57,7 +58,18 @@ struct Planes {
   const int32_t *comm_table;
   const real *interp_table;  // [162][9][5][8][12][6]
   double *halo_out;          // [R][nb_comm][kHaloFields]: message records of this shard's edge houses, or NULL
+
+  template <typename O>
+  DRSIM_HD O *rows() const { return static_cast<O *>(obs); }
 };
+
+// Observation-row element type O: `real`, or __nv_bfloat16 on an fp32 handle built with DRSIM_OBS_BF16.  A row value is
+// computed in `real` as always and rounded to nearest-even where it is stored (the implicit float -> __nv_bfloat16
+// conversion is __float2bfloat16_rn).  put2 stores columns 2 k, 2 k + 1 of a row with one 8- / 4-byte store.
+DRSIM_D void put2(float *row, int k, float a, float b) { reinterpret_cast<float2 *>(row)[k] = make_float2(a, b); }
+DRSIM_D void put2(__nv_bfloat16 *row, int k, float a, float b) {
+  reinterpret_cast<__nv_bfloat162 *>(row)[k] = __floats2bfloat162_rn(a, b);
+}
 
 // One packed record per (scheduled step, replica): every env-level value of that step that does NOT
 // depend on the step's cluster power, pre-computed by k_schedule_pack with the very expressions of
@@ -910,8 +922,8 @@ DRSIM_D real own_sso_norm(const Planes<real> &pl, const SimParams &p, size_t o, 
 // own-state part of the observation row (utils/norm.py:71-146).  `what` selects the columns
 // written: bit0 = those that depend on the house only, bit1 = those that need the env epilogue
 // (cluster power, signal, solar gain, outdoor temperature).
-template <typename real>
-DRSIM_D int obs_own(real *row, const SimParams &p, uint32_t f, real sso_n, real ta20, real tm20, real tg20,
+template <typename real, typename O>
+DRSIM_D int obs_own(O *row, const SimParams &p, uint32_t f, real sso_n, real ta20, real tm20, real tg20,
                     const EnvBroadcast<real> &e, const real ratio[4], int what = 3) {
   int i = 0;
   const bool hs = what & 1, ev = what & 2;
@@ -1374,11 +1386,11 @@ __global__ void k_env(Planes<real> pl, SimParams p, StepIn in, const double *acc
 
 // General path, kernel 4: rewards + observation rows for a chunk of kObsChunk houses.
 // Neighbour messages are gathered from global memory (any table); rows are assembled in shared
-// memory and written back with coalesced 128-bit stores.
-template <typename real>
+// memory and written back with coalesced 128-bit stores (2-byte stores where bf16 rows leave a chunk unaligned).
+template <typename real, typename O = real>
 __global__ void __launch_bounds__(kObsChunk) k_obs(Planes<real> pl, SimParams p, StepIn in, int chunks) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  real *tile = reinterpret_cast<real *>(smem_raw);
+  O *tile = reinterpret_cast<O *>(smem_raw);
   pdl_wait();
   pdl_trigger();
   const int r = blockIdx.x / chunks, c = blockIdx.x % chunks;
@@ -1395,7 +1407,7 @@ __global__ void __launch_bounds__(kObsChunk) k_obs(Planes<real> pl, SimParams p,
   e.pen_max = (real)pl.pen_max[r];
   const size_t rb = (size_t)r * p.Ns;
   if (n < p.Ns) {
-    real *row = tile + (size_t)threadIdx.x * D;
+    O *row = tile + (size_t)threadIdx.x * D;
     if (n < p.N) {
       const size_t o = rb + n;
       const real ta = pl.t_air[o], tm = pl.t_mass[o], tgt = pl.target[o];
@@ -1449,9 +1461,16 @@ __global__ void __launch_bounds__(kObsChunk) k_obs(Planes<real> pl, SimParams p,
   if (D == 0) return;
   __syncthreads();
   const int rows = min(kObsChunk, p.Ns - c * kObsChunk);
-  const size_t bytes = (size_t)rows * D * sizeof(real);  // rows % 4 == 0 -> multiple of 16
+  const size_t bytes = (size_t)rows * D * sizeof(O);  // rows % 4 == 0 -> multiple of 16 for 4- and 8-byte elements
+  O *gdst = pl.template rows<O>() + (rb + (size_t)c * kObsChunk) * D;
+  if (sizeof(O) == 2 && ((bytes | reinterpret_cast<uintptr_t>(gdst)) & 15)) {   // bf16 rows of odd D
+    const unsigned short *src = reinterpret_cast<const unsigned short *>(tile);
+    unsigned short *dst = reinterpret_cast<unsigned short *>(gdst);
+    for (size_t i = threadIdx.x; i < bytes / 2; i += blockDim.x) dst[i] = src[i];
+    return;
+  }
   const uint4 *src = reinterpret_cast<const uint4 *>(tile);
-  uint4 *dst = reinterpret_cast<uint4 *>(pl.obs + (rb + (size_t)c * kObsChunk) * D);
+  uint4 *dst = reinterpret_cast<uint4 *>(gdst);
   for (size_t i = threadIdx.x; i < bytes / 16; i += blockDim.x) dst[i] = src[i];
 }
 
@@ -1519,7 +1538,7 @@ template <> struct FusedOcc<float> { static constexpr int min_ctas = DRSIM_FUSED
 // DIRECT: the whole tile's observation rows fit the staging buffer; each thread writes the rows of
 // its own 4 houses straight from registers and one TMA bulk store per tile ships them.
 // ------------------------------------------------------------------------------------------
-template <typename real, bool DIRECT>
+template <typename real, bool DIRECT, typename O = real>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1527,7 +1546,7 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
   Own4<real> *s_own = reinterpret_cast<Own4<real> *>(smem_raw + g.off_own);
   EnvBroadcast<real> *s_env = reinterpret_cast<EnvBroadcast<real> *>(smem_raw + g.off_env);
   double *s_wp = reinterpret_cast<double *>(smem_raw + g.off_wp);  // [warps][max_segs][kRed]
-  real *s_tile = reinterpret_cast<real *>(smem_raw + g.off_tile);
+  O *s_tile = reinterpret_cast<O *>(smem_raw + g.off_tile);
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int Ns = p.Ns, D = p.obs_dim;
@@ -1621,7 +1640,7 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
         const int n0 = s0 - e_loc * Ns;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          real *row = s_tile + (size_t)(s0 + j) * D;
+          O *row = s_tile + (size_t)(s0 + j) * D;
           if (j < h.valid) {
             const uint32_t f = (h.flags >> (8 * j)) & 0xffu;
             real ratio[4] = {0, 0, 0, 0};
@@ -1651,7 +1670,7 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
         fence_proxy_async_smem();
         __syncthreads();
         if (threadIdx.x == 0) {
-          bulk_store_s2g(pl.obs + base * D, s_tile, (uint32_t)((size_t)slots * D * sizeof(real)));
+          bulk_store_s2g(pl.template rows<O>() + base * D, s_tile, (uint32_t)((size_t)slots * D * sizeof(O)));
           store_pending = true;
         }
       } else {
@@ -1664,7 +1683,7 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
           for (int i = threadIdx.x; i < rows; i += kThreads) {
             const int s = cb + i;
             const int e = (int)fast_div((uint32_t)s, p.fd_ns), n = s - e * Ns;
-            real *row = s_tile + (size_t)i * D;
+            O *row = s_tile + (size_t)i * D;
             if (n < p.N) {
               const Own4<real> o = s_own[s];
               const Msg4<real> m = s_msg[s];
@@ -1690,7 +1709,7 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
           fence_proxy_async_smem();
           __syncthreads();
           if (threadIdx.x == 0) {
-            bulk_store_s2g(pl.obs + (base + cb) * D, s_tile, (uint32_t)((size_t)rows * D * sizeof(real)));
+            bulk_store_s2g(pl.template rows<O>() + (base + cb) * D, s_tile, (uint32_t)((size_t)rows * D * sizeof(O)));
             store_pending = true;
           }
         }
@@ -1718,14 +1737,14 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
 // barrier; the two env-dependent columns, the neighbour messages and the rewards after the second.
 // Each warp ships its own 128 rows with one TMA bulk store (no CTA barrier in front of it).
 // ------------------------------------------------------------------------------------------
-template <typename real>
+template <typename real, typename O = real>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   Msg4<real> *s_msg_base = reinterpret_cast<Msg4<real> *>(smem_raw + g.off_msg);  // [2][slots] if need_msg
   EnvBroadcast<real> *s_env = reinterpret_cast<EnvBroadcast<real> *>(smem_raw + g.off_env);
   double *s_wp = reinterpret_cast<double *>(smem_raw + g.off_wp);  // [warps][max_segs][kRed]
-  real *s_tile = reinterpret_cast<real *>(smem_raw + g.off_tile);
+  O *s_tile = reinterpret_cast<O *>(smem_raw + g.off_tile);
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int Ns = p.Ns, D = p.obs_dim;
@@ -1776,20 +1795,19 @@ k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
           s_msg[s0 + j] = m;
         }
         if (D > 0) {
-          real *row = s_tile + (size_t)(s0 + j) * D;
+          O *row = s_tile + (size_t)(s0 + j) * D;
           if (plain) {
             // own_dim == 10, even D: rows are 8-byte aligned -> 64-bit shared stores
             if constexpr (sizeof(real) == 4) {
-              float2 *r2 = reinterpret_cast<float2 *>(row);
               const float tg = h.target[j] - 20.f;
               const bool ok = j < h.valid;
-              r2[0] = make_float2(ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
-              r2[1] = make_float2(ok ? sso_n : 0.f, ok ? 1.f : 0.f);
-              r2[3] = make_float2(ok ? p.hf.deadband : 0.f, ok ? (h.ta[j] + tg) * 0.2f : 0.f);
-              r2[4] = make_float2(ok ? (h.tm[j] + tg) * 0.2f : 0.f, ok ? tg * 0.2f : 0.f);
+              put2(row, 0, ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
+              put2(row, 1, ok ? sso_n : 0.f, ok ? 1.f : 0.f);
+              put2(row, 3, ok ? p.hf.deadband : 0.f, ok ? (h.ta[j] + tg) * 0.2f : 0.f);
+              put2(row, 4, ok ? (h.tm[j] + tg) * 0.2f : 0.f, ok ? tg * 0.2f : 0.f);
               if (!ok) {
-                r2[2] = make_float2(0.f, 0.f);
-                for (int q = 5; q < D / 2; ++q) r2[q] = make_float2(0.f, 0.f);
+                put2(row, 2, 0.f, 0.f);
+                for (int q = 5; q < D / 2; ++q) put2(row, q, 0.f, 0.f);
               }
             }
           } else if (j < h.valid) {
@@ -1858,17 +1876,16 @@ k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           if (j < h.valid) {
-            real *row = s_tile + (size_t)(s0 + j) * D;
+            O *row = s_tile + (size_t)(s0 + j) * D;
             if (plain) {
               if constexpr (sizeof(real) == 4) {
-                float2 *r2 = reinterpret_cast<float2 *>(row);
-                r2[2] = make_float2(e.power_n, e.signal_n);
+                put2(row, 2, e.power_n, e.signal_n);
                 if (g.need_msg) {
                   for (int k = 0; k < p.nb_comm; ++k) {
                     const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                     const float4 mk = *reinterpret_cast<const float4 *>(&s_msg[e_loc * Ns + nb]);
-                    r2[5 + 2 * k] = make_float2(mk.x, mk.y);
-                    r2[6 + 2 * k] = make_float2(mk.z, mk.w);
+                    put2(row, 5 + 2 * k, mk.x, mk.y);
+                    put2(row, 6 + 2 * k, mk.z, mk.w);
                   }
                 }
               }
@@ -1897,7 +1914,7 @@ k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
       const int w0 = warp * 128;
       if (lane == 0 && w0 < slots) {
         const int nrows = min(128, slots - w0);
-        bulk_store_s2g(pl.obs + (base + w0) * D, s_tile + (size_t)w0 * D, (uint32_t)((size_t)nrows * D * sizeof(real)));
+        bulk_store_s2g(pl.template rows<O>() + (base + w0) * D, s_tile + (size_t)w0 * D, (uint32_t)((size_t)nrows * D * sizeof(O)));
         store_pending = true;
       }
     }
@@ -2090,7 +2107,7 @@ DRSIM_D uint32_t act_word_polled(const uint8_t *actions, size_t off, uint32_t st
 
 // POLL = copy-engine mode of drsim_step_host (StepIn::act_poll_err): a separate instantiation, so the
 // device-resident step does not carry the branch (measured: 0.6 us of 39 on C4)
-template <int MODE, bool POLL = false>
+template <int MODE, bool POLL = false, typename O = float>
 __global__ void __launch_bounds__(kThreads, DRSIM_FUSED_MINCTAS)
 k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   typedef float real;
@@ -2102,7 +2119,7 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   double *s_wp_base = reinterpret_cast<double *>(smem_raw + g.off_wp);
   double *s_sold_base = reinterpret_cast<double *>(smem_raw + g.off_sold);  // [2][E] previous signal
   EnvStage *s_stage_base = reinterpret_cast<EnvStage *>(smem_raw + g.off_stage);  // [2][E] schedule record + metrics
-  real *s_tile = reinterpret_cast<real *>(smem_raw + g.off_tile);
+  O *s_tile = reinterpret_cast<O *>(smem_raw + g.off_tile);
   float *s_in = reinterpret_cast<float *>(smem_raw + g.off_in);        // [kInPlanes][kTileSlots]
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -2271,17 +2288,16 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
           s_msg[s0 + j] = m;
         }
         if (D > 0) {
-          real *row = s_tile + (size_t)(s0 + j) * D;
+          O *row = s_tile + (size_t)(s0 + j) * D;
           if (plain) {
-            float2 *r2 = reinterpret_cast<float2 *>(row);
             const float tg = h.target[j] - 20.f;
-            r2[0] = make_float2(ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
-            r2[1] = make_float2(ok ? sso_n : 0.f, ok ? 1.f : 0.f);
-            r2[3] = make_float2(ok ? p.hf.deadband : 0.f, ok ? (h.ta[j] + tg) * 0.2f : 0.f);
-            r2[4] = make_float2(ok ? (h.tm[j] + tg) * 0.2f : 0.f, ok ? tg * 0.2f : 0.f);
+            put2(row, 0, ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
+            put2(row, 1, ok ? sso_n : 0.f, ok ? 1.f : 0.f);
+            put2(row, 3, ok ? p.hf.deadband : 0.f, ok ? (h.ta[j] + tg) * 0.2f : 0.f);
+            put2(row, 4, ok ? (h.tm[j] + tg) * 0.2f : 0.f, ok ? tg * 0.2f : 0.f);
             if (!ok) {
-              r2[2] = make_float2(0.f, 0.f);
-              for (int q = 5; q < D / 2; ++q) r2[q] = make_float2(0.f, 0.f);
+              put2(row, 2, 0.f, 0.f);
+              for (int q = 5; q < D / 2; ++q) put2(row, q, 0.f, 0.f);
             }
           } else if (ok) {
             EnvBroadcast<real> none{};
@@ -2418,16 +2434,15 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           if (j < h.valid) {
-            real *row = s_tile + (size_t)(s0 + j) * D;
+            O *row = s_tile + (size_t)(s0 + j) * D;
             if (plain) {
-              float2 *r2 = reinterpret_cast<float2 *>(row);
-              r2[2] = make_float2(e.power_n, e.signal_n);
+              put2(row, 2, e.power_n, e.signal_n);
               if (need_msg) {
                 for (int k = 0; k < p.nb_comm; ++k) {
                   const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                   const float4 mk = *reinterpret_cast<const float4 *>(&s_msg[e_loc * Ns + nb]);
-                  r2[5 + 2 * k] = make_float2(mk.x, mk.y);
-                  r2[6 + 2 * k] = make_float2(mk.z, mk.w);
+                  put2(row, 5 + 2 * k, mk.x, mk.y);
+                  put2(row, 6 + 2 * k, mk.z, mk.w);
                 }
               }
               continue;
@@ -2455,7 +2470,7 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
         // the tile's previous step stored the same rows: its global writes must have landed, or they could
         // overwrite this step's (waited for here, a whole step after that store was issued)
         if (st > 0) bulk_store_wait_all();
-        bulk_store_s2g_hint(pl.obs + (base + w0) * D, s_tile + (size_t)w0 * D, (uint32_t)((size_t)nrows * D * sizeof(real)),
+        bulk_store_s2g_hint(pl.template rows<O>() + (base + w0) * D, s_tile + (size_t)w0 * D, (uint32_t)((size_t)nrows * D * sizeof(O)),
                             pol_stream);
         store_pending = true;
       }
@@ -2500,7 +2515,7 @@ constexpr int kRowGroup = 16;  // rows per warp-level TMA store in k_fused_rows 
 
 // STAGED = inputs prefetched one tile ahead into thread-private shared-memory slots (needs 44 B of
 // shared memory per house slot); false = 128-bit register loads at the top of the tile (large clusters)
-template <bool STAGED, bool POLL = false>
+template <bool STAGED, bool POLL = false, typename O = float>
 __global__ void __launch_bounds__(kThreads, 2)
 k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   typedef float real;
@@ -2512,7 +2527,7 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   EnvBroadcast<real> *s_env_base = reinterpret_cast<EnvBroadcast<real> *>(smem_raw + g.off_env);
   double *s_wp_base = reinterpret_cast<double *>(smem_raw + g.off_wp);
   double *s_sold_base = reinterpret_cast<double *>(smem_raw + g.off_sold);
-  real *s_stage = reinterpret_cast<real *>(smem_raw + g.off_tile);         // [warps][kRowGroup][D]
+  O *s_stage = reinterpret_cast<O *>(smem_raw + g.off_tile);         // [warps][kRowGroup][D]
   EnvStage *s_rec_base = reinterpret_cast<EnvStage *>(smem_raw + g.off_stage);  // [2][E] schedule record + metrics
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -2520,7 +2535,7 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   const int tile_slots = g.envs_per_tile * Ns;
   const int s0 = threadIdx.x * kHousesPerThread;
   const int w0 = warp * 128;
-  real *stage = s_stage + (size_t)warp * kRowGroup * D;
+  O *stage = s_stage + (size_t)warp * kRowGroup * D;
   bool store_pending = false;
   int parity = 0;
 
@@ -2703,18 +2718,18 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
       const int s = gs + row;
       if (s < slots) {
         const int e = (int)fast_div((uint32_t)s, p.fd_ns), n = s - e * Ns;
-        float2 *r2 = reinterpret_cast<float2 *>(stage + (size_t)row * D);
+        O *orow = stage + (size_t)row * D;
         if (n < p.N) {
           if (half == 0) {
             const float4 o = s_own[s];
             const float4 m = s_msg[s];
             const EnvBroadcast<real> ev = s_env[e];
             const uint32_t f = (uint32_t)o.w;
-            r2[0] = make_float2((float)(f & 1u), (float)((f >> 1) & 1u));
-            r2[1] = make_float2(m.y, 1.f);
-            r2[2] = make_float2(ev.power_n, ev.signal_n);
-            r2[3] = make_float2(p.hf.deadband, o.x);
-            r2[4] = make_float2(o.y, o.z);
+            put2(orow, 0, (float)(f & 1u), (float)((f >> 1) & 1u));
+            put2(orow, 1, m.y, 1.f);
+            put2(orow, 2, ev.power_n, ev.signal_n);
+            put2(orow, 3, p.hf.deadband, o.x);
+            put2(orow, 4, o.y, o.z);
           }
           const float4 *mb = s_msg + e * Ns;
           const int k0 = half ? nb_lo : 0, k1 = half ? nbc : nb_lo;
@@ -2724,25 +2739,25 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
             const float4 *src = mb + (half ? n + 1 - nb_lo : n - nb_lo);
             for (int q = k0; q < k1; ++q) {
               const float4 mk = src[q];
-              r2[5 + 2 * q] = make_float2(mk.x, mk.y);
-              r2[6 + 2 * q] = make_float2(mk.z, mk.w);
+              put2(orow, 5 + 2 * q, mk.x, mk.y);
+              put2(orow, 6 + 2 * q, mk.z, mk.w);
             }
           } else {
             for (int q = k0; q < k1; ++q) {
               const float4 mk = mb[neighbour_of(p, pl.comm_table, r0 + e, n, q)];
-              r2[5 + 2 * q] = make_float2(mk.x, mk.y);
-              r2[6 + 2 * q] = make_float2(mk.z, mk.w);
+              put2(orow, 5 + 2 * q, mk.x, mk.y);
+              put2(orow, 6 + 2 * q, mk.z, mk.w);
             }
           }
         } else {
-          for (int q = half; q < D / 2; q += 2) r2[q] = make_float2(0.f, 0.f);
+          for (int q = half; q < D / 2; q += 2) put2(orow, q, 0.f, 0.f);
         }
       }
       fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
         const int nrows = min(kRowGroup, slots - gs);
-        bulk_store_s2g(pl.obs + (base + gs) * D, stage, (uint32_t)((size_t)nrows * D * sizeof(real)));
+        bulk_store_s2g(pl.template rows<O>() + (base + gs) * D, stage, (uint32_t)((size_t)nrows * D * sizeof(O)));
         store_pending = true;
       }
     }
@@ -2764,6 +2779,7 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
 // ------------------------------------------------------------------------------------------
 constexpr int kSmallWarps = 4;   // clusters per CTA
 
+template <typename O = float>
 __global__ void __launch_bounds__(kSmallWarps * 32) k_small(Planes<float> pl, SimParams p, StepIn in) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int r = (int)blockIdx.x * kSmallWarps + warp;
@@ -2859,13 +2875,13 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small(Planes<float> pl, Si
     // this house's message record (building.py:102-139 through norm.py:31-60), read by its neighbours through shuffles
     const float m0 = ok ? ta * 0.2f : 0.f, m1 = ok ? sso_n : 0.f, m2 = (ok && (f & 1u)) ? pmax_n : 0.f, m3 = ok ? pmax_n : 0.f;
     if (D > 0) {
-      float2 *row = reinterpret_cast<float2 *>(pl.obs + o * D);
+      O *row = pl.template rows<O>() + o * D;
       if (slot) {
-        row[0] = make_float2(ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
-        row[1] = make_float2(ok ? sso_n : 0.f, ok ? 1.f : 0.f);
-        row[2] = ok ? make_float2(e.power_n, e.signal_n) : make_float2(0.f, 0.f);
-        row[3] = make_float2(ok ? p.hf.deadband : 0.f, ok ? (ta + tg20) * 0.2f : 0.f);
-        row[4] = make_float2(ok ? (tm + tg20) * 0.2f : 0.f, ok ? tg20 * 0.2f : 0.f);
+        put2(row, 0, ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
+        put2(row, 1, ok ? sso_n : 0.f, ok ? 1.f : 0.f);
+        put2(row, 2, ok ? e.power_n : 0.f, ok ? e.signal_n : 0.f);
+        put2(row, 3, ok ? p.hf.deadband : 0.f, ok ? (ta + tg20) * 0.2f : 0.f);
+        put2(row, 4, ok ? (tm + tg20) * 0.2f : 0.f, ok ? tg20 * 0.2f : 0.f);
       }
       if (need_msg) {
         for (int q = 0; q < nbc; ++q) {      // (every lane takes part in the shuffles)
@@ -2873,12 +2889,12 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small(Planes<float> pl, Si
           const float v0 = __shfl_sync(0xffffffffu, m0, nb), v1 = __shfl_sync(0xffffffffu, m1, nb),
                       v2 = __shfl_sync(0xffffffffu, m2, nb), v3 = __shfl_sync(0xffffffffu, m3, nb);
           if (slot) {
-            row[5 + 2 * q] = ok ? make_float2(v0, v1) : make_float2(0.f, 0.f);
-            row[6 + 2 * q] = ok ? make_float2(v2, v3) : make_float2(0.f, 0.f);
+            put2(row, 5 + 2 * q, ok ? v0 : 0.f, ok ? v1 : 0.f);
+            put2(row, 6 + 2 * q, ok ? v2 : 0.f, ok ? v3 : 0.f);
           }
         }
       } else if (slot && !ok) {
-        for (int q = 5; q < D / 2; ++q) row[q] = make_float2(0.f, 0.f);
+        for (int q = 5; q < D / 2; ++q) put2(row, q, 0.f, 0.f);
       }
     }
     // ---- env planes + running metrics (one lane; the staged record of the fused kernels, built in registers) ----
@@ -2981,7 +2997,7 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small_gen(Planes<real> pl,
     // this house's message record (building.py:102-139 through norm.py:31-60): its neighbours read it through shuffles
     const real m0 = ok ? div5(Rep<real>::dev(ta, tg)) : (real)0, m1 = ok ? sso_n : (real)0,
                m2 = (ok && (f & 1u)) ? pmax_n : (real)0, m3 = ok ? pmax_n : (real)0;
-    real *row = pl.obs + o * D;
+    real *row = pl.template rows<real>() + o * D;
     int q = 0;
     if (ok) {
       real ratio[4] = {0, 0, 0, 0};
@@ -3017,7 +3033,7 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small_gen(Planes<real> pl,
       snap.on[i] = (uint8_t)(f & 1u);
       snap.lockout[i] = (uint8_t)((f >> 1) & 1u);
       if (snap_obs && D > 0) {
-        const real *src = pl.obs + o * D;
+        const real *src = pl.template rows<real>() + o * D;
         real *dst = snap_obs + i * D;
         for (int k = 0; k < D; ++k) dst[k] = src[k];
       }

@@ -181,7 +181,7 @@ DRSIM_D void ld4i_cg(const int32_t *p, int v[4]) {
 }
 
 // PLAIN = fp32 build, 10-column rows without neighbour messages (TarMAC layout / nb_comm = 0)
-template <typename real, bool PLAIN>
+template <typename real, bool PLAIN, typename O = real>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerCtx peer) {
   static_assert(!PLAIN || sizeof(real) == 4, "the plain variant is fp32 only");
@@ -558,7 +558,7 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
   };
 
   if constexpr (PLAIN) {
-    float *s_tile = reinterpret_cast<float *>(smem_raw + g.off_rows);
+    O *s_tile = reinterpret_cast<O *>(smem_raw + g.off_rows);
     bool store_pending = false;
     const int w0 = warp * 128;
     for (int tile = t_lo; tile < t_hi; ++tile) {
@@ -596,12 +596,12 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
           const uint32_t f = (flags >> (8 * j)) & 0xffu;
           const float sso_n = (float)fast_div((uint32_t)sso[j], p.fd_dur);          // norm.py:40-43, :79-82
           const float t20 = tg[j] - 20.f;
-          float2 *r2 = reinterpret_cast<float2 *>(s_tile + (size_t)(s0 + j) * 10);
-          r2[0] = make_float2(ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
-          r2[1] = make_float2(ok ? sso_n : 0.f, ok ? 1.f : 0.f);
-          r2[2] = make_float2(ok ? e.power_n : 0.f, ok ? e.signal_n : 0.f);
-          r2[3] = make_float2(ok ? p.hf.deadband : 0.f, ok ? (ta[j] + t20) * 0.2f : 0.f);
-          r2[4] = make_float2(ok ? (tm[j] + t20) * 0.2f : 0.f, ok ? t20 * 0.2f : 0.f);
+          O *row = s_tile + (size_t)(s0 + j) * 10;
+          put2(row, 0, ok ? (float)(f & 1u) : 0.f, ok ? (float)((f >> 1) & 1u) : 0.f);
+          put2(row, 1, ok ? sso_n : 0.f, ok ? 1.f : 0.f);
+          put2(row, 2, ok ? e.power_n : 0.f, ok ? e.signal_n : 0.f);
+          put2(row, 3, ok ? p.hf.deadband : 0.f, ok ? (ta[j] + t20) * 0.2f : 0.f);
+          put2(row, 4, ok ? (tm[j] + t20) * 0.2f : 0.f, ok ? t20 * 0.2f : 0.f);
         }
         store4(pl.reward + off, rw);
       }
@@ -609,7 +609,8 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
       __syncwarp();
       if (lane == 0 && w0 < slots) {
         const int nrows = min(128, slots - w0);
-        bulk_store_s2g(pl.obs + (rb + (size_t)c * kTileSlots + w0) * 10, s_tile + (size_t)w0 * 10, (uint32_t)(nrows * 40));
+        bulk_store_s2g(pl.template rows<O>() + (rb + (size_t)c * kTileSlots + w0) * 10, s_tile + (size_t)w0 * 10,
+                       (uint32_t)(nrows * 10 * sizeof(O)));
         store_pending = true;
       }
     }
@@ -617,7 +618,7 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
     if (lane == 0 && store_pending) bulk_store_wait_read();
     stamp(5);
   } else {
-    real *rows_w = reinterpret_cast<real *>(smem_raw + g.off_rows) + (size_t)warp * g.nbuf * kShardGroup * D;
+    O *rows_w = reinterpret_cast<O *>(smem_raw + g.off_rows) + (size_t)warp * g.nbuf * kShardGroup * D;
     const bool halo = needs_halo(p);
     int grp = 0;   // row groups this warp has shipped (selects the staging buffer)
     for (int tile = t_lo; tile < t_hi; ++tile) {
@@ -632,7 +633,7 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
         const int ng0 = c * kTileSlots + hs0;            // ... inside the cluster
         if (ng0 >= Ns) break;                            // warp-uniform: nothing of this group exists
         const int n = ng0 + lane, hs = hs0 + lane;
-        real *row = rows_w + ((size_t)(grp % g.nbuf) * kShardGroup + lane) * D;
+        O *row = rows_w + ((size_t)(grp % g.nbuf) * kShardGroup + lane) * D;
         if (D > 0) {
           // the bulk store that last used this staging buffer must have finished reading it
           if (lane == 0 && grp >= g.nbuf) {
@@ -699,8 +700,8 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
           __syncwarp();
           if (lane == 0) {
             const int nrows = min(kShardGroup, Ns - ng0);   // multiple of 4: the byte count is a multiple of 16
-            bulk_store_s2g(pl.obs + (rb + ng0) * D, rows_w + (size_t)(grp % g.nbuf) * kShardGroup * D,
-                           (uint32_t)((size_t)nrows * D * sizeof(real)));
+            bulk_store_s2g(pl.template rows<O>() + (rb + ng0) * D, rows_w + (size_t)(grp % g.nbuf) * kShardGroup * D,
+                           (uint32_t)((size_t)nrows * D * sizeof(O)));
           }
           ++grp;
         }

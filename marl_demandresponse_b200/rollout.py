@@ -32,7 +32,7 @@ class RolloutBuffer:
         R, N, Ns, D = sim.R, sim.N, sim.Ns, sim.D
         self.R, self.N, self.Ns, self.D = R, N, Ns, D
         dev = f"cuda:{sim.device}"
-        self.obs = torch.zeros((self.T + 1, R, Ns, D), dtype=torch.float32, device=dev)
+        self.obs = torch.zeros((self.T + 1, R, Ns, D), dtype=torch.bfloat16 if sim.obs_bf16 else torch.float32, device=dev)
         self.actions = torch.zeros((self.T, R, Ns), dtype=torch.uint8, device=dev)
         self.probs = torch.zeros((self.T, R, Ns), dtype=torch.float32, device=dev)
         self.rewards = torch.zeros((self.T, R, Ns), dtype=torch.float32, device=dev)

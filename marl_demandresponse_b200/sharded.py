@@ -63,7 +63,7 @@ def halo_lookup(gathered, n_global: int, rank: int, world: int, nb_comm: int, ho
 class ShardedClusterEnv:
     def __init__(self, env_props: Any, n_replicas: int = 1, rank: int = 0, world: int = 1, device: int = 0,
                  precision: str = "f32", obs_layout: str = "tarmac", policy: str = "external", noise: str = "philox",
-                 seed: int = 0, group=None, exchange: str = "nccl"):
+                 seed: int = 0, group=None, exchange: str = "nccl", obs_dtype: str = "float32"):
         self.props = as_props(env_props)
         self.rank, self.world, self.group = int(rank), int(world), group
         self.n_global = int(self.props.cluster_prop.nb_agents)
@@ -71,7 +71,7 @@ class ShardedClusterEnv:
         if self.hi <= self.lo:
             raise ValueError("more ranks than 4-house blocks")
         cfg = flatten_config(self.props, n_replicas, precision, obs_layout, policy, noise, seed, "split",
-                             house_offset=self.lo, n_house_local=self.hi - self.lo)
+                             house_offset=self.lo, n_house_local=self.hi - self.lo, obs_dtype=obs_dtype)
         self.sim = DrSim(cfg, device)
         self.device = device
         self._v = self.sim.views()
