@@ -8,31 +8,8 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 
-def _prop(n, **over):
-    p = {"start_datetime": "2021-06-15T11:58:20", "start_datetime_mode": "fixed", "time_step": 4.0,
-         "cluster_prop": {"nb_agents": n, "house_prop": {"target_temp": 19.0}}}
-    for path, v in over.items():
-        d = p
-        keys = path.split("/")
-        for k in keys[:-1]:
-            d = d.setdefault(k, {})
-        d[keys[-1]] = v
-    return p
-
-
-def _oracle_run(prop, st, actions, od_noise, perlin):
-    from oracle.np_oracle import NpOracle
-
-    R = st["t_air"].shape[0]
-    orc = NpOracle(prop, R)
-    orc.set_state(st)
-    from oracle.np_oracle import from_epoch
-
-    orc.power_grid_step([from_epoch(e) for e in orc.state["epoch"]], perlin[0])   # PowerGrid.step at reset
-    rew = []
-    for t in range(actions.shape[0]):
-        rew.append(orc.step(actions[t], od_noise[t], perlin[t + 1]))
-    return orc, np.array(rew)
+from oracle_driver import OracleDriver, od_noise as _od_noise, oracle_run as _oracle_run, perlin as _perlin
+from oracle_driver import prop as _prop
 
 
 @pytest.mark.parametrize("n,R,layout,path", [(100, 24, "hand_engineered", "auto"), (1000, 6, "tarmac", "auto"),
@@ -48,7 +25,6 @@ def test_batched_env_philox_matches_oracle(n, R, layout, path):
 
     from marl_demandresponse_b200 import BatchedEnv
     from marl_demandresponse_b200.batched import synthetic_state
-    from oracle import philox
 
     T, seed, off = 12, 77, 1000
     prop = _prop(n)
@@ -59,13 +35,9 @@ def test_batched_env_philox_matches_oracle(n, R, layout, path):
     acts = (rng.random((T, R, n)) < 0.5).astype(np.uint8)
     # the values the device streams must produce
     epoch0 = int(st["epoch"][0])
-    sp = {"nb_octaves": 5, "octaves_step": 5, "period": 300}
-    od_noise = np.array([[philox.od_noise(seed, off + r, t, 1.0) for r in range(R)] for t in range(T)])
-    perlin = np.zeros((T + 1, R))
-    for t in range(T + 1):
-        tsec = (epoch0 + 4 * t) % 86400
-        for r in range(R):
-            perlin[t, r] = philox.perlin(seed, off + r, tsec / sp["period"], sp["nb_octaves"], sp["octaves_step"])
+    reps = [off + r for r in range(R)]
+    od_noise = _od_noise(seed, reps, range(T))
+    perlin = _perlin(seed, reps, [epoch0 + 4 * t for t in range(T + 1)])
     rewards = []
     for t in range(T):
         obs, rew = env.step(torch.as_tensor(acts[t], device="cuda"))
@@ -198,8 +170,15 @@ def test_fused_kernel_variants_match_general_path(R, n, layout, tile_envs, varia
             if tile_envs is not None:
                 assert info["envs_per_tile"] == min(tile_envs, 1024 // env.sim.Ns), info
         env.reset(copy.deepcopy(st))
-        for t in range(T):
-            env.step(torch.as_tensor(acts[t], device="cuda"))
+        if path == "fused":   # every step re-anchored on the oracle on three replicas (first, last, mid-tile)
+            drv = OracleDriver(env, prop, st)
+            assert len(drv.picks) == 3, drv.picks
+            for t in range(T):
+                drv.step(acts[t])
+            drv.check_metrics()
+        else:
+            for t in range(T):
+                env.step(torch.as_tensor(acts[t], device="cuda"))
         torch.cuda.synchronize()
         out[path] = {k: env.state[k].clone() for k in
                      ("signal", "od_temp", "epoch", "sso", "flags", "power", "dt_air", "dt_mass", "reward", "obs", "metrics")}
@@ -685,7 +664,6 @@ def test_full_size_c4_spot_check_against_oracle():
 
     from marl_demandresponse_b200 import BatchedEnv
     from marl_demandresponse_b200.batched import synthetic_state
-    from oracle import philox
 
     n, R, T, seed = 1000, 2048, 8, 1234
     prop = _prop(n)
@@ -706,8 +684,8 @@ def test_full_size_c4_spot_check_against_oracle():
     pick = [0, 777, 2047]
     sub = {k: (v[pick] if np.asarray(v).shape[:1] == (R,) else v) for k, v in st.items()}
     epoch0 = int(st["epoch"][0])
-    od_noise = np.array([[philox.od_noise(seed, r, t, 1.0) for r in pick] for t in range(T)])
-    perlin = np.array([[philox.perlin(seed, r, ((epoch0 + 4 * t) % 86400) / 300, 5, 5) for r in pick] for t in range(T + 1)])
+    od_noise = _od_noise(seed, pick, range(T))
+    perlin = _perlin(seed, pick, [epoch0 + 4 * t for t in range(T + 1)])
     a_np = np.stack([a[pick].cpu().numpy() for a in acts])
     orc, _ = _oracle_run(prop, sub, a_np, od_noise, perlin)
     for k in ("on", "lockout", "sso"):
@@ -726,7 +704,6 @@ def test_edge_sizes_match_oracle(n, R, precision):
 
     from marl_demandresponse_b200 import BatchedEnv
     from marl_demandresponse_b200.batched import synthetic_state
-    from oracle import philox
 
     T, seed = 6, 3
     prop = _prop(n, **{"reward_prop/penalty_props/mode": "mixture", "cluster_prop/house_prop/deadband": 0.4})
@@ -735,8 +712,8 @@ def test_edge_sizes_match_oracle(n, R, precision):
     env.reset(copy.deepcopy(st))
     acts = (np.random.default_rng(4).random((T, R, n)) < 0.5).astype(np.uint8)
     epoch0 = int(st["epoch"][0])
-    od_noise = np.array([[philox.od_noise(seed, r, t, 1.0) for r in range(R)] for t in range(T)])
-    perlin = np.array([[philox.perlin(seed, r, ((epoch0 + 4 * t) % 86400) / 300, 5, 5) for r in range(R)] for t in range(T + 1)])
+    od_noise = _od_noise(seed, range(R), range(T))
+    perlin = _perlin(seed, range(R), [epoch0 + 4 * t for t in range(T + 1)])
     rew = []
     for t in range(T):
         _, r_ = env.step(torch.as_tensor(acts[t], device="cuda"))
@@ -759,7 +736,6 @@ def test_maximum_size_single_cluster_of_one_million_houses():
 
     from marl_demandresponse_b200.batched import synthetic_state
     from marl_demandresponse_b200.sharded import ShardedClusterEnv
-    from oracle import philox
 
     n, T, seed = 1_000_000, 3, 5
     prop = _prop(n)
@@ -769,8 +745,8 @@ def test_maximum_size_single_cluster_of_one_million_houses():
     env.sim.refresh(True)
     acts = (np.random.default_rng(6).random((T, 1, n)) < 0.5).astype(np.uint8)
     epoch0 = int(st["epoch"][0])
-    od_noise = np.array([[philox.od_noise(seed, 0, t, 1.0)] for t in range(T)])
-    perlin = np.array([[philox.perlin(seed, 0, ((epoch0 + 4 * t) % 86400) / 300, 5, 5)] for t in range(T + 1)])
+    od_noise = _od_noise(seed, [0], range(T))
+    perlin = _perlin(seed, [0], [epoch0 + 4 * t for t in range(T + 1)])
     for t in range(T):
         env.step(torch.as_tensor(acts[t], device="cuda"))
     orc, rew_ref = _oracle_run(prop, copy.deepcopy(st), acts, od_noise, perlin)
@@ -810,9 +786,9 @@ def test_device_reset_matches_numpy_restatement(mode, precision):
         assert np.all(got["on"] == 1) and np.allclose(got["t_air"], 20.0, rtol=0, atol=1e-5)
     # continue from the device-drawn state and compare with the oracle started from the restated one
     acts = (np.random.default_rng(0).random((T, R, n)) < 0.5).astype(np.uint8)
-    od_noise = np.array([[philox.od_noise(seed, off + r, t, 1.0) for r in range(R)] for t in range(T)])
-    perlin = np.array([[philox.perlin(seed, off + r, ((int(want["epoch"][r]) + 4 * t) % 86400) / 300, 5, 5) for r in range(R)]
-                       for t in range(T + 1)])
+    reps = [off + r for r in range(R)]
+    od_noise = _od_noise(seed, reps, range(T))
+    perlin = _perlin(seed, reps, [np.asarray(want["epoch"]) + 4 * t for t in range(T + 1)])
     for t in range(T):
         env.step(torch.as_tensor(acts[t], device="cuda"))
     if mode == "reference":

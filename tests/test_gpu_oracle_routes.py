@@ -1,0 +1,394 @@
+"""Every step-kernel route, and the in-kernel step loop, against the fp64 NumPy oracle.
+
+The step has one specification, ``oracle/np_oracle.py``, and many implementations; the host picks one from the
+shape and the configuration (``plan_fused``, ``launch_tile``, ``launch_tma``, ``small_handle`` and the ``taped``
+condition of ``drsim_run_tape`` in ``drsim_api.cu``).  Each case below names the kernel it means to run and fails if
+the planner stops sending it there: ``fused_info()`` gives the variant and the clusters per tile, ``launch_count``
+the launches per step, and where the ABI says nothing (which ``k_fused_tma<MODE>`` specialisation, ``k_small``) the
+test restates the host condition and the case table states the expected outcome.
+
+* ``test_route_matches_oracle``: a mode matrix over the routes (a covering design, not the full product), 24 steps
+  re-anchored on the oracle at every step, and the same steps free-running.
+* ``test_seeded_sweep_matches_oracle``: random (R, N, layout, modes) from a fixed list of seeds.
+* ``test_in_kernel_loop_matches_oracle``: ``run(T, tape, rotate=True)`` on the loop routes: one step kernel per
+  schedule block, bit-identical to one launch per step, and free-running against the oracle.
+
+Tolerances and the replicas compared are those of ``oracle_driver``.
+"""
+import copy
+import os
+
+import numpy as np
+import pytest
+
+from oracle_driver import OracleDriver, prop, same_state
+
+pytestmark = pytest.mark.gpu
+
+T_STEPS = 24   # a 40 s lock-out is 10 steps of 4 s: lock-outs expire and re-arm within the run
+
+# neighbours_2D: N -> (row_size, max_communication_distance); the table is 2 d (d + 1) wide
+NB_2D = {12: (4, 1), 100: (10, 1), 300: (15, 1), 1000: (25, 2), 1300: (26, 2), 2500: (50, 2)}
+
+
+def config(n, pen="individual_L2", sig="perlin", state="none", msg="none", nb="neighbours", c=10, start=None, dist=None,
+           **extra):
+    """Properties of one matrix cell.  The deadband keeps ``common_max_error`` non-zero and the lock-out FSM busy."""
+    over = {"cluster_prop/house_prop/deadband": 0.4,
+            "reward_prop/penalty_props/mode": pen,
+            "reward_prop/penalty_props/alpha_common_max": 1.0,
+            "power_grid_prop/signal_properties/mode": sig,
+            "state_prop/solar_gain": state in ("solar", "all"),
+            "state_prop/thermal": state == "all",
+            "state_prop/hvac": state == "all",
+            "cluster_prop/message_prop/thermal": msg == "th_hvac",
+            "cluster_prop/message_prop/hvac": msg == "th_hvac",
+            "cluster_prop/agents_comm_prop/mode": nb,
+            "cluster_prop/agents_comm_prop/max_nb_agents_communication": c}
+    if nb == "neighbours_2D":
+        row, d = NB_2D[n]
+        dist = d if dist is None else dist
+        over["cluster_prop/agents_comm_prop/row_size"] = row
+        over["cluster_prop/agents_comm_prop/max_communication_distance"] = dist
+    if start is not None:
+        over["start_datetime"] = start
+    over.update(extra)
+    return prop(n, **over)
+
+
+def dims(p, layout):
+    """(own columns, message columns, row width, messages in the rows?) as ``fill_params`` / ``plan_fused`` derive them."""
+    from marl_demandresponse_b200.core import comm_width
+    from marl_demandresponse_b200.properties import as_props
+
+    sp, mp = p["state_prop"], p["cluster_prop"]["message_prop"]
+    own = 10 + 2 * sp["hvac"] + sp["solar_gain"] + 5 * sp["thermal"]
+    msg = 4 + 4 * mp["thermal"] + 3 * mp["hvac"]
+    c = comm_width(as_props(p))
+    D = {"none": 0, "tarmac": own, "hand_engineered": own + c * msg}[layout]
+    return own, msg, D, layout == "hand_engineered" and c > 0
+
+
+def tma_mode(p, layout, e):
+    """The ``k_fused_tma`` specialisation ``launch_tma`` picks for a scheduled step (no injected noise) with external
+    actions: 1 = plain rows without messages, one cluster per tile, individual penalty; 2 = plain rows with messages,
+    several clusters per tile, individual penalty; 0 = everything else."""
+    own, msg, D, need_msg = dims(p, layout)
+    plain = own == 10 and msg == 4 and D % 2 == 0 and D > 0
+    common = plain and p["reward_prop"]["penalty_props"]["mode"] == "individual_L2"
+    if common and not need_msg and e == 1:
+        return 1
+    if common and need_msg and e > 1:
+        return 2
+    return 0
+
+
+def small_fp32(sim, p, layout):
+    """``small_handle``: clusters of at most 32 plane slots in at most 256 replicas, plain columns."""
+    own, msg, D, need_msg = dims(p, layout)
+    if sim.real != np.float32 or sim.fused_info()["variant"] == "none" or sim.Ns > 32 or sim.R > 256:
+        return False
+    if D == 0:
+        return True
+    if own != 10 or D % 2:
+        return False
+    return msg == 4 if need_msg else D == 10
+
+
+def small_fp64(sim):
+    """``small64_handle``: the fp64 build's ``k_small_gen`` takes any observation options."""
+    return sim.real == np.float64 and sim.fused_info()["variant"] != "none" and sim.Ns <= 32 and sim.R <= 256
+
+
+# route -> (precision, R, N, layout, path, environment, expected)
+#   expected: variant = fused_info()["variant"]; e = clusters per tile; launches = kernel launches per step;
+#   mode = k_fused_tma<MODE> (restated from launch_tma); small = k_small / k_small_gen (restated from small_handle)
+ROUTES = {
+    "k_fused_tma<1>": ("f32", 12, 1000, "tarmac", "auto", {}, dict(variant="staged", e=1, launches=1, mode=1)),
+    "k_fused_tma<2>": ("f32", 30, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 3},
+                       dict(variant="staged", e=3, launches=1, mode=2)),
+    "k_fused_tma<0>/1-per-tile": ("f32", 9, 300, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 1},
+                                  dict(variant="staged", e=1, launches=1, mode=0)),
+    "k_fused_tma<0>/3-per-tile": ("f32", 30, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 3},
+                                  dict(variant="staged", e=3, launches=1, mode=0)),
+    "k_fused_rows<staged>": ("f32", 60, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 7},
+                             dict(variant="staged_rows", e=7, launches=1)),
+    "k_fused_rows<unstaged>": ("f32", 6, 1000, "hand_engineered", "auto", {}, dict(variant="staged_rows", e=1, launches=1)),
+    "general/rows-fallback": ("f32", 60, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 7},
+                              dict(variant="staged_rows", e=7, launches=4)),
+    "k_fused/chunked": ("f32", 3, 1000, "hand_engineered", "auto", {}, dict(variant="chunked", e=1, launches=1)),
+    # 85 clusters per tile: their schedule records do not fit next to the TMA planes (rows of at most 16 columns)
+    "k_fused_direct": ("f32", 300, 10, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 85},
+                       dict(variant="direct", e=85, launches=1, small=False)),
+    "k_small": ("f32", 7, 10, "hand_engineered", "auto", {}, dict(launches=1, small=True)),
+    "k_shard": ("f32", 2, 2500, "hand_engineered", "auto", {}, dict(variant="none", launches=1)),
+    "four-kernel": ("f32", 24, 100, "hand_engineered", "split", {"DRSIM_NO_SHARD_KERNEL": 1},
+                    dict(variant="none", launches=4)),
+    "k_fused_direct<double>": ("f64", 24, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 2},
+                               dict(variant="direct", e=2, launches=1)),
+    "k_fused<double>/chunked": ("f64", 3, 1000, "hand_engineered", "auto", {}, dict(variant="chunked", e=1, launches=1)),
+    "k_small_gen<double>": ("f64", 7, 10, "hand_engineered", "auto", {}, dict(launches=1, small=True)),
+    "k_shard<double>": ("f64", 3, 1300, "hand_engineered", "auto", {}, dict(variant="none", launches=1)),
+}
+
+# the mode matrix: every value of every axis on every route that can take it, plus penalty x clusters per tile
+# (the k_fused_tma<0> routes with one and three clusters per tile), flags x odd D and neighbour mode x clusters per tile.
+# Routes that cannot take a value: k_fused_tma<1|2> and k_fused_rows only run the individual penalty with plain rows
+# (a common penalty there is the rows fallback / k_fused_tma<0>); k_small takes plain rows only.
+MATRIX = {
+    "k_fused_tma<1>": [dict(sig="perlin"), dict(sig="sinusoidals"), dict(sig="regular_steps"), dict(sig="flat"),
+                       dict(sig="perlin", layout="hand_engineered", c=0)],
+    "k_fused_tma<2>": [dict(sig="perlin", nb="neighbours", c=1), dict(sig="sinusoidals", nb="random_fixed", c=3),
+                       dict(sig="regular_steps", nb="closed_groups", c=5), dict(sig="flat", nb="neighbours_2D", c=10)],
+    "k_fused_tma<0>/1-per-tile": [
+        dict(pen="common_L2", sig="perlin", nb="neighbours", c=1),
+        dict(pen="common_max_error", sig="sinusoidals", state="solar", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", state="all", nb="closed_groups", c=5),
+        dict(sig="flat", state="solar", nb="neighbours_2D"),
+        dict(pen="mixture", sig="perlin", c=0),
+        dict(pen="common_L2", sig="sinusoidals", state="solar", layout="tarmac")],
+    "k_fused_tma<0>/3-per-tile": [
+        dict(pen="common_L2", sig="perlin", nb="neighbours", c=2),
+        dict(pen="common_max_error", sig="sinusoidals", state="solar", msg="th_hvac", nb="random_fixed", c=2),
+        dict(pen="mixture", sig="regular_steps", state="all", nb="neighbours_2D"),
+        dict(sig="flat", state="solar", nb="closed_groups", c=3),
+        dict(pen="common_max_error", sig="flat", c=0),
+        dict(sig="sinusoidals", layout="tarmac")],
+    "k_fused_rows<staged>": [dict(sig="perlin", c=10), dict(sig="sinusoidals", nb="random_fixed", c=7),
+                             dict(sig="regular_steps", nb="closed_groups", c=9), dict(sig="flat", nb="neighbours_2D", dist=2)],
+    "k_fused_rows<unstaged>": [dict(sig="perlin", c=10), dict(sig="sinusoidals", nb="random_fixed", c=10),
+                               dict(sig="regular_steps", nb="closed_groups", c=9), dict(sig="flat", nb="neighbours_2D", dist=2)],
+    "general/rows-fallback": [dict(pen="common_L2", sig="perlin"), dict(pen="common_max_error", sig="sinusoidals", nb="random_fixed"),
+                              dict(pen="mixture", sig="regular_steps", nb="closed_groups", c=9),
+                              dict(pen="common_L2", sig="flat", nb="neighbours_2D", dist=2)],
+    "k_fused/chunked": [
+        dict(pen="common_L2", sig="perlin", state="solar", nb="neighbours", c=10),
+        dict(pen="common_max_error", sig="sinusoidals", state="all", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", msg="th_hvac", nb="closed_groups", c=9),
+        dict(sig="flat", state="solar", msg="th_hvac", nb="neighbours_2D"),
+        dict(sig="perlin", state="all", msg="th_hvac", c=1)],
+    "k_fused_direct": [   # (no room for message flags or a 2-D neighbourhood in rows of 16 columns)
+        dict(pen="common_L2", sig="perlin", layout="tarmac"),
+        dict(pen="common_max_error", sig="sinusoidals", state="solar", layout="tarmac"),
+        dict(pen="mixture", sig="regular_steps", state="all", layout="tarmac"),
+        dict(sig="flat", c=1),
+        dict(pen="common_max_error", sig="perlin", nb="random_fixed", c=1),
+        dict(pen="mixture", sig="sinusoidals", nb="closed_groups", c=1),
+        dict(sig="regular_steps", state="solar", c=0)],
+    "k_small": [dict(pen="common_L2", sig="perlin", c=9), dict(pen="common_max_error", sig="sinusoidals", nb="random_fixed", c=3),
+                dict(pen="mixture", sig="regular_steps", nb="closed_groups", c=4), dict(sig="flat", c=0),
+                dict(sig="perlin", c=1)],
+    "k_shard": [
+        dict(pen="common_L2", sig="perlin", c=10),
+        dict(pen="common_max_error", sig="sinusoidals", state="solar", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", state="all", nb="closed_groups", c=10),
+        dict(sig="flat", state="solar", nb="neighbours_2D"),
+        dict(pen="mixture", sig="perlin", layout="tarmac"),
+        dict(sig="sinusoidals", c=1), dict(pen="common_L2", sig="flat", c=0)],
+    "four-kernel": [
+        dict(pen="common_L2", sig="perlin", state="solar", c=1),
+        dict(pen="common_max_error", sig="sinusoidals", state="all", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", msg="th_hvac", nb="closed_groups", c=10),
+        dict(sig="flat", nb="neighbours_2D", c=0)],
+    "k_fused_direct<double>": [
+        dict(pen="common_L2", sig="perlin", c=10),
+        dict(pen="common_max_error", sig="sinusoidals", state="solar", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", state="all", nb="closed_groups", c=4),
+        dict(sig="flat", state="solar", nb="neighbours_2D"),
+        dict(sig="perlin", c=1), dict(sig="sinusoidals", c=0)],
+    "k_fused<double>/chunked": [
+        dict(pen="common_L2", sig="perlin", c=10),
+        dict(pen="common_max_error", sig="sinusoidals", state="all", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", state="solar", nb="closed_groups", c=9),
+        dict(sig="flat", state="solar", msg="th_hvac", nb="neighbours_2D")],
+    "k_small_gen<double>": [
+        dict(pen="common_L2", sig="perlin", state="solar", c=9),
+        dict(pen="common_max_error", sig="sinusoidals", state="all", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", msg="th_hvac", nb="closed_groups", c=4),
+        dict(sig="flat", c=0), dict(sig="perlin", nb="neighbours_2D", n=12)],
+    "k_shard<double>": [
+        dict(pen="common_L2", sig="perlin", c=10),
+        dict(pen="common_max_error", sig="sinusoidals", state="solar", msg="th_hvac", nb="random_fixed", c=3),
+        dict(pen="mixture", sig="regular_steps", state="all", nb="closed_groups", c=10),
+        dict(sig="flat", state="solar", nb="neighbours_2D"), dict(sig="sinusoidals", c=1)],
+}
+# neighbours_2D needs N % row_size == 0: the 10-house routes take it at N = 12 (its own case)
+MATRIX["k_small"].append(dict(sig="perlin", nb="neighbours_2D", n=12, c=10))
+
+CASES = [pytest.param(route, i, id=f"{route}-{i}") for route in ROUTES for i in range(len(MATRIX[route]))]
+
+
+def _make(route, cell, monkeypatch, seed=21):
+    """The handle of one matrix cell, its properties and initial state; asserts the route it takes."""
+    from marl_demandresponse_b200 import BatchedEnv
+    from marl_demandresponse_b200.batched import synthetic_state
+
+    precision, R, N, layout, path, env_vars, expect = ROUTES[route]
+    cell = dict(cell)
+    layout = cell.pop("layout", layout)
+    N = cell.pop("n", N)
+    for k, v in env_vars.items():
+        monkeypatch.setenv(k, str(v))
+    p = config(N, **cell)
+    env = BatchedEnv(p, R, precision=precision, obs_layout=layout, noise="philox", seed=seed, path=path)
+    info = env.sim.fused_info()
+    print(route, cell, info)
+    if "variant" in expect:
+        assert info["variant"] == expect["variant"], (route, info)
+    if "e" in expect:
+        assert info["envs_per_tile"] == expect["e"], (route, info)
+    if "mode" in expect:
+        assert tma_mode(p, layout, info["envs_per_tile"]) == expect["mode"], (route, dims(p, layout))
+    if "small" in expect:
+        small = small_fp32(env.sim, p, layout) if precision == "f32" else small_fp64(env.sim)
+        assert small == expect["small"], (route, info, dims(p, layout))
+    st = synthetic_state(p, R, seed=seed + 1)
+    env.reset(copy.deepcopy(st))
+    return env, p, st, expect
+
+
+@pytest.mark.parametrize("route,i", CASES)
+def test_route_matches_oracle(route, i, monkeypatch):
+    """24 steps of one matrix cell: every step re-anchored on the oracle (the single-step error), the trajectory
+    free-running against the oracle, the running metrics, and the launches of each step."""
+    env, p, st, expect = _make(route, MATRIX[route][i], monkeypatch)
+    R, N = env.n_replicas, env.n_houses
+    drv = OracleDriver(env, p, st)
+    drv.start_free()
+    acts = (np.random.default_rng(100 + i).random((T_STEPS, R, N)) < 0.5).astype(np.uint8)
+    launches = [drv.step(acts[t]) for t in range(T_STEPS)]
+    # the first step generates the 64-step schedule block (two kernels), then one route's launches per step
+    assert launches == [expect["launches"] + 2] + [expect["launches"]] * (T_STEPS - 1), launches
+    drv.check_metrics()
+    drv.check_free()
+
+
+SWEEP_SEEDS = list(range(20))
+
+
+@pytest.mark.parametrize("seed", SWEEP_SEEDS)
+def test_seeded_sweep_matches_oracle(seed):
+    """Random (R, N, layout, modes) on whatever route the planner picks, re-anchored on the oracle at every step."""
+    from marl_demandresponse_b200 import BatchedEnv
+    from marl_demandresponse_b200.batched import synthetic_state
+
+    rng = np.random.default_rng(1000 + seed)
+    N = int(rng.choice([1, 2, 3, 5, 9, 10, 12, 33, 64, 100, 127, 128, 250, 300, 333, 512, 1000, 1023, 1024, 1300]))
+    R = int(rng.integers(1, max(2, min(3000, 300000 // N))))
+    layout = str(rng.choice(["tarmac", "hand_engineered", "none"]))
+    precision = str(rng.choice(["f32", "f64"], p=[0.7, 0.3]))
+    c = int(rng.choice([0, 1, 3, 4, 10, 11]))
+    nb = str(rng.choice(["neighbours", "random_fixed", "closed_groups", "neighbours_2D"]))
+    # (closed_groups: a last group one house short makes the reference's table point past the cluster)
+    if nb == "neighbours_2D" and N not in NB_2D or nb == "closed_groups" and (c > N - 1 or N % (c + 1) == c):
+        nb = "neighbours"
+    cell = dict(pen=str(rng.choice(["individual_L2", "common_L2", "common_max_error", "mixture"])),
+                sig=str(rng.choice(["perlin", "sinusoidals", "regular_steps", "flat"])),
+                state=str(rng.choice(["none", "solar", "all"])), msg=str(rng.choice(["none", "th_hvac"])), nb=nb, c=c)
+    p = config(N, **cell)
+    env = BatchedEnv(p, R, precision=precision, obs_layout=layout, noise="philox", seed=seed)
+    print(seed, R, N, layout, precision, cell, env.sim.fused_info())
+    st = synthetic_state(p, R, seed=seed)
+    env.reset(copy.deepcopy(st))
+    drv = OracleDriver(env, p, st)
+    T = 12
+    acts = (rng.random((T, R, N)) < 0.5).astype(np.uint8)
+    for t in range(T):
+        drv.step(acts[t])
+    drv.check_metrics()
+
+
+def _loop_launches(first_step, T, block_base):
+    """Launches of ``drsim_run_tape`` on a loop route: one step kernel per 64-step schedule block, plus the two schedule
+    kernels when the run enters a block that has not been generated (``block_base`` = start of the current block)."""
+    n, s, base = 0, first_step, block_base
+    while s < first_step + T:
+        if base is None or not base <= s < base + 64:
+            base, n = s, n + 2
+        k = min(first_step + T - s, base + 64 - s)
+        n, s = n + 1, s + k
+    return n
+
+
+# route, R, N, layout, environment, cell, steps before the run, run length, expected (fp32: the loop is fp32 only)
+LOOP_CASES = [
+    ("k_small", 7, 10, "hand_engineered", {}, dict(c=9), 0, 70, dict(small=True)),
+    ("k_small", 7, 10, "hand_engineered", {}, dict(pen="common_max_error", nb="closed_groups", c=4, sig="sinusoidals"), 5, 100,
+     dict(small=True)),
+    ("k_small", 5, 10, "hand_engineered", {}, dict(pen="mixture", nb="random_fixed", c=3, sig="flat",
+                                                   start="2021-12-31T23:58:20"), 0, 70, dict(small=True)),
+    ("k_fused_tma<1>", 400, 1000, "tarmac", {}, dict(sig="perlin", start="2021-06-15T23:58:20"), 0, 70,
+     dict(variant="staged", e=1, mode=1)),
+    ("k_fused_tma<1>", 640, 1000, "tarmac", {}, dict(sig="sinusoidals"), 5, 100, dict(variant="staged", e=1, mode=1)),
+    ("k_fused_tma<2>", 1800, 100, "hand_engineered", {"DRSIM_TILE_ENVS": 3}, dict(c=2, sig="regular_steps", nb="random_fixed",
+                                                                                 start="2021-12-31T23:58:20"), 0, 70,
+     dict(variant="staged", e=3, mode=2)),
+    ("k_fused_tma<0>", 400, 1000, "tarmac", {}, dict(pen="common_L2", state="solar", start="2021-12-31T23:58:20"), 0, 70,
+     dict(variant="staged", e=1, mode=0)),
+    ("k_fused_tma<0>", 300, 300, "hand_engineered", {"DRSIM_TILE_ENVS": 1},
+     dict(pen="common_max_error", state="solar", msg="th_hvac", nb="closed_groups", c=3, sig="sinusoidals"), 5, 100,
+     dict(variant="staged", e=1, mode=0)),
+    ("k_fused_tma<0>", 1800, 100, "hand_engineered", {"DRSIM_TILE_ENVS": 3},
+     dict(pen="mixture", state="all", nb="neighbours_2D", sig="perlin", start="2021-06-15T23:58:20"), 0, 70,
+     dict(variant="staged", e=3, mode=0)),
+    ("k_fused_tma<0>", 6100, 100, "tarmac", {}, dict(pen="common_max_error", sig="flat"), 5, 100,
+     dict(variant="staged", mode=0)),
+    ("k_fused_rows", 4096, 100, "hand_engineered", {}, dict(c=10, sig="sinusoidals", start="2021-06-15T23:58:20"), 0, 70,
+     dict(variant="staged_rows")),
+    ("k_fused_rows", 4096, 100, "hand_engineered", {}, dict(c=10, nb="random_fixed", sig="perlin"), 5, 100,
+     dict(variant="staged_rows")),
+]
+
+
+@pytest.mark.parametrize("route,R,N,layout,env_vars,cell,pre,T,expect",
+                         [pytest.param(*c, id=f"{c[0]}-{i}") for i, c in enumerate(LOOP_CASES)])
+def test_in_kernel_loop_matches_oracle(route, R, N, layout, env_vars, cell, pre, T, expect, monkeypatch):
+    """``run(T, tape, rotate=True)`` with the step loop inside the kernel: one step kernel per schedule block, the same
+    bits as one launch per step (``DRSIM_NO_STREAM=1``), and the trajectory free-running against the oracle."""
+    import datetime as _dt
+
+    import torch
+
+    from marl_demandresponse_b200 import BatchedEnv
+    from marl_demandresponse_b200.batched import synthetic_state
+
+    for k, v in env_vars.items():
+        monkeypatch.setenv(k, str(v))
+    p = config(N, **cell)
+    env = BatchedEnv(p, R, obs_layout=layout, noise="philox", seed=31)
+    info = env.sim.fused_info()
+    print(route, cell, info)
+    for k in ("variant", "e"):
+        if k in expect:
+            assert info[{"e": "envs_per_tile"}.get(k, k)] == expect[k], info
+    if "mode" in expect:
+        assert tma_mode(p, layout, info["envs_per_tile"]) == expect["mode"], dims(p, layout)
+    if "small" in expect:
+        assert small_fp32(env.sim, p, layout) == expect["small"], info
+    if route == "k_fused_rows":   # the loop takes k_fused_rows on at least two tiles per CTA (the `taped` condition)
+        assert (min(info["grid"], info["tiles"] // 2)) * 10 >= info["grid"] * 9, info
+    start = _dt.datetime.fromisoformat(cell["start"]) if "start" in cell else None
+    st = synthetic_state(p, R, seed=4, start=start)
+    env.reset(copy.deepcopy(st))
+    planes = 3
+    tape = (torch.rand((planes, R, N), device="cuda", generator=torch.Generator(device="cuda").manual_seed(6)) < 0.5)
+    tape = tape.to(torch.uint8)
+    tape_np = tape.cpu().numpy()
+    drv = OracleDriver(env, p, st)
+    for t in range(pre):
+        drv.step(tape_np[t % planes], check=False)
+    twin = copy.deepcopy(env)
+    drv.start_free()
+    l0 = env.sim.launch_count
+    env.run(T, tape, rotate=True)
+    torch.cuda.synchronize()
+    # (the first of the steps before the run generated the block that starts at step 0; set_state invalidates it)
+    assert env.sim.launch_count - l0 == _loop_launches(pre, T, 0 if pre else None), (env.sim.launch_count - l0, pre, T)
+    monkeypatch.setenv("DRSIM_NO_STREAM", "1")
+    twin.run(T, tape, rotate=True)
+    monkeypatch.delenv("DRSIM_NO_STREAM")
+    torch.cuda.synchronize()
+    same_state(env, twin)
+    for k in range(T):
+        drv.advance_free(tape_np[k % planes])
+    drv.check_free(f"{route}: run({T}) from step {pre}")
