@@ -51,8 +51,14 @@ enum { DRSIM_OBS_NONE = 0, DRSIM_OBS_HAND_ENGINEERED = 1, DRSIM_OBS_TARMAC = 2 }
 /* element type of the observation rows: the build's `real`, or bfloat16 (fp32 build only).  A bf16 row element is
  * the fp32 element the kernels compute, rounded to nearest-even where it is stored; nothing else changes. */
 enum { DRSIM_OBS_F32 = 0, DRSIM_OBS_BF16 = 1 };
-/* neighbour source: arithmetic ring (agent_communication_builder.py:63-85) or explicit table */
-enum { DRSIM_COMM_RING = 0, DRSIM_COMM_TABLE = 1 };
+/* neighbour source: arithmetic ring (agent_communication_builder.py:63-85), explicit table, or a fresh uniform
+ * sample per step (`random_sample`, cluster.py:96-99): neighbour k of house n in the rows written after the handle's
+ * d-th step (d = drsim_step_count; rows of drsim_reset / drsim_refresh use the current count) is output k of a
+ * sparse partial Fisher-Yates shuffle of the other houses driven by Philox4x32-10 keyed (seed, global replica,
+ * global house, d, purpose 7 | block << 8) -- see drsim_comm_sample and DESIGN.md.  Replicas only: a house-sharded
+ * handle rejects it.  nb_comm <= DRSIM_MAX_SAMPLE_COMM in this mode (the swap record is per-thread). */
+enum { DRSIM_COMM_RING = 0, DRSIM_COMM_TABLE = 1, DRSIM_COMM_SAMPLE = 2 };
+#define DRSIM_MAX_SAMPLE_COMM 32
 /* where per-step noise comes from when the matching pointer of drsim_step_args is NULL */
 enum { DRSIM_NOISE_ZERO = 0, DRSIM_NOISE_PHILOX = 1 };
 /* action source: caller-provided, or restated controllers
@@ -242,6 +248,15 @@ int drsim_reset(drsim_t *h, const drsim_reset_args *args, void *stream);
 /* Cluster.agent_communicators (cluster.py:66-70): explicit neighbour table, host int32
  * [n_house][nb_comm] (per_replica = 0) or [n_rep][n_house][nb_comm] (per_replica = 1). */
 int drsim_set_comm_table(drsim_t *h, const int32_t *table, int per_replica, void *stream);
+
+/* DRSIM_COMM_SAMPLE handle: writes the neighbour table of draw `draw` -- device int32 [n_rep][n_house][nb_comm],
+ * global house ids -- on `stream`.  draw < 0: the draw behind the current observation rows (= drsim_step_count).
+ * This is what a TarMAC policy attends over.  DRSIM_E_STATE on a handle of another mode. */
+int drsim_comm_sample(drsim_t *h, int64_t draw, int32_t *d_out, void *stream);
+
+/* steps taken since creation or the last drsim_reset (drsim_step, drsim_run, step_host, rollout, sharded steps);
+ * drsim_clone copies it */
+int64_t drsim_step_count(const drsim_t *h);
 
 /* PowerInterpolator.values (interpolation.py:88-90) re-ordered to
  * [162][9][5][8][12][6] (see DESIGN.md), host fp64. */
@@ -444,6 +459,9 @@ void drsim_host_civil(int64_t epoch, int32_t out7[7]); /* year, month, day, hour
 void drsim_host_thermal_coefs(double Ua, double Ca, double Cm, double Hm, int32_t dt, double out12[12]);
 /* Philox4x32-10 block, for cross-checking the NumPy restatement */
 void drsim_host_philox(uint64_t seed, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t out4[4]);
+/* the DRSIM_COMM_SAMPLE draw of one house: out[0..c) = its c sampled neighbours (global ids), the device's code.
+ * Requires 1 <= c <= min(n_global - 1, DRSIM_MAX_SAMPLE_COMM); otherwise out is left untouched. */
+void drsim_host_comm_sample(uint64_t seed, int64_t rep, int64_t house, int64_t draw, int64_t n_global, int c, int32_t *out);
 
 const char *drsim_last_error(void);
 int drsim_abi_version(void);

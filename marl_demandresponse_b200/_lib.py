@@ -25,7 +25,8 @@ BASE = {"constant": 0, "interpolation": 1}
 SIG = {"flat": 0, "sinusoidals": 1, "regular_steps": 2, "perlin": 3}
 OBS = {"none": 0, "hand_engineered": 1, "tarmac": 2}
 OBS_DTYPE = {"float32": 0, "bfloat16": 1}
-COMM_RING, COMM_TABLE = 0, 1
+COMM_RING, COMM_TABLE, COMM_SAMPLE = 0, 1, 2
+MAX_SAMPLE_COMM = 32   # DRSIM_MAX_SAMPLE_COMM: nb_comm bound of the `random_sample` mode
 NOISE = {"zero": 0, "philox": 1}
 POLICY = {"external": 0, "deadband_bangbang": 1, "bangbang": 2, "always_on": 3, "greedy_myopic": 4}
 PATH = {"auto": 0, "fused": 1, "split": 2}
@@ -153,6 +154,8 @@ def lib():
         "drsim_reset": (C.c_int, [hp, C.POINTER(ResetArgs), C.c_void_p]),
         "drsim_set_comm_table": (C.c_int, [hp, C.c_void_p, C.c_int, C.c_void_p]),
         "drsim_set_interp_table": (C.c_int, [hp, C.c_void_p, C.c_void_p]),
+        "drsim_comm_sample": (C.c_int, [hp, _i64, C.c_void_p, C.c_void_p]),
+        "drsim_step_count": (C.c_int64, [hp]),
         "drsim_step": (C.c_int, [hp, C.POINTER(StepArgs), C.c_void_p]),
         "drsim_run": (C.c_int, [hp, C.POINTER(StepArgs), C.c_int, C.c_size_t, C.c_void_p]),
         "drsim_run_tape": (C.c_int, [hp, C.POINTER(StepArgs), C.c_int, C.c_size_t, C.c_int, C.c_void_p]),
@@ -182,6 +185,7 @@ def lib():
         "drsim_host_civil": (None, [_i64, C.POINTER(_i32 * 7)]),
         "drsim_host_thermal_coefs": (None, [_d, _d, _d, _d, _i32, C.POINTER(_d * 12)]),
         "drsim_host_philox": (None, [_u64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32 * 4)]),
+        "drsim_host_comm_sample": (None, [_u64, _i64, _i64, _i64, _i64, C.c_int, C.c_void_p]),
         "drsim_last_error": (C.c_char_p, []),
         "drsim_abi_version": (C.c_int, []),
         "drsim_sizeof": (C.c_int, [C.c_int]),
@@ -205,7 +209,7 @@ EXPORTED_SYMBOLS = [
     "drsim_step_finish", "drsim_step_sharded", "drsim_step_finish_gathered", "drsim_step_host", "drsim_step_host_full", "drsim_snapshot", "drsim_step_host_snapshot",
     "drsim_ipc_export", "drsim_ipc_attach", "drsim_peer_status", "drsim_peer_attach_local", "drsim_policy_step", "drsim_rollout_transition", "drsim_launch_count", "drsim_fused_info", "drsim_cluster_summary", "drsim_metrics_update", "drsim_host_solar_gain", "drsim_host_od_temp",
     "drsim_host_civil", "drsim_host_thermal_coefs", "drsim_host_philox", "drsim_last_error", "drsim_abi_version",
-    "drsim_sizeof",
+    "drsim_sizeof", "drsim_comm_sample", "drsim_step_count", "drsim_host_comm_sample",
 ]
 
 

@@ -98,10 +98,12 @@ class BatchedEnv:
                              rep_offset=rep_offset, obs_dtype=obs_dtype)
         self.sim = DrSim(cfg, device)
         self.device = device
-        mode = self.props.cluster_prop.agents_comm_prop.mode
+        self.comm_mode = self.props.cluster_prop.agents_comm_prop.mode
         self.comm_width = comm_width(self.props)
+        # a table mode's static table is drawn once: here when the rows carry messages, else at the first
+        # neighbour_index(); `random_sample` draws on the device every step instead (no table)
         self._table: Optional[np.ndarray] = None
-        if mode != "neighbours" and obs_layout == "hand_engineered" and self.comm_width > 0:
+        if self._table_mode() and obs_layout == "hand_engineered":
             self._table = self._static_table()
             self.sim.set_comm_table(self._table)
         if interp_table is not None:
@@ -109,15 +111,24 @@ class BatchedEnv:
         self._v = self.sim.views()
 
     # ---- neighbour index tensor (TarMAC attention mask / message routing) -----------------
+    def _table_mode(self) -> bool:
+        return self.comm_mode not in ("neighbours", "random_sample") and self.comm_width > 0
+
     def _static_table(self) -> np.ndarray:
         from .environment import build_comm_table
 
         return build_comm_table(self.props)
 
-    def neighbour_index(self):
-        """Static ``[N, c]`` int32 neighbour tensor on the device."""
+    def neighbour_index(self, draw: Optional[int] = None):
+        """int32 neighbour tensor on the device.  ``random_sample``: ``[R, N, c]``, the neighbours behind the current
+        observation rows, or those of draw ``draw`` (the draw index is the step count the rows were written at, see
+        ``DrSim.step_count``).  Other modes: the mode's static ``[N, c]`` table."""
         import torch
 
+        if self.comm_mode == "random_sample":
+            return self.sim.comm_sample(draw)
+        if self._table is None and self._table_mode():
+            self._table = self._static_table()
         t = self._table if self._table is not None else ring_table(self.n_houses, self.comm_width)
         return torch.as_tensor(t, device=f"cuda:{self.device}")
 

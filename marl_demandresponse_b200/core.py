@@ -111,9 +111,12 @@ def flatten_config(props: Any, n_rep: int = 1, precision: str = "f32", obs_layou
     c.obs_dtype = _lib.OBS_DTYPE[obs_dtype]
     c.nb_comm = comm_width(p)
     mode = p.cluster_prop.agents_comm_prop.mode
-    if comm_table is None:
-        comm_table = mode != "neighbours"
-    c.comm_mode = _lib.COMM_TABLE if comm_table else _lib.COMM_RING
+    if comm_table is None and mode == "random_sample":
+        c.comm_mode = _lib.COMM_SAMPLE     # drawn on the device every step (drsim_comm_sample)
+    else:
+        if comm_table is None:
+            comm_table = mode != "neighbours"
+        c.comm_mode = _lib.COMM_TABLE if comm_table else _lib.COMM_RING
     st, mp = p.state_prop, p.cluster_prop.message_prop
     c.state_solar_gain, c.state_thermal, c.state_hvac = int(st.solar_gain), int(st.thermal), int(st.hvac)
     c.message_thermal, c.message_hvac = int(mp.thermal), int(mp.hvac)
@@ -518,6 +521,24 @@ class DrSim:
     @property
     def launch_count(self) -> int:
         return int(self._L.drsim_launch_count(self._h))
+
+    @property
+    def step_count(self) -> int:
+        """Steps taken since creation or the last device reset (``drsim_step_count``)."""
+        return int(self._L.drsim_step_count(self._h))
+
+    def comm_sample(self, draw: Optional[int] = None, out=None, stream=None):
+        """``random_sample`` handle (``COMM_SAMPLE``): the neighbour table of draw ``draw`` -- default the draw behind
+        the current observation rows, i.e. :attr:`step_count` -- as an int32 CUDA tensor ``[R, N, nb_comm]``
+        (``drsim_comm_sample``)."""
+        import torch
+
+        c = int(self.ptrs.nb_comm)
+        if out is None:
+            out = torch.empty((self.R, self.N, c), dtype=torch.int32, device=f"cuda:{self.device}")
+        assert out.dtype == torch.int32 and out.is_contiguous() and out.numel() == self.R * self.N * c
+        _lib.check(self._L.drsim_comm_sample(self._h, -1 if draw is None else int(draw), self._ptr(out), self._stream(stream)))
+        return out
 
     def fused_info(self) -> Dict[str, int]:
         """Geometry of the fused step kernel chosen for this handle (``drsim_fused_info``)."""

@@ -219,10 +219,19 @@ static int fill_params(const drsim_config &c, SimParams &p, std::string &why) {
     why = "obs_dtype = DRSIM_OBS_BF16 needs an observation layout (obs_layout = none writes no rows)";
     return -1;
   }
+  if (c.comm_mode != DRSIM_COMM_RING && c.comm_mode != DRSIM_COMM_TABLE && c.comm_mode != DRSIM_COMM_SAMPLE) {
+    why = "comm_mode";
+    return -1;
+  }
   if (p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0 && p.N != p.n_global &&
       (p.comm_mode != DRSIM_COMM_RING || p.N < p.nb_comm)) {
-    why = "house-sharded cluster with neighbour messages: only the ring (`neighbours`) mode is exchanged as a halo, and every "
-          "shard must hold at least nb_comm houses";
+    why = "house-sharded cluster with neighbour messages: only the ring (`neighbours`) mode is exchanged as a halo (table "
+          "modes and `random_sample` are replicas only), and every shard must hold at least nb_comm houses";
+    return -1;
+  }
+  if (p.comm_mode == DRSIM_COMM_SAMPLE && (p.nb_comm > DRSIM_MAX_SAMPLE_COMM || p.nb_comm > p.n_global - 1)) {
+    why = "comm_mode = DRSIM_COMM_SAMPLE (`random_sample`) needs nb_comm <= min(n_house - 1, DRSIM_MAX_SAMPLE_COMM = " +
+          std::to_string(DRSIM_MAX_SAMPLE_COMM) + "), got " + std::to_string(p.nb_comm);
     return -1;
   }
   if (p.base_mode == DRSIM_BASE_INTERPOLATION && (p.interp_k < 1 || p.interp_period < 1)) { why = "interp props"; return -1; }
@@ -236,6 +245,12 @@ static int fill_params(const drsim_config &c, SimParams &p, std::string &why) {
   p.hf.neg_inv_opl = (float)(-1.0 / (1.0 + p.latent)); p.hf.rew_scale = (float)(p.alpha_temp / p.norm_temp);
   if (c.lockout_duration < 1) { why = "lockout_duration must be >= 1 s"; return -1; }
   return 0;
+}
+
+// the rows carry `random_sample` neighbours: the step kernels are launched in their sampled instantiation (a compile-time
+// flag, so the table / ring instantiations are the code they were); planning and routing ignore it
+static bool sample_rows(const SimParams &p) {
+  return p.comm_mode == DRSIM_COMM_SAMPLE && p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0;
 }
 
 static void plan_fused(drsim_handle *h, int e_cap = 1 << 30) {
@@ -322,38 +337,40 @@ static void plan_fused(drsim_handle *h, int e_cap = 1 << 30) {
 template <typename real>
 static int plan_shard(drsim_handle *h);
 
-// O = observation-row element type (real, or __nv_bfloat16 on an fp32 handle with DRSIM_OBS_BF16)
-template <typename real, typename O>
+// O = observation-row element type (real, or __nv_bfloat16 on an fp32 handle with DRSIM_OBS_BF16); S = the rows carry
+// sampled neighbours (sample_rows)
+template <typename real, typename O, bool S>
 static int configure_fused(drsim_handle *h, bool direct, int &per_sm) {
   using Of = std::conditional_t<sizeof(O) == 8, float, O>;   // row type of the fp32-only kernels (never run on fp64)
   const bool f = h->fused_ok;
   if (f && h->geom.use_rows) {
     if (sizeof(real) == 4) {
-      auto kern = h->geom.in_stride ? k_fused_rows<true, false, Of> : k_fused_rows<false, false, Of>;
+      auto kern = h->geom.in_stride ? k_fused_rows<true, false, Of, S> : k_fused_rows<false, false, Of, S>;
       CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
       if (h->geom.in_stride)
-        CU_TRY(cudaFuncSetAttribute(k_fused_rows<true, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+        CU_TRY(cudaFuncSetAttribute(k_fused_rows<true, true, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
       CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, h->geom.smem_bytes));
     }
-    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   } else if (f && direct && h->geom.use_tma) {
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    // (MODE 1 writes no messages: it is never launched with S)
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, false, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
     CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, false, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, true, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
     CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_tma<0, false, Of>, kThreads, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, true, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_tma<0, false, Of, S>, kThreads, h->geom.smem_bytes));
   } else if (f && direct) {
-    CU_TRY(cudaFuncSetAttribute(k_fused_direct<real, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_direct<real, O>, kThreads, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused_direct<real, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_direct<real, O, S>, kThreads, h->geom.smem_bytes));
   } else if (f) {
-    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused<real, false, O>, kThreads, h->geom.smem_bytes));
+    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused<real, false, O, S>, kThreads, h->geom.smem_bytes));
   }
   const size_t obs_smem = (size_t)kObsChunk * h->p.obs_dim * sizeof(O);
   if (obs_smem > 48 * 1024)
-    CU_TRY(cudaFuncSetAttribute(k_obs<real, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem));
+    CU_TRY(cudaFuncSetAttribute(k_obs<real, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem));
   return 0;
 }
 
@@ -362,10 +379,12 @@ static int configure_kernels(drsim_handle *h) {
   const bool direct = h->geom.chunk_rows == h->geom.envs_per_tile * h->p.Ns || h->p.obs_dim == 0;
   int per_sm = 0;
   int rc;
+  const bool smp = sample_rows(h->p);
   if constexpr (sizeof(real) == 4) {
-    rc = h->obs_bytes == 2 ? configure_fused<float, __nv_bfloat16>(h, direct, per_sm) : configure_fused<float, float>(h, direct, per_sm);
+    if (smp) rc = h->obs_bytes == 2 ? configure_fused<float, __nv_bfloat16, true>(h, direct, per_sm) : configure_fused<float, float, true>(h, direct, per_sm);
+    else rc = h->obs_bytes == 2 ? configure_fused<float, __nv_bfloat16, false>(h, direct, per_sm) : configure_fused<float, float, false>(h, direct, per_sm);
   } else {
-    rc = configure_fused<real, real>(h, direct, per_sm);
+    rc = smp ? configure_fused<real, real, true>(h, direct, per_sm) : configure_fused<real, real, false>(h, direct, per_sm);
   }
   if (rc) return rc;
   if (h->fused_ok) {
@@ -953,9 +972,10 @@ static int launch_env_phase(drsim_handle *h, const StepIn &in, const double *acc
   PeerCtx pc = make_peer(h);
   if (acc || n_parts >= 0) pc.world = 1;  // explicit partials (or the handle's own): no peer wait
   launch_pdl(k_env<real>, (p.R + 127) / 128, 128, 0, s, pl, p, in, (const double *)(acc ? acc : pl.acc), acc ? n_parts : 1, pc);
-  auto kobs = k_obs<real, real>;
+  const bool smp = sample_rows(p);
+  auto kobs = smp ? k_obs<real, real, true> : k_obs<real, real>;
   if constexpr (sizeof(real) == 4) {
-    if (h->obs_bytes == 2) kobs = k_obs<float, __nv_bfloat16>;
+    if (h->obs_bytes == 2) kobs = smp ? k_obs<float, __nv_bfloat16, true> : k_obs<float, __nv_bfloat16>;
   }
   launch_pdl(kobs, p.R * h->obs_chunks, kObsChunk, (size_t)kObsChunk * p.obs_dim * h->obs_bytes, s, pl, p, in, h->obs_chunks);
   h->launches += 2;
@@ -1004,15 +1024,18 @@ static int plan_shard(drsim_handle *h) {
     bool done = false;
     if constexpr (sizeof(real) == 4) {
       const bool bf = h->obs_bytes == 2;
+      const bool smp = sample_rows(p);
       auto kern = plain ? (bf ? k_shard<float, true, __nv_bfloat16> : k_shard<float, true>)
-                        : (bf ? k_shard<float, false, __nv_bfloat16> : k_shard<float, false>);
+                        : smp ? (bf ? k_shard<float, false, __nv_bfloat16, true> : k_shard<float, false, float, true>)
+                              : (bf ? k_shard<float, false, __nv_bfloat16> : k_shard<float, false>);
       CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
       CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
       done = true;
     }
     if (!done) {
-      CU_TRY(cudaFuncSetAttribute(k_shard<real, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shard<real, false>, kThreads, g.smem_bytes));
+      auto kern = sample_rows(p) ? k_shard<real, false, real, true> : k_shard<real, false>;
+      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
     }
     if (per_sm >= min_ctas || g.t_smem == 0) break;
   }
@@ -1061,11 +1084,12 @@ static int launch_shard(drsim_handle *h, StepIn in, cudaStream_t s) {
   sc.dbg = h->shard_dbg;
   PeerCtx pc = make_peer(h);
   if (!needs_halo(p)) pc.rowll = reinterpret_cast<unsigned long long *const *>(h->slab + h->o_peer_tab + 64 * 8);
-  auto kern = k_shard<real, false>;
+  const bool smp = sample_rows(p);
+  auto kern = smp ? k_shard<real, false, real, true> : k_shard<real, false>;
   if constexpr (sizeof(real) == 4) {
     const bool bf = h->obs_bytes == 2;
     if (shard_plain(h)) kern = bf ? k_shard<float, true, __nv_bfloat16> : k_shard<float, true>;
-    else if (bf) kern = k_shard<float, false, __nv_bfloat16>;
+    else if (bf) kern = smp ? k_shard<float, false, __nv_bfloat16, true> : k_shard<float, false, __nv_bfloat16>;
   }
   launch_pdl(kern, h->shard_grid, kThreads, (size_t)h->shard.smem_bytes, s, pl, p, in, h->shard, sc, pc);
   h->launches++;
@@ -1080,8 +1104,9 @@ static int exchange_error(const drsim_handle *h) {
   return 0;
 }
 
-// picks the compile-time specialisation of the production kernel (see k_fused_tma); O = row element type
-template <typename O>
+// picks the compile-time specialisation of the production kernel (see k_fused_tma); O = row element type, S = sampled
+// neighbours (MODE 1 writes no messages)
+template <typename O, bool S>
 static void launch_tma(drsim_handle *h, const StepIn &in, cudaStream_t s) {
   const Planes<float> pl = make_planes<float>(h);
   const SimParams &p = h->p;
@@ -1095,22 +1120,22 @@ static void launch_tma(drsim_handle *h, const StepIn &in, cudaStream_t s) {
     if (poll) launch_pdl(k_fused_tma<1, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
     else launch_pdl(k_fused_tma<1, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
   } else if (common && g.need_msg && g.envs_per_tile > 1) {
-    if (poll) launch_pdl(k_fused_tma<2, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<2, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    if (poll) launch_pdl(k_fused_tma<2, true, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    else launch_pdl(k_fused_tma<2, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
   } else {
-    if (poll) launch_pdl(k_fused_tma<0, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<0, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    if (poll) launch_pdl(k_fused_tma<0, true, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+    else launch_pdl(k_fused_tma<0, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
   }
 }
 
-template <typename O>
+template <typename O, bool S>
 static void launch_rows(drsim_handle *h, const StepIn &in, cudaStream_t s) {
   const Planes<float> pl = make_planes<float>(h);
   const int grid = h->launch_grid ? h->launch_grid : h->fused_grid;
   if (h->geom.in_stride && in.act_poll_err)
-    launch_pdl(k_fused_rows<true, true, O>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-  else if (h->geom.in_stride) launch_pdl(k_fused_rows<true, false, O>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-  else launch_pdl(k_fused_rows<false, false, O>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
+    launch_pdl(k_fused_rows<true, true, O, S>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
+  else if (h->geom.in_stride) launch_pdl(k_fused_rows<true, false, O, S>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
+  else launch_pdl(k_fused_rows<false, false, O, S>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
 }
 
 // steps the wide-row kernel cannot take (injected noise, on-device policies, common penalty modes)
@@ -1145,16 +1170,21 @@ static bool small64_handle(const drsim_handle *h) {
   return !getenv("DRSIM_NO_SMALL") && h->real_bytes == 8 && h->fused_ok && p.Ns <= 32 && p.N == p.n_global && p.R <= 256;
 }
 
-// one launch of the tile kernel chosen for this handle, rows of element type O
-template <typename real, typename O>
-static void launch_tile(drsim_handle *h, const StepIn &in, bool rows_ok, cudaStream_t s) {
+// one launch of the tile kernel chosen for this handle, rows of element type O, sampled neighbours S
+template <typename real, typename O, bool S>
+static void launch_tile_as(drsim_handle *h, const StepIn &in, bool rows_ok, cudaStream_t s) {
   const Planes<real> pl = make_planes<real>(h);
   if constexpr (sizeof(real) == 4) {
-    if (rows_ok) { launch_rows<O>(h, in, s); return; }
-    if (h->fused_direct && h->geom.use_tma) { launch_tma<O>(h, in, s); return; }
+    if (rows_ok) { launch_rows<O, S>(h, in, s); return; }
+    if (h->fused_direct && h->geom.use_tma) { launch_tma<O, S>(h, in, s); return; }
   }
-  if (h->fused_direct) k_fused_direct<real, O><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
-  else k_fused<real, false, O><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
+  if (h->fused_direct) k_fused_direct<real, O, S><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
+  else k_fused<real, false, O, S><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
+}
+template <typename real, typename O>
+static void launch_tile(drsim_handle *h, const StepIn &in, bool rows_ok, cudaStream_t s) {
+  if (sample_rows(h->p)) launch_tile_as<real, O, true>(h, in, rows_ok, s);
+  else launch_tile_as<real, O, false>(h, in, rows_ok, s);
 }
 
 template <typename real>
@@ -1175,7 +1205,8 @@ static int launch_fused(drsim_handle *h, const StepIn &in, cudaStream_t s) {
         if (int rc = snap_targets(h, so, &so_obs)) return rc;
         h->snap_fused = true;
       }
-      launch_pdl(k_small_gen<double>, (p.R + kSmallWarps - 1) / kSmallWarps, kSmallWarps * 32, 0, s, pl, p, in, so,
+      launch_pdl(sample_rows(p) ? k_small_gen<double, true> : k_small_gen<double>, (p.R + kSmallWarps - 1) / kSmallWarps,
+                 kSmallWarps * 32, 0, s, pl, p, in, so,
                  reinterpret_cast<double *>(so_obs));
       h->launches++;
       CU_TRY(cudaGetLastError());
@@ -1190,8 +1221,9 @@ static int launch_fused(drsim_handle *h, const StepIn &in, cudaStream_t s) {
         launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
         h->launches++;
       }
-      launch_pdl(h->obs_bytes == 2 ? k_small<__nv_bfloat16> : k_small<float>, (p.R + kSmallWarps - 1) / kSmallWarps,
-                 kSmallWarps * 32, 0, s, pl, p, in);
+      auto kern = h->obs_bytes == 2 ? k_small<__nv_bfloat16> : k_small<float>;
+      if (sample_rows(p)) kern = h->obs_bytes == 2 ? k_small<__nv_bfloat16, true> : k_small<float, true>;
+      launch_pdl(kern, (p.R + kSmallWarps - 1) / kSmallWarps, kSmallWarps * 32, 0, s, pl, p, in);
       h->launches++;
       CU_TRY(cudaGetLastError());
       return 0;
@@ -2100,6 +2132,27 @@ extern "C" void drsim_host_civil(int64_t epoch, int32_t out7[7]) {
 extern "C" void drsim_host_thermal_coefs(double Ua, double Ca, double Cm, double Hm, int32_t dt, double out12[12]) {
   thermal_coefs(Ua, Ca, Cm, Hm, dt, out12);
 }
+extern "C" int drsim_comm_sample(drsim_t *h, int64_t draw, int32_t *d_out, void *stream) {
+  if (!h || !d_out) return fail(DRSIM_E_ARG, "null argument");
+  const SimParams &p = h->p;
+  if (p.comm_mode != DRSIM_COMM_SAMPLE || p.nb_comm < 1)
+    return fail(DRSIM_E_STATE, "drsim_comm_sample: the handle was not created with comm_mode = DRSIM_COMM_SAMPLE and nb_comm > 0");
+  CU_TRY(cudaSetDevice(h->device));
+  const int64_t n = (int64_t)p.R * p.N;
+  k_comm_sample<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(p, (uint32_t)(draw < 0 ? h->step : draw), d_out);
+  CU_TRY(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int64_t drsim_step_count(const drsim_t *h) { return h ? h->step : -1; }
+
+extern "C" void drsim_host_comm_sample(uint64_t seed, int64_t rep, int64_t house, int64_t draw, int64_t n_global, int c,
+                                       int32_t *out) {
+  if (!out || c < 1 || c > DRSIM_MAX_SAMPLE_COMM || c > n_global - 1 || house < 0 || house >= n_global) return;
+  CommSampler smp(seed, (uint32_t)rep, (uint32_t)house, (uint32_t)draw, (uint32_t)n_global);
+  for (int k = 0; k < c; ++k) out[k] = smp.next();
+}
+
 extern "C" void drsim_host_philox(uint64_t seed, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t out4[4]) {
   const U4 r = philox4x32_10(seed, c0, c1, c2, c3);
   out4[0] = r.x; out4[1] = r.y; out4[2] = r.z; out4[3] = r.w;

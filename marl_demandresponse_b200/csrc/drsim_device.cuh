@@ -133,6 +133,47 @@ DRSIM_HD U4 philox4x32_10(uint64_t key, uint32_t c0, uint32_t c1, uint32_t c2, u
 }
 
 enum : uint32_t { PURPOSE_OD = 1, PURPOSE_PERLIN = 2, PURPOSE_INTERP = 3, PURPOSE_RESET = 4, PURPOSE_RESET_ENV = 5 };
+// (6 = PURPOSE_POLICY, drsim_actor.cuh)
+constexpr uint32_t PURPOSE_NEIGHBOUR = 7;
+
+// `random_sample` neighbours (cluster.py:96-99: random.sample(ids without n, c) per agent per step): a uniformly
+// random ordered c-tuple of distinct houses other than `house`, as a sparse partial Fisher-Yates shuffle of the
+// M = n_global - 1 other ids.  Step j draws r_j = j + mulhi(u_j, M - j) (Lemire's map without rejection: each value
+// has probability within (M - j) / 2^32 <= M / 2^32 of uniform), swaps positions j and r_j of the virtual identity
+// array and outputs the value now at position j, mapped past the house itself (v + (v >= house)).  Only the swaps are
+// recorded: the value at a position p >= j is `held` of the last earlier step whose r_i was p, else p.  The words u_j
+// are philox4x32_10(seed, rep, house, draw, PURPOSE_NEIGHBOUR | (j / 4) << 8), four per block.  next() yields
+// outputs 0, 1, ... in turn; pick(k) advances to output k (both halves of a row split over two lanes).
+struct CommSampler {
+  uint64_t seed;
+  uint32_t rep, house, draw, M;
+  int j;
+  U4 blk;
+  int32_t pos[DRSIM_MAX_SAMPLE_COMM], held[DRSIM_MAX_SAMPLE_COMM];
+  DRSIM_HD CommSampler(uint64_t seed_, uint32_t rep_, uint32_t house_, uint32_t draw_, uint32_t n_global)
+      : seed(seed_), rep(rep_), house(house_), draw(draw_), M(n_global - 1u), j(0), blk{0, 0, 0, 0} {}
+  DRSIM_HD int next() {
+    const int w = j & 3;
+    if (w == 0) blk = philox4x32_10(seed, rep, house, draw, PURPOSE_NEIGHBOUR | ((uint32_t)(j >> 2) << 8));
+    const uint32_t u = w == 0 ? blk.x : w == 1 ? blk.y : w == 2 ? blk.z : blk.w;
+    uint32_t hi, lo;
+    mulhilo32(u, M - (uint32_t)j, hi, lo);
+    const int r = j + (int)hi;
+    int v = r, hj = j;
+    for (int i = 0; i < j; ++i) {   // ascending: the last swap that wrote a position wins
+      v = pos[i] == r ? held[i] : v;
+      hj = pos[i] == j ? held[i] : hj;
+    }
+    pos[j] = r;
+    held[j] = hj;
+    ++j;
+    return v + (v >= (int)house ? 1 : 0);
+  }
+  DRSIM_HD int pick(int k) {
+    while (j < k) next();
+    return next();
+  }
+};
 
 DRSIM_HD double u01_open_closed(uint32_t x) { return ((double)x + 1.0) * 2.3283064365386963e-10; }  // (0,1]
 

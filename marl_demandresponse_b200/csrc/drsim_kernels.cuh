@@ -911,6 +911,34 @@ DRSIM_D int neighbour_of(const SimParams &p, const int32_t *table, int r, int n,
   return __ldg(table + base + (size_t)n * p.nb_comm + k);
 }
 
+// Draw index of the rows a kernel writes (DRSIM_COMM_SAMPLE): the handle's step count as the rows see it -- in.step + 1
+// after step 0 of the launch, + k + 1 after step k of an in-kernel block, in.step for a refresh (advance = 0)
+DRSIM_D uint32_t rows_draw(const StepIn &in, int k = 0) { return (uint32_t)(in.step + (in.advance ? k + 1 : 0)); }
+
+// Neighbours of one row.  SMP = false: neighbour_of, unchanged.  SMP = true (DRSIM_COMM_SAMPLE): the row's draw,
+// computed once as the row's message loop asks for k = 0, 1, ... (a later k runs the draw up to it).
+template <bool SMP>
+struct RowNbrs {
+  DRSIM_D RowNbrs(const SimParams &, int, int, uint32_t) {}
+  DRSIM_D int operator()(const SimParams &p, const int32_t *table, int r, int n, int k) { return neighbour_of(p, table, r, n, k); }
+};
+template <>
+struct RowNbrs<true> {
+  CommSampler s;
+  DRSIM_D RowNbrs(const SimParams &p, int r, int n, uint32_t draw)
+      : s(p.seed, (uint32_t)(p.rep_offset + r), (uint32_t)(p.house_offset + n), draw, (uint32_t)p.n_global) {}
+  DRSIM_D int operator()(const SimParams &, const int32_t *, int, int, int k) { return s.pick(k); }
+};
+
+// neighbour table of one draw, [R][N][nb_comm] (drsim_comm_sample)
+__global__ void k_comm_sample(SimParams p, uint32_t draw, int32_t *out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (int64_t)p.R * p.N) return;
+  const int r = (int)(i / p.N), n = (int)(i - (int64_t)r * p.N);
+  RowNbrs<true> nb(p, r, n, draw);
+  for (int k = 0; k < p.nb_comm; ++k) out[i * p.nb_comm + k] = nb(p, nullptr, r, n, k);
+}
+
 // int(seconds_since_off / lockout_duration) of the house's OWN hvac (norm.py:79-82); messages use the default
 // duration (norm.py:40-43) and keep fast_div
 template <typename real>
@@ -1387,7 +1415,7 @@ __global__ void k_env(Planes<real> pl, SimParams p, StepIn in, const double *acc
 // General path, kernel 4: rewards + observation rows for a chunk of kObsChunk houses.
 // Neighbour messages are gathered from global memory (any table); rows are assembled in shared
 // memory and written back with coalesced 128-bit stores (2-byte stores where bf16 rows leave a chunk unaligned).
-template <typename real, typename O = real>
+template <typename real, typename O = real, bool SMP = false>
 __global__ void __launch_bounds__(kObsChunk) k_obs(Planes<real> pl, SimParams p, StepIn in, int chunks) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   O *tile = reinterpret_cast<O *>(smem_raw);
@@ -1421,8 +1449,9 @@ __global__ void __launch_bounds__(kObsChunk) k_obs(Planes<real> pl, SimParams p,
                               Rep<real>::minus20(tm, tgt), tgt - (real)20, e, ratio);
         if (p.obs_layout == DRSIM_OBS_HAND_ENGINEERED) {
           const bool halo = needs_halo(p);
+          RowNbrs<SMP> nbr(p, r, n, rows_draw(in));
           for (int k = 0; k < p.nb_comm; ++k) {
-            int nb = neighbour_of(p, pl.comm_table, r, n + (halo ? (int)p.house_offset : 0), k);
+            int nb = nbr(p, pl.comm_table, r, n + (halo ? (int)p.house_offset : 0), k);
             if (halo) {
               // ring neighbour by GLOBAL index; outside this shard it comes from the exchanged halo
               nb -= (int)p.house_offset;
@@ -1538,7 +1567,7 @@ template <> struct FusedOcc<float> { static constexpr int min_ctas = DRSIM_FUSED
 // DIRECT: the whole tile's observation rows fit the staging buffer; each thread writes the rows of
 // its own 4 houses straight from registers and one TMA bulk store per tile ships them.
 // ------------------------------------------------------------------------------------------
-template <typename real, bool DIRECT, typename O = real>
+template <typename real, bool DIRECT, typename O = real, bool SMP = false>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1650,8 +1679,9 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
                                   Rep<real>::minus20(h.ta[j], h.target[j]), Rep<real>::minus20(h.tm[j], h.target[j]),
                                   h.target[j] - (real)20, e, ratio);
             if (g.need_msg) {
+              RowNbrs<SMP> nbr(p, r0 + e_loc, n0 + j, rows_draw(in));
               for (int k = 0; k < p.nb_comm; ++k) {
-                const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
+                const int nb = nbr(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                 const Msg4<real> mk = s_msg[e_loc * Ns + nb];
                 row[q++] = mk.dT; row[q++] = mk.sso_n; row[q++] = mk.p_n; row[q++] = mk.pmax_n;
                 if (p.msg_thermal)
@@ -1693,8 +1723,9 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
               int q = obs_own<real>(row, p, (uint32_t)o.flags, m.sso_n, Rep<real>::minus20(o.ta, o.target),
                                     Rep<real>::minus20(o.tm, o.target), o.target - (real)20, s_env[e], ratio);
               if (g.need_msg) {
+                RowNbrs<SMP> nbr(p, r0 + e, n, rows_draw(in));
                 for (int k = 0; k < p.nb_comm; ++k) {
-                  const int nb = neighbour_of(p, pl.comm_table, r0 + e, n, k);
+                  const int nb = nbr(p, pl.comm_table, r0 + e, n, k);
                   const Msg4<real> mk = s_msg[e * Ns + nb];
                   row[q++] = mk.dT; row[q++] = mk.sso_n; row[q++] = mk.p_n; row[q++] = mk.pmax_n;
                   if (p.msg_thermal)
@@ -1737,7 +1768,7 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
 // barrier; the two env-dependent columns, the neighbour messages and the rewards after the second.
 // Each warp ships its own 128 rows with one TMA bulk store (no CTA barrier in front of it).
 // ------------------------------------------------------------------------------------------
-template <typename real, typename O = real>
+template <typename real, typename O = real, bool SMP = false>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1881,8 +1912,9 @@ k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
               if constexpr (sizeof(real) == 4) {
                 put2(row, 2, e.power_n, e.signal_n);
                 if (g.need_msg) {
+                  RowNbrs<SMP> nbr(p, r0 + e_loc, n0 + j, rows_draw(in));
                   for (int k = 0; k < p.nb_comm; ++k) {
-                    const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
+                    const int nb = nbr(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                     const float4 mk = *reinterpret_cast<const float4 *>(&s_msg[e_loc * Ns + nb]);
                     put2(row, 5 + 2 * k, mk.x, mk.y);
                     put2(row, 6 + 2 * k, mk.z, mk.w);
@@ -1893,8 +1925,9 @@ k_fused_direct(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
             }
             int q = obs_own<real>(row, p, 0u, (real)0, (real)0, (real)0, (real)0, e, nullptr, 2);
             if (g.need_msg) {
+              RowNbrs<SMP> nbr(p, r0 + e_loc, n0 + j, rows_draw(in));
               for (int k = 0; k < p.nb_comm; ++k) {
-                const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
+                const int nb = nbr(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                 const Msg4<real> mk = s_msg[e_loc * Ns + nb];
                 row[q++] = mk.dT; row[q++] = mk.sso_n; row[q++] = mk.p_n; row[q++] = mk.pmax_n;
                 if (p.msg_thermal)
@@ -2107,7 +2140,7 @@ DRSIM_D uint32_t act_word_polled(const uint8_t *actions, size_t off, uint32_t st
 
 // POLL = copy-engine mode of drsim_step_host (StepIn::act_poll_err): a separate instantiation, so the
 // device-resident step does not carry the branch (measured: 0.6 us of 39 on C4)
-template <int MODE, bool POLL = false, typename O = float>
+template <int MODE, bool POLL = false, typename O = float, bool SMP = false>
 __global__ void __launch_bounds__(kThreads, DRSIM_FUSED_MINCTAS)
 k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   typedef float real;
@@ -2438,8 +2471,9 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
             if (plain) {
               put2(row, 2, e.power_n, e.signal_n);
               if (need_msg) {
+                RowNbrs<SMP> nbr(p, r0 + e_loc, n0 + j, rows_draw(in, st));
                 for (int k = 0; k < p.nb_comm; ++k) {
-                  const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
+                  const int nb = nbr(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                   const float4 mk = *reinterpret_cast<const float4 *>(&s_msg[e_loc * Ns + nb]);
                   put2(row, 5 + 2 * k, mk.x, mk.y);
                   put2(row, 6 + 2 * k, mk.z, mk.w);
@@ -2449,8 +2483,9 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
             }
             int q = obs_own<real>(row, p, 0u, 0.f, 0.f, 0.f, 0.f, e, nullptr, 2);
             if (need_msg) {
+              RowNbrs<SMP> nbr(p, r0 + e_loc, n0 + j, rows_draw(in, st));
               for (int k = 0; k < p.nb_comm; ++k) {
-                const int nb = neighbour_of(p, pl.comm_table, r0 + e_loc, n0 + j, k);
+                const int nb = nbr(p, pl.comm_table, r0 + e_loc, n0 + j, k);
                 const Msg4<real> mk = s_msg[e_loc * Ns + nb];
                 row[q++] = mk.dT; row[q++] = mk.sso_n; row[q++] = mk.p_n; row[q++] = mk.pmax_n;
                 if (p.msg_thermal)
@@ -2515,7 +2550,7 @@ constexpr int kRowGroup = 16;  // rows per warp-level TMA store in k_fused_rows 
 
 // STAGED = inputs prefetched one tile ahead into thread-private shared-memory slots (needs 44 B of
 // shared memory per house slot); false = 128-bit register loads at the top of the tile (large clusters)
-template <bool STAGED, bool POLL = false, typename O = float>
+template <bool STAGED, bool POLL = false, typename O = float, bool SMP = false>
 __global__ void __launch_bounds__(kThreads, 2)
 k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   typedef float real;
@@ -2743,8 +2778,9 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
               put2(orow, 6 + 2 * q, mk.z, mk.w);
             }
           } else {
+            RowNbrs<SMP> nbr(p, r0 + e, n, rows_draw(in, st));   // (the second half runs the draw through the first)
             for (int q = k0; q < k1; ++q) {
-              const float4 mk = mb[neighbour_of(p, pl.comm_table, r0 + e, n, q)];
+              const float4 mk = mb[nbr(p, pl.comm_table, r0 + e, n, q)];
               put2(orow, 5 + 2 * q, mk.x, mk.y);
               put2(orow, 6 + 2 * q, mk.z, mk.w);
             }
@@ -2779,7 +2815,7 @@ k_fused_rows(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
 // ------------------------------------------------------------------------------------------
 constexpr int kSmallWarps = 4;   // clusters per CTA
 
-template <typename O = float>
+template <typename O = float, bool SMP = false>
 __global__ void __launch_bounds__(kSmallWarps * 32) k_small(Planes<float> pl, SimParams p, StepIn in) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int r = (int)blockIdx.x * kSmallWarps + warp;
@@ -2884,8 +2920,9 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small(Planes<float> pl, Si
         put2(row, 4, ok ? (tm + tg20) * 0.2f : 0.f, ok ? tg20 * 0.2f : 0.f);
       }
       if (need_msg) {
+        RowNbrs<SMP> nbr(p, r, lane, rows_draw(in, k));
         for (int q = 0; q < nbc; ++q) {      // (every lane takes part in the shuffles)
-          const int nb = ok ? neighbour_of(p, pl.comm_table, r, lane, q) : 0;
+          const int nb = ok ? nbr(p, pl.comm_table, r, lane, q) : 0;
           const float v0 = __shfl_sync(0xffffffffu, m0, nb), v1 = __shfl_sync(0xffffffffu, m1, nb),
                       v2 = __shfl_sync(0xffffffffu, m2, nb), v3 = __shfl_sync(0xffffffffu, m3, nb);
           if (slot) {
@@ -2925,7 +2962,7 @@ constexpr int kSnapEnv = 8;   // od_temp, signal, power, solar, base_power, epoc
 // tile kernel (three active threads, a serial fp64 epilogue between two CTA barriers).
 // `snap` / `snap_obs` (optional, mapped pinned host memory): the host snapshot of drsim_step_host_snapshot is written
 // by the same lanes -- no second kernel and no D2H copy behind the step, one synchronisation for the whole call.
-template <typename real>
+template <typename real, bool SMP = false>
 __global__ void __launch_bounds__(kSmallWarps * 32) k_small_gen(Planes<real> pl, SimParams p, StepIn in, SnapPtrs snap, real *snap_obs) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int r = (int)blockIdx.x * kSmallWarps + warp;
@@ -3008,8 +3045,9 @@ __global__ void __launch_bounds__(kSmallWarps * 32) k_small_gen(Planes<real> pl,
       for (int k = 0; k < D; ++k) row[k] = (real)0;
     }
     if (need_msg) {
+      RowNbrs<SMP> nbr(p, r, lane, rows_draw(in));
       for (int k = 0; k < nbc; ++k) {      // (every lane takes part in the shuffles)
-        const int nb = ok ? neighbour_of(p, pl.comm_table, r, lane, k) : 0;
+        const int nb = ok ? nbr(p, pl.comm_table, r, lane, k) : 0;
         const real v0 = __shfl_sync(0xffffffffu, m0, nb), v1 = __shfl_sync(0xffffffffu, m1, nb),
                    v2 = __shfl_sync(0xffffffffu, m2, nb), v3 = __shfl_sync(0xffffffffu, m3, nb);
         if (ok) {

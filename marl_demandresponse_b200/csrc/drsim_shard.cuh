@@ -181,7 +181,7 @@ DRSIM_D void ld4i_cg(const int32_t *p, int v[4]) {
 }
 
 // PLAIN = fp32 build, 10-column rows without neighbour messages (TarMAC layout / nb_comm = 0)
-template <typename real, bool PLAIN, typename O = real>
+template <typename real, bool PLAIN, typename O = real, bool SMP = false>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerCtx peer) {
   static_assert(!PLAIN || sizeof(real) == 4, "the plain variant is fp32 only");
@@ -659,8 +659,9 @@ k_shard(Planes<real> pl, SimParams p, StepIn in, ShardGeom g, ShardCtx sc, PeerC
             int i = obs_own<real>(row, p, f, own_sso_norm<real>(pl, p, o, sso), Rep<real>::minus20(ta, tgt),
                                   Rep<real>::minus20(tm, tgt), tgt - (real)20, e, ratio);
             if (p.obs_layout == DRSIM_OBS_HAND_ENGINEERED) {
+              RowNbrs<SMP> nbr(p, r, n, rows_draw(in));
               for (int k = 0; k < p.nb_comm; ++k) {
-                int nb = neighbour_of(p, pl.comm_table, r, n + (halo ? (int)p.house_offset : 0), k);
+                int nb = nbr(p, pl.comm_table, r, n + (halo ? (int)p.house_offset : 0), k);
                 if (halo) {
                   // ring neighbour by GLOBAL index; outside this shard it comes from the exchanged halo
                   nb -= (int)p.house_offset;

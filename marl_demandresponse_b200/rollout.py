@@ -26,6 +26,7 @@ class RolloutBuffer:
         import torch
 
         sim = env.sim
+        self._env = env
         if sim.real is not __import__("numpy").float32 or not sim.D:
             raise ValueError("the on-device rollout needs the fp32 build with an observation layout")
         self.sim, self.T = sim, int(horizon)
@@ -38,6 +39,7 @@ class RolloutBuffer:
         self.rewards = torch.zeros((self.T, R, Ns), dtype=torch.float32, device=dev)
         self.done = torch.zeros((self.T,), dtype=torch.bool, device=dev)
         self.filled = 0
+        self.draw0 = 0   # step count of the handle when obs[0] was written (`random_sample` draw index of obs[0])
 
     # ---- Transition fields (mappo.py:23-35), [R, N, ...] views of step t ---------------------
     def state(self, t: int):
@@ -54,6 +56,13 @@ class RolloutBuffer:
 
     def reward(self, t: int):
         return self.rewards[t, :, :self.N]
+
+    def neighbour_index(self, t: int):
+        """``random_sample`` handle: the ``[R, N, c]`` neighbour table behind ``obs[t]`` (its draw is
+        ``draw0 + t``); other modes: the handle's static table."""
+        if self._env.comm_mode == "random_sample":
+            return self.sim.comm_sample(self.draw0 + int(t))
+        return self._env.neighbour_index()
 
     def others_actions(self, t: int):
         """``[R, N, N - 1]``: for every agent the actions of all OTHER agents of its cluster in id order
@@ -91,6 +100,7 @@ def collect(env, weights, buf: RolloutBuffer, n_steps: Optional[int] = None, see
         raise ValueError("n_steps exceeds the buffer's horizon")
     net = sim.actor_net(weights, precision)
     buf.obs[0].copy_(sim.views()["obs_padded"])     # state_0 = the rows of the last step / reset (one copy per segment)
+    buf.draw0 = sim.step_count
     seed = env.seed if seed is None else int(seed)
     st = sim._stream(stream)
     slot = _lib.RolloutSlot()

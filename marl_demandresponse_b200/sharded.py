@@ -70,8 +70,13 @@ class ShardedClusterEnv:
         self.lo, self.hi = house_shard(self.n_global, rank, world)
         if self.hi <= self.lo:
             raise ValueError("more ranks than 4-house blocks")
+        mode = self.props.cluster_prop.agents_comm_prop.mode
+        if mode == "random_sample" and obs_layout == "hand_engineered":
+            raise ValueError("`random_sample` neighbour messages are drawn from the whole cluster every step: they are "
+                             "available on replicas (BatchedEnv), not on a cluster split across GPUs")
         cfg = flatten_config(self.props, n_replicas, precision, obs_layout, policy, noise, seed, "split",
-                             house_offset=self.lo, n_house_local=self.hi - self.lo, obs_dtype=obs_dtype)
+                             comm_table=mode != "neighbours", house_offset=self.lo, n_house_local=self.hi - self.lo,
+                             obs_dtype=obs_dtype)
         self.sim = DrSim(cfg, device)
         self.device = device
         self._v = self.sim.views()
