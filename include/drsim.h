@@ -429,6 +429,22 @@ int64_t drsim_launch_count(const drsim_t *h);
  * caps the clusters per tile instead of the built-in round-count heuristic. */
 int drsim_fused_info(const drsim_t *h, int32_t out[6]);
 
+/* Route of the last step launched on this handle (diagnostics and tests), -1 before the first step (a refresh counts):
+ * which kernels ran it.  A handle's steps take different routes: refreshes, interpolator firings, injected noise,
+ * polled actions or per-HVAC lock-out durations move a step off the tile kernel that drsim_fused_info reports. */
+#define DRSIM_ROUTE_FOUR_KERNEL 0          /* k_house + k_reduce + k_env + k_obs */
+#define DRSIM_ROUTE_SHARD 1                /* k_shard */
+#define DRSIM_ROUTE_FUSED 2                /* k_fused (rows staged in CTA-wide chunks) */
+#define DRSIM_ROUTE_FUSED_DIRECT 3         /* k_fused_direct */
+#define DRSIM_ROUTE_FUSED_TMA0 4           /* k_fused_tma<0> */
+#define DRSIM_ROUTE_FUSED_TMA1 5           /* k_fused_tma<1> */
+#define DRSIM_ROUTE_FUSED_TMA2 6           /* k_fused_tma<2> */
+#define DRSIM_ROUTE_FUSED_ROWS_STAGED 7    /* k_fused_rows<staged> */
+#define DRSIM_ROUTE_FUSED_ROWS_UNSTAGED 8  /* k_fused_rows<unstaged> */
+#define DRSIM_ROUTE_SMALL 9                /* k_small */
+#define DRSIM_ROUTE_SMALL_GEN 10           /* k_small_gen<double> */
+int drsim_step_route(const drsim_t *h);
+
 /* Per-cluster summary behind the reference's UI feed (ClientManagerService.update_data,
  * server/app/services/client_manager_service.py:147-197; description values :64-118): one launch,
  * d_out = device [R][DRSIM_SUMMARY_FIELDS] fp64 =

@@ -178,6 +178,7 @@ def lib():
         "drsim_rollout_transition": (C.c_int, [hp, C.POINTER(ActorNet), _u64, C.POINTER(RolloutSlot), C.c_void_p]),
         "drsim_launch_count": (C.c_int64, [hp]),
         "drsim_fused_info": (C.c_int, [hp, C.POINTER(_i32 * 6)]),
+        "drsim_step_route": (C.c_int, [hp]),
         "drsim_cluster_summary": (C.c_int, [hp, C.c_void_p, C.c_void_p]),
         "drsim_metrics_update": (C.c_int, [hp, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
         "drsim_host_solar_gain": (C.c_double, [_i64, _d, _d]),
@@ -207,7 +208,7 @@ EXPORTED_SYMBOLS = [
     "drsim_create", "drsim_destroy", "drsim_clone", "drsim_buffers", "drsim_set_state", "drsim_get_state", "drsim_reset",
     "drsim_set_comm_table", "drsim_set_interp_table", "drsim_step", "drsim_run", "drsim_run_tape", "drsim_refresh", "drsim_step_begin",
     "drsim_step_finish", "drsim_step_sharded", "drsim_step_finish_gathered", "drsim_step_host", "drsim_step_host_full", "drsim_snapshot", "drsim_step_host_snapshot",
-    "drsim_ipc_export", "drsim_ipc_attach", "drsim_peer_status", "drsim_peer_attach_local", "drsim_policy_step", "drsim_rollout_transition", "drsim_launch_count", "drsim_fused_info", "drsim_cluster_summary", "drsim_metrics_update", "drsim_host_solar_gain", "drsim_host_od_temp",
+    "drsim_ipc_export", "drsim_ipc_attach", "drsim_peer_status", "drsim_peer_attach_local", "drsim_policy_step", "drsim_rollout_transition", "drsim_launch_count", "drsim_fused_info", "drsim_step_route", "drsim_cluster_summary", "drsim_metrics_update", "drsim_host_solar_gain", "drsim_host_od_temp",
     "drsim_host_civil", "drsim_host_thermal_coefs", "drsim_host_philox", "drsim_last_error", "drsim_abi_version",
     "drsim_sizeof", "drsim_comm_sample", "drsim_step_count", "drsim_host_comm_sample",
 ]

@@ -548,6 +548,14 @@ class DrSim:
         return {"variant": names[out[0]], "envs_per_tile": out[1], "tiles": out[2], "grid": out[3],
                 "smem_bytes": out[4], "ctas_per_sm": out[5]}
 
+    @property
+    def last_route(self) -> str:
+        """Kernels of the last step launched on this handle (``drsim_step_route``; "none" before the first)."""
+        names = ("four-kernel", "k_shard", "k_fused", "k_fused_direct", "k_fused_tma<0>", "k_fused_tma<1>", "k_fused_tma<2>",
+                 "k_fused_rows<staged>", "k_fused_rows<unstaged>", "k_small", "k_small_gen")
+        r = self._L.drsim_step_route(self._h)
+        return "none" if r < 0 else names[r]
+
     def cluster_summary(self, out=None, stream=None):
         """``drsim_cluster_summary``: fp64 CUDA tensor ``[R, 8]`` = locked HVACs, sum Ta, sum (Ta - target),
         sum |Ta - target|, sum Tm, sum target, running HVACs, N  (the UI feed's aggregates,

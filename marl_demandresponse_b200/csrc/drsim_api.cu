@@ -69,7 +69,8 @@ struct drsim_handle {
   size_t o_dur = 0;
   int chunks = 1;       // CTAs per cluster in the general path
   int obs_chunks = 1;   // k_obs CTAs per cluster
-  bool fused_ok = false, fused_direct = false;
+  bool fused_ok = false;   // plan_fused found a tile kernel for this shape (taken while fused_ready)
+  bool fused_direct = false;   // ... whose tile's rows fit the staging buffer at once (k_fused_direct, not k_fused)
   FusedGeom geom{};
   int fused_grid = 0;
   int64_t step = 0;
@@ -95,7 +96,6 @@ struct drsim_handle {
   unsigned char *h_snap = nullptr, *h_snap_dev = nullptr;
   size_t snap_bytes = 0, snap_obs_off = 0;
   bool snap_next = false, snap_fused = false;   // transient: the next small-cluster step writes the host snapshot itself
-  int launch_grid = 0;                       // transient: grid of the next fused launch (tape stream), 0 = fused_grid
   unsigned long long *actor_dbg = nullptr;   // DRSIM_ACTOR_DBG: phase stamps of CTA 0 of the last k_actor3x launch
   unsigned long long *shard_dbg = nullptr;   // DRSIM_SHARD_DBG: per-CTA time stamps of the last k_shard launch
   int *h_peer_err = nullptr, *h_peer_err_dev = nullptr;   // mapped: set by a kernel whose exchange wait timed out
@@ -114,6 +114,7 @@ struct drsim_handle {
   double *mirror_next = nullptr;   // the next fused step writes its per-cluster results [R][4] straight to this mapped host buffer
   unsigned char *actor_image = nullptr;   // packed weight operands of drsim_policy_step (k_actor_pack)
   bool broken = false;             // a step was committed with missing inputs: refuse to step until state is re-injected
+  int last_route = -1;             // StepRoute of the last step launched (drsim_step_route)
 
   template <typename T>
   T *at(size_t off) const {
@@ -247,10 +248,25 @@ static int fill_params(const drsim_config &c, SimParams &p, std::string &why) {
   return 0;
 }
 
-// the rows carry `random_sample` neighbours: the step kernels are launched in their sampled instantiation (a compile-time
-// flag, so the table / ring instantiations are the code they were); planning and routing ignore it
-static bool sample_rows(const SimParams &p) {
-  return p.comm_mode == DRSIM_COMM_SAMPLE && p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0;
+// Template arguments of a handle's step kernels: real = the build (fp32 / fp64); O = observation-row element (real, or
+// __nv_bfloat16 on an fp32 handle with DRSIM_OBS_BF16); S = the rows carry `random_sample` neighbours, drawn in the
+// kernel (a compile-time flag, so the table / ring instantiations are the code they were; planning and routing ignore it)
+template <typename Real, typename Obs, bool Sampled>
+struct KernelTypes {
+  using real = Real;
+  using O = Obs;
+  static constexpr bool S = Sampled;
+};
+
+// calls f(KernelTypes<...>{}) with the handle's template arguments: the one place they are derived from the handle
+template <typename F>
+static int with_kernel_types(const drsim_handle *h, F &&f) {
+  const SimParams &p = h->p;
+  const bool s = p.comm_mode == DRSIM_COMM_SAMPLE && p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0;
+  if (h->real_bytes == 8) return s ? f(KernelTypes<double, double, true>{}) : f(KernelTypes<double, double, false>{});
+  if (h->obs_bytes == 2)
+    return s ? f(KernelTypes<float, __nv_bfloat16, true>{}) : f(KernelTypes<float, __nv_bfloat16, false>{});
+  return s ? f(KernelTypes<float, float, true>{}) : f(KernelTypes<float, float, false>{});
 }
 
 static void plan_fused(drsim_handle *h, int e_cap = 1 << 30) {
@@ -331,73 +347,66 @@ static void plan_fused(drsim_handle *h, int e_cap = 1 << 30) {
     }
   }
   h->geom = g;
+  h->fused_direct = g.chunk_rows == g.envs_per_tile * p.Ns || p.obs_dim == 0;
   h->fused_ok = true;
 }
 
-template <typename real>
 static int plan_shard(drsim_handle *h);
 
-// O = observation-row element type (real, or __nv_bfloat16 on an fp32 handle with DRSIM_OBS_BF16); S = the rows carry
-// sampled neighbours (sample_rows)
-template <typename real, typename O, bool S>
-static int configure_fused(drsim_handle *h, bool direct, int &per_sm) {
-  using Of = std::conditional_t<sizeof(O) == 8, float, O>;   // row type of the fp32-only kernels (never run on fp64)
-  const bool f = h->fused_ok;
-  if (f && h->geom.use_rows) {
-    if (sizeof(real) == 4) {
-      auto kern = h->geom.in_stride ? k_fused_rows<true, false, Of, S> : k_fused_rows<false, false, Of, S>;
-      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      if (h->geom.in_stride)
-        CU_TRY(cudaFuncSetAttribute(k_fused_rows<true, true, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, h->geom.smem_bytes));
+// k_greedy sorts a cluster in shared memory: its width rounded up to a power of two, 24 bytes an entry
+static int greedy_n2(const SimParams &p) {
+  int n2 = 1;
+  while (n2 < p.N) n2 <<= 1;
+  return n2;
+}
+
+// shared-memory attributes of the tile kernel plan_fused chose (and its resident CTAs per SM), k_obs and k_greedy
+template <typename K>
+static int configure_step_kernels(drsim_handle *h, int &per_sm) {
+  using real = typename K::real;
+  using O = typename K::O;
+  constexpr bool S = K::S;
+  const FusedGeom &g = h->geom;
+  if constexpr (sizeof(real) == 4) {
+    if (h->fused_ok && g.use_rows) {
+      auto kern = g.in_stride ? k_fused_rows<true, false, O, S> : k_fused_rows<false, false, O, S>;
+      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      if (g.in_stride)
+        CU_TRY(cudaFuncSetAttribute(k_fused_rows<true, true, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
+    } else if (h->fused_ok && g.use_tma) {
+      // (MODE 1 writes no messages: it is never launched with S)
+      CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, false, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, false, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, false, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, true, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, true, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, true, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_tma<0, false, O, S>, kThreads, g.smem_bytes));
     }
-    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  } else if (f && direct && h->geom.use_tma) {
-    // (MODE 1 writes no messages: it is never launched with S)
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, false, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, false, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, false, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<0, true, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<1, true, Of>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaFuncSetAttribute(k_fused_tma<2, true, Of, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_tma<0, false, Of, S>, kThreads, h->geom.smem_bytes));
-  } else if (f && direct) {
-    CU_TRY(cudaFuncSetAttribute(k_fused_direct<real, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused_direct<real, O, S>, kThreads, h->geom.smem_bytes));
-  } else if (f) {
-    CU_TRY(cudaFuncSetAttribute(k_fused<real, false, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->geom.smem_bytes));
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_fused<real, false, O, S>, kThreads, h->geom.smem_bytes));
+  }
+  if (h->fused_ok && !g.use_rows && !g.use_tma) {
+    auto kern = h->fused_direct ? k_fused_direct<real, O, S> : k_fused<real, O, S>;
+    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
   }
   const size_t obs_smem = (size_t)kObsChunk * h->p.obs_dim * sizeof(O);
   if (obs_smem > 48 * 1024)
     CU_TRY(cudaFuncSetAttribute(k_obs<real, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem));
+  if (h->p.policy == DRSIM_POLICY_GREEDY_MYOPIC) {
+    const size_t sm = (size_t)greedy_n2(h->p) * 24;
+    if (sm > 200 * 1024) return fail(DRSIM_E_ARG, "greedy-myopic: cluster too large for the shared-memory sort");
+    if (sm > 48 * 1024) CU_TRY(cudaFuncSetAttribute(k_greedy<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+  }
   return 0;
 }
 
-template <typename real>
 static int configure_kernels(drsim_handle *h) {
-  const bool direct = h->geom.chunk_rows == h->geom.envs_per_tile * h->p.Ns || h->p.obs_dim == 0;
   int per_sm = 0;
-  int rc;
-  const bool smp = sample_rows(h->p);
-  if constexpr (sizeof(real) == 4) {
-    if (smp) rc = h->obs_bytes == 2 ? configure_fused<float, __nv_bfloat16, true>(h, direct, per_sm) : configure_fused<float, float, true>(h, direct, per_sm);
-    else rc = h->obs_bytes == 2 ? configure_fused<float, __nv_bfloat16, false>(h, direct, per_sm) : configure_fused<float, float, false>(h, direct, per_sm);
-  } else {
-    rc = smp ? configure_fused<real, real, true>(h, direct, per_sm) : configure_fused<real, real, false>(h, direct, per_sm);
-  }
-  if (rc) return rc;
+  if (int rc = with_kernel_types(h, [&](auto k) { return configure_step_kernels<decltype(k)>(h, per_sm); })) return rc;
   if (h->fused_ok) {
-    h->fused_direct = direct;
     if (per_sm < 1) { h->fused_ok = false; }
     else { h->fused_grid = std::min(h->geom.n_tiles, per_sm * h->sm_count); h->fused_per_sm = per_sm; }
-  }
-  if (h->p.policy == DRSIM_POLICY_GREEDY_MYOPIC) {
-    int n2 = 1;
-    while (n2 < h->p.N) n2 <<= 1;
-    const size_t sm = (size_t)n2 * 24;
-    if (sm > 200 * 1024) return fail(DRSIM_E_ARG, "greedy-myopic: cluster too large for the shared-memory sort");
-    if (sm > 48 * 1024) CU_TRY(cudaFuncSetAttribute(k_greedy<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
   }
   return 0;
 }
@@ -505,7 +514,7 @@ extern "C" int drsim_create(const drsim_config *cfg, int device, drsim_t **out) 
   if (const char *m = getenv("DRSIM_HOST_ACTIONS"))
     h->host_actions_mode = !strcmp(m, "zerocopy") ? 1 : (!strcmp(m, "dma") ? 2 : 0);
   plan_fused(h);
-  int rc = cfg->precision == DRSIM_F64 ? configure_kernels<double>(h) : configure_kernels<float>(h);
+  int rc = configure_kernels(h);
   if (rc) { drsim_destroy(h); return rc; }
   const int e_max0 = p.Ns <= kTileSlots ? std::min(p.R, kTileSlots / p.Ns) : 0;
   if (e_max0 > 1 && cfg->path != DRSIM_PATH_SPLIT && p.N == p.n_global) {
@@ -522,8 +531,7 @@ extern "C" int drsim_create(const drsim_config *cfg, int device, drsim_t **out) 
       plan_fused(h, e);
       if (!h->fused_ok) continue;
       const FusedGeom &g = h->geom;
-      const bool direct = g.chunk_rows == g.envs_per_tile * p.Ns || p.obs_dim == 0;
-      const bool lean = g.use_rows || direct;   // the chunked k_fused variant is markedly slower
+      const bool lean = g.use_rows || h->fused_direct;   // the chunked k_fused variant is markedly slower
       const int per_sm = rb == 8 ? 1 : std::max(1, std::min(2, (int)(226 * 1024 / std::max(1, g.smem_bytes))));
       const long resident = (long)per_sm * h->sm_count;
       const long rounds = (g.n_tiles + resident - 1) / resident;
@@ -535,15 +543,15 @@ extern "C" int drsim_create(const drsim_config *cfg, int device, drsim_t **out) 
       if (e >= 1) best_e = std::min(e, e_max);
     }
     plan_fused(h, best_e);
-    rc = cfg->precision == DRSIM_F64 ? configure_kernels<double>(h) : configure_kernels<float>(h);
+    rc = configure_kernels(h);
     if (rc) { drsim_destroy(h); return rc; }
     if (!h->fused_ok) {  // the chosen tile did not configure: back to the largest one
       plan_fused(h);
-      rc = cfg->precision == DRSIM_F64 ? configure_kernels<double>(h) : configure_kernels<float>(h);
+      rc = configure_kernels(h);
       if (rc) { drsim_destroy(h); return rc; }
     }
   }
-  rc = cfg->precision == DRSIM_F64 ? plan_shard<double>(h) : plan_shard<float>(h);
+  rc = plan_shard(h);
   if (rc) { drsim_destroy(h); return rc; }
   if (cfg->path == DRSIM_PATH_FUSED && !h->fused_ok) {
     drsim_destroy(h);
@@ -581,7 +589,7 @@ extern "C" int drsim_clone(const drsim_t *src, drsim_t **out) {
   h->sched_valid = src->sched_valid;
   h->sched_base = src->sched_base;
   h->xseq = src->xseq;
-  if (src->has_dur) { h->has_dur = true; h->fused_ok = false; }
+  h->has_dur = src->has_dur;
   h->shard = src->shard; h->shard_grid = src->shard_grid; h->shard_ok = src->shard_ok;
   *out = h;
   return 0;
@@ -710,8 +718,7 @@ static int set_state_t(drsim_handle *h, const drsim_host_state *st, cudaStream_t
     UP_HOUSE(lockout_duration, int32_t, h->o_dur)
     if (differs != h->has_dur) {
       h->has_dur = differs;
-      if (differs) h->fused_ok = false;
-      if ((rc = plan_shard<real>(h))) return rc;   // (the plain variant is out while the plane is live)
+      if ((rc = plan_shard(h))) return rc;   // (the plain variant is out while the plane is live)
     }
   }
 #undef UP_HOUSE
@@ -948,49 +955,153 @@ static void launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t sme
   cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
-template <typename real>
-static int launch_house_phase(drsim_handle *h, const StepIn &in, cudaStream_t s) {
-  const Planes<real> pl = make_planes<real>(h);
-  const SimParams &p = h->p;
-  if (p.policy == DRSIM_POLICY_GREEDY_MYOPIC && in.advance && !in.actions) {
-    int n2 = 1;
-    while (n2 < p.N) n2 <<= 1;
-    launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
-    h->launches++;
-  }
-  launch_pdl(k_house<real>, p.R * h->chunks, kThreads, 0, s, pl, p, in, h->chunks);
-  launch_pdl(k_reduce<real>, p.R, 128, 0, s, pl, p, in, h->chunks, make_peer(h));
-  h->launches += 2;
-  CU_TRY(cudaGetLastError());
-  return 0;
-}
+// ---- step routes ------------------------------------------------------------------------------
+// The kernels a step runs on.  The values are the DRSIM_ROUTE_* of drsim.h (drsim_step_route).
+enum class StepRoute : int {
+  FourKernel = DRSIM_ROUTE_FOUR_KERNEL,   // k_house + k_reduce + k_env + k_obs: every step any other route cannot take
+  Shard = DRSIM_ROUTE_SHARD,              // k_shard: clusters larger than a tile, house-sharded clusters, steps off the tile path
+  FusedChunked = DRSIM_ROUTE_FUSED,       // k_fused: the tile's rows staged in CTA-wide chunks
+  FusedDirect = DRSIM_ROUTE_FUSED_DIRECT,
+  Tma0 = DRSIM_ROUTE_FUSED_TMA0,
+  Tma1 = DRSIM_ROUTE_FUSED_TMA1,
+  Tma2 = DRSIM_ROUTE_FUSED_TMA2,
+  RowsStaged = DRSIM_ROUTE_FUSED_ROWS_STAGED,
+  RowsUnstaged = DRSIM_ROUTE_FUSED_ROWS_UNSTAGED,
+  Small = DRSIM_ROUTE_SMALL,
+  SmallGen = DRSIM_ROUTE_SMALL_GEN,
+};
 
-template <typename real>
-static int launch_env_phase(drsim_handle *h, const StepIn &in, const double *acc, int n_parts, cudaStream_t s) {
-  const Planes<real> pl = make_planes<real>(h);
-  const SimParams &p = h->p;
-  PeerCtx pc = make_peer(h);
-  if (acc || n_parts >= 0) pc.world = 1;  // explicit partials (or the handle's own): no peer wait
-  launch_pdl(k_env<real>, (p.R + 127) / 128, 128, 0, s, pl, p, in, (const double *)(acc ? acc : pl.acc), acc ? n_parts : 1, pc);
-  const bool smp = sample_rows(p);
-  auto kobs = smp ? k_obs<real, real, true> : k_obs<real, real>;
-  if constexpr (sizeof(real) == 4) {
-    if (h->obs_bytes == 2) kobs = smp ? k_obs<float, __nv_bfloat16, true> : k_obs<float, __nv_bfloat16>;
-  }
-  launch_pdl(kobs, p.R * h->obs_chunks, kObsChunk, (size_t)kObsChunk * p.obs_dim * h->obs_bytes, s, pl, p, in, h->obs_chunks);
-  h->launches += 2;
-  CU_TRY(cudaGetLastError());
-  return 0;
-}
+// What a step is, as far as its route goes.  Known before make_in builds its StepIn: make_in sets the schedule
+// pointers exactly when the step advances without injected noise.
+struct StepKind {
+  bool advance;    // a step of the power grid (not a refresh)
+  bool interp;     // the interpolator fires on this step
+  bool injected;   // outdoor-temperature or perlin noise comes from the caller (no scheduled records)
+  bool poll;       // copy-engine actions, polled word by word by the kernel (drsim_step_host)
+};
 
+// the tile kernels run the handle's fused plan; per-HVAC lock-out durations take the general path while they differ
+static bool fused_ready(const drsim_handle *h) { return h->fused_ok && !h->has_dur; }
 
-// ---- single-kernel step of the general path (drsim_shard.cuh) ---------------------------------
 static bool shard_plain(const drsim_handle *h) {
   return h->real_bytes == 4 && h->p.obs_dim == 10 && h->p.own_dim == 10 && !h->has_dur;
 }
 
-template <typename real>
-static int plan_shard(drsim_handle *h) {
+// can a step run as ONE k_shard launch?  (refreshes, the NCCL-gathered exchange and a halo without attached peers stay
+// on the four-kernel path)
+static bool shard_step_ok(const drsim_handle *h) {
+  if (!h->shard_ok) return false;
+  if (needs_halo(h->p) && h->peer_world < 2) return false;
+  return true;
+}
+
+// Clusters that fit a warp (<= 32 plane slots) in a handful of replicas: the latency-oriented kernels (one house per
+// lane) instead of the tile kernels (four houses per thread).  k_small (fp32) takes plain columns only; k_small_gen
+// (the fp64 build: the drop-in Environment) any observation / message option.
+static bool small_cluster(const drsim_handle *h) {
+  const SimParams &p = h->p;
+  if (getenv("DRSIM_NO_SMALL") || p.Ns > 32 || p.N != p.n_global || p.R > 256) return false;
+  if (h->real_bytes == 8 || p.obs_dim == 0) return true;
+  if (p.own_dim != 10 || (p.obs_dim & 1)) return false;
+  const bool msgs = p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0;
+  return msgs ? (p.msg_dim == 4 && p.obs_dim == 10 + 4 * p.nb_comm) : p.obs_dim == 10;
+}
+
+// The tile kernel plan_fused chose.  k_fused_tma is specialised by the step: MODE 1 = plain rows without messages, one
+// cluster per tile; MODE 2 = plain rows with messages, several clusters per tile (both for scheduled steps with external
+// actions and the individual penalty); MODE 0 = everything else.
+static StepRoute tile_route(const drsim_handle *h, bool scheduled) {
+  const SimParams &p = h->p;
+  const FusedGeom &g = h->geom;
+  if (g.use_rows) return g.in_stride ? StepRoute::RowsStaged : StepRoute::RowsUnstaged;
+  if (!g.use_tma) return h->fused_direct ? StepRoute::FusedDirect : StepRoute::FusedChunked;
+  const bool plain = p.own_dim == 10 && p.msg_dim == 4 && (p.obs_dim % 2) == 0 && p.obs_dim > 0;
+  const bool common = plain && scheduled && p.policy == DRSIM_POLICY_EXTERNAL && p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
+  if (common && !g.need_msg && g.envs_per_tile == 1) return StepRoute::Tma1;
+  if (common && g.need_msg && g.envs_per_tile > 1) return StepRoute::Tma2;
+  return StepRoute::Tma0;
+}
+
+static bool is_tma(StepRoute r) { return r == StepRoute::Tma0 || r == StepRoute::Tma1 || r == StepRoute::Tma2; }
+
+// the route of one step of this handle
+static StepRoute step_route(const drsim_handle *h, const StepKind &k) {
+  const SimParams &p = h->p;
+  const bool scheduled = k.advance && !k.injected;
+  if (fused_ready(h) && k.advance && !k.interp) {
+    if ((h->real_bytes == 8 || (scheduled && !k.poll)) && small_cluster(h))
+      return h->real_bytes == 8 ? StepRoute::SmallGen : StepRoute::Small;
+    const StepRoute t = tile_route(h, scheduled);
+    // k_fused_rows takes scheduled steps with the actions in the action plane (external, or written there by k_greedy)
+    // and the individual penalty
+    const bool rows_ok = scheduled && (p.policy == DRSIM_POLICY_EXTERNAL || p.policy == DRSIM_POLICY_GREEDY_MYOPIC) &&
+                         p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
+    if ((t == StepRoute::RowsStaged || t == StepRoute::RowsUnstaged) && !rows_ok) return StepRoute::FourKernel;
+    return t;
+  }
+  if (k.advance && p.N == p.n_global && shard_step_ok(h)) return StepRoute::Shard;
+  return StepRoute::FourKernel;
+}
+
+// ---- launches ---------------------------------------------------------------------------------
+// greedy-myopic policy: k_greedy writes this step's actions into the action plane, ahead of the step kernels
+static void launch_greedy(drsim_handle *h, const StepIn &in, cudaStream_t s) {
+  const SimParams &p = h->p;
+  if (p.policy != DRSIM_POLICY_GREEDY_MYOPIC || !in.advance || in.actions) return;
+  const int n2 = greedy_n2(p);
+  with_kernel_types(h, [&](auto k) {
+    using real = typename decltype(k)::real;
+    launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, make_planes<real>(h), p, n2);
+    return 0;
+  });
+  h->launches++;
+}
+
+static int launch_house_phase(drsim_handle *h, const StepIn &in, cudaStream_t s) {
+  const SimParams &p = h->p;
+  with_kernel_types(h, [&](auto k) {
+    using real = typename decltype(k)::real;
+    const Planes<real> pl = make_planes<real>(h);
+    launch_pdl(k_house<real>, p.R * h->chunks, kThreads, 0, s, pl, p, in, h->chunks);
+    launch_pdl(k_reduce<real>, p.R, 128, 0, s, pl, p, in, h->chunks, make_peer(h));
+    return 0;
+  });
+  h->launches += 2;
+  CU_TRY(cudaGetLastError());
+  return 0;
+}
+
+static int launch_env_phase(drsim_handle *h, const StepIn &in, const double *acc, int n_parts, cudaStream_t s) {
+  const SimParams &p = h->p;
+  PeerCtx pc = make_peer(h);
+  if (acc || n_parts >= 0) pc.world = 1;  // explicit partials (or the handle's own): no peer wait
+  with_kernel_types(h, [&](auto k) {
+    using K = decltype(k);
+    using real = typename K::real;
+    const Planes<real> pl = make_planes<real>(h);
+    launch_pdl(k_env<real>, (p.R + 127) / 128, 128, 0, s, pl, p, in, (const double *)(acc ? acc : pl.acc), acc ? n_parts : 1, pc);
+    launch_pdl(k_obs<real, typename K::O, K::S>, p.R * h->obs_chunks, kObsChunk, (size_t)kObsChunk * p.obs_dim * h->obs_bytes,
+               s, pl, p, in, h->obs_chunks);
+    return 0;
+  });
+  h->launches += 2;
+  CU_TRY(cudaGetLastError());
+  return 0;
+}
+
+// ---- single-kernel step of the general path (drsim_shard.cuh) ---------------------------------
+template <typename K>
+static auto shard_kernel(const drsim_handle *h) {
+  auto kern = k_shard<typename K::real, false, typename K::O, K::S>;
+  if constexpr (sizeof(typename K::real) == 4) {
+    if (shard_plain(h)) kern = k_shard<float, true, typename K::O>;   // (plain rows carry no messages)
+  }
+  return kern;
+}
+
+template <typename K>
+static int plan_shard_as(drsim_handle *h) {
+  using real = typename K::real;
   const SimParams &p = h->p;
   ShardGeom g{};
   h->shard_ok = false;
@@ -1018,25 +1129,12 @@ static int plan_shard(drsim_handle *h) {
   const int per_cta0 = (g.n_tiles + cap0 - 1) / cap0;
   g.t_smem = (int)std::min<size_t>(per_cta0, (budget - g.off_saved) / g.tile_bytes);
   if (const char *e = getenv("DRSIM_SHARD_TSMEM")) g.t_smem = std::max(0, std::min(g.t_smem, atoi(e)));
+  const auto kern = shard_kernel<K>(h);
   int per_sm = 0;
   for (;; --g.t_smem) {
     g.smem_bytes = g.off_saved + g.t_smem * g.tile_bytes;
-    bool done = false;
-    if constexpr (sizeof(real) == 4) {
-      const bool bf = h->obs_bytes == 2;
-      const bool smp = sample_rows(p);
-      auto kern = plain ? (bf ? k_shard<float, true, __nv_bfloat16> : k_shard<float, true>)
-                        : smp ? (bf ? k_shard<float, false, __nv_bfloat16, true> : k_shard<float, false, float, true>)
-                              : (bf ? k_shard<float, false, __nv_bfloat16> : k_shard<float, false>);
-      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
-      done = true;
-    }
-    if (!done) {
-      auto kern = sample_rows(p) ? k_shard<real, false, real, true> : k_shard<real, false>;
-      CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
-      CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
-    }
+    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes));
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, g.smem_bytes));
     if (per_sm >= min_ctas || g.t_smem == 0) break;
   }
   if (per_sm < 1) return 0;
@@ -1049,24 +1147,13 @@ static int plan_shard(drsim_handle *h) {
   return 0;
 }
 
-// can this step run as ONE k_shard launch?  (refreshes, the NCCL-gathered exchange and a halo without
-// attached peers stay on the four-kernel path)
-static bool shard_step_ok(const drsim_handle *h) {
-  if (!h->shard_ok) return false;
-  if (needs_halo(h->p) && h->peer_world < 2) return false;
-  return true;
+static int plan_shard(drsim_handle *h) {
+  return with_kernel_types(h, [&](auto k) { return plan_shard_as<decltype(k)>(h); });
 }
 
-template <typename real>
-static int launch_shard(drsim_handle *h, StepIn in, cudaStream_t s) {
-  const Planes<real> pl = make_planes<real>(h);
+template <typename K>
+static void launch_shard(drsim_handle *h, StepIn in, cudaStream_t s) {
   const SimParams &p = h->p;
-  if (p.policy == DRSIM_POLICY_GREEDY_MYOPIC && in.advance && !in.actions) {
-    int n2 = 1;
-    while (n2 < p.N) n2 <<= 1;
-    launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
-    h->launches++;
-  }
   if (needs_halo(p)) {   // the peers push their edge-house records into this rank's halo inbox (reduce_cluster)
     const int L = p.nb_comm / 2;
     const size_t per_rank = (size_t)p.R * p.nb_comm * kHaloFields;
@@ -1084,17 +1171,8 @@ static int launch_shard(drsim_handle *h, StepIn in, cudaStream_t s) {
   sc.dbg = h->shard_dbg;
   PeerCtx pc = make_peer(h);
   if (!needs_halo(p)) pc.rowll = reinterpret_cast<unsigned long long *const *>(h->slab + h->o_peer_tab + 64 * 8);
-  const bool smp = sample_rows(p);
-  auto kern = smp ? k_shard<real, false, real, true> : k_shard<real, false>;
-  if constexpr (sizeof(real) == 4) {
-    const bool bf = h->obs_bytes == 2;
-    if (shard_plain(h)) kern = bf ? k_shard<float, true, __nv_bfloat16> : k_shard<float, true>;
-    else if (bf) kern = smp ? k_shard<float, false, __nv_bfloat16, true> : k_shard<float, false, __nv_bfloat16>;
-  }
-  launch_pdl(kern, h->shard_grid, kThreads, (size_t)h->shard.smem_bytes, s, pl, p, in, h->shard, sc, pc);
-  h->launches++;
-  CU_TRY(cudaGetLastError());
-  return 0;
+  launch_pdl(shard_kernel<K>(h), h->shard_grid, kThreads, (size_t)h->shard.smem_bytes, s, make_planes<typename K::real>(h), p,
+             in, h->shard, sc, pc);
 }
 
 static int exchange_error(const drsim_handle *h) {
@@ -1104,151 +1182,71 @@ static int exchange_error(const drsim_handle *h) {
   return 0;
 }
 
-// picks the compile-time specialisation of the production kernel (see k_fused_tma); O = row element type, S = sampled
-// neighbours (MODE 1 writes no messages)
-template <typename O, bool S>
-static void launch_tma(drsim_handle *h, const StepIn &in, cudaStream_t s) {
-  const Planes<float> pl = make_planes<float>(h);
+// the one kernel of a single-kernel route; grid = the persistent grid of the tile kernels
+template <typename K>
+static void launch_step_kernel(drsim_handle *h, StepRoute r, const StepIn &in, int grid, const SnapPtrs &snap,
+                               unsigned char *snap_obs, cudaStream_t s) {
+  using real = typename K::real;
+  using O = typename K::O;
+  constexpr bool S = K::S;
+  const Planes<real> pl = make_planes<real>(h);
   const SimParams &p = h->p;
   const FusedGeom &g = h->geom;
-  const int grid = h->launch_grid ? h->launch_grid : h->fused_grid;
-  const bool plain = p.own_dim == 10 && p.msg_dim == 4 && (p.obs_dim % 2) == 0 && p.obs_dim > 0;
-  const bool common = plain && in.sched_od != nullptr && p.policy == DRSIM_POLICY_EXTERNAL &&
-                      p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
-  const bool poll = in.act_poll_err != nullptr;   // copy-engine mode of drsim_step_host
-  if (common && !g.need_msg && g.envs_per_tile == 1) {
-    if (poll) launch_pdl(k_fused_tma<1, true, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<1, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-  } else if (common && g.need_msg && g.envs_per_tile > 1) {
-    if (poll) launch_pdl(k_fused_tma<2, true, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<2, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-  } else {
-    if (poll) launch_pdl(k_fused_tma<0, true, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
-    else launch_pdl(k_fused_tma<0, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+  const int small_grid = (p.R + kSmallWarps - 1) / kSmallWarps;
+  const bool poll = in.act_poll_err != nullptr;
+  switch (r) {
+    case StepRoute::Shard: launch_shard<K>(h, in, s); return;
+    case StepRoute::FusedChunked: k_fused<real, O, S><<<grid, kThreads, g.smem_bytes, s>>>(pl, p, in, g); return;
+    case StepRoute::FusedDirect: k_fused_direct<real, O, S><<<grid, kThreads, g.smem_bytes, s>>>(pl, p, in, g); return;
+    default: break;
   }
-}
-
-template <typename O, bool S>
-static void launch_rows(drsim_handle *h, const StepIn &in, cudaStream_t s) {
-  const Planes<float> pl = make_planes<float>(h);
-  const int grid = h->launch_grid ? h->launch_grid : h->fused_grid;
-  if (h->geom.in_stride && in.act_poll_err)
-    launch_pdl(k_fused_rows<true, true, O, S>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-  else if (h->geom.in_stride) launch_pdl(k_fused_rows<true, false, O, S>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-  else launch_pdl(k_fused_rows<false, false, O, S>, grid, kThreads, h->geom.smem_bytes, s, pl, h->p, in, h->geom);
-}
-
-// steps the wide-row kernel cannot take (injected noise, on-device policies, common penalty modes)
-// run on the general path
-template <typename real>
-static int launch_house_phase(drsim_handle *h, const StepIn &in, cudaStream_t s);
-template <typename real>
-static int launch_env_phase(drsim_handle *h, const StepIn &in, const double *acc, int n_parts, cudaStream_t s);
-template <typename real>
-static int launch_chunked_fallback(drsim_handle *h, const StepIn &in, cudaStream_t s) {
-  int rc = launch_house_phase<real>(h, in, s);
-  if (rc) return rc;
-  return launch_env_phase<real>(h, in, nullptr, 1, s);
-}
-
-// A handle whose clusters fit a warp (<= 32 plane slots) in a handful of replicas: the latency-oriented kernel k_small
-// (one house per lane) instead of the tile kernels (four houses per thread).  fp32, plain columns only.
-static bool small_handle(const drsim_handle *h) {
-  const SimParams &p = h->p;
-  if (getenv("DRSIM_NO_SMALL") || h->real_bytes != 4 || !h->fused_ok || p.Ns > 32 || p.N != p.n_global || p.R > 256) return false;
-  if (p.obs_dim == 0) return true;
-  if (p.own_dim != 10 || (p.obs_dim & 1)) return false;
-  const bool msgs = p.obs_layout == DRSIM_OBS_HAND_ENGINEERED && p.nb_comm > 0;
-  return msgs ? (p.msg_dim == 4 && p.obs_dim == 10 + 4 * p.nb_comm) : p.obs_dim == 10;
+  if constexpr (sizeof(real) == 8) {
+    if (r == StepRoute::SmallGen)
+      launch_pdl(k_small_gen<double, S>, small_grid, kSmallWarps * 32, 0, s, pl, p, in, snap, reinterpret_cast<double *>(snap_obs));
+  } else {
+    switch (r) {
+      case StepRoute::Tma0:
+        launch_pdl(poll ? k_fused_tma<0, true, O, S> : k_fused_tma<0, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+        break;
+      case StepRoute::Tma1:
+        launch_pdl(poll ? k_fused_tma<1, true, O> : k_fused_tma<1, false, O>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+        break;
+      case StepRoute::Tma2:
+        launch_pdl(poll ? k_fused_tma<2, true, O, S> : k_fused_tma<2, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+        break;
+      case StepRoute::RowsStaged:
+        launch_pdl(poll ? k_fused_rows<true, true, O, S> : k_fused_rows<true, false, O, S>, grid, kThreads, g.smem_bytes, s, pl,
+                   p, in, g);
+        break;
+      case StepRoute::RowsUnstaged:   // (inputs through registers: never a polled step, see can_dma in step_host_impl)
+        launch_pdl(k_fused_rows<false, false, O, S>, grid, kThreads, g.smem_bytes, s, pl, p, in, g);
+        break;
+      case StepRoute::Small: launch_pdl(k_small<O, S>, small_grid, kSmallWarps * 32, 0, s, pl, p, in); break;
+      default: break;
+    }
+  }
 }
 
 static int snap_targets(drsim_handle *h, SnapPtrs &o, unsigned char **obs_dev);
 
-// ... and the fp64 build (the drop-in Environment): k_small_gen<double>, any observation / message option
-static bool small64_handle(const drsim_handle *h) {
-  const SimParams &p = h->p;
-  return !getenv("DRSIM_NO_SMALL") && h->real_bytes == 8 && h->fused_ok && p.Ns <= 32 && p.N == p.n_global && p.R <= 256;
-}
-
-// one launch of the tile kernel chosen for this handle, rows of element type O, sampled neighbours S
-template <typename real, typename O, bool S>
-static void launch_tile_as(drsim_handle *h, const StepIn &in, bool rows_ok, cudaStream_t s) {
-  const Planes<real> pl = make_planes<real>(h);
-  if constexpr (sizeof(real) == 4) {
-    if (rows_ok) { launch_rows<O, S>(h, in, s); return; }
-    if (h->fused_direct && h->geom.use_tma) { launch_tma<O, S>(h, in, s); return; }
+// the launches of one step on route r
+static int launch_step(drsim_handle *h, StepRoute r, const StepIn &in, int grid, cudaStream_t s) {
+  h->last_route = (int)r;
+  launch_greedy(h, in, s);
+  if (r == StepRoute::FourKernel) {
+    if (int rc = launch_house_phase(h, in, s)) return rc;
+    return launch_env_phase(h, in, nullptr, 1, s);
   }
-  if (h->fused_direct) k_fused_direct<real, O, S><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
-  else k_fused<real, false, O, S><<<h->fused_grid, kThreads, h->geom.smem_bytes, s>>>(pl, h->p, in, h->geom);
-}
-template <typename real, typename O>
-static void launch_tile(drsim_handle *h, const StepIn &in, bool rows_ok, cudaStream_t s) {
-  if (sample_rows(h->p)) launch_tile_as<real, O, true>(h, in, rows_ok, s);
-  else launch_tile_as<real, O, false>(h, in, rows_ok, s);
-}
-
-template <typename real>
-static int launch_fused(drsim_handle *h, const StepIn &in, cudaStream_t s) {
-  const Planes<real> pl = make_planes<real>(h);
-  const SimParams &p = h->p;
-  if constexpr (sizeof(real) == 8) {
-    if (small64_handle(h) && in.advance && in.do_interp <= 0 && !pl.dur) {
-      if (p.policy == DRSIM_POLICY_GREEDY_MYOPIC && !in.actions) {
-        int n2 = 1;
-        while (n2 < p.N) n2 <<= 1;
-        launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
-        h->launches++;
-      }
-      SnapPtrs so{};
-      unsigned char *so_obs = nullptr;
-      if (h->snap_next) {
-        if (int rc = snap_targets(h, so, &so_obs)) return rc;
-        h->snap_fused = true;
-      }
-      launch_pdl(sample_rows(p) ? k_small_gen<double, true> : k_small_gen<double>, (p.R + kSmallWarps - 1) / kSmallWarps,
-                 kSmallWarps * 32, 0, s, pl, p, in, so,
-                 reinterpret_cast<double *>(so_obs));
-      h->launches++;
-      CU_TRY(cudaGetLastError());
-      return 0;
-    }
+  SnapPtrs snap{};
+  unsigned char *snap_obs = nullptr;
+  if (r == StepRoute::SmallGen && h->snap_next) {   // k_small_gen writes the host snapshot itself
+    if (int rc = snap_targets(h, snap, &snap_obs)) return rc;
+    h->snap_fused = true;
   }
-  if constexpr (sizeof(real) == 4) {
-    if (small_handle(h) && in.sched_rec && in.advance && in.do_interp <= 0 && !in.act_poll_err && !pl.dur) {
-      if (p.policy == DRSIM_POLICY_GREEDY_MYOPIC && !in.actions) {
-        int n2 = 1;
-        while (n2 < p.N) n2 <<= 1;
-        launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
-        h->launches++;
-      }
-      auto kern = h->obs_bytes == 2 ? k_small<__nv_bfloat16> : k_small<float>;
-      if (sample_rows(p)) kern = h->obs_bytes == 2 ? k_small<__nv_bfloat16, true> : k_small<float, true>;
-      launch_pdl(kern, (p.R + kSmallWarps - 1) / kSmallWarps, kSmallWarps * 32, 0, s, pl, p, in);
-      h->launches++;
-      CU_TRY(cudaGetLastError());
-      return 0;
-    }
-  }
-  if (p.policy == DRSIM_POLICY_GREEDY_MYOPIC && in.advance && !in.actions) {
-    int n2 = 1;
-    while (n2 < p.N) n2 <<= 1;
-    launch_pdl(k_greedy<real>, p.R, std::min(1024, std::max(32, n2)), (size_t)n2 * 24, s, pl, p, n2);
-    h->launches++;
-  }
-  // (greedy-myopic actions were just written into the action plane by k_greedy: external to the step kernel)
-  const bool rows_ok = h->geom.use_rows && in.sched_od != nullptr &&
-                       (p.policy == DRSIM_POLICY_EXTERNAL || p.policy == DRSIM_POLICY_GREEDY_MYOPIC) &&
-                       p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
-  if (h->geom.use_rows && !rows_ok) return launch_chunked_fallback<real>(h, in, s);
-  if constexpr (sizeof(real) == 4) {
-    if (h->obs_bytes == 2) {
-      launch_tile<float, __nv_bfloat16>(h, in, rows_ok, s);
-      h->launches++;
-      CU_TRY(cudaGetLastError());
-      return 0;
-    }
-  }
-  launch_tile<real, real>(h, in, rows_ok, s);
+  with_kernel_types(h, [&](auto k) {
+    launch_step_kernel<decltype(k)>(h, r, in, grid, snap, snap_obs, s);
+    return 0;
+  });
   h->launches++;
   CU_TRY(cudaGetLastError());
   return 0;
@@ -1307,20 +1305,12 @@ static int run_step(drsim_handle *h, const drsim_step_args *a, int advance, int 
   if (h->broken)
     return fail(DRSIM_E_STATE, "an earlier host-buffer step was committed with missing actions: re-inject the state "
                                "(drsim_set_state / drsim_reset) before stepping again");
+  const StepKind kind{advance != 0, do_interp > 0, a && (a->od_noise || a->perlin), h->act_poll_next};
+  const StepRoute r = step_route(h, kind);
   h->xseq++;
   const StepIn in = make_in(h, a, advance, do_interp, s);
-  const bool dbl = h->real_bytes == 8;
-  int rc;
-  if (h->fused_ok && do_interp <= 0 && advance) {
-    rc = dbl ? launch_fused<double>(h, in, s) : launch_fused<float>(h, in, s);
-  } else if (advance && h->p.N == h->p.n_global && shard_step_ok(h)) {
-    rc = dbl ? launch_shard<double>(h, in, s) : launch_shard<float>(h, in, s);   // one launch instead of four
-  } else {
-    if (h->p.N != h->p.n_global) return fail(DRSIM_E_STATE, "house-sharded cluster: use drsim_step_begin / drsim_step_finish");
-    rc = dbl ? launch_house_phase<double>(h, in, s) : launch_house_phase<float>(h, in, s);
-    if (rc) return rc;
-    rc = dbl ? launch_env_phase<double>(h, in, nullptr, 1, s) : launch_env_phase<float>(h, in, nullptr, 1, s);
-  }
+  if (h->p.N != h->p.n_global) return fail(DRSIM_E_STATE, "house-sharded cluster: use drsim_step_begin / drsim_step_finish");
+  const int rc = launch_step(h, r, in, h->fused_grid, s);
   // the packed schedule records chain each step to the one before it (previous signal / outdoor
   // temperature, base power): any step that did not follow the schedule ends their validity
   if (!(advance && in.sched_rec && do_interp <= 0)) h->sched_valid = false;
@@ -1378,32 +1368,28 @@ extern "C" int drsim_run_tape(drsim_t *h, const drsim_step_args *args, int n_ste
   // (its next step's first tile must not be the tile it is still updating): it runs on min(resident CTAs, tiles / 2)
   // CTAs, and only when that costs at most a tenth of the resident grid.
   const SimParams &p = h->p;
-  const bool small = small_handle(h);
-  const int sgrid = h->fused_ok ? std::min(h->fused_grid, h->geom.n_tiles / 2) : 0;
-  const bool tma_path = h->fused_direct && h->geom.use_tma && !h->geom.use_rows;
-  const bool rows_path = tape && h->geom.use_rows && h->geom.in_stride && p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2 &&
-                         sgrid * 10 >= h->fused_grid * 9;
+  const StepRoute r = step_route(h, StepKind{true, false, false, false});
+  const int sgrid = fused_ready(h) ? std::min(h->fused_grid, h->geom.n_tiles / 2) : 0;
+  const bool loop_route = r == StepRoute::Small || is_tma(r) ||
+                          (r == StepRoute::RowsStaged && tape && sgrid * 10 >= h->fused_grid * 9);
   const bool policy_ok = tape ? p.policy == DRSIM_POLICY_EXTERNAL
                               : (p.policy != DRSIM_POLICY_EXTERNAL && p.policy != DRSIM_POLICY_GREEDY_MYOPIC);
-  const bool taped = n_steps > 1 && h->fused_ok && h->real_bytes == 4 && (small || tma_path || rows_path) && policy_ok &&
-                     p.base_mode == DRSIM_BASE_CONSTANT && !h->mirror_next &&
+  const bool taped = n_steps > 1 && loop_route && policy_ok && p.base_mode == DRSIM_BASE_CONSTANT && !h->mirror_next &&
                      !h->act_poll_next && !h->obs_override && !h->reward_override && !h->broken && !getenv("DRSIM_NO_STREAM");
   int first = 0;
   if (taped) {
+    const int grid = r == StepRoute::RowsStaged ? sgrid : h->fused_grid;
     a.actions = tape;
     while (first < n_steps) {
       h->xseq++;
       StepIn in = make_in(h, &a, 1, 0, (cudaStream_t)stream);   // (re)generates the schedule block when the step leaves it
-      if (!in.sched_rec) break;                                  // no scheduled records (should not happen): per-step loop
       const int k = (int)std::min<int64_t>(n_steps - first, h->sched_base + drsim_handle::kSched - h->step);
       in.stream_steps = k;
       in.tape_planes = tape_planes;
       in.tape_first = first;
       in.tape_stride = action_stride;
       if (k == 1 && tape) in.actions = tape + (size_t)(tape_planes > 0 ? first % tape_planes : first) * action_stride;
-      h->launch_grid = (small || tma_path) ? 0 : sgrid;
-      const int rc = launch_fused<float>(h, in, (cudaStream_t)stream);
-      h->launch_grid = 0;
+      const int rc = launch_step(h, r, in, grid, (cudaStream_t)stream);
       if (rc) return rc;
       h->step += k;
       first += k;
@@ -1436,8 +1422,9 @@ extern "C" int drsim_step_begin(drsim_t *h, const drsim_step_args *args, void *s
   h->xseq++;
   const StepIn in = make_in(h, args, 1, h->pending_interp, (cudaStream_t)stream);
   h->pending_in = in;
-  return h->real_bytes == 8 ? launch_house_phase<double>(h, in, (cudaStream_t)stream)
-                            : launch_house_phase<float>(h, in, (cudaStream_t)stream);
+  h->last_route = (int)StepRoute::FourKernel;
+  launch_greedy(h, in, (cudaStream_t)stream);
+  return launch_house_phase(h, in, (cudaStream_t)stream);
 }
 
 static int step_finish_impl(drsim_handle *h, const double *acc, const double *halo, int n_parts, int rank,
@@ -1465,8 +1452,7 @@ static int step_finish_impl(drsim_handle *h, const double *acc, const double *ha
                                "(drsim_step_finish_gathered) or use the peer exchange");
     }
   }
-  int rc = h->real_bytes == 8 ? launch_env_phase<double>(h, in, acc, n_parts, stream)
-                              : launch_env_phase<float>(h, in, acc, n_parts, stream);
+  int rc = launch_env_phase(h, in, acc, n_parts, stream);
   if (!rc) h->step++;
   return rc;
 }
@@ -1489,8 +1475,7 @@ extern "C" int drsim_step_sharded(drsim_t *h, const drsim_step_args *args, void 
     const int di = interp_decision(h);
     h->xseq++;
     const StepIn in = make_in(h, args, 1, di, (cudaStream_t)stream);
-    const int rc = h->real_bytes == 8 ? launch_shard<double>(h, in, (cudaStream_t)stream)
-                                      : launch_shard<float>(h, in, (cudaStream_t)stream);
+    const int rc = launch_step(h, StepRoute::Shard, in, h->fused_grid, (cudaStream_t)stream);
     // the packed schedule records chain each step to the one before it: a step off the schedule ends their validity
     if (!(in.sched_rec && di <= 0)) h->sched_valid = false;
     if (!rc) h->step++;
@@ -1506,17 +1491,6 @@ extern "C" int drsim_step_finish_gathered(drsim_t *h, const double *acc_gathered
   if (!h) return fail(DRSIM_E_ARG, "null handle");
   if (!acc_gathered) return fail(DRSIM_E_ARG, "acc_gathered is required");
   return step_finish_impl(h, acc_gathered, halo_gathered, n_parts, rank, (cudaStream_t)stream);
-}
-
-// true when this step will run on one of the staged fused kernels with the scheduled (fast) env path:
-// those prefetch their inputs one tile ahead (so actions can be read in place from mapped host memory)
-// and mirror the per-cluster results into the mapped result buffer
-static bool staged_fast_step(const drsim_handle *h, int do_interp, bool injected) {
-  if (!h->fused_ok || h->real_bytes != 4 || do_interp > 0 || injected) return false;
-  const SimParams &p = h->p;
-  if (h->geom.use_rows)
-    return (p.policy == DRSIM_POLICY_EXTERNAL || p.policy == DRSIM_POLICY_GREEDY_MYOPIC) && p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
-  return h->fused_direct && h->geom.use_tma;
 }
 
 // Host-buffer step.  On the staged fused path the action transfer overlaps the kernel instead of
@@ -1607,7 +1581,12 @@ static int step_host_impl(drsim_t *h, const uint8_t *actions, const double *od_n
   drsim_step_args a{};
   const int tsi_before = h->t_since_interp;
   const int di = interp_decision(h);
-  const bool staged = staged_fast_step(h, di, od_noise || perlin);
+  // The staged tile kernels (k_fused_tma, k_fused_rows) prefetch their inputs one tile ahead, so they can read the
+  // actions in place from mapped host memory, and they mirror the per-cluster results into mapped host memory.
+  // `polled` is the route of this step if its actions are polled; only k_fused_rows<unstaged> has no polling variant.
+  const bool injected = od_noise || perlin;
+  const StepRoute polled = step_route(h, StepKind{true, di > 0, injected, true});
+  const bool staged = !injected && (is_tma(polled) || polled == StepRoute::RowsStaged || polled == StepRoute::RowsUnstaged);
   bool dma_poll = false;
   // small inputs: staged in the handle's pinned mapped page and read in place by the kernels (the call ends with a
   // stream synchronisation, so the page is free again when it returns)
@@ -1640,7 +1619,7 @@ static int step_host_impl(drsim_t *h, const uint8_t *actions, const double *od_n
     // Needs the stream sync this call ends with (env_out), so the next copy cannot overtake this kernel.
     const size_t act_bytes = (size_t)p.R * p.N;
     const bool can_dma = mapped && h->copy_stream && h->h_poll_err_dev && env_out && h->h_env_dev &&
-                         (!h->geom.use_rows || h->geom.in_stride > 0);
+                         polled != StepRoute::RowsUnstaged;
     const bool want_dma = h->host_actions_mode == 2 || (h->host_actions_mode == 0 && act_bytes >= ((size_t)256 << 10));
     if (can_dma && want_dma) {
       CU_TRY(cudaMemcpyAsync(h->slab + h->o_act_stage, actions, act_bytes, cudaMemcpyHostToDevice, h->copy_stream));
@@ -1816,8 +1795,7 @@ extern "C" int drsim_reset(drsim_t *h, const drsim_reset_args *ra, void *stream)
   h->t_since_interp = h->p.interp_period + 1;
   if (h->has_dur) {   // the device reset draws no lock-out noise: back to the common duration
     h->has_dur = false;
-    const int rc = h->real_bytes == 8 ? plan_shard<double>(h) : plan_shard<float>(h);
-    if (rc) return rc;
+    if (int rc = plan_shard(h)) return rc;
   }
   // artificial ratio: power_grid.py:46-49 draws ratio * range^(2u - 1); range == 1 in every shipped config
   {
@@ -2069,21 +2047,20 @@ extern "C" int64_t drsim_launch_count(const drsim_t *h) { return h ? h->launches
 
 extern "C" int drsim_fused_info(const drsim_t *h, int32_t out[6]) {
   if (!h || !out) return fail(DRSIM_E_ARG, "null argument");
-  int variant = 0;
-  if (h->fused_ok) {
-    if (h->geom.use_rows) variant = 4;
-    else if (h->fused_direct && h->geom.use_tma) variant = 3;
-    else if (h->fused_direct) variant = 2;
-    else variant = 1;
-  }
+  const bool f = fused_ready(h);
+  const StepRoute t = tile_route(h, true);
+  int variant = 0;   // none, chunked, direct, staged (k_fused_tma), staged_rows (k_fused_rows)
+  if (f) variant = t == StepRoute::FusedChunked ? 1 : t == StepRoute::FusedDirect ? 2 : is_tma(t) ? 3 : 4;
   out[0] = variant;
-  out[1] = h->fused_ok ? h->geom.envs_per_tile : 0;
-  out[2] = h->fused_ok ? h->geom.n_tiles : 0;
-  out[3] = h->fused_ok ? h->fused_grid : 0;
-  out[4] = h->fused_ok ? h->geom.smem_bytes : 0;
-  out[5] = h->fused_ok ? h->fused_per_sm : 0;
+  out[1] = f ? h->geom.envs_per_tile : 0;
+  out[2] = f ? h->geom.n_tiles : 0;
+  out[3] = f ? h->fused_grid : 0;
+  out[4] = f ? h->geom.smem_bytes : 0;
+  out[5] = f ? h->fused_per_sm : 0;
   return 0;
 }
+
+extern "C" int drsim_step_route(const drsim_t *h) { return h ? h->last_route : -1; }
 
 template <typename real>
 static int summary_impl(drsim_t *h, double *d_out, cudaStream_t st) {

@@ -1563,11 +1563,12 @@ template <typename real> struct FusedOcc { static constexpr int min_ctas = 1; };
 template <> struct FusedOcc<float> { static constexpr int min_ctas = DRSIM_FUSED_MINCTAS; };
 
 // ------------------------------------------------------------------------------------------
-// Fused path: one persistent kernel per step (always a real step: refreshes use the general path).
-// DIRECT: the whole tile's observation rows fit the staging buffer; each thread writes the rows of
-// its own 4 houses straight from registers and one TMA bulk store per tile ships them.
+// Fused path, chunked variant: one persistent kernel per step (always a real step: refreshes use the
+// general path) for tiles whose observation rows do not fit the staging buffer at once.  Phase 1 parks
+// every house's message and own-column record in shared memory; phase 3 assembles the rows from them
+// g.chunk_rows at a time, one TMA bulk store per chunk.
 // ------------------------------------------------------------------------------------------
-template <typename real, bool DIRECT, typename O = real, bool SMP = false>
+template <typename real, typename O = real, bool SMP = false>
 __global__ void __launch_bounds__(kThreads, FusedOcc<real>::min_ctas)
 k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1602,25 +1603,21 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
       const int r = r0 + e_loc;
       const int n0 = s0 - e_loc * Ns;
       house4_step<real, true>(pl, p, kc, in, base + s0, min(4, p.N - n0), (real)pl.od_temp[r], (real)pl.solar_next[r], h, red);
-      if (g.need_msg || !DIRECT) {
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const uint32_t f = (h.flags >> (8 * j)) & 0xffu;
-          const real pmax = qdiv(h.cap[j], kc.cop, kc.inv_cop);
-          Msg4<real> m;
-          m.dT = div5(Rep<real>::dev(h.ta[j], h.target[j]));                  // norm.py:39
-          m.sso_n = (real)fast_div((uint32_t)h.sso[j], p.fd_dur);             // norm.py:40-43
-          m.p_n = qdiv((f & 1u) ? pmax : (real)0, kc.nrs, kc.inv_nrs);
-          m.pmax_n = qdiv(pmax, kc.nrs, kc.inv_nrs);
-          if (j >= h.valid) { m.dT = m.sso_n = m.p_n = m.pmax_n = 0; }
-          s_msg[s0 + j] = m;
-          if (!DIRECT) {
-            Own4<real> o;
-            o.ta = h.ta[j]; o.tm = h.tm[j]; o.target = h.target[j]; o.flags = (real)f;
-            if (j >= h.valid) { o.ta = o.tm = o.target = o.flags = 0; }
-            s_own[s0 + j] = o;
-          }
-        }
+      for (int j = 0; j < 4; ++j) {
+        const uint32_t f = (h.flags >> (8 * j)) & 0xffu;
+        const real pmax = qdiv(h.cap[j], kc.cop, kc.inv_cop);
+        Msg4<real> m;
+        m.dT = div5(Rep<real>::dev(h.ta[j], h.target[j]));                  // norm.py:39
+        m.sso_n = (real)fast_div((uint32_t)h.sso[j], p.fd_dur);             // norm.py:40-43
+        m.p_n = qdiv((f & 1u) ? pmax : (real)0, kc.nrs, kc.inv_nrs);
+        m.pmax_n = qdiv(pmax, kc.nrs, kc.inv_nrs);
+        if (j >= h.valid) { m.dT = m.sso_n = m.p_n = m.pmax_n = 0; }
+        s_msg[s0 + j] = m;
+        Own4<real> o;
+        o.ta = h.ta[j]; o.tm = h.tm[j]; o.target = h.target[j]; o.flags = (real)f;
+        if (j >= h.valid) { o.ta = o.tm = o.target = o.flags = 0; }
+        s_own[s0 + j] = o;
       }
     }
     // segmented warp reduction over clusters (lanes of one cluster are contiguous)
@@ -1665,27 +1662,34 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) rw[j] = j < h.valid ? house_reward<real>(p, kc, h.ta[j], h.target[j], e) : (real)0;
       store4(pl.reward + base + s0, rw);
-      if (DIRECT && D > 0) {
-        const int n0 = s0 - e_loc * Ns;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          O *row = s_tile + (size_t)(s0 + j) * D;
-          if (j < h.valid) {
-            const uint32_t f = (h.flags >> (8 * j)) & 0xffu;
+    }
+    if (D > 0) {
+      for (int cb = 0; cb < slots; cb += g.chunk_rows) {
+        const int rows = min(g.chunk_rows, slots - cb);
+        if (cb > 0) {
+          if (threadIdx.x == 0) bulk_store_wait_read();
+          __syncthreads();
+        }
+        for (int i = threadIdx.x; i < rows; i += kThreads) {
+          const int s = cb + i;
+          const int e = (int)fast_div((uint32_t)s, p.fd_ns), n = s - e * Ns;
+          O *row = s_tile + (size_t)i * D;
+          if (n < p.N) {
+            const Own4<real> o = s_own[s];
+            const Msg4<real> m = s_msg[s];
             real ratio[4] = {0, 0, 0, 0};
             if (p.st_thermal)
-              for (int k = 0; k < 4; ++k) ratio[k] = pl.ratio[k][base + s0 + j];
-            int q = obs_own<real>(row, p, f, (real)fast_div((uint32_t)h.sso[j], p.fd_dur),
-                                  Rep<real>::minus20(h.ta[j], h.target[j]), Rep<real>::minus20(h.tm[j], h.target[j]),
-                                  h.target[j] - (real)20, e, ratio);
+              for (int k = 0; k < 4; ++k) ratio[k] = pl.ratio[k][base + s];
+            int q = obs_own<real>(row, p, (uint32_t)o.flags, m.sso_n, Rep<real>::minus20(o.ta, o.target),
+                                  Rep<real>::minus20(o.tm, o.target), o.target - (real)20, s_env[e], ratio);
             if (g.need_msg) {
-              RowNbrs<SMP> nbr(p, r0 + e_loc, n0 + j, rows_draw(in));
+              RowNbrs<SMP> nbr(p, r0 + e, n, rows_draw(in));
               for (int k = 0; k < p.nb_comm; ++k) {
-                const int nb = nbr(p, pl.comm_table, r0 + e_loc, n0 + j, k);
-                const Msg4<real> mk = s_msg[e_loc * Ns + nb];
+                const int nb = nbr(p, pl.comm_table, r0 + e, n, k);
+                const Msg4<real> mk = s_msg[e * Ns + nb];
                 row[q++] = mk.dT; row[q++] = mk.sso_n; row[q++] = mk.p_n; row[q++] = mk.pmax_n;
                 if (p.msg_thermal)
-                  for (int t = 0; t < 4; ++t) row[q++] = (real)pl.ratio[t][base + e_loc * Ns + nb];
+                  for (int t = 0; t < 4; ++t) row[q++] = (real)pl.ratio[t][base + e * Ns + nb];
                 if (p.msg_hvac) { row[q++] = (real)p.cop; row[q++] = (real)p.latent; row[q++] = (real)p.dcap; }
               }
             }
@@ -1693,56 +1697,11 @@ k_fused(Planes<real> pl, SimParams p, StepIn in, FusedGeom g) {
             for (int q = 0; q < D; ++q) row[q] = (real)0;
           }
         }
-      }
-    }
-    if (D > 0) {
-      if (DIRECT) {
         fence_proxy_async_smem();
         __syncthreads();
         if (threadIdx.x == 0) {
-          bulk_store_s2g(pl.template rows<O>() + base * D, s_tile, (uint32_t)((size_t)slots * D * sizeof(O)));
+          bulk_store_s2g(pl.template rows<O>() + (base + cb) * D, s_tile, (uint32_t)((size_t)rows * D * sizeof(O)));
           store_pending = true;
-        }
-      } else {
-        for (int cb = 0; cb < slots; cb += g.chunk_rows) {
-          const int rows = min(g.chunk_rows, slots - cb);
-          if (cb > 0) {
-            if (threadIdx.x == 0) bulk_store_wait_read();
-            __syncthreads();
-          }
-          for (int i = threadIdx.x; i < rows; i += kThreads) {
-            const int s = cb + i;
-            const int e = (int)fast_div((uint32_t)s, p.fd_ns), n = s - e * Ns;
-            O *row = s_tile + (size_t)i * D;
-            if (n < p.N) {
-              const Own4<real> o = s_own[s];
-              const Msg4<real> m = s_msg[s];
-              real ratio[4] = {0, 0, 0, 0};
-              if (p.st_thermal)
-                for (int k = 0; k < 4; ++k) ratio[k] = pl.ratio[k][base + s];
-              int q = obs_own<real>(row, p, (uint32_t)o.flags, m.sso_n, Rep<real>::minus20(o.ta, o.target),
-                                    Rep<real>::minus20(o.tm, o.target), o.target - (real)20, s_env[e], ratio);
-              if (g.need_msg) {
-                RowNbrs<SMP> nbr(p, r0 + e, n, rows_draw(in));
-                for (int k = 0; k < p.nb_comm; ++k) {
-                  const int nb = nbr(p, pl.comm_table, r0 + e, n, k);
-                  const Msg4<real> mk = s_msg[e * Ns + nb];
-                  row[q++] = mk.dT; row[q++] = mk.sso_n; row[q++] = mk.p_n; row[q++] = mk.pmax_n;
-                  if (p.msg_thermal)
-                    for (int t = 0; t < 4; ++t) row[q++] = (real)pl.ratio[t][base + e * Ns + nb];
-                  if (p.msg_hvac) { row[q++] = (real)p.cop; row[q++] = (real)p.latent; row[q++] = (real)p.dcap; }
-                }
-              }
-            } else {
-              for (int q = 0; q < D; ++q) row[q] = (real)0;
-            }
-          }
-          fence_proxy_async_smem();
-          __syncthreads();
-          if (threadIdx.x == 0) {
-            bulk_store_s2g(pl.template rows<O>() + (base + cb) * D, s_tile, (uint32_t)((size_t)rows * D * sizeof(O)));
-            store_pending = true;
-          }
         }
       }
     }

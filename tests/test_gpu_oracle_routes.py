@@ -1,11 +1,11 @@
 """Every step-kernel route, and the in-kernel step loop, against the fp64 NumPy oracle.
 
 The step has one specification, ``oracle/np_oracle.py``, and many implementations; the host picks one from the
-shape and the configuration (``plan_fused``, ``launch_tile``, ``launch_tma``, ``small_handle`` and the ``taped``
-condition of ``drsim_run_tape`` in ``drsim_api.cu``).  Each case below names the kernel it means to run and fails if
-the planner stops sending it there: ``fused_info()`` gives the variant and the clusters per tile, ``launch_count``
-the launches per step, and where the ABI says nothing (which ``k_fused_tma<MODE>`` specialisation, ``k_small``) the
-test restates the host condition and the case table states the expected outcome.
+shape and the configuration (``plan_fused`` and ``step_route`` in ``drsim_api.cu``).  The routes: the four-kernel
+path (``k_house`` + ``k_reduce`` + ``k_env`` + ``k_obs``), ``k_shard``, chunked ``k_fused``, ``k_fused_direct``,
+``k_fused_tma<0|1|2>``, ``k_fused_rows<staged|unstaged>``, ``k_small`` and ``k_small_gen<double>``.  Each case below
+names the route it means to run and fails if the host stops sending it there: ``last_route`` gives the kernels the
+step ran on, ``fused_info()`` the tile variant and the clusters per tile, ``launch_count`` the launches per step.
 
 * ``test_route_matches_oracle``: a mode matrix over the routes (a covering design, not the full product), 24 steps
   re-anchored on the oracle at every step, and the same steps free-running.
@@ -56,79 +56,37 @@ def config(n, pen="individual_L2", sig="perlin", state="none", msg="none", nb="n
     return prop(n, **over)
 
 
-def dims(p, layout):
-    """(own columns, message columns, row width, messages in the rows?) as ``fill_params`` / ``plan_fused`` derive them."""
-    from marl_demandresponse_b200.core import comm_width
-    from marl_demandresponse_b200.properties import as_props
-
-    sp, mp = p["state_prop"], p["cluster_prop"]["message_prop"]
-    own = 10 + 2 * sp["hvac"] + sp["solar_gain"] + 5 * sp["thermal"]
-    msg = 4 + 4 * mp["thermal"] + 3 * mp["hvac"]
-    c = comm_width(as_props(p))
-    D = {"none": 0, "tarmac": own, "hand_engineered": own + c * msg}[layout]
-    return own, msg, D, layout == "hand_engineered" and c > 0
-
-
-def tma_mode(p, layout, e):
-    """The ``k_fused_tma`` specialisation ``launch_tma`` picks for a scheduled step (no injected noise) with external
-    actions: 1 = plain rows without messages, one cluster per tile, individual penalty; 2 = plain rows with messages,
-    several clusters per tile, individual penalty; 0 = everything else."""
-    own, msg, D, need_msg = dims(p, layout)
-    plain = own == 10 and msg == 4 and D % 2 == 0 and D > 0
-    common = plain and p["reward_prop"]["penalty_props"]["mode"] == "individual_L2"
-    if common and not need_msg and e == 1:
-        return 1
-    if common and need_msg and e > 1:
-        return 2
-    return 0
-
-
-def small_fp32(sim, p, layout):
-    """``small_handle``: clusters of at most 32 plane slots in at most 256 replicas, plain columns."""
-    own, msg, D, need_msg = dims(p, layout)
-    if sim.real != np.float32 or sim.fused_info()["variant"] == "none" or sim.Ns > 32 or sim.R > 256:
-        return False
-    if D == 0:
-        return True
-    if own != 10 or D % 2:
-        return False
-    return msg == 4 if need_msg else D == 10
-
-
-def small_fp64(sim):
-    """``small64_handle``: the fp64 build's ``k_small_gen`` takes any observation options."""
-    return sim.real == np.float64 and sim.fused_info()["variant"] != "none" and sim.Ns <= 32 and sim.R <= 256
-
-
 # route -> (precision, R, N, layout, path, environment, expected)
-#   expected: variant = fused_info()["variant"]; e = clusters per tile; launches = kernel launches per step;
-#   mode = k_fused_tma<MODE> (restated from launch_tma); small = k_small / k_small_gen (restated from small_handle)
+#   expected: route = last_route after a step; variant = fused_info()["variant"]; e = clusters per tile;
+#   launches = kernel launches per step
 ROUTES = {
-    "k_fused_tma<1>": ("f32", 12, 1000, "tarmac", "auto", {}, dict(variant="staged", e=1, launches=1, mode=1)),
+    "k_fused_tma<1>": ("f32", 12, 1000, "tarmac", "auto", {}, dict(route="k_fused_tma<1>", variant="staged", e=1, launches=1)),
     "k_fused_tma<2>": ("f32", 30, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 3},
-                       dict(variant="staged", e=3, launches=1, mode=2)),
+                       dict(route="k_fused_tma<2>", variant="staged", e=3, launches=1)),
     "k_fused_tma<0>/1-per-tile": ("f32", 9, 300, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 1},
-                                  dict(variant="staged", e=1, launches=1, mode=0)),
+                                  dict(route="k_fused_tma<0>", variant="staged", e=1, launches=1)),
     "k_fused_tma<0>/3-per-tile": ("f32", 30, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 3},
-                                  dict(variant="staged", e=3, launches=1, mode=0)),
+                                  dict(route="k_fused_tma<0>", variant="staged", e=3, launches=1)),
     "k_fused_rows<staged>": ("f32", 60, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 7},
-                             dict(variant="staged_rows", e=7, launches=1)),
-    "k_fused_rows<unstaged>": ("f32", 6, 1000, "hand_engineered", "auto", {}, dict(variant="staged_rows", e=1, launches=1)),
+                             dict(route="k_fused_rows<staged>", variant="staged_rows", e=7, launches=1)),
+    "k_fused_rows<unstaged>": ("f32", 6, 1000, "hand_engineered", "auto", {},
+                               dict(route="k_fused_rows<unstaged>", variant="staged_rows", e=1, launches=1)),
     "general/rows-fallback": ("f32", 60, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 7},
-                              dict(variant="staged_rows", e=7, launches=4)),
-    "k_fused/chunked": ("f32", 3, 1000, "hand_engineered", "auto", {}, dict(variant="chunked", e=1, launches=1)),
+                              dict(route="four-kernel", variant="staged_rows", e=7, launches=4)),
+    "k_fused/chunked": ("f32", 3, 1000, "hand_engineered", "auto", {}, dict(route="k_fused", variant="chunked", e=1, launches=1)),
     # 85 clusters per tile: their schedule records do not fit next to the TMA planes (rows of at most 16 columns)
     "k_fused_direct": ("f32", 300, 10, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 85},
-                       dict(variant="direct", e=85, launches=1, small=False)),
-    "k_small": ("f32", 7, 10, "hand_engineered", "auto", {}, dict(launches=1, small=True)),
-    "k_shard": ("f32", 2, 2500, "hand_engineered", "auto", {}, dict(variant="none", launches=1)),
+                       dict(route="k_fused_direct", variant="direct", e=85, launches=1)),
+    "k_small": ("f32", 7, 10, "hand_engineered", "auto", {}, dict(route="k_small", launches=1)),
+    "k_shard": ("f32", 2, 2500, "hand_engineered", "auto", {}, dict(route="k_shard", variant="none", launches=1)),
     "four-kernel": ("f32", 24, 100, "hand_engineered", "split", {"DRSIM_NO_SHARD_KERNEL": 1},
-                    dict(variant="none", launches=4)),
+                    dict(route="four-kernel", variant="none", launches=4)),
     "k_fused_direct<double>": ("f64", 24, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 2},
-                               dict(variant="direct", e=2, launches=1)),
-    "k_fused<double>/chunked": ("f64", 3, 1000, "hand_engineered", "auto", {}, dict(variant="chunked", e=1, launches=1)),
-    "k_small_gen<double>": ("f64", 7, 10, "hand_engineered", "auto", {}, dict(launches=1, small=True)),
-    "k_shard<double>": ("f64", 3, 1300, "hand_engineered", "auto", {}, dict(variant="none", launches=1)),
+                               dict(route="k_fused_direct", variant="direct", e=2, launches=1)),
+    "k_fused<double>/chunked": ("f64", 3, 1000, "hand_engineered", "auto", {},
+                                dict(route="k_fused", variant="chunked", e=1, launches=1)),
+    "k_small_gen<double>": ("f64", 7, 10, "hand_engineered", "auto", {}, dict(route="k_small_gen", launches=1)),
+    "k_shard<double>": ("f64", 3, 1300, "hand_engineered", "auto", {}, dict(route="k_shard", variant="none", launches=1)),
 }
 
 # the mode matrix: every value of every axis on every route that can take it, plus penalty x clusters per tile
@@ -237,11 +195,6 @@ def _make(route, cell, monkeypatch, seed=21):
         assert info["variant"] == expect["variant"], (route, info)
     if "e" in expect:
         assert info["envs_per_tile"] == expect["e"], (route, info)
-    if "mode" in expect:
-        assert tma_mode(p, layout, info["envs_per_tile"]) == expect["mode"], (route, dims(p, layout))
-    if "small" in expect:
-        small = small_fp32(env.sim, p, layout) if precision == "f32" else small_fp64(env.sim)
-        assert small == expect["small"], (route, info, dims(p, layout))
     st = synthetic_state(p, R, seed=seed + 1)
     env.reset(copy.deepcopy(st))
     return env, p, st, expect
@@ -256,11 +209,47 @@ def test_route_matches_oracle(route, i, monkeypatch):
     drv = OracleDriver(env, p, st)
     drv.start_free()
     acts = (np.random.default_rng(100 + i).random((T_STEPS, R, N)) < 0.5).astype(np.uint8)
-    launches = [drv.step(acts[t]) for t in range(T_STEPS)]
+    launches = [drv.step(acts[0])]
+    assert env.sim.last_route == expect["route"], (route, MATRIX[route][i], env.sim.fused_info())
+    launches += [drv.step(acts[t]) for t in range(1, T_STEPS)]
     # the first step generates the 64-step schedule block (two kernels), then one route's launches per step
     assert launches == [expect["launches"] + 2] + [expect["launches"]] * (T_STEPS - 1), launches
     drv.check_metrics()
     drv.check_free()
+
+
+@pytest.mark.parametrize("clear", ["set_state", "reset"])
+@pytest.mark.parametrize("route", ["k_fused_tma<1>", "k_small", "k_small_gen<double>"])
+def test_common_lockout_durations_restore_the_planned_route(route, clear, monkeypatch):
+    """Per-house lock-out durations that differ take the general path; once they are common again (``set_state`` at
+    the common duration, or a device reset) the handle is back on its planned route, with the bits of a fresh handle
+    in the same state."""
+    import torch
+
+    env, p, st, expect = _make(route, MATRIX[route][0], monkeypatch)
+    R, N = env.n_replicas, env.n_houses
+    info = env.sim.fused_info()
+    dur = int(env.sim.cfg.lockout_duration)
+    rng = np.random.default_rng(3)
+    mixed = np.full((R, N), dur, dtype=np.int32)
+    mixed[:, ::2] = 2 * dur
+    env.set_state({"lockout_duration": mixed})
+    env.step(torch.as_tensor((rng.random((R, N)) < 0.5).astype(np.uint8), device="cuda"))
+    assert env.sim.last_route in ("k_shard", "four-kernel"), env.sim.last_route
+    assert env.sim.fused_info()["variant"] == "none"
+    if clear == "set_state":
+        env.set_state({"lockout_duration": np.full((R, N), dur, dtype=np.int32)})
+    else:
+        env.reset(device_mode="synthetic")
+    assert env.sim.fused_info() == info
+    fresh = copy.deepcopy(env)
+    for t in range(3):
+        acts = torch.as_tensor((rng.random((R, N)) < 0.5).astype(np.uint8), device="cuda")
+        env.step(acts)
+        fresh.step(acts)
+        torch.cuda.synchronize()
+        assert env.sim.last_route == fresh.sim.last_route == expect["route"], (t, env.sim.last_route)
+        same_state(env, fresh)
 
 
 SWEEP_SEEDS = list(range(20))
@@ -312,32 +301,36 @@ def _loop_launches(first_step, T, block_base):
 
 # route, R, N, layout, environment, cell, steps before the run, run length, expected (fp32: the loop is fp32 only)
 LOOP_CASES = [
-    ("k_small", 7, 10, "hand_engineered", {}, dict(c=9), 0, 70, dict(small=True)),
+    ("k_small", 7, 10, "hand_engineered", {}, dict(c=9), 0, 70, dict()),
     ("k_small", 7, 10, "hand_engineered", {}, dict(pen="common_max_error", nb="closed_groups", c=4, sig="sinusoidals"), 5, 100,
-     dict(small=True)),
+     dict()),
     ("k_small", 5, 10, "hand_engineered", {}, dict(pen="mixture", nb="random_fixed", c=3, sig="flat",
-                                                   start="2021-12-31T23:58:20"), 0, 70, dict(small=True)),
+                                                   start="2021-12-31T23:58:20"), 0, 70, dict()),
     ("k_fused_tma<1>", 400, 1000, "tarmac", {}, dict(sig="perlin", start="2021-06-15T23:58:20"), 0, 70,
-     dict(variant="staged", e=1, mode=1)),
-    ("k_fused_tma<1>", 640, 1000, "tarmac", {}, dict(sig="sinusoidals"), 5, 100, dict(variant="staged", e=1, mode=1)),
+     dict(variant="staged", e=1)),
+    ("k_fused_tma<1>", 640, 1000, "tarmac", {}, dict(sig="sinusoidals"), 5, 100, dict(variant="staged", e=1)),
     ("k_fused_tma<2>", 1800, 100, "hand_engineered", {"DRSIM_TILE_ENVS": 3}, dict(c=2, sig="regular_steps", nb="random_fixed",
                                                                                  start="2021-12-31T23:58:20"), 0, 70,
-     dict(variant="staged", e=3, mode=2)),
+     dict(variant="staged", e=3)),
     ("k_fused_tma<0>", 400, 1000, "tarmac", {}, dict(pen="common_L2", state="solar", start="2021-12-31T23:58:20"), 0, 70,
-     dict(variant="staged", e=1, mode=0)),
+     dict(variant="staged", e=1)),
     ("k_fused_tma<0>", 300, 300, "hand_engineered", {"DRSIM_TILE_ENVS": 1},
      dict(pen="common_max_error", state="solar", msg="th_hvac", nb="closed_groups", c=3, sig="sinusoidals"), 5, 100,
-     dict(variant="staged", e=1, mode=0)),
+     dict(variant="staged", e=1)),
     ("k_fused_tma<0>", 1800, 100, "hand_engineered", {"DRSIM_TILE_ENVS": 3},
      dict(pen="mixture", state="all", nb="neighbours_2D", sig="perlin", start="2021-06-15T23:58:20"), 0, 70,
-     dict(variant="staged", e=3, mode=0)),
+     dict(variant="staged", e=3)),
     ("k_fused_tma<0>", 6100, 100, "tarmac", {}, dict(pen="common_max_error", sig="flat"), 5, 100,
-     dict(variant="staged", mode=0)),
+     dict(variant="staged")),
     ("k_fused_rows", 4096, 100, "hand_engineered", {}, dict(c=10, sig="sinusoidals", start="2021-06-15T23:58:20"), 0, 70,
      dict(variant="staged_rows")),
     ("k_fused_rows", 4096, 100, "hand_engineered", {}, dict(c=10, nb="random_fixed", sig="perlin"), 5, 100,
      dict(variant="staged_rows")),
 ]
+
+
+# the loop takes k_fused_rows in its staged variant only
+LOOP_ROUTE = {"k_fused_rows": "k_fused_rows<staged>"}
 
 
 @pytest.mark.parametrize("route,R,N,layout,env_vars,cell,pre,T,expect",
@@ -361,10 +354,6 @@ def test_in_kernel_loop_matches_oracle(route, R, N, layout, env_vars, cell, pre,
     for k in ("variant", "e"):
         if k in expect:
             assert info[{"e": "envs_per_tile"}.get(k, k)] == expect[k], info
-    if "mode" in expect:
-        assert tma_mode(p, layout, info["envs_per_tile"]) == expect["mode"], dims(p, layout)
-    if "small" in expect:
-        assert small_fp32(env.sim, p, layout) == expect["small"], info
     if route == "k_fused_rows":   # the loop takes k_fused_rows on at least two tiles per CTA (the `taped` condition)
         assert (min(info["grid"], info["tiles"] // 2)) * 10 >= info["grid"] * 9, info
     start = _dt.datetime.fromisoformat(cell["start"]) if "start" in cell else None
@@ -382,6 +371,7 @@ def test_in_kernel_loop_matches_oracle(route, R, N, layout, env_vars, cell, pre,
     l0 = env.sim.launch_count
     env.run(T, tape, rotate=True)
     torch.cuda.synchronize()
+    assert env.sim.last_route == LOOP_ROUTE.get(route, route), (env.sim.last_route, info)
     # (the first of the steps before the run generated the block that starts at step 0; set_state invalidates it)
     assert env.sim.launch_count - l0 == _loop_launches(pre, T, 0 if pre else None), (env.sim.launch_count - l0, pre, T)
     monkeypatch.setenv("DRSIM_NO_STREAM", "1")
