@@ -62,7 +62,8 @@ enum { DRSIM_COMM_RING = 0, DRSIM_COMM_TABLE = 1, DRSIM_COMM_SAMPLE = 2 };
 /* where per-step noise comes from when the matching pointer of drsim_step_args is NULL */
 enum { DRSIM_NOISE_ZERO = 0, DRSIM_NOISE_PHILOX = 1 };
 /* action source: caller-provided, or restated controllers
- * (controllers/bangbang_controllers.py:18-89, greedy_myopic_controller.py:67-104) */
+ * (controllers/bangbang_controllers.py:18-89, greedy_myopic_controller.py:67-104).  Greedy-myopic sorts the whole
+ * cluster in shared memory: replicas only (a house-sharded handle rejects it) and n_house <= 8192. */
 enum {
   DRSIM_POLICY_EXTERNAL = 0,
   DRSIM_POLICY_DEADBAND_BANGBANG = 1,

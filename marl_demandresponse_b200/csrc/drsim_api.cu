@@ -230,6 +230,11 @@ static int fill_params(const drsim_config &c, SimParams &p, std::string &why) {
           "modes and `random_sample` are replicas only), and every shard must hold at least nb_comm houses";
     return -1;
   }
+  if (c.policy == DRSIM_POLICY_GREEDY_MYOPIC && p.N != p.n_global) {
+    why = "policy = DRSIM_POLICY_GREEDY_MYOPIC on a house-sharded cluster: the greedy scan sorts the whole cluster "
+          "against its signal, so it runs on replicas only (n_house_local == n_house_global)";
+    return -1;
+  }
   if (p.comm_mode == DRSIM_COMM_SAMPLE && (p.nb_comm > DRSIM_MAX_SAMPLE_COMM || p.nb_comm > p.n_global - 1)) {
     why = "comm_mode = DRSIM_COMM_SAMPLE (`random_sample`) needs nb_comm <= min(n_house - 1, DRSIM_MAX_SAMPLE_COMM = " +
           std::to_string(DRSIM_MAX_SAMPLE_COMM) + "), got " + std::to_string(p.nb_comm);
@@ -394,9 +399,13 @@ static int configure_step_kernels(drsim_handle *h, int &per_sm) {
   if (obs_smem > 48 * 1024)
     CU_TRY(cudaFuncSetAttribute(k_obs<real, O, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)obs_smem));
   if (h->p.policy == DRSIM_POLICY_GREEDY_MYOPIC) {
+    constexpr int kGreedySmem = 200 * 1024;
     const size_t sm = (size_t)greedy_n2(h->p) * 24;
-    if (sm > 200 * 1024) return fail(DRSIM_E_ARG, "greedy-myopic: cluster too large for the shared-memory sort");
-    if (sm > 48 * 1024) CU_TRY(cudaFuncSetAttribute(k_greedy<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    if (sm > kGreedySmem) return fail(DRSIM_E_ARG, "greedy-myopic: cluster too large for the shared-memory sort");
+    // the cap, whatever this handle's size: the attribute belongs to the kernel, so a smaller handle created later must
+    // not lower it under a larger one's launch; and the kernel's static shared memory counts against the 48 KB default
+    // too (2048 slots = exactly 48 KB of dynamic memory does not launch without the attribute)
+    CU_TRY(cudaFuncSetAttribute(k_greedy<real>, cudaFuncAttributeMaxDynamicSharedMemorySize, kGreedySmem));
   }
   return 0;
 }

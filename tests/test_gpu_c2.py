@@ -123,3 +123,32 @@ def test_c2_fp32_on_the_oracle_action_tape():
     np.testing.assert_allclose(got["power"], s["power"], rtol=1e-6)
     np.testing.assert_allclose(env.reward.double().cpu().numpy(), rew, rtol=1e-5, atol=1e-5 * 2)
     np.testing.assert_allclose(env.obs.double().cpu().numpy(), orc.obs_vectors(), rtol=1e-5, atol=1e-5)
+
+
+def test_c2_fp32_greedy_on_the_device():
+    """The production fp32 build with greedy-myopic on the device, as benchmarked.  Every step the action plane
+    ``k_greedy`` wrote is the restated greedy on the device's own inputs (fp32 deviation from the set-point as the key,
+    capacities, lock-out bits, the signal before the step), and the discrete state is those actions through the lock-out
+    state machine.  The continuous state under these actions is ``test_c2_fp32_on_the_oracle_action_tape``'s."""
+    from marl_demandresponse_b200 import BatchedEnv
+    from marl_demandresponse_b200.batched import synthetic_state
+    from oracle.np_oracle import hvac_fsm
+    from oracle_driver import check_greedy_plane, controller_actions, controller_inputs
+
+    prop, table = _prop(), _table()
+    st = synthetic_state(prop, R, seed=21)
+    env = BatchedEnv(prop, R, precision="f32", policy="greedy_myopic", noise="philox", seed=SEED, interp_table=table)
+    env.reset(copy.deepcopy(st))
+    s = env.get_state(["on", "lockout", "sso"])
+    on, lock, sso = s["on"], s["lockout"], s["sso"]
+    n_on = []
+    for t in range(T):
+        want = controller_actions("greedy_myopic", 0.0, 2.5, **controller_inputs(env))
+        env.step(None)
+        check_greedy_plane(env, want, f"step {t}")
+        on, lock, sso = hvac_fsm(on, lock, sso, want, 4, 40)
+        got = env.get_state(["on", "lockout", "sso"])
+        for k, v in (("on", on), ("lockout", lock), ("sso", sso)):
+            assert np.array_equal(got[k].astype(np.int64), v.astype(np.int64)), (t, k)
+        n_on.append(int(want.sum()))
+    assert 0 < min(n_on) and max(n_on) < N, (min(n_on), max(n_on))   # the signal splits the cluster every step

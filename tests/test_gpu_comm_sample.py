@@ -12,8 +12,8 @@ import numpy as np
 import pytest
 
 import comm_sample_np
-from oracle_driver import OracleDriver, same_state
-from test_gpu_oracle_routes import LOOP_ROUTE, ROUTES, T_STEPS, _loop_launches, config
+from oracle_driver import ROUTES, OracleDriver, config, loop_launches, same_state
+from test_gpu_oracle_routes import LOOP_ROUTE, T_STEPS
 
 pytestmark = pytest.mark.gpu
 
@@ -229,7 +229,7 @@ def test_in_kernel_loop(route, R, N, env_vars, cell, pre, T, monkeypatch):
     env.run(T, tape, rotate=True)
     torch.cuda.synchronize()
     assert env.sim.last_route == LOOP_ROUTE.get(route, route), (env.sim.last_route, info)
-    assert env.sim.launch_count - l0 == _loop_launches(pre, T, 0 if pre else None)
+    assert env.sim.launch_count - l0 == loop_launches(pre, T, 0 if pre else None)
     monkeypatch.setenv("DRSIM_NO_STREAM", "1")
     twin.run(T, tape, rotate=True)
     monkeypatch.delenv("DRSIM_NO_STREAM")

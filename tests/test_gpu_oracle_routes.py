@@ -21,73 +21,11 @@ import os
 import numpy as np
 import pytest
 
-from oracle_driver import OracleDriver, prop, same_state
+from oracle_driver import NB_2D, ROUTES, OracleDriver, config, loop_launches, same_state
 
 pytestmark = pytest.mark.gpu
 
 T_STEPS = 24   # a 40 s lock-out is 10 steps of 4 s: lock-outs expire and re-arm within the run
-
-# neighbours_2D: N -> (row_size, max_communication_distance); the table is 2 d (d + 1) wide
-NB_2D = {12: (4, 1), 100: (10, 1), 300: (15, 1), 1000: (25, 2), 1300: (26, 2), 2500: (50, 2)}
-
-
-def config(n, pen="individual_L2", sig="perlin", state="none", msg="none", nb="neighbours", c=10, start=None, dist=None,
-           **extra):
-    """Properties of one matrix cell.  The deadband keeps ``common_max_error`` non-zero and the lock-out FSM busy."""
-    over = {"cluster_prop/house_prop/deadband": 0.4,
-            "reward_prop/penalty_props/mode": pen,
-            "reward_prop/penalty_props/alpha_common_max": 1.0,
-            "power_grid_prop/signal_properties/mode": sig,
-            "state_prop/solar_gain": state in ("solar", "all"),
-            "state_prop/thermal": state == "all",
-            "state_prop/hvac": state == "all",
-            "cluster_prop/message_prop/thermal": msg == "th_hvac",
-            "cluster_prop/message_prop/hvac": msg == "th_hvac",
-            "cluster_prop/agents_comm_prop/mode": nb,
-            "cluster_prop/agents_comm_prop/max_nb_agents_communication": c}
-    if nb == "neighbours_2D":
-        row, d = NB_2D[n]
-        dist = d if dist is None else dist
-        over["cluster_prop/agents_comm_prop/row_size"] = row
-        over["cluster_prop/agents_comm_prop/max_communication_distance"] = dist
-    if start is not None:
-        over["start_datetime"] = start
-    over.update(extra)
-    return prop(n, **over)
-
-
-# route -> (precision, R, N, layout, path, environment, expected)
-#   expected: route = last_route after a step; variant = fused_info()["variant"]; e = clusters per tile;
-#   launches = kernel launches per step
-ROUTES = {
-    "k_fused_tma<1>": ("f32", 12, 1000, "tarmac", "auto", {}, dict(route="k_fused_tma<1>", variant="staged", e=1, launches=1)),
-    "k_fused_tma<2>": ("f32", 30, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 3},
-                       dict(route="k_fused_tma<2>", variant="staged", e=3, launches=1)),
-    "k_fused_tma<0>/1-per-tile": ("f32", 9, 300, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 1},
-                                  dict(route="k_fused_tma<0>", variant="staged", e=1, launches=1)),
-    "k_fused_tma<0>/3-per-tile": ("f32", 30, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 3},
-                                  dict(route="k_fused_tma<0>", variant="staged", e=3, launches=1)),
-    "k_fused_rows<staged>": ("f32", 60, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 7},
-                             dict(route="k_fused_rows<staged>", variant="staged_rows", e=7, launches=1)),
-    "k_fused_rows<unstaged>": ("f32", 6, 1000, "hand_engineered", "auto", {},
-                               dict(route="k_fused_rows<unstaged>", variant="staged_rows", e=1, launches=1)),
-    "general/rows-fallback": ("f32", 60, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 7},
-                              dict(route="four-kernel", variant="staged_rows", e=7, launches=4)),
-    "k_fused/chunked": ("f32", 3, 1000, "hand_engineered", "auto", {}, dict(route="k_fused", variant="chunked", e=1, launches=1)),
-    # 85 clusters per tile: their schedule records do not fit next to the TMA planes (rows of at most 16 columns)
-    "k_fused_direct": ("f32", 300, 10, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 85},
-                       dict(route="k_fused_direct", variant="direct", e=85, launches=1)),
-    "k_small": ("f32", 7, 10, "hand_engineered", "auto", {}, dict(route="k_small", launches=1)),
-    "k_shard": ("f32", 2, 2500, "hand_engineered", "auto", {}, dict(route="k_shard", variant="none", launches=1)),
-    "four-kernel": ("f32", 24, 100, "hand_engineered", "split", {"DRSIM_NO_SHARD_KERNEL": 1},
-                    dict(route="four-kernel", variant="none", launches=4)),
-    "k_fused_direct<double>": ("f64", 24, 100, "hand_engineered", "auto", {"DRSIM_TILE_ENVS": 2},
-                               dict(route="k_fused_direct", variant="direct", e=2, launches=1)),
-    "k_fused<double>/chunked": ("f64", 3, 1000, "hand_engineered", "auto", {},
-                                dict(route="k_fused", variant="chunked", e=1, launches=1)),
-    "k_small_gen<double>": ("f64", 7, 10, "hand_engineered", "auto", {}, dict(route="k_small_gen", launches=1)),
-    "k_shard<double>": ("f64", 3, 1300, "hand_engineered", "auto", {}, dict(route="k_shard", variant="none", launches=1)),
-}
 
 # the mode matrix: every value of every axis on every route that can take it, plus penalty x clusters per tile
 # (the k_fused_tma<0> routes with one and three clusters per tile), flags x odd D and neighbour mode x clusters per tile.
@@ -287,18 +225,6 @@ def test_seeded_sweep_matches_oracle(seed):
     drv.check_metrics()
 
 
-def _loop_launches(first_step, T, block_base):
-    """Launches of ``drsim_run_tape`` on a loop route: one step kernel per 64-step schedule block, plus the two schedule
-    kernels when the run enters a block that has not been generated (``block_base`` = start of the current block)."""
-    n, s, base = 0, first_step, block_base
-    while s < first_step + T:
-        if base is None or not base <= s < base + 64:
-            base, n = s, n + 2
-        k = min(first_step + T - s, base + 64 - s)
-        n, s = n + 1, s + k
-    return n
-
-
 # route, R, N, layout, environment, cell, steps before the run, run length, expected (fp32: the loop is fp32 only)
 LOOP_CASES = [
     ("k_small", 7, 10, "hand_engineered", {}, dict(c=9), 0, 70, dict()),
@@ -373,7 +299,7 @@ def test_in_kernel_loop_matches_oracle(route, R, N, layout, env_vars, cell, pre,
     torch.cuda.synchronize()
     assert env.sim.last_route == LOOP_ROUTE.get(route, route), (env.sim.last_route, info)
     # (the first of the steps before the run generated the block that starts at step 0; set_state invalidates it)
-    assert env.sim.launch_count - l0 == _loop_launches(pre, T, 0 if pre else None), (env.sim.launch_count - l0, pre, T)
+    assert env.sim.launch_count - l0 == loop_launches(pre, T, 0 if pre else None), (env.sim.launch_count - l0, pre, T)
     monkeypatch.setenv("DRSIM_NO_STREAM", "1")
     twin.run(T, tape, rotate=True)
     monkeypatch.delenv("DRSIM_NO_STREAM")

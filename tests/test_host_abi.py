@@ -47,6 +47,21 @@ def test_create_fails_loudly_without_gpu_or_on_bad_config():
         assert rc != 0 and not h.value, "must not fall back to a CPU path"
 
 
+def test_house_sharded_greedy_myopic_is_refused():
+    """Greedy-myopic sorts the whole cluster against the cluster's signal: a handle holding part of the houses refuses
+    it before it looks for a device (each shard would fill the whole signal on its own)."""
+    from marl_demandresponse_b200 import flatten_config
+
+    L = _lib.lib()
+    h = C.c_void_p()
+    p = {"cluster_prop": {"nb_agents": 64}}
+    cfg = flatten_config(p, 2, "f32", "tarmac", policy="greedy_myopic", path="split", house_offset=32, n_house_local=32)
+    assert cfg.policy == _lib.POLICY["greedy_myopic"]
+    rc = L.drsim_create(C.byref(cfg), 0, C.byref(h))
+    msg = L.drsim_last_error().decode()
+    assert rc == -1 and not h.value and "house-sharded cluster: the greedy scan sorts the whole cluster" in msg, (rc, msg)
+
+
 def _epochs():
     rng = np.random.default_rng(3)
     base = np_oracle.to_epoch(dt.datetime(2019, 1, 1))
