@@ -1016,7 +1016,7 @@ static bool small_cluster(const drsim_handle *h) {
   return msgs ? (p.msg_dim == 4 && p.obs_dim == 10 + 4 * p.nb_comm) : p.obs_dim == 10;
 }
 
-// The tile kernel plan_fused chose.  k_fused_tma is specialised by the step: MODE 1 = plain rows without messages, one
+// The tile kernel plan_fused chose.  k_fused_tma is specialised by the step: MODE 1 = plain 10-column rows without messages, one
 // cluster per tile; MODE 2 = plain rows with messages, several clusters per tile (both for scheduled steps with external
 // actions and the individual penalty); MODE 0 = everything else.
 static StepRoute tile_route(const drsim_handle *h, bool scheduled) {
@@ -1026,7 +1026,7 @@ static StepRoute tile_route(const drsim_handle *h, bool scheduled) {
   if (!g.use_tma) return h->fused_direct ? StepRoute::FusedDirect : StepRoute::FusedChunked;
   const bool plain = p.own_dim == 10 && p.msg_dim == 4 && (p.obs_dim % 2) == 0 && p.obs_dim > 0;
   const bool common = plain && scheduled && p.policy == DRSIM_POLICY_EXTERNAL && p.penalty_mode == DRSIM_PEN_INDIVIDUAL_L2;
-  if (common && !g.need_msg && g.envs_per_tile == 1) return StepRoute::Tma1;
+  if (common && !g.need_msg && g.envs_per_tile == 1 && p.obs_dim == 10) return StepRoute::Tma1;
   if (common && g.need_msg && g.envs_per_tile > 1) return StepRoute::Tma2;
   return StepRoute::Tma0;
 }
@@ -2042,6 +2042,23 @@ extern "C" int drsim_debug_shard_times(drsim_t *h, unsigned long long *host_out,
   const int n = std::min(max_ctas, h->shard_grid);
   cudaMemcpy(host_out, h->shard_dbg, (size_t)n * 128, cudaMemcpyDeviceToHost);
   return n;
+}
+
+// diagnostics, not part of the documented ABI: per-warp phase cycles of the k_fused_tma step loop [cta][warp][kTilePhases]
+// (house update, own rows, barrier wait, fold + reward, row store, epilogue, tile-steps), summed over the launches since
+// the last reset.  Returns the number of CTA slots copied; 0 unless the library was built with -DDRSIM_TILE_DBG.
+extern "C" int drsim_debug_tile_phases(unsigned long long *host_out, int max_ctas, int reset) {
+#ifdef DRSIM_TILE_DBG
+  const int n = std::min(max_ctas, kTileDbgCtas);
+  if (host_out && n > 0 && cudaMemcpyFromSymbol(host_out, g_tile_dbg, (size_t)n * sizeof(g_tile_dbg[0])) != cudaSuccess) return 0;
+  void *dev = nullptr;
+  if (reset && (cudaGetSymbolAddress(&dev, g_tile_dbg) != cudaSuccess || cudaMemset(dev, 0, sizeof(g_tile_dbg)) != cudaSuccess))
+    return 0;
+  return n;
+#else
+  (void)host_out; (void)max_ctas; (void)reset;
+  return 0;
+#endif
 }
 
 // diagnostics, not part of the documented ABI: clock64 stamps [tile < 8][producer, consumer, MMA warp][16] of CTA 0 of the

@@ -2039,6 +2039,35 @@ DRSIM_D void env_stage_store(const Planes<real> &pl, const SimParams &p, int r, 
 
 constexpr int kInPlanes = 12;  // fp32 planes staged by TMA: Ta, Tm, sso, target, cap, 6 coefficients (+1 spare)
 
+// Phase counters of the k_fused_tma step loop (build with -DDRSIM_TILE_DBG, read by drsim_debug_tile_phases and
+// profiles/tools/tile_phases.py): every warp accumulates the clock() cycles of each phase of a tile-step over the
+// launch, and lane 0 adds them to g_tile_dbg[cta][warp][phase].  In the default build the marks compile to nothing.
+enum TilePhase { kPhHouse, kPhRows, kPhBarrier, kPhFold, kPhStore, kPhEpilogue, kPhSteps, kTilePhases = 8 };
+#ifdef DRSIM_TILE_DBG
+constexpr int kTileDbgCtas = 1024;
+__device__ unsigned long long g_tile_dbg[kTileDbgCtas][kThreads / 32][kTilePhases];
+struct TileClock {   // 32-bit counters (a launch is a few million cycles per warp): few registers in the debug build
+  unsigned t, acc[kTilePhases];
+  DRSIM_D TileClock() : t((unsigned)clock()) {
+#pragma unroll
+    for (int k = 0; k < kTilePhases; ++k) acc[k] = 0;
+  }
+  DRSIM_D void mark(int k) { const unsigned n = (unsigned)clock(); acc[k] += n - t; t = n; }
+  DRSIM_D void step() { ++acc[kPhSteps]; }
+  DRSIM_D void flush() {
+    if ((threadIdx.x & 31) == 0 && blockIdx.x < kTileDbgCtas)
+#pragma unroll
+      for (int k = 0; k < kTilePhases; ++k) atomicAdd(&g_tile_dbg[blockIdx.x][threadIdx.x >> 5][k], (unsigned long long)acc[k]);
+  }
+};
+#else
+struct TileClock {
+  DRSIM_D void mark(int) {}
+  DRSIM_D void step() {}
+  DRSIM_D void flush() {}
+};
+#endif
+
 // ------------------------------------------------------------------------------------------
 // Fused path, fp32 production kernel with TMA-staged inputs.
 //
@@ -2097,6 +2126,68 @@ DRSIM_D uint32_t act_word_polled(const uint8_t *actions, size_t off, uint32_t st
   return v;
 }
 
+// Observation rows of MODE 1 of k_fused_tma (plain 10-column rows, no messages).  A thread's four rows are contiguous in
+// the tile's staging rows: 160 bytes in fp32, 80 in bf16.  Before the tile barrier the thread writes all of them with
+// 16-byte stores, the power / signal columns (4, 5) as zeros; after the fold own_rows10_patch puts those two columns
+// into the valid rows.  fp32: at a 160-byte lane stride lanes t and t + 4 of a quarter-warp would hit the same banks, so
+// lanes with bit 2 set assemble their houses in the order 2, 3, 0, 1: their k-th store lands 80 bytes (20 banks) away
+// from that of lane t and each 16-byte store takes one wavefront per quarter-warp.  bf16 needs no swap: an 80-byte
+// lane stride already puts the eight lanes of a quarter-warp on distinct banks.
+template <typename O>
+DRSIM_D void own_rows10(O *rows, const House4<float> &h, const SimParams &p, int lane) {
+  const int sw = (sizeof(O) == 4 && (lane & 4)) ? 2 : 0;
+  float v[40];
+#pragma unroll
+  for (int jv = 0; jv < 4; ++jv) {   // row jv of the thread's store order holds house jv ^ sw
+    const int j = jv ^ sw;
+    const float ta = sw ? h.ta[jv ^ 2] : h.ta[jv];
+    const float tm = sw ? h.tm[jv ^ 2] : h.tm[jv];
+    const float target = sw ? h.target[jv ^ 2] : h.target[jv];
+    const int sso = sw ? h.sso[jv ^ 2] : h.sso[jv];
+    const uint32_t f = (h.flags >> (8 * j)) & 0xffu;
+    const float sso_n = (float)fast_div((uint32_t)sso, p.fd_dur);            // norm.py:40-43, :79-82
+    const bool ok = j < h.valid;
+    const float tg = target - 20.f;
+    float *r = v + 10 * jv;
+    r[0] = ok ? (float)(f & 1u) : 0.f;
+    r[1] = ok ? (float)((f >> 1) & 1u) : 0.f;
+    r[2] = ok ? sso_n : 0.f;
+    r[3] = ok ? 1.f : 0.f;
+    r[4] = 0.f;
+    r[5] = 0.f;
+    r[6] = ok ? p.hf.deadband : 0.f;
+    r[7] = ok ? (ta + tg) * 0.2f : 0.f;
+    r[8] = ok ? (tm + tg) * 0.2f : 0.f;
+    r[9] = ok ? tg * 0.2f : 0.f;
+  }
+  if constexpr (sizeof(O) == 4) {
+    float4 *dst = reinterpret_cast<float4 *>(rows);
+#pragma unroll
+    for (int k = 0; k < 10; ++k)
+      dst[k < 5 ? k + 5 * (sw >> 1) : k - 5 * (sw >> 1)] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
+  } else {
+    auto pk = [&](int i) {
+      const __nv_bfloat162 b = __floats2bfloat162_rn(v[i], v[i + 1]);
+      return *reinterpret_cast<const uint32_t *>(&b);
+    };
+    uint4 *dst = reinterpret_cast<uint4 *>(rows);
+#pragma unroll
+    for (int k = 0; k < 5; ++k) dst[k] = make_uint4(pk(8 * k), pk(8 * k + 2), pk(8 * k + 4), pk(8 * k + 6));
+  }
+}
+
+// columns 4, 5 of the thread's valid rows.  The k-th store goes to row (k + lane / 4) % 4 (fp32: 8-byte stores, taken by
+// half-warps) or (k + lane / 8) % 4 (bf16: 4-byte stores), which spreads each store over all 32 banks.
+template <typename O>
+DRSIM_D void own_rows10_patch(O *rows, int valid, int lane, float power_n, float signal_n) {
+  const int rot = sizeof(O) == 4 ? lane >> 2 : lane >> 3;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const int j = (k + rot) & 3;
+    if (j < valid) put2(rows + 10 * j, 2, power_n, signal_n);
+  }
+}
+
 // POLL = copy-engine mode of drsim_step_host (StepIn::act_poll_err): a separate instantiation, so the
 // device-resident step does not carry the branch (measured: 0.6 us of 39 on C4)
 template <int MODE, bool POLL = false, typename O = float, bool SMP = false>
@@ -2115,7 +2206,7 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
   float *s_in = reinterpret_cast<float *>(smem_raw + g.off_in);        // [kInPlanes][kTileSlots]
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int Ns = p.Ns, D = p.obs_dim;
+  const int Ns = p.Ns, D = MODE == 1 ? 10 : p.obs_dim;   // MODE 1 runs on 10-column rows only (tile_route)
   const int tile_slots = g.envs_per_tile * Ns;
   const KC<real> kc(p);
   const bool fast = MODE ? true : in.sched_od != nullptr;
@@ -2193,6 +2284,7 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
     if (fast) fetch_env(blockIdx.x, 0);
   }
 
+  TileClock clk;
   // Tile-major step loop: a tile runs through all n_steps steps before the CTA moves to its next tile.
   // Between two steps of a tile the thread's updated state goes back into its own staging slots, the static
   // planes stay there, the next step's action word, (od, solar) pair and schedule record are fetched while
@@ -2260,11 +2352,15 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
       reinterpret_cast<int4 *>(s_in)[(size_t)2 * (kTileSlots / 4) + threadIdx.x] = make_int4(h.sso[0], h.sso[1], h.sso[2], h.sso[3]);
       s_flags[threadIdx.x] = h.flags;
     }
+    clk.mark(kPhHouse);
     // the previous tile's row store must have drained the warp's staging rows before they are rewritten
     // (waited for here, after the house update, not at the top of the tile)
     if (lane == 0 && store_pending) bulk_store_wait_read();
     __syncwarp();
-    if (active) {
+    clk.mark(kPhStore);
+    if (MODE == 1 && active) {
+      own_rows10(s_tile + (size_t)s0 * 10, h, p, lane);
+    } else if (active) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         const uint32_t f = (h.flags >> (8 * j)) & 0xffu;
@@ -2337,8 +2433,10 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
         for (int k = 0; k < kRed; ++k) dst[k] = (double)red[k];
       }
     }
+    clk.mark(kPhRows);
     if (fast && threadIdx.x < E) cp_async_wait_all();  // this tile's records (issued a whole tile ago) are in s_stage
     __syncthreads();
+    clk.mark(kPhBarrier);
     // every warp is past the previous tile's phase 3: the other parity of s_stage is free again
     if (fast) {
       if (more) {
@@ -2422,7 +2520,10 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
         if (j >= h.valid) rw[j] = 0.f;
       }
       st4_hint(pl.reward + base + s0, rw, pol_stream);
-      if (D > 0) {
+      clk.mark(kPhFold);
+      if (MODE == 1) {
+        own_rows10_patch(s_tile + (size_t)s0 * 10, h.valid, lane, e.power_n, e.signal_n);
+      } else if (D > 0) {
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           if (j < h.valid) {
@@ -2469,6 +2570,7 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
         store_pending = true;
       }
     }
+    clk.mark(kPhStore);
     // off the critical path: env planes + running metrics of cluster threadIdx.x
     if (threadIdx.x < E && fast) {
       double a[kRed] = {0, 0, 0, 0, 0};
@@ -2476,9 +2578,12 @@ k_fused_tma(Planes<float> pl, SimParams p, StepIn in, FusedGeom g) {
       double *m_next = more ? (s_stage_base + (size_t)(parity ^ 1) * g.envs_per_tile + threadIdx.x)->m : nullptr;
       env_stage_store<real>(pl, p, r0 + threadIdx.x, s_stage[threadIdx.x], a, in.host_env, m_next);
     }
+    clk.mark(kPhEpilogue);
+    clk.step();
   }
   // shared memory must outlive the reads of the last row store; its global writes complete with the grid
   if (lane == 0 && store_pending) bulk_store_wait_read();
+  clk.flush();
 }
 
 // ------------------------------------------------------------------------------------------
