@@ -2015,7 +2015,8 @@ static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t see
     a.K2 = (a.h1 + 1 + 7) / 8 * 8; a.N2 = (a.h2 + 1 + 15) / 16 * 16;
     a.K3 = (a.h2 + 1 + 7) / 8 * 8;
     if (a.N1 + a.N2 + kActN3 > 256)
-      return fail(DRSIM_E_ARG, "drsim_policy_step: h1 + h2 too wide for two tile slots in tensor memory (<= 111 each, 224 together)");
+      return fail(DRSIM_E_ARG, "drsim_policy_step: h1 + h2 too wide for two tile slots in tensor memory (N1 + N2 + 16 <= 256 "
+                               "columns, N1 = h1 + 1 and N2 = h2 + 1 each rounded up to 16)");
     a.off_w1 = take(a.N1 * a.K1 * 4); a.off_w2 = take(a.N2 * a.K2 * 4);
     a.off_vec = take(kActN3 * a.K3 * 4);          // output-layer operand
     a.off_a1 = take(2 * kActRows * a.K1 * 4);     // two tile slots: observation operand (canonical layout)

@@ -33,7 +33,12 @@ class RolloutBuffer:
         R, N, Ns, D = sim.R, sim.N, sim.Ns, sim.D
         self.R, self.N, self.Ns, self.D = R, N, Ns, D
         dev = f"cuda:{sim.device}"
-        self.obs = torch.zeros((self.T + 1, R, Ns, D), dtype=torch.bfloat16 if sim.obs_bf16 else torch.float32, device=dev)
+        # obs[t] is one contiguous plane; the transition needs each plane on a 16-byte boundary, which a bf16 plane of
+        # odd width (R Ns D 2 bytes) does not keep by itself: planes are spaced by a stride padded to 16 bytes
+        dtype, per16 = (torch.bfloat16, 8) if sim.obs_bf16 else (torch.float32, 4)
+        stride = (R * Ns * D + per16 - 1) // per16 * per16
+        flat = torch.zeros((self.T + 1) * stride, dtype=dtype, device=dev)
+        self.obs = flat.as_strided((self.T + 1, R, Ns, D), (stride, Ns * D, D, 1))
         self.actions = torch.zeros((self.T, R, Ns), dtype=torch.uint8, device=dev)
         self.probs = torch.zeros((self.T, R, Ns), dtype=torch.float32, device=dev)
         self.rewards = torch.zeros((self.T, R, Ns), dtype=torch.float32, device=dev)

@@ -300,7 +300,7 @@ def _torch_actor(D, h1, h2, seed):
 
 @pytest.mark.parametrize("R,n,layout,h1,h2,nb_comm", [
     (300, 100, "hand_engineered", 100, 100, 10), (7, 1000, "tarmac", 100, 100, 10), (33, 37, "hand_engineered", 64, 48, 10),
-    (5, 9, "tarmac", 111, 96, 10),                      # widest layers that fit the tensor memory (no spare columns)
+    (5, 9, "tarmac", 111, 96, 10),                      # wide layers: 240 of the 256 TMEM columns of a k_actor2 tile slot
     (520, 100, "hand_engineered", 100, 100, 10),        # three tiles per CTA: every pipeline slot is recycled
     (1100, 100, "tarmac", 32, 16, 10),                  # narrow layers: a single chunk, nothing through the spare columns
     (40, 100, "hand_engineered", 100, 100, 3),          # D = 22: the 4-chunk instantiation of the row handling

@@ -27,8 +27,14 @@ def _actor(D, seed=3):
     return fc
 
 
-@pytest.mark.parametrize("R,n,layout", [(64, 100, "hand_engineered"), (5, 1000, "tarmac"), (9, 37, "hand_engineered"), (3, 2500, "tarmac")])
-def test_collect_equals_policy_step_plus_step(R, n, layout):
+@pytest.mark.parametrize("R,n,layout,state_prop,obs_dtype", [
+    pytest.param(64, 100, "hand_engineered", {}, "float32", id="64-100-hand_engineered"),
+    pytest.param(5, 1000, "tarmac", {}, "float32", id="5-1000-tarmac"),
+    pytest.param(9, 37, "hand_engineered", {}, "float32", id="9-37-hand_engineered"),
+    pytest.param(3, 2500, "tarmac", {}, "float32", id="3-2500-tarmac"),
+    # bf16 rows of odd width (D = 11): one plane is 6600 bytes, off the 16-byte grid the transition needs
+    pytest.param(3, 100, "tarmac", {"solar_gain": True}, "bfloat16", id="3-100-tarmac-solar-bfloat16")])
+def test_collect_equals_policy_step_plus_step(R, n, layout, state_prop, obs_dtype):
     import torch
 
     from marl_demandresponse_b200 import BatchedEnv
@@ -36,15 +42,16 @@ def test_collect_equals_policy_step_plus_step(R, n, layout):
     from marl_demandresponse_b200.rollout import RolloutBuffer
 
     T = 7
-    prop = _prop(n)
+    prop = {**_prop(n), "state_prop": state_prop}
     st = synthetic_state(prop, R, seed=4)
-    a = BatchedEnv(prop, R, obs_layout=layout, noise="philox", seed=17)
-    b = BatchedEnv(prop, R, obs_layout=layout, noise="philox", seed=17)
+    a = BatchedEnv(prop, R, obs_layout=layout, noise="philox", seed=17, obs_dtype=obs_dtype)
+    b = BatchedEnv(prop, R, obs_layout=layout, noise="philox", seed=17, obs_dtype=obs_dtype)
     a.reset(copy.deepcopy(st))
     b.reset(copy.deepcopy(st))
     weights = BatchedEnv.actor_weights(_actor(a.sim.D))
     buf = RolloutBuffer(a, T)
     a.collect(weights, buf, done_last=True)
+    assert all(buf.obs[t].is_contiguous() and buf.obs[t].data_ptr() % 16 == 0 for t in range(T + 1))
     states, actions, probs, rewards = [], [], [], []
     for t in range(T):
         states.append(b.obs.clone())
