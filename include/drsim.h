@@ -199,7 +199,11 @@ typedef struct drsim_ptrs {
 
 #define DRSIM_N_ACC 6 /* P, sum pen/N, max pen, sum dT, sum dT^2, interpolated base-power sum */
 
-#define DRSIM_N_METRICS 6 /* steps, sum reward/N, sum |Ta-target|/N, sum (Ta-target)^2/N, sum |P-S|, sum (P-S)^2 */
+/* Running metrics, summed over steps per replica.  Each step adds: 1, sum_i reward_i / N, |sum_i (Ta_i - target_i)| / N
+ * (the absolute value of the mean offset), sum_i (Ta_i - target_i)^2 / N, |P - S_old|, (P - S_old)^2; Ta after the step,
+ * P the cluster power after it, S_old the regulation signal before it, i over the N houses of the whole cluster.
+ * drsim_reset zeroes them; drsim_set_state leaves them alone. */
+#define DRSIM_N_METRICS 6
 
 /* Per-step inputs, all DEVICE pointers; NULL selects the handle's own source. */
 typedef struct drsim_step_args {

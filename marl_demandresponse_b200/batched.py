@@ -138,7 +138,8 @@ class BatchedEnv:
         """Inject ``state`` (default: the seeded synthetic state), compute the first regulation
         signal (``PowerGrid.step`` at reset, environment.py:66-68) and return the observations.
         ``device_mode`` = "reference" | "synthetic" draws the state on the GPU instead
-        (``drsim_reset``: the reference's reset distributions from Philox streams)."""
+        (``drsim_reset``: the reference's reset distributions from Philox streams).  Either way a new episode
+        begins: the running metrics (``metrics``) start again from zero."""
         if device_mode is not None:
             self.sim.reset_device(self.props, self.seed if seed is None else seed, device_mode, quirk_ua)
             self.sim.refresh(True)
@@ -146,10 +147,12 @@ class BatchedEnv:
         if state is None:
             state = synthetic_state(self.props, self.n_replicas, self.seed if seed is None else seed, self.rep_offset)
         self.sim.set_state(state)
+        self._v["metrics"].zero_()   # on the current stream, like drsim_reset
         self.sim.refresh(True)
         return self.obs
 
     def set_state(self, state: Dict[str, np.ndarray]) -> None:
+        """Overwrite the given planes (restoring a state mid-episode): the running metrics keep counting."""
         self.sim.set_state(state)
 
     def get_state(self, keys=None) -> Dict[str, np.ndarray]:

@@ -7,6 +7,9 @@ from typing import Dict
 
 from . import _lib
 
+# the running sums of BatchedEnv.metrics; each step adds 1, mean_i reward_i, |sum_i (Ta_i - target_i)| / N,
+# sum_i (Ta_i - target_i)^2 / N, |P - S_old| and (P - S_old)^2 (Ta and cluster power P after the step, S_old the
+# regulation signal before it)
 METRIC_NAMES = ("steps", "sum_mean_reward", "sum_abs_mean_temp_offset", "sum_mean_sq_temp_error",
                 "sum_abs_signal_error", "sum_sq_signal_error")
 
@@ -21,7 +24,11 @@ def replica_shard(n_replicas_total: int, rank: int, world: int):
 
 def reduce_rollout_metrics(metrics, group=None) -> Dict[str, float]:
     """``metrics``: this rank's ``[R_local, N_METRICS]`` running sums (``BatchedEnv.metrics``).
-    Returns the job-wide per-replica-step averages (identical on every rank)."""
+    Returns the job-wide per-replica-step averages (identical on every rank).
+
+    Made for replica-sharded runs, where each rank holds different replicas.  On a house-sharded cluster
+    (``ShardedClusterEnv``) every rank holds the same whole-cluster rows: the averages still come out right, but
+    ``replicas`` and ``replica_steps`` are ``world`` times too large."""
     import torch
     import torch.distributed as dist
 

@@ -93,7 +93,8 @@ class ShardedClusterEnv:
             dist.barrier(group=group)
 
     def reset(self, state: Optional[Dict[str, np.ndarray]] = None, seed: int = 1234):
-        """``state``: full-cluster state dict (every rank passes the same one) or None = synthetic."""
+        """``state``: full-cluster state dict (every rank passes the same one) or None = synthetic.  A new episode
+        begins: the running metrics (``state["metrics"]``) start again from zero."""
         if state is None:
             state = synthetic_state(self.props, self.sim.R, seed)
         local = {}
@@ -101,6 +102,7 @@ class ShardedClusterEnv:
             v = np.asarray(v)
             local[k] = v[:, self.lo:self.hi] if v.ndim == 2 else v
         self.sim.set_state(local)
+        self._v["metrics"].zero_()   # on the current stream, like drsim_reset
         return self
 
     def step(self, actions=None):

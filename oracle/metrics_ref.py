@@ -51,3 +51,51 @@ class RefMetrics:
         return {"rmse_sig_per_ag": float(np.sqrt(self.v["cumul_squared_error_sig"] / d) / self.n),
                 "rmse_temp": float(np.sqrt(self.v["cumul_squared_error_temp"] / (d * self.n))),
                 "rms_max_error_temp": float(np.sqrt(self.v["cumul_squared_max_error_temp"] / d))}
+
+
+# Metrics.reset (:222-235) zeroes these and leaves the squared sums alone
+RESET_FIELDS = [f for f in FIELDS if f not in ("cumul_squared_error_temp", "cumul_squared_error_sig",
+                                               "cumul_squared_max_error_temp")]
+
+
+class BatchedRefMetrics:
+    """``RefMetrics`` of R clusters at once: the same expressions in the same order of updates, with the per-house
+    loop of ``update`` as fp64 sums over the house axis of ``[R, N]`` arrays.  ``values`` is ``[R, 12]`` in the order
+    of ``FIELDS``."""
+
+    def __init__(self, n_replicas: int, nb_agents: int, start_stats_from: int = 0):
+        self.n = int(nb_agents)
+        self.start = int(start_stats_from)
+        self.values = np.zeros((int(n_replicas), len(FIELDS)))
+
+    def update(self, t_air_next, target, rewards, signal_old, power_new, od_old, power_old, time_step: int) -> None:
+        """``t_air_next, target, rewards``: ``[R, N]`` after the step; ``signal_old, od_old, power_old``: ``[R]``, the
+        observation BEFORE the step; ``power_new``: ``[R]``, cluster power after it (see ``RefMetrics.update``)."""
+        v, n = self.values, self.n
+        ix = FIELDS.index
+        temp_error = np.asarray(t_air_next, dtype=np.float64) - np.asarray(target, dtype=np.float64) / n
+        v[:, ix("cumul_temp_offset")] += temp_error.sum(axis=1)
+        v[:, ix("cumul_temp_error")] += np.abs(temp_error).sum(axis=1)
+        v[:, ix("max_temp_error")] = np.maximum(v[:, ix("max_temp_error")], temp_error.max(axis=1))
+        v[:, ix("cumul_avg_reward")] += (np.asarray(rewards, dtype=np.float64) / n).sum(axis=1)
+        if time_step >= self.start:
+            v[:, ix("cumul_squared_error_temp")] += (temp_error ** 2).sum(axis=1)
+        signal_error = (np.asarray(signal_old, dtype=np.float64) - np.asarray(power_new, dtype=np.float64)) / (n ** 2)
+        v[:, ix("cumul_signal_offset")] += n * signal_error
+        v[:, ix("cumul_signal_error")] += n * np.abs(signal_error)
+        v[:, ix("cumul_OD_temp")] += od_old
+        v[:, ix("cumul_signal")] += signal_old
+        v[:, ix("cumul_cons")] += power_old
+        if time_step >= self.start:
+            v[:, ix("cumul_squared_error_sig")] += np.asarray(signal_old, dtype=np.float64) ** 2
+            v[:, ix("cumul_squared_max_error_temp")] = v[:, ix("max_temp_error")] ** 2
+
+    def reset(self) -> None:                                                   # :222-235
+        self.values[:, [FIELDS.index(f) for f in RESET_FIELDS]] = 0.0
+
+    def rms(self, time_step: int) -> dict:
+        d = time_step - self.start
+        v, ix = self.values, FIELDS.index
+        return {"rmse_sig_per_ag": np.sqrt(v[:, ix("cumul_squared_error_sig")] / d) / self.n,
+                "rmse_temp": np.sqrt(v[:, ix("cumul_squared_error_temp")] / (d * self.n)),
+                "rms_max_error_temp": np.sqrt(v[:, ix("cumul_squared_max_error_temp")] / d)}

@@ -18,8 +18,17 @@ follows from them (1e-6 relative: an fp32 sum of up to 1000 terms).
 Outdoor temperature, signal and base power are fp64 env scalars in both builds: 1e-9 relative.  Temperatures: one
 fp32 step of the difference-form update is at rounding level, 4e-6 absolute (``test_per_step_error_fp32_is_at_rounding
 _level``); free-running fp32 trajectories get the 2e-4 drift allowance of the batched oracle tests; the fp64 build
-replays the reference's literal arithmetic, 1e-9.  Rewards, observations and the running metrics: the BASELINE.json
-north star, rtol 1e-5 of (|value| + natural scale 1) in fp32, and 1e-9 of the same in fp64.
+replays the reference's literal arithmetic, 1e-9.  Rewards and observations: the BASELINE.json north star, rtol 1e-5
+of (|value| + natural scale 1) in fp32, and 1e-9 of the same in fp64.
+
+Running metrics (the six sums of ``DRSIM_N_METRICS``).  Every checked step's increment is compared on ALL replicas
+with ``metric_increments`` of the device's own planes before and after the step, and on the picked replicas with the
+oracle's post-step state; ``check_metrics`` / ``check_free`` compare the sums since the start with the oracle's
+increments, summed.  The step count is exact; the mean reward takes the reward tolerance; sum |d| / N and sum d^2 / N
+take rtol 1e-5 of those natural scales in fp32 (fp32 sums over at most one tile), plus the temperature tolerance
+propagated against the oracle; |P - S_old| takes the power tolerance of P, and (P - S_old)^2 that error propagated.
+fp64: 1e-9 of the same scales against the oracle, 1e-12 against the device's own planes.  Each comparison also allows
+the rounding of the two readings of the running sums it differences (``check_metric_delta``).
 """
 from __future__ import annotations
 
@@ -204,6 +213,62 @@ def oracle_run(env_prop, st, actions, od, pe):
     return orc, np.array(rew)
 
 
+# ---- running metrics ---------------------------------------------------------------------------
+def step_planes(env):
+    """What the running metrics of one step are made of, read from the device after the step: the deviation ``d`` =
+    Ta - target (fp32: the deviation plane; fp64: ``t_air - target``) and ``reward`` ``[R, N]``, cluster ``power`` and
+    ``signal`` ``[R]``; fp64 host arrays."""
+    import torch
+
+    torch.cuda.synchronize()
+    v = env.state
+    f64 = lambda t: t.double().cpu().numpy()   # noqa: E731
+    d = f64(v["dt_air"]) if v["temp_is_deviation"] else f64(v["t_air"]) - f64(v["target"])
+    return dict(d=d, reward=f64(v["reward"]), power=f64(v["power"]), signal=f64(v["signal"]))
+
+
+def metric_increments(signal_before, after):
+    """fp64 restatement of what one step adds to each replica's six running sums (``DRSIM_N_METRICS``): ``[R, 6]`` =
+    ``[1, mean_i reward_i, |sum_i d_i| / N, sum_i d_i^2 / N, |P - S_old|, (P - S_old)^2]`` with ``d`` and the reward
+    after the step over the N real houses (``after`` as :func:`step_planes` returns it), ``P`` the cluster power after
+    the step and ``S_old`` = ``signal_before`` ``[R]``, the regulation signal the step's reward was charged against."""
+    d = np.asarray(after["d"], dtype=np.float64)
+    n = d.shape[1]
+    ps = np.asarray(after["power"], dtype=np.float64) - np.asarray(signal_before, dtype=np.float64)
+    return np.stack([np.ones(d.shape[0]), np.asarray(after["reward"], dtype=np.float64).mean(axis=1),
+                     np.abs(d.sum(axis=1)) / n, (d * d).sum(axis=1) / n, np.abs(ps), ps * ps], axis=1)
+
+
+def metric_tolerance(signal_before, after, rel, p_rel, temp=0.0, s_rel=0.0, rew_rel=None):
+    """``[R, 6]`` allowed error of :func:`metric_increments`: field 0 exact; the reward mean ``rew_rel`` (default
+    ``rel``) of (mean |reward| + 1); the deviation sums ``rel`` of their natural scales sum |d| / N and sum d^2 / N, plus
+    a temperature error ``temp`` per house propagated; |P - S_old| a relative error ``p_rel`` of P (and ``s_rel`` of
+    S_old), and its square that error propagated."""
+    d = np.asarray(after["d"], dtype=np.float64)
+    P = np.abs(np.asarray(after["power"], dtype=np.float64))
+    abs_ps = np.abs(P - np.asarray(signal_before, dtype=np.float64))
+    mean_abs_d = np.abs(d).mean(axis=1)
+    dp = p_rel * P + s_rel * np.abs(signal_before)
+    rew_rel = rel if rew_rel is None else rew_rel
+    return np.stack([np.zeros(d.shape[0]), rew_rel * (np.abs(after["reward"]).mean(axis=1) + 1.0),
+                     rel * mean_abs_d + temp, rel * (d * d).mean(axis=1) + 2.0 * temp * mean_abs_d + temp * temp,
+                     dp, 2.0 * abs_ps * dp + dp * dp], axis=1)
+
+
+def check_metric_delta(delta, want, tol, what, rows=None, sums=None, n_terms=1):
+    """``delta`` (device) against ``want`` (restated) ``[R, 6]``, within ``tol``; field 0 exactly.  ``delta`` is the
+    difference of two readings of the running sums ``sums = (m_before, m_after)``: it and the ``n_terms`` additions it
+    spans round at the ulp of those sums (the whole error when the increment is exact, e.g. |P - S_old| of a cluster
+    with every HVAC off, P = 0)."""
+    rows = list(range(delta.shape[0])) if rows is None else list(rows)
+    assert np.array_equal(delta[:, 0], want[:, 0]), f"{what}: metric steps {delta[:, 0]} != {want[:, 0]}"
+    if sums is not None:
+        tol = tol + (n_terms + 2) * np.finfo(np.float64).eps * (np.abs(sums[0]) + np.abs(sums[1]))
+    bad = np.argwhere(~(np.abs(delta - want) <= tol))
+    assert bad.size == 0, (f"{what}: running metrics differ at (replica, field) "
+                           f"{[(rows[i], int(f), float(delta[i, f]), float(want[i, f])) for i, f in bad[:6]]}")
+
+
 def pick_replicas(R, envs_per_tile):
     """First replica, last replica (ragged last tile) and one in the middle of a multi-cluster tile."""
     e = max(1, envs_per_tile)
@@ -213,9 +278,17 @@ def pick_replicas(R, envs_per_tile):
 
 
 def tolerances(precision, anchored):
+    """``temp``: absolute temperature error; ``rel``: rewards, observations, metrics; ``power``: relative error of the
+    cluster power against the oracle."""
     if precision == "f64":
-        return {"temp": 1e-9, "rel": 1e-9}
-    return {"temp": 4e-6 if anchored else 2e-4, "rel": 1e-5}
+        return {"temp": 1e-9, "rel": 1e-9, "power": 1e-9}
+    return {"temp": 4e-6 if anchored else 2e-4, "rel": 1e-5, "power": 1e-6}
+
+
+def own_plane_tolerance(precision):
+    """(rel, p_rel) of the running metrics against :func:`metric_increments` of the device's own planes: fp32 sums over
+    at most one tile in fp32; fp64 the same values summed in another order."""
+    return (1e-12, 1e-12) if precision == "f64" else (1e-5, 1e-6)
 
 
 class OracleDriver:
@@ -243,7 +316,8 @@ class OracleDriver:
         self.disc = {k: s[k].astype(np.int64) for k in ("on", "lockout", "sso")}
         self.epoch = s["epoch"].astype(np.int64)
         self.metrics0 = env.metrics.double().cpu().numpy().copy()
-        self.rew_sum = np.zeros(len(self.picks))
+        self.inc_sum = np.zeros((len(self.picks), 6))   # the oracle's metric increments and their tolerances, summed
+        self.inc_tol = np.zeros((len(self.picks), 6))
         self.n_steps = 0
         self.free = None
 
@@ -334,6 +408,7 @@ class OracleDriver:
         import torch
 
         before = self.env.get_state() if check else None
+        m_before = self.env.metrics.double().cpu().numpy() if check else None
         on_device = acts is None
         if on_device:
             acts = self._controller(controller_inputs(self.env))
@@ -354,20 +429,39 @@ class OracleDriver:
             od, pe = self._noise(self.step_index, self.epoch[self.picks])
             rew_ref = orc.step(acts[self.picks], od, pe)
             self._check_picked(got, orc, rew, rew_ref, obs, True, what)
-            self.rew_sum += rew_ref.mean(axis=1)
-            self._rew_scale = getattr(self, "_rew_scale", 0.0) + np.abs(rew_ref).mean(axis=1) + 1.0
+            self._check_step_metrics(before["signal"], m_before, orc.state, rew_ref, what)
         self.step_index += 1
         self.n_steps += 1
         return launches
 
+    def _check_step_metrics(self, signal_before, m_before, s, rew_ref, what):
+        """What the step added to the running metrics: on every replica against :func:`metric_increments` of the
+        device's own planes, on the picked replicas against the oracle's post-step state ``s``."""
+        m_after = self.env.metrics.double().cpu().numpy()
+        delta = m_after - m_before
+        after = step_planes(self.env)
+        rel, p_rel = own_plane_tolerance(self.precision)
+        tol = tolerances(self.precision, True)
+        check_metric_delta(delta, metric_increments(signal_before, after),
+                           metric_tolerance(signal_before, after, rel, p_rel, rew_rel=tol["rel"]), f"{what}: own planes",
+                           sums=(m_before, m_after))
+        pk = self.picks
+        o_after = dict(d=s["t_air"] - s["target"], reward=rew_ref, power=s["power"])
+        want = metric_increments(signal_before[pk], o_after)
+        o_tol = metric_tolerance(signal_before[pk], o_after, tol["rel"], tol["power"], tol["temp"])
+        check_metric_delta(delta[pk], want, o_tol, f"{what}: oracle", pk, sums=(m_before[pk], m_after[pk]))
+        self.inc_sum += want
+        self.inc_tol += o_tol
+
     def check_metrics(self):
-        """Running metrics since the driver started: the step count exactly (all replicas), the sum of the mean
-        rewards on the picked replicas (the per-step reward tolerance, summed)."""
-        m = self.env.metrics.double().cpu().numpy() - self.metrics0
+        """Running metrics since the driver started: the step count exactly (all replicas), all six sums on the picked
+        replicas against the oracle's increments (their per-step tolerances, summed)."""
+        now = self.env.metrics.double().cpu().numpy()
+        m = now - self.metrics0
         assert np.all(m[:, 0] == self.n_steps), m[:, 0]
-        rel = tolerances(self.precision, True)["rel"]
-        err = np.abs(m[self.picks, 1] - self.rew_sum)
-        assert np.all(err <= rel * self._rew_scale), (m[self.picks, 1], self.rew_sum)
+        pk = self.picks
+        check_metric_delta(m[pk], self.inc_sum, self.inc_tol, "running metrics since the start", pk,
+                           sums=(self.metrics0[pk], now[pk]), n_terms=self.n_steps)
 
     # ---- free-running -------------------------------------------------------------------------
     def start_free(self):
@@ -375,15 +469,20 @@ class OracleDriver:
         self.free = self._oracle(self.env.get_state())
         self.free_metrics0 = self.env.metrics.double().cpu().numpy().copy()
         self.free_rew = None
-        self.free_rew_sum = np.zeros(len(self.picks))
-        self.free_rew_scale = np.zeros(len(self.picks))
+        self.free_inc = np.zeros((len(self.picks), 6))   # the free oracle's metric increments and tolerances, summed
+        self.free_tol = np.zeros((len(self.picks), 6))
         self.free_steps = 0
 
     def _advance_free_one(self, acts_picked):
         od, pe = self._noise(self.step_index, self.epoch[self.picks])
+        signal_before = np.array(self.free.state["signal"], dtype=np.float64)
         self.free_rew = self.free.step(acts_picked, od, pe)
-        self.free_rew_sum += self.free_rew.mean(axis=1)
-        self.free_rew_scale += np.abs(self.free_rew).mean(axis=1) + 1.0
+        s = self.free.state
+        after = dict(d=s["t_air"] - s["target"], reward=self.free_rew, power=s["power"])
+        tol = tolerances(self.precision, False)
+        self.free_inc += metric_increments(signal_before, after)
+        # the free oracle's signal is compared to 1e-9 relative, its temperatures with the drift allowance
+        self.free_tol += metric_tolerance(signal_before, after, tol["rel"], tol["power"], tol["temp"], s_rel=1e-9)
         self.free_steps += 1
 
     def advance_free(self, acts):
@@ -397,11 +496,12 @@ class OracleDriver:
         got, rew, obs = self._gpu()
         self._check_all_replicas(got, what)
         self._check_picked(got, self.free, rew, self.free_rew, obs, False, what)
-        m = self.env.metrics.double().cpu().numpy() - self.free_metrics0
+        now = self.env.metrics.double().cpu().numpy()
+        m = now - self.free_metrics0
         assert np.all(m[:, 0] == self.free_steps), m[:, 0]
-        rel = tolerances(self.precision, False)["rel"]
-        err = np.abs(m[self.picks, 1] - self.free_rew_sum)
-        assert np.all(err <= rel * self.free_rew_scale), (what, m[self.picks, 1], self.free_rew_sum)
+        pk = self.picks
+        check_metric_delta(m[pk], self.free_inc, self.free_tol, f"{what}: running metrics", pk,
+                           sums=(self.free_metrics0[pk], now[pk]), n_terms=self.free_steps)
 
 
 def same_state(a, b):

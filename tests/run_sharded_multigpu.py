@@ -39,7 +39,8 @@ def main():
             torch.cuda.synchronize()
             if exchange == "peer":
                 env.sim.peer_status()
-            results[exchange] = {k: env.state[k].clone() for k in ("dt_air", "sso", "flags", "reward", "power", "signal", "obs")}
+            results[exchange] = {k: env.state[k].clone()
+                                 for k in ("dt_air", "sso", "flags", "reward", "power", "signal", "obs", "metrics")}
             # timing of the exchange variants (device events, max over ranks)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             dist.barrier(); torch.cuda.synchronize()
@@ -70,6 +71,12 @@ def main():
         torch.testing.assert_close(ws["reward"][:, lo:hi], results["peer"]["reward"], rtol=1e-6, atol=1e-7)
         # observation rows, including the neighbour messages that cross the shard edges
         torch.testing.assert_close(ws["obs"][:, lo:hi], results["peer"]["obs"], rtol=1e-6, atol=1e-7)
+        # running metrics: whole-cluster sums on every rank (partials folded in another order)
+        wm, pm = ws["metrics"], results["peer"]["metrics"]
+        assert torch.equal(wm[:, 0], pm[:, 0]) and bool((wm[:, 0] == T).all()), f"{layout}: metric step counts"
+        mtol = 1e-5 * wm.abs()
+        mtol[:, 1] += 1e-5 * T
+        assert bool(((pm - wm).abs() <= mtol).all()), f"{layout}: running metrics differ from the unsharded cluster"
     dist.barrier()
     if rank == 0:
         print("sharded multi-GPU check OK", flush=True)

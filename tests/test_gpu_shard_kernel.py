@@ -150,8 +150,17 @@ def _sharded_vs_whole(layout, base_mode, W, n, R, T, no_shard_kernel=False, rese
         for p_ in parts:
             p_.sim.peer_status()
         ws = whole.state
+        wm = ws["metrics"].cpu().numpy()
+        # every reset starts the running metrics from zero: one episode's steps, whole-cluster sums on every shard
+        # (folded in another order: fp32 tolerance of the summed values, the reward sum also of 1 per step)
+        assert np.all(wm[:, 0] == T), (episode, wm[:, 0])
+        mtol = 1e-5 * np.abs(wm)
+        mtol[:, 1] += 1e-5 * T
         for p_ in parts:
             ps = p_.state
+            pm = ps["metrics"].cpu().numpy()
+            assert np.array_equal(pm[:, 0], wm[:, 0]), (layout, base_mode, episode, p_.rank)
+            assert np.all(np.abs(pm - wm) <= mtol), (layout, base_mode, episode, p_.rank, pm, wm)
             for k in ("sso", "flags", "dt_air", "dt_mass"):
                 assert torch.equal(ws[k][:, p_.lo:p_.hi], ps[k]), (layout, base_mode, episode, k)
             for k in ("power", "signal", "od_temp", "base_power"):

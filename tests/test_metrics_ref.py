@@ -40,6 +40,43 @@ def test_restatement_matches_the_real_metrics_class(path):
         assert abs(rms[k] - v) <= 1e-12 * max(1.0, abs(v)), k
 
 
+def test_batched_restatement_matches_the_per_house_loop():
+    """``BatchedRefMetrics`` (the ``[R, N]`` form the device metrics are checked against) against ``RefMetrics``
+    cluster by cluster: random states, several clusters, squared sums collected from step 5 on, ``Metrics.reset``
+    half-way through."""
+    from oracle.metrics_ref import FIELDS, RESET_FIELDS, BatchedRefMetrics, RefMetrics
+
+    rng = np.random.default_rng(11)
+    R, N, T, start = 5, 37, 14, 5
+    bm = BatchedRefMetrics(R, N, start)
+    refs = [RefMetrics(N, start) for _ in range(R)]
+    for t in range(T):
+        if t == 8:
+            bm.reset()
+            for m in refs:
+                for f in RESET_FIELDS:
+                    m.v[f] = 0.0
+        target = 19.0 + np.abs(rng.normal(0.0, 0.5, (R, N)))
+        t_air = target + rng.uniform(-2.0, 4.0, (R, N))
+        rew = -rng.uniform(0.0, 2.0, (R, N))
+        sig, p_new, p_old = (rng.uniform(0.5, 1.5, R) * 6000.0 * N for _ in range(3))
+        od = rng.uniform(25.0, 35.0, R)
+        bm.update(t_air, target, rew, sig, p_new, od, p_old, t)
+        for r, m in enumerate(refs):
+            m.update(t_air[r], target[r], rew[r], sig[r], p_new[r], od[r], p_old[r], t)
+        want = np.array([m.row() for m in refs])
+        # offsets may cancel across steps: their scale is the matching sum of absolute values
+        scale = np.abs(want)
+        for signed, absolute in (("cumul_temp_offset", "cumul_temp_error"), ("cumul_signal_offset", "cumul_signal_error")):
+            scale[:, FIELDS.index(signed)] = want[:, FIELDS.index(absolute)]
+        err = np.abs(bm.values - want)
+        assert np.all(err <= 1e-13 * (1.0 + scale)), (t, np.argwhere(err > 1e-13 * (1.0 + scale)).tolist())
+    rms = bm.rms(T)
+    for r, m in enumerate(refs):
+        for k, v in m.rms(T).items():
+            assert abs(rms[k][r] - v) <= 1e-13 * max(1.0, abs(v)), (r, k)
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("path", FILES, ids=[os.path.basename(f)[8:-5] for f in FILES])
 def test_device_metrics_match_the_real_metrics_class(path):
