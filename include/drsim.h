@@ -384,7 +384,16 @@ typedef struct drsim_actor_net {
   int32_t h1, h2;       /* 1 .. 111 each */
   /* 0 = one TF32 pass per product (|dp| <= 5e-3 against an fp32 forward), 1 = "3xTF32": every operand split into
    * hi + lo TF32 halves, three tensor-core passes per product, fp32-grade probabilities (|dp| ~ 1e-6).
-   * On a handle with bfloat16 rows (DRSIM_OBS_BF16) only 1 is accepted: the 3xTF32 actor widens the rows as it loads
+   * 2 = "f16x3": the same three passes on fp16 halves (tcgen05 kind::f16, K = 16: half the tensor-core instructions of
+   * 3xTF32) -- A_hi W_hi + A_lo W_d + A_hi W_lo with A_lo = fp16((x - A_hi) 2^11), W_d = fp16(W_hi 2^-11) and the weights
+   * scaled per output neuron by an exact power of two, undone after the layer -- at the same fp32-grade accuracy.  fp16 has
+   * 11 significant bits like TF32 but a narrow range: an observation element or hidden activation of a live row with
+   * |x| >= 65520 cannot be split.  The kernel detects it and sets a flag of the handle; drsim_actor_status (which
+   * synchronises the stream) and the next drsim_policy_step / drsim_rollout_transition then fail once with DRSIM_E_STATE
+   * naming f16x3.  The actions and probabilities of every actor launch since the previous successful check are then not
+   * valid (those of the rows concerned are wrong).  fp16 operands halve the weights' shared memory, so every obs_dim <= 64
+   * and h1, h2 <= 128 is accepted.  Any other value fails with DRSIM_E_ARG.
+   * On a handle with bfloat16 rows (DRSIM_OBS_BF16) 1 and 2 are accepted: those actors widen the rows as they load
    * them, with results bit-identical to the same actor on the widened fp32 rows; 0 fails with DRSIM_E_ARG. */
   int32_t precision;
   int32_t pad_;
@@ -398,6 +407,10 @@ typedef struct drsim_actor_net {
  * the drawn action (the PPO ratio's denominator) and prob_on[R][stride] the probability of action 1. */
 int drsim_policy_step(drsim_t *h, const drsim_actor_net *net, uint64_t seed, float *prob_drawn, float *prob_on,
                       void *stream);
+
+/* Synchronises `stream` and reports (DRSIM_E_STATE, once) whether an f16x3 actor launch (precision = 2) met an operand
+ * outside the fp16 range since the last report. */
+int drsim_actor_status(drsim_t *h, void *stream);
 
 /* One transition of an MA-PPO rollout ENTIRELY on the device, stored where the caller wants it (SURVEY 8f-2):
  * MAPPO.select_actions (mappo.py:83-97) on state_t, Environment.step (environment.py:72-108) on the drawn actions and

@@ -246,7 +246,8 @@ class BatchedEnv:
         """``MAPPO.select_actions`` (mappo.py:83-97) for all ``R * N`` agents in one kernel: actor
         forward on the current observation rows (tcgen05 TF32 GEMMs), softmax, categorical draw from a
         Philox uniform keyed (seed, replica, house, step).  The drawn actions land in the action plane
-        (``state["actions"]``); returns ``(actions u8 [R,N], prob_of_drawn_action f32 [R,N] | None)``."""
+        (``state["actions"]``); returns ``(actions u8 [R,N], prob_of_drawn_action f32 [R,N] | None)``.
+        ``precision``: "tf32x3" (default), "f16x3" or "tf32", see :meth:`DrSim.policy_step`."""
         import torch
 
         sim = self.sim
@@ -260,7 +261,8 @@ class BatchedEnv:
 
     def rollout_step(self, weights, seed: Optional[int] = None, precision: str = "tf32x3"):
         """One transition of a rollout entirely on the device: actor + draw, then the environment
-        step on the drawn actions.  Returns ``(obs', reward, actions, prob_of_drawn_action)``."""
+        step on the drawn actions.  Returns ``(obs', reward, actions, prob_of_drawn_action)``.  ``precision`` as for
+        :meth:`policy_step`."""
         actions, prob = self.policy_step(weights, seed, precision=precision)
         self.sim.step(None)
         return self._v["obs"], self._v["reward"], actions, prob
@@ -268,7 +270,9 @@ class BatchedEnv:
     def collect(self, weights, buf, n_steps=None, seed: Optional[int] = None, done_last: bool = False,
                 precision: str = "tf32x3"):
         """A rollout segment entirely on the device, stored in a :class:`~.rollout.RolloutBuffer` (SURVEY 8f-2:
-        ``select_actions`` + ``env.step`` + ``store_transition`` of mappo.py:83-127 per transition, one C call)."""
+        ``select_actions`` + ``env.step`` + ``store_transition`` of mappo.py:83-127 per transition, one C call).
+        ``precision`` as for :meth:`policy_step`; with "f16x3" the segment ends with ``actor_status``, which raises if an
+        operand left the fp16 range during the segment."""
         from .rollout import collect
 
         return collect(self, weights, buf, n_steps, seed, done_last, precision=precision)

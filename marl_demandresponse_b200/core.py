@@ -497,7 +497,7 @@ class DrSim:
         _lib.check(self._L.drsim_step_host_snapshot(self._h, *args, C.byref(v), self._stream(stream)))
         return self._snapshot_arrays(v)
 
-    ACTOR_PRECISION = {"tf32": 0, "tf32x3": 1}
+    ACTOR_PRECISION = {"tf32": 0, "tf32x3": 1, "f16x3": 2}
 
     def actor_net(self, weights, precision: str = "tf32x3") -> "_lib.ActorNet":
         w1, b1, w2, b2, w3, b3 = weights
@@ -511,12 +511,19 @@ class DrSim:
         """``drsim_policy_step``: the reference's MA-PPO actor + categorical draw on the observation rows.
         ``weights`` = (w1, b1, w2, b2, w3, b3) contiguous fp32 CUDA tensors in ``torch.nn.Linear`` layout;
         ``prob_drawn`` / ``prob_on``: optional fp32 CUDA tensors ``[R, Ns]``; ``precision``: "tf32x3" (three
-        tensor-core passes per product on hi / lo operand halves: fp32-grade probabilities) or "tf32" (one pass)."""
+        tensor-core passes per product on hi / lo operand halves: fp32-grade probabilities), "f16x3" (the same three
+        passes on fp16 halves with scaled weights: fp32-grade, half the tensor-core instructions; an observation element or
+        hidden activation with |x| >= 65520 is reported by ``actor_status`` and fails the next call) or "tf32" (one pass)."""
         w1, b1, w2, b2, w3, b3 = weights
         net = self.actor_net(weights, precision)
         assert tuple(w1.shape) == (net.h1, self.D) and tuple(w2.shape) == (net.h2, net.h1) and tuple(w3.shape) == (2, net.h2)
         _lib.check(self._L.drsim_policy_step(self._h, C.byref(net), int(seed) & (2 ** 64 - 1), self._ptr(prob_drawn),
                                              self._ptr(prob_on), self._stream(stream)))
+
+    def actor_status(self, stream=None) -> None:
+        """``drsim_actor_status``: synchronise and raise if an "f16x3" actor launch met an operand outside the fp16 range
+        since the last report (its actions and probabilities are then not valid)."""
+        _lib.check(self._L.drsim_actor_status(self._h, self._stream(stream)))
 
     @property
     def launch_count(self) -> int:

@@ -17,6 +17,7 @@
 // weights are converted once per CTA; only the 128 x D observation tile moves per iteration.
 #pragma once
 
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include "drsim_device.cuh"
@@ -45,6 +46,8 @@ struct ActorArgs {
   int off_w3, w_bytes;     // k_actor3x: the fp32 output layer in the image; size of one (hi or lo) weight block
   unsigned long long seed;
   long long step, rep_offset;
+  int off_sc;              // k_actor3h: 2^-s of each layer-1 output column [N1] in the image
+  int *range_err;          // k_actor3h: mapped host flag, set when a live row's operand overflows fp16
 };
 
 // byte offset of element (row, k) of a K-major fp32 operand with `rows` rows in the canonical layout
@@ -488,6 +491,95 @@ DRSIM_D void tmem_wait_ld_dep(uint32_t r[16]) {
       a.dbg[(it * 3 + role) * 16 + (slot)] = (unsigned long long)clock64();                       \
   } while (0)
 
+// consumers of k_actor3h (warps 8-11, one thread per row): the consumer role of k_actor3x, statement for statement (kept
+// inline there so that its code stays as tuned) -- ReLU + the 2-wide output layer in plain fp32 FMAs straight from the
+// tcgen05.ld registers of the R2 slot, softmax, Philox draw
+DRSIM_D void act3_consumers(const ActorArgs &a, const unsigned char *smem, uint32_t R2, uint32_t lane_off, int n_my, int tid,
+                            int warp, uint64_t *bar2, uint64_t *r2_free, uint64_t *wbar) {
+  const int t = tid & 127, role = 1;
+  const float *w3 = reinterpret_cast<const float *>(smem + a.off_w3);   // [2][N2] zero-padded, then b3[2]
+  const int ng2 = (a.h2 + 15) >> 4;
+  if (n_my > 0) mbar_wait_bounded(wbar, 0);
+  for (int it = 0; it < n_my; ++it) {
+    const int s = it & 1;
+    const int tile = (int)blockIdx.x + it * (int)gridDim.x;
+    const uint32_t src = R2 + (uint32_t)(s * a.N2) + lane_off;
+    float acc0 = w3[2 * a.N2], acc1 = w3[2 * a.N2 + 1];
+    ACT3_STAMP(0);
+    mbar_wait_bounded(bar2 + s, (uint32_t)((it >> 1) & 1));
+    tc_fence_after();
+    ACT3_STAMP(1);
+    // rounds of two 16-column granules; the next round's loads fly under this round's arithmetic, two accumulators
+    // per logit keep the FMA chains short
+    float acc2 = 0.f, acc3 = 0.f;
+    uint32_t r[2][2][16];
+    const int nrounds = (ng2 + 1) >> 1;
+    tmem_ld16_issue(src, r[0][0]);
+    if (1 < ng2) tmem_ld16_issue(src + 16u, r[0][1]);
+#pragma unroll
+    for (int rd = 0; rd < (kAct3MaxChunks + 1); ++rd) {
+      if (rd < nrounds) {
+        const int g = 2 * rd;
+        const bool two = g + 1 < ng2;
+        tmem_wait_ld_dep(r[rd & 1][0]);
+        if (two) tmem_wait_ld_dep(r[rd & 1][1]);
+        if (rd + 1 < nrounds) {
+          tmem_ld16_issue(src + (uint32_t)(16 * g + 32), r[(rd + 1) & 1][0]);
+          if (g + 3 < ng2) tmem_ld16_issue(src + (uint32_t)(16 * g + 48), r[(rd + 1) & 1][1]);
+        } else {                   // the slot's last loads have completed: GEMM2 of tile it + 2 may overwrite it
+          tc_fence_before();
+          mbar_arrive(r2_free + s);
+          ACT3_STAMP(2);
+        }
+        const float4 *wa = reinterpret_cast<const float4 *>(w3 + 16 * g), *wb = reinterpret_cast<const float4 *>(w3 + a.N2 + 16 * g);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const float4 u = wa[q], v = wb[q];
+          const float x0 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 1]), 0.f),
+                      x2 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 3]), 0.f);
+          acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
+          acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
+        }
+        if (two) {
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            const float4 u = wa[4 + q], v = wb[4 + q];
+            const float x0 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 1]), 0.f),
+                        x2 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 3]), 0.f);
+            acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
+            acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
+          }
+        }
+      }
+    }
+    {
+      const float l0 = acc0 + acc2, l1 = acc1 + acc3;
+      const long long row = (long long)tile * kActRows + t;
+      if (row < a.rows) {
+        // replica / house of the row: 32-bit division whenever the row index allows it (the 64-bit one is ~100 instructions)
+        const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
+        const int n = (int)(row - rr * a.Ns);
+        uint8_t act = 0;
+        float p_draw = 0.f, p1 = 0.f;
+        if (n < a.N) {
+          const float m = fmaxf(l0, l1);                      // F.softmax(dim=1), network.py:34
+          const float e0 = expf(l0 - m), e1 = expf(l1 - m);
+          const float p0 = e0 / (e0 + e1);
+          p1 = e1 / (e0 + e1);
+          const U4 u = philox4x32_10(a.seed, (uint32_t)(a.rep_offset + rr), (uint32_t)n, (uint32_t)a.step, PURPOSE_POLICY);
+          const float uf = (float)(u.x >> 8) * 5.9604644775390625e-8f;   // 24 random bits: [0, 1) exactly
+          act = uf < p0 ? 0 : 1;
+          p_draw = act ? p1 : p0;
+        }
+        a.actions[row] = act;
+        if (a.prob) a.prob[row] = p_draw;
+        if (a.prob_on) a.prob_on[row] = p1;
+      }
+    }
+    ACT3_STAMP(3);
+  }
+}
+
 // O = element type of the observation rows.  bf16 rows are widened in the producers' load: a bf16 value is exact in
 // TF32, so its hi half is the value itself, its lo half zero, and the products equal those on the widened fp32 rows.
 template <int PRE, typename O = float>   // PRE: 16-byte K chunks per thread in the observation operand (>= K1 / 8)
@@ -753,6 +845,310 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3x(ActorArgs a) {
       }
       ACT3_STAMP(3);
     }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0)
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*s_tmem), "r"((uint32_t)kAct2TmemCols) : "memory");
+}
+
+// ------------------------------------------------------------------------------------------------
+// k_actor3h: the "f16x3" precision -- k_actor3x's roles, pipeline and consumers, with all three passes of a product on fp16
+// halves (kind::f16, K = 16 per instruction instead of 8: C4's 100 x 100 actor issues 24 MMAs per tile instead of 45).
+//
+// Split, into ONE fp32 accumulator.  An fp16 value has 11 significant bits like TF32, so hi + lo carries 22 bits:
+//   A_hi = fp16(x),  A_lo = fp16((x - A_hi) 2^11);   W' = W 2^s  (s per output neuron: the row's largest |w| in [2^13, 2^14)),
+//   W_hi = fp16(W'), W_d = fp16(W_hi 2^-11), W_lo = fp16(W' - W_hi);     A_hi W_hi + A_lo W_d + A_hi W_lo  ~  x W'.
+// The per-neuron scale keeps W_hi, W_d and W_lo normal fp16 numbers however small or large the weights are.  It is a power of
+// two, so it commutes with ReLU and is undone exactly: by the producers for layer 1 (2^-s per column, from the image), through the
+// output-layer weights for layer 2 (the image holds w3 2^-s: relu(acc) (w3 2^-s) is the same fp32 product as relu(acc 2^-s) w3).
+// Range: an A value of a live row -- an observation element, or a hidden activation once its scale is undone -- with
+// |x| >= 65520 has no fp16 hi half.  The producers detect it and set the mapped host flag a.range_err; the host reports it
+// (drsim_actor_status, and the next drsim_policy_step / drsim_rollout_transition fails).  Padding slots (house >= N) and rows past
+// the end enter as zero rows, so whatever they hold never sets it.
+// Layouts: layer-1 A and all weights in the canonical no-swizzle K-major layout for 16-bit elements (8 per 16-byte core-matrix
+// row; LBO / SBO as for fp32).  Layer-2 A lives in tensor memory IN PLACE of R1: the 16 fp32 columns of granule g (K values
+// 16 g ... 16 g + 15) become 8 columns of packed hi pairs, [16 g, 16 g + 8), and 8 of packed lo pairs, [16 g + 8, 16 g + 16),
+// written by the one thread that read the granule.  Tensor memory: R1 | R2[0] | R2[1] = N1 + 2 N2 <= 400 columns.
+// Image (k_actor_pack3h): [w1_hi | w2_hi | w1_d | w2_d | w1_lo | w2_lo | 2^-s of layer 1 [N1] | w3 2^-s [2][N2] zero-padded, b3[2]].
+// ------------------------------------------------------------------------------------------------
+constexpr float kF16Overflow = 65520.f;   // the smallest |x| that fp16 round-to-nearest-even turns into infinity
+
+// byte offset of element (row, k) of a K-major 16-bit operand with `rows` rows in the canonical layout
+DRSIM_D int umma_kmajor_off16(int rows, int row, int k) {
+  return (k >> 3) * (rows >> 3) * 128 + (row >> 3) * 128 + (row & 7) * 16 + (k & 7) * 2;
+}
+DRSIM_D uint32_t umma_instr_desc_f16(int M, int N) {
+  // c_format F32 = 1 [4,6), a/b_format F16 = 0, K-major A and B, n_dim = N >> 3 [17,23), m_dim = M >> 4 [24,29)
+  return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+DRSIM_D void umma_f16_ss(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %6, %7, %8}, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "l"(da), "l"(db), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u)
+      : "memory");
+}
+DRSIM_D void umma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t db, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, {%5, %6, %7, %8}, p;\n\t"
+      "}\n" ::"r"(tmem_d),
+      "r"(tmem_a), "l"(db), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u)
+      : "memory");
+}
+// the hi and the 2^11-scaled lo fp16 halves of two values, packed in pairs (the first value in the low 16 bits)
+DRSIM_D void split_f16x2(float x0, float x1, uint32_t &hi, uint32_t &lo) {
+  const __half2 h = __floats2half2_rn(x0, x1);
+  const float2 f = __half22float2(h);
+  const __half2 l = __floats2half2_rn((x0 - f.x) * 2048.f, (x1 - f.y) * 2048.f);
+  hi = *reinterpret_cast<const uint32_t *>(&h);
+  lo = *reinterpret_cast<const uint32_t *>(&l);
+}
+
+// Row n of the augmented operand [W | b] (+ the one-regenerating row n_out when `gen_one`) as W_hi / W_d / W_lo at img + off,
+// + w_bytes, + 2 w_bytes, scaled by the row's 2^s; returns 2^-s.  One warp per row.  s <= 126 keeps 2^s and 2^-s normal
+// (weights below 2^-112 then lose fp16 precision instead); s >= -114 holds for every finite weight.
+DRSIM_D float pack_row_f16x3(unsigned char *img, int w_bytes, int off, const float *w, const float *b, int n, int n_out, int n_in,
+                             int Np, int Kp, bool gen_one, int lane) {
+  auto val = [&](int k) -> float {
+    if (n < n_out) return k < n_in ? __ldg(w + (size_t)n * n_in + k) : (k == n_in ? __ldg(b + n) : 0.f);
+    return (n == n_out && gen_one && k == n_in) ? 1.f : 0.f;
+  };
+  float m = 0.f;
+  for (int k = lane; k < Kp; k += 32) m = fmaxf(m, fabsf(val(k)));
+  for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  int e = 0;
+  if (m > 0.f) frexpf(m, &e);                                     // m = f 2^e, f in [0.5, 1)
+  const int s = m > 0.f ? min(14 - e, 126) : 0;
+  const float up = __int_as_float((127 + s) << 23), down = __int_as_float((127 - s) << 23);
+  for (int k = lane; k < Kp; k += 32) {
+    const float v = val(k) * up;
+    const __half hi = __float2half_rn(v);
+    const float hf = __half2float(hi);
+    const int o = off + umma_kmajor_off16(Np, n, k);
+    *reinterpret_cast<__half *>(img + o) = hi;
+    *reinterpret_cast<__half *>(img + w_bytes + o) = __float2half_rn(hf * 0.00048828125f);   // W_hi 2^-11
+    *reinterpret_cast<__half *>(img + 2 * w_bytes + o) = __float2half_rn(v - hf);
+  }
+  return down;
+}
+
+// the image of k_actor3h, once per launch: one warp per output neuron of layers 1 and 2
+__global__ void k_actor_pack3h(ActorArgs a, unsigned char *image) {
+  pdl_trigger();
+  const int lane = threadIdx.x & 31, wid = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), nw = (int)(gridDim.x * blockDim.x >> 5);
+  float *sc1 = reinterpret_cast<float *>(image + a.off_sc), *w3 = reinterpret_cast<float *>(image + a.off_w3);
+  for (int r = wid; r < a.N1 + a.N2; r += nw) {
+    if (r < a.N1) {
+      const float down = pack_row_f16x3(image, a.w_bytes, a.off_w1, a.w1, a.b1, r, a.h1, a.D, a.N1, a.K1, true, lane);
+      if (lane == 0) sc1[r] = down;
+    } else {
+      const int n = r - a.N1;
+      const float down = pack_row_f16x3(image, a.w_bytes, a.off_w2, a.w2, a.b2, n, a.h2, a.h1, a.N2, a.K2, false, lane);
+      if (lane < 2) w3[lane * a.N2 + n] = n < a.h2 ? __ldg(a.w3 + (size_t)lane * a.h2 + n) * down : 0.f;
+    }
+  }
+  if (blockIdx.x == 0 && threadIdx.x < 2) w3[2 * a.N2 + threadIdx.x] = __ldg(a.b3 + threadIdx.x);
+}
+
+// PRE: 16-byte chunks (8 fp16 values) of the observation operand per producer thread, ceil(K1 / 16) with K1 = D + 1 rounded up
+// to 16; the instantiations 1 / 2 / 4 / 5 cover the observation widths of k_actor3x's 2 / 4 / 7 / 9.  O as for k_actor3x.
+template <int PRE, typename O = float>
+__global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
+  extern __shared__ __align__(1024) unsigned char smem[];
+  // mbarriers as in k_actor3x
+  uint64_t *s_bar = reinterpret_cast<uint64_t *>(smem + a.off_bar);
+  uint64_t *a1_ready = s_bar, *bar1 = s_bar + 1, *a2_ready = s_bar + 2, *bar2 = s_bar + 7, *r2_free = s_bar + 9, *wbar = s_bar + 11;
+  uint32_t *s_tmem = reinterpret_cast<uint32_t *>(s_bar + 12);
+  const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0), role = warp < 8 ? 0 : (warp < 12 ? 1 : 2);
+  const int t = tid & 127, part = (tid >> 7) & 1;
+  const int n_tiles = (int)((a.rows + kActRows - 1) / kActRows);
+  const int n_my = blockIdx.x < n_tiles ? (n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+  unsigned char *s_a1h = smem + a.off_a1, *s_a1l = s_a1h + kActRows * a.K1 * 2;   // observation operand, hi and lo
+
+  if (tid == 0) {
+    mbar_init(a1_ready, 256);
+    mbar_init(bar1, 1);
+    for (int k = 0; k < kAct3MaxChunks; ++k) mbar_init(a2_ready + k, 256);
+    mbar_init(bar2, 1);
+    mbar_init(bar2 + 1, 1);
+    mbar_init(r2_free, 128);
+    mbar_init(r2_free + 1, 128);
+    mbar_init(wbar, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
+                     (uint32_t)__cvta_generic_to_shared(s_tmem)),
+                 "r"((uint32_t)kAct2TmemCols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  pdl_trigger();
+  pdl_wait();
+  if (tid == 0) {
+    mbar_expect_tx(wbar, (uint32_t)a.off_a1);
+    bulk_load_g2s(smem, a.image, (uint32_t)a.off_a1, wbar);
+  }
+  const uint32_t tmem = *s_tmem;
+  const uint32_t R1 = tmem, R2 = tmem + (uint32_t)a.N1;             // R2 slot s at R2 + s * N2
+  const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
+  const int ng = a.K2 >> 4, nchunk = (ng + 1) >> 1;                  // 16-value granules / 32-column chunks of R1
+
+  if (role == 0) {
+    // ---------------------------------------------------------------- producers
+    const int nch = a.K1 >> 3, c_lo = part ? nch / 2 : 0, c_hi = part ? nch : nch / 2;   // this thread's 16-byte K chunks
+    const float *sc1 = reinterpret_cast<const float *>(smem + a.off_sc);
+    float pre[PRE * 8];
+    bool pre_live = false, bad = false;
+    auto fetch = [&](int tile) {
+      const long long row = (long long)tile * kActRows + t;
+      bool live = row < a.rows;
+      if (live) {
+        const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
+        live = row - rr * a.Ns < a.N;
+      }
+      pre_live = live;
+      const O *g = static_cast<const O *>(a.obs) + (size_t)(live ? row : 0) * a.D;
+      if ((a.D & 1) == 0) {
+#pragma unroll
+        for (int j = 0; j < PRE * 4; ++j) {
+          const int k = c_lo * 8 + 2 * j;
+          float2 v = make_float2(0.f, 0.f);
+          if (live && k < c_hi * 8 && k < a.D) {
+            if constexpr (sizeof(O) == 2) v = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162 *>(g + k)));
+            else v = __ldg(reinterpret_cast<const float2 *>(g + k));
+          }
+          pre[2 * j] = v.x;
+          pre[2 * j + 1] = v.y;
+        }
+      } else {
+#pragma unroll
+        for (int j = 0; j < PRE * 8; ++j) {
+          const int k = c_lo * 8 + j;
+          pre[j] = (live && k < c_hi * 8 && k < a.D) ? (float)__ldg(g + k) : 0.f;
+        }
+      }
+    };
+    if (n_my > 0) fetch((int)blockIdx.x);
+    for (int it = 0; it < n_my; ++it) {
+      const int tile = (int)blockIdx.x + it * (int)gridDim.x;
+      const bool live = pre_live;
+      float mx = 0.f;   // largest |A value| of this row in this thread's columns
+      ACT3_STAMP(0);
+      // layer-1 operand: [obs | 1 | 0 ...] as hi + lo, one 16-byte store per K chunk (8 values; conflict-free)
+#pragma unroll
+      for (int j = 0; j < PRE; ++j) {
+        const int c = c_lo + j;
+        if (c < c_hi) {
+          uint32_t h[4], l[4];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            const float v0 = (8 * c + 2 * i == a.D) ? 1.f : pre[8 * j + 2 * i];
+            const float v1 = (8 * c + 2 * i + 1 == a.D) ? 1.f : pre[8 * j + 2 * i + 1];
+            mx = fmaxf(mx, fmaxf(fabsf(v0), fabsf(v1)));
+            split_f16x2(v0, v1, h[i], l[i]);
+          }
+          const int off = c * (kActRows * 16) + t * 16;
+          *reinterpret_cast<uint4 *>(s_a1h + off) = make_uint4(h[0], h[1], h[2], h[3]);
+          *reinterpret_cast<uint4 *>(s_a1l + off) = make_uint4(l[0], l[1], l[2], l[3]);
+        }
+      }
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      mbar_arrive(a1_ready);
+      ACT3_STAMP(1);
+      if (it + 1 < n_my) fetch(tile + (int)gridDim.x);
+      ACT3_STAMP(2);
+      // layer-2 operand: A2 = relu(D1 2^-s) as packed hi | lo pairs in place of each granule, published chunk by chunk.  bar1
+      // also covers GEMM2 of the previous tile, the last reader of R1.
+      mbar_wait_bounded(bar1, (uint32_t)(it & 1));
+      tc_fence_after();
+      ACT3_STAMP(3);
+      uint32_t r[2][16];
+      const uint32_t src = R1 + lane_off;
+      if (part < ng) tmem_ld16_issue(src + (uint32_t)(16 * part), r[0]);
+#pragma unroll
+      for (int k = 0; k < kAct3MaxChunks; ++k) {
+        if (k < nchunk) {
+          const int g = 2 * k + part;
+          if (g < ng) {
+            tmem_wait_ld_dep(r[k & 1]);
+            if (k + 1 < nchunk && g + 2 < ng) tmem_ld16_issue(src + (uint32_t)(16 * (g + 2)), r[(k + 1) & 1]);
+            const float4 *sc = reinterpret_cast<const float4 *>(sc1 + 16 * g);
+            uint32_t o[16];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              const float4 u = sc[q];
+              const float x0 = fmaxf(__uint_as_float(r[k & 1][4 * q]) * u.x, 0.f), x1 = fmaxf(__uint_as_float(r[k & 1][4 * q + 1]) * u.y, 0.f),
+                          x2 = fmaxf(__uint_as_float(r[k & 1][4 * q + 2]) * u.z, 0.f), x3 = fmaxf(__uint_as_float(r[k & 1][4 * q + 3]) * u.w, 0.f);
+              mx = fmaxf(mx, fmaxf(fmaxf(x0, x1), fmaxf(x2, x3)));
+              split_f16x2(x0, x1, o[2 * q], o[8 + 2 * q]);
+              split_f16x2(x2, x3, o[2 * q + 1], o[9 + 2 * q]);
+            }
+            tmem_st16(src + (uint32_t)(16 * g), o);
+            tmem_wait_st();
+          }
+          tc_fence_before();
+          mbar_arrive(a2_ready + k);
+          ACT3_STAMP(4 + k);
+        }
+      }
+      bad |= live && mx >= kF16Overflow;
+    }
+    if (bad) *reinterpret_cast<volatile int *>(a.range_err) = 1;
+  } else if (role == 2) {
+    // ---------------------------------------------------------------- MMA warp: one thread issues everything
+    if (n_my > 0 && elect_one_lane()) {
+      const uint32_t idesc1 = umma_instr_desc_f16(kActRows, a.N1), idesc2 = umma_instr_desc_f16(kActRows, a.N2);
+      const uint32_t w1h = (uint32_t)__cvta_generic_to_shared(smem + a.off_w1), w2h = (uint32_t)__cvta_generic_to_shared(smem + a.off_w2);
+      const uint32_t wb = (uint32_t)a.w_bytes;   // W_hi, W_d, W_lo blocks
+      const uint32_t a1h = (uint32_t)__cvta_generic_to_shared(s_a1h), a1l = (uint32_t)__cvta_generic_to_shared(s_a1l);
+      const uint32_t lbo_a = (kActRows / 8) * 128, lbo_w1 = (a.N1 / 8) * 128, lbo_w2 = (a.N2 / 8) * 128;
+      const int ks1 = a.K1 >> 4;
+      mbar_wait_bounded(wbar, 0);
+      for (int it = 0; it < n_my; ++it) {
+        const int s = it & 1;
+        const uint32_t d2 = R2 + (uint32_t)(s * a.N2);
+        mbar_wait_bounded(a1_ready, (uint32_t)(it & 1));
+        tc_fence_after();
+        ACT3_STAMP(0);
+        for (int ks = 0; ks < ks1; ++ks) {      // layer 1: hi.hi, lo.d, hi.lo
+          const uint64_t dah = umma_smem_desc(a1h + ks * 2 * lbo_a, lbo_a, 128), dal = umma_smem_desc(a1l + ks * 2 * lbo_a, lbo_a, 128);
+          const uint32_t wk = w1h + ks * 2 * lbo_w1;
+          umma_f16_ss(R1, dah, umma_smem_desc(wk, lbo_w1, 128), idesc1, ks > 0);
+          umma_f16_ss(R1, dal, umma_smem_desc(wk + wb, lbo_w1, 128), idesc1, 1);
+          umma_f16_ss(R1, dah, umma_smem_desc(wk + 2 * wb, lbo_w1, 128), idesc1, 1);
+        }
+        umma_commit(bar1);
+        ACT3_STAMP(1);
+        for (int k = 0; k < nchunk; ++k) {      // layer 2: A2 from tensor memory, chunk by chunk
+          mbar_wait_bounded(a2_ready + k, (uint32_t)(it & 1));
+          if (k == 0 && it >= 2) mbar_wait_bounded(r2_free + s, (uint32_t)(((it >> 1) & 1) ^ 1));
+          tc_fence_after();
+          ACT3_STAMP(2 + k);
+          const int ge = min(2 * k + 2, ng);
+          for (int g = 2 * k; g < ge; ++g) {
+            const uint32_t wk = w2h + g * 2 * lbo_w2, ah = R1 + (uint32_t)(16 * g);
+            umma_f16_ts(d2, ah, umma_smem_desc(wk, lbo_w2, 128), idesc2, g > 0);
+            umma_f16_ts(d2, ah + 8u, umma_smem_desc(wk + wb, lbo_w2, 128), idesc2, 1);
+            umma_f16_ts(d2, ah, umma_smem_desc(wk + 2 * wb, lbo_w2, 128), idesc2, 1);
+          }
+        }
+        umma_commit(bar2 + s);
+        ACT3_STAMP(7);
+      }
+    }
+  } else {
+    act3_consumers(a, smem, R2, lane_off, n_my, tid, warp, bar2, r2_free, wbar);
   }
   tc_fence_before();
   __syncthreads();

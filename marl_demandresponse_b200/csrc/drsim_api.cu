@@ -96,9 +96,10 @@ struct drsim_handle {
   unsigned char *h_snap = nullptr, *h_snap_dev = nullptr;
   size_t snap_bytes = 0, snap_obs_off = 0;
   bool snap_next = false, snap_fused = false;   // transient: the next small-cluster step writes the host snapshot itself
-  unsigned long long *actor_dbg = nullptr;   // DRSIM_ACTOR_DBG: phase stamps of CTA 0 of the last k_actor3x launch
+  unsigned long long *actor_dbg = nullptr;   // DRSIM_ACTOR_DBG: phase stamps of CTA 0 of the last k_actor3x / k_actor3h launch
   unsigned long long *shard_dbg = nullptr;   // DRSIM_SHARD_DBG: per-CTA time stamps of the last k_shard launch
   int *h_peer_err = nullptr, *h_peer_err_dev = nullptr;   // mapped: set by a kernel whose exchange wait timed out
+  int *h_actor_err = nullptr, *h_actor_err_dev = nullptr; // mapped: set by k_actor3h when an operand overflows fp16
   int pending_interp = 0;  // decision of drsim_step_begin, consumed by drsim_step_finish
   StepIn pending_in{};
   // pinned staging for drsim_step_host; h_env_dev = the same memory as the device sees it (mapped)
@@ -515,6 +516,9 @@ extern "C" int drsim_create(const drsim_config *cfg, int device, drsim_t **out) 
     h->h_peer_err = h->h_poll_err + 1;
     h->h_peer_err_dev = h->h_poll_err_dev + 1;
     *h->h_peer_err = 0;
+    h->h_actor_err = h->h_poll_err + 2;
+    h->h_actor_err_dev = h->h_poll_err_dev + 2;
+    *h->h_actor_err = 0;
     if (cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking) != cudaSuccess) {
       h->copy_stream = nullptr;
       cudaGetLastError();
@@ -1917,6 +1921,21 @@ extern "C" int drsim_peer_status(drsim_t *h, void *stream) {
 static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const void *obs_in, uint8_t *actions_out,
                             float *prob_drawn, float *prob_on, void *stream);
 
+// the range flag of the f16x3 actor (k_actor3h), reported once and cleared
+static int actor_range_error(drsim_t *h) {
+  if (!h->h_actor_err || !*reinterpret_cast<volatile int *>(h->h_actor_err)) return 0;
+  *reinterpret_cast<volatile int *>(h->h_actor_err) = 0;
+  return fail(DRSIM_E_STATE, "f16x3 actor: an observation element or hidden activation of a live row was outside the fp16 range "
+                             "(|x| >= 65520) in an earlier launch: its actions and probabilities are not valid; use precision = 1 (3xTF32)");
+}
+
+extern "C" int drsim_actor_status(drsim_t *h, void *stream) {
+  if (!h) return fail(DRSIM_E_ARG, "null handle");
+  CU_TRY(cudaSetDevice(h->device));
+  CU_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+  return actor_range_error(h);
+}
+
 extern "C" int drsim_policy_step(drsim_t *h, const drsim_actor_net *net, uint64_t seed, float *prob_drawn, float *prob_on,
                                  void *stream) {
   return policy_step_impl(h, net, seed, nullptr, nullptr, prob_drawn, prob_on, stream);
@@ -1951,15 +1970,18 @@ extern "C" int drsim_rollout_transition(drsim_t *h, const drsim_actor_net *net, 
 static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const void *obs_in, uint8_t *actions_out,
                             float *prob_drawn, float *prob_on, void *stream) {
   if (!h || !net) return fail(DRSIM_E_ARG, "null argument");
+  if (int rc = actor_range_error(h)) return rc;
   const SimParams &p = h->p;
+  if (net->precision < 0 || net->precision > 2)
+    return fail(DRSIM_E_ARG, "drsim_policy_step: precision must be 0 (tf32), 1 (tf32x3) or 2 (f16x3)");
   if (h->real_bytes != 4) return fail(DRSIM_E_ARG, "drsim_policy_step needs the fp32 build (observation rows are its input)");
   if (p.obs_dim < 1 || p.obs_dim > 64) return fail(DRSIM_E_ARG, "drsim_policy_step: obs_dim must be in [1, 64]");
   if (net->h1 < 1 || net->h1 > 128 || net->h2 < 1 || net->h2 > 128) return fail(DRSIM_E_ARG, "drsim_policy_step: h1, h2 in [1, 128]");
   if (!net->w1 || !net->b1 || !net->w2 || !net->b2 || !net->w3 || !net->b3) return fail(DRSIM_E_ARG, "drsim_policy_step: null weight pointer");
   const bool bf16 = h->obs_bytes == 2;
-  if (bf16 && net->precision != 1)
-    return fail(DRSIM_E_ARG, "drsim_policy_step: bfloat16 observation rows need precision = 1 (3xTF32); the single-pass actor "
-                             "stages fp32 rows");
+  if (bf16 && net->precision == 0)
+    return fail(DRSIM_E_ARG, "drsim_policy_step: bfloat16 observation rows need precision = 1 (3xTF32) or 2 (f16x3); the "
+                             "single-pass actor stages fp32 rows");
   CU_TRY(cudaSetDevice(h->device));
   ActorArgs a{};
   a.obs = obs_in ? obs_in : static_cast<const void *>(h->slab + h->o_obs);
@@ -2006,6 +2028,43 @@ static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t see
                         : pre <= 7 ? k_actor3x<7, __nv_bfloat16>
                                    : k_actor3x<kAct3PreChunks, __nv_bfloat16>)
                      : (pre <= 2 ? k_actor3x<2> : pre <= 4 ? k_actor3x<4> : pre <= 7 ? k_actor3x<7> : k_actor3x<kAct3PreChunks>);
+    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
+    launch_pdl(kern, std::min(tiles, h->sm_count), kAct3Threads, (size_t)a.smem_bytes, (cudaStream_t)stream, a);
+    h->launches++;
+  } else if (net->precision == 2) {
+    // f16x3: fp16 hi / d / lo operands with per-neuron power-of-two scales, k_actor3x's roles (see k_actor3h).  K is a multiple
+    // of 16 (UMMA_K of kind::f16).  The widest accepted shape (D = 64, h1 = h2 = 128) takes 222,592 bytes of shared memory and
+    // N1 + 2 N2 = 400 tensor-memory columns: no width within the limits above is refused.
+    if (!h->h_actor_err_dev) return fail(DRSIM_E_CUDA, "drsim_policy_step: f16x3 needs mapped host memory for its range flag");
+    a.K1 = (a.D + 1 + 15) / 16 * 16; a.N1 = (a.h1 + 1 + 15) / 16 * 16;
+    a.K2 = a.N1; a.N2 = (a.h2 + 15) / 16 * 16;
+    a.K3 = a.N2;
+    a.off_w1 = take(a.N1 * a.K1 * 2); a.off_w2 = take(a.N2 * a.K2 * 2);
+    a.w_bytes = off;                              // one (hi, d or lo) weight block
+    off = 3 * a.w_bytes;
+    a.off_sc = take(a.N1 * 4);                    // 2^-s of the layer-1 columns
+    a.off_w3 = take((2 * a.N2 + 2) * 4);          // output layer, fp32, carrying the layer-2 2^-s
+    a.off_vec = a.off_w3;
+    a.off_a1 = off;                               // = size of the packed image
+    take(2 * kActRows * a.K1 * 2);                // observation operand, hi and lo
+    a.off_a2 = off;
+    a.off_bar = take(128);
+    a.smem_bytes = off;
+    a.range_err = h->h_actor_err_dev;
+    if (!h->actor_image) CU_TRY(cudaMalloc(&h->actor_image, 256 * 1024));
+    a.image = h->actor_image;
+    if (!h->actor_dbg && getenv("DRSIM_ACTOR_DBG")) {
+      CU_TRY(cudaMalloc(&h->actor_dbg, 8 * 3 * 16 * 8));
+      CU_TRY(cudaMemset(h->actor_dbg, 0, 8 * 3 * 16 * 8));
+    }
+    a.dbg = h->actor_dbg;
+    k_actor_pack3h<<<(a.N1 + a.N2 + 15) / 16, 512, 0, (cudaStream_t)stream>>>(a, h->actor_image);
+    const int pre = a.K1 / 16;                    // 16-byte chunks (8 fp16 values) per producer thread
+    auto kern = bf16 ? (pre <= 1   ? k_actor3h<1, __nv_bfloat16>
+                        : pre <= 2 ? k_actor3h<2, __nv_bfloat16>
+                        : pre <= 4 ? k_actor3h<4, __nv_bfloat16>
+                                   : k_actor3h<5, __nv_bfloat16>)
+                     : (pre <= 1 ? k_actor3h<1> : pre <= 2 ? k_actor3h<2> : pre <= 4 ? k_actor3h<4> : k_actor3h<5>);
     CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
     launch_pdl(kern, std::min(tiles, h->sm_count), kAct3Threads, (size_t)a.smem_bytes, (cudaStream_t)stream, a);
     h->launches++;
@@ -2063,7 +2122,7 @@ extern "C" int drsim_debug_tile_phases(unsigned long long *host_out, int max_cta
 }
 
 // diagnostics, not part of the documented ABI: clock64 stamps [tile < 8][producer, consumer, MMA warp][16] of CTA 0 of the
-// last k_actor3x launch (DRSIM_ACTOR_DBG=1)
+// last k_actor3x / k_actor3h launch (DRSIM_ACTOR_DBG=1)
 extern "C" int drsim_debug_actor_times(drsim_t *h, unsigned long long *host_out) {
   if (!h || !h->actor_dbg || !host_out) return 0;
   cudaMemcpy(host_out, h->actor_dbg, 8 * 3 * 16 * 8, cudaMemcpyDeviceToHost);

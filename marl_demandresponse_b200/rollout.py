@@ -98,7 +98,9 @@ def collect(env, weights, buf: RolloutBuffer, n_steps: Optional[int] = None, see
             done_last: bool = False, stream=None, precision: str = "tf32x3") -> RolloutBuffer:
     """``n_steps`` (default: the buffer's horizon) rollout transitions on the device, stored in ``buf``:
     per transition ONE C call (``drsim_rollout_transition``: actor + categorical draw, then the environment step
-    writing reward and next observation rows straight into the buffer)."""
+    writing reward and next observation rows straight into the buffer).  ``precision``: the actor's, see
+    ``DrSim.policy_step``; "f16x3" ends the segment with ``DrSim.actor_status`` (a synchronisation), which raises if an
+    operand left the fp16 range: the segment's actions and probabilities are then not valid."""
     sim = env.sim
     T = buf.T if n_steps is None else int(n_steps)
     if T > buf.T:
@@ -121,4 +123,6 @@ def collect(env, weights, buf: RolloutBuffer, n_steps: Optional[int] = None, see
     if done_last and T:
         buf.done[T - 1] = True
     buf.filled = T
+    if precision == "f16x3":
+        sim.actor_status(stream)
     return buf

@@ -1,6 +1,7 @@
-"""Per-role phase time lines of k_actor3x (CTA 0, first 8 tiles), from the clock64 stamps of DRSIM_ACTOR_DBG=1.
+"""Per-role phase time lines of k_actor3x ("tf32x3") or k_actor3h ("f16x3") (CTA 0, first 8 tiles), from the clock64
+stamps of DRSIM_ACTOR_DBG=1.  Both kernels stamp the same phases; k_actor3h's chunks are 32 columns of R1 as well.
 
-    DRSIM_ACTOR_DBG=1 python profiles/tools/actor_phases.py [c3|c4]
+    DRSIM_ACTOR_DBG=1 python profiles/tools/actor_phases.py [c3|c4] [tf32x3|f16x3]
 """
 import ctypes as C, os, sys
 os.environ["DRSIM_ACTOR_DBG"] = "1"
@@ -10,6 +11,7 @@ from bench import env_prop_for
 from marl_demandresponse_b200 import BatchedEnv
 from marl_demandresponse_b200 import _lib
 which = sys.argv[1] if len(sys.argv) > 1 else "c4"
+precision = sys.argv[2] if len(sys.argv) > 2 else "tf32x3"
 R, N, layout = (4096, 100, "hand_engineered") if which == "c3" else (2048, 1000, "tarmac")
 env = BatchedEnv(env_prop_for(N), R, obs_layout=layout, noise="philox", seed=1)
 env.reset()
@@ -18,7 +20,7 @@ D = env.sim.D
 fc = torch.nn.ModuleList([torch.nn.Linear(D, 100), torch.nn.Linear(100, 100), torch.nn.Linear(100, 2)]).cuda()
 w = BatchedEnv.actor_weights(fc)
 for _ in range(4):
-    env.policy_step(w, precision="tf32x3")
+    env.policy_step(w, precision=precision)
 torch.cuda.synchronize()
 L = _lib.lib()
 L.drsim_debug_actor_times.restype = C.c_int
@@ -30,7 +32,7 @@ t0 = int(buf[0][buf[0] > 0].min())
 names = {0: ["start", "a1 arrived", "fetch issued", "bar1 passed", "chunk0", "chunk1", "chunk2", "chunk3", "chunk4"],
          1: ["wait bar2", "bar2 passed", "R2 drained", "tile done"],
          2: ["a1 ready", "GEMM1 issued", "c0 ready", "c1 ready", "c2 ready", "c3 ready", "c4 ready", "GEMM2 committed"]}
-print(f"{which}: clock64 cycles since the first stamp of CTA 0 (producer warp 0 / consumer warp 8 / MMA warp)")
+print(f"{which} {precision}: clock64 cycles since the first stamp of CTA 0 (producer warp 0 / consumer warp 8 / MMA warp)")
 for it in range(8):
     for role, rn in ((0, "prod"), (2, "mma "), (1, "cons")):
         row = buf[it][role]
