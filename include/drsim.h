@@ -155,6 +155,8 @@ typedef struct drsim_host_state {
   double *artificial_ratio;        /* PowerGridProperties.artificial_ratio (post-draw)    */
   double *max_power;               /* Cluster.max_power                                   */
   int32_t *t_since_interp;         /* PowerGrid.time_since_last_interp                    */
+  /* t_since_interp: the interpolator fires for all replicas of a handle on the same step, so drsim_set_state
+   * takes one counter for the handle and fails with DRSIM_E_ARG when the values differ across replicas. */
   /* optional [n_rep][n_house][12]: precomputed output of drsim_host_thermal_coefs for each house
    * (set_state only).  When NULL the library derives it from Ua, Ca, Cm, Hm with libm; a caller
    * that wants the constants of building.py:196-206 bit-identical to NumPy's passes its own. */

@@ -73,6 +73,16 @@ def synthetic_state(props: Any, n_rep: int, seed: int = 1234, rep_offset: int = 
     return st
 
 
+def reset_counter(props: Any, state: Dict[str, np.ndarray], n_rep: int) -> Dict[str, np.ndarray]:
+    """``state`` with the interpolator's counter of a new episode: the reference builds a new ``PowerGrid`` at every
+    reset, whose counter starts at ``interp_update_period + 1`` (power_grid.py:64-66), so the interpolator fires at
+    the reset.  A state that carries ``t_since_interp`` keeps its own."""
+    if "t_since_interp" in state:
+        return state
+    period = as_props(props).power_grid_prop.base_power_props.interp_update_period
+    return {**state, "t_since_interp": np.full(n_rep, period + 1, dtype=np.int32)}
+
+
 class BatchedEnv:
     """R independent replicas of the reference's cluster environment on one GPU.
 
@@ -139,14 +149,16 @@ class BatchedEnv:
         signal (``PowerGrid.step`` at reset, environment.py:66-68) and return the observations.
         ``device_mode`` = "reference" | "synthetic" draws the state on the GPU instead
         (``drsim_reset``: the reference's reset distributions from Philox streams).  Either way a new episode
-        begins: the running metrics (``metrics``) start again from zero."""
+        begins: the running metrics (``metrics``) start again from zero, and an interpolated base power is
+        computed afresh (the counter starts at ``interp_update_period + 1`` unless ``state`` carries
+        ``t_since_interp``)."""
         if device_mode is not None:
             self.sim.reset_device(self.props, self.seed if seed is None else seed, device_mode, quirk_ua)
             self.sim.refresh(True)
             return self.obs
         if state is None:
             state = synthetic_state(self.props, self.n_replicas, self.seed if seed is None else seed, self.rep_offset)
-        self.sim.set_state(state)
+        self.sim.set_state(reset_counter(self.props, state, self.n_replicas))
         self._v["metrics"].zero_()   # on the current stream, like drsim_reset
         self.sim.refresh(True)
         return self.obs

@@ -813,6 +813,12 @@ static int set_state_t(drsim_handle *h, const drsim_host_state *st, cudaStream_t
 
 extern "C" int drsim_set_state(drsim_t *h, const drsim_host_state *st, void *stream) {
   if (!h || !st) return fail(DRSIM_E_ARG, "null argument");
+  // the interpolator fires for the whole handle at once (interp_decision): one counter, common to all replicas
+  if (st->t_since_interp)
+    for (int r = 1; r < h->p.R; ++r)
+      if (st->t_since_interp[r] != st->t_since_interp[0])
+        return fail(DRSIM_E_ARG, "set_state: t_since_interp must be the same on every replica (the interpolator fires "
+                                 "for all replicas of a handle on the same step)");
   CU_TRY(cudaSetDevice(h->device));
   h->sched_valid = false;
   h->broken = false;

@@ -669,7 +669,9 @@ DRSIM_D EnvBroadcast<real> env_epilogue_compute(const Planes<real> &pl, const Si
       const double factor = p.n_global <= p.interp_k ? 1.0 : (double)p.n_global / (double)p.interp_k;
       e.base_power = interp_sum * factor;
       e.t_since_interp = 0;
-    } else if (in.advance) {
+    } else {
+      // every power-grid step adds dt (power_grid.py:150), also a refresh that recomputes the signal without
+      // firing: the plane stays equal to the host counter interp_decision advanced
       e.t_since_interp += p.dt;
     }
   }

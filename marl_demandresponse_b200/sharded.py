@@ -18,7 +18,7 @@ from typing import Any, Dict, Optional
 
 import numpy as np
 
-from .batched import synthetic_state
+from .batched import reset_counter, synthetic_state
 from .core import DrSim, flatten_config
 from .properties import as_props
 
@@ -94,14 +94,16 @@ class ShardedClusterEnv:
 
     def reset(self, state: Optional[Dict[str, np.ndarray]] = None, seed: int = 1234):
         """``state``: full-cluster state dict (every rank passes the same one) or None = synthetic.  A new episode
-        begins: the running metrics (``state["metrics"]``) start again from zero."""
+        begins: the running metrics (``state["metrics"]``) start again from zero, and the interpolator's counter at
+        ``interp_update_period + 1`` unless ``state`` carries ``t_since_interp`` (its first step fires it, as the
+        reference's reset would: a house-sharded handle has no refresh)."""
         if state is None:
             state = synthetic_state(self.props, self.sim.R, seed)
         local = {}
         for k, v in state.items():
             v = np.asarray(v)
             local[k] = v[:, self.lo:self.hi] if v.ndim == 2 else v
-        self.sim.set_state(local)
+        self.sim.set_state(reset_counter(self.props, local, self.sim.R))
         self._v["metrics"].zero_()   # on the current stream, like drsim_reset
         return self
 

@@ -21,6 +21,12 @@ _level``); free-running fp32 trajectories get the 2e-4 drift allowance of the ba
 replays the reference's literal arithmetic, 1e-9.  Rewards and observations: the BASELINE.json north star, rtol 1e-5
 of (|value| + natural scale 1) in fp32, and 1e-9 of the same in fp64.
 
+Interpolated base power (``table`` given).  The oracle is built with the table and gets the Philox ids of the sampled
+houses.  On a firing step the device's base power is checked against ``interp_ref`` on the device's own post-step
+planes (fp32: ``interp_ref``'s first-principles bound; fp64: 1e-12 relative) and then handed to the oracle, so that the
+fp32 interpolation error is not carried through the signal (the ``regular_steps`` Heaviside), observations and
+metrics.  The counter ``t_since_interp`` is compared exactly.
+
 Running metrics (the six sums of ``DRSIM_N_METRICS``).  Every checked step's increment is compared on ALL replicas
 with ``metric_increments`` of the device's own planes before and after the step, and on the picked replicas with the
 oracle's post-step state; ``check_metrics`` / ``check_free`` compare the sums since the start with the oracle's
@@ -295,7 +301,7 @@ class OracleDriver:
     """Steps ``env`` with external actions, or under its on-device controller, and compares it with the oracle (see
     the module docstring)."""
 
-    def __init__(self, env, env_prop, st0, step_index=0, picks=None):
+    def __init__(self, env, env_prop, st0, step_index=0, picks=None, table=None):
         from oracle.config import normalize_env_prop
 
         self.env, self.env_prop = env, env_prop
@@ -320,6 +326,13 @@ class OracleDriver:
         self.inc_tol = np.zeros((len(self.picks), 6))
         self.n_steps = 0
         self.free = None
+        # interpolated base power: the oracle is built with the table, and on a firing step the device's base power is
+        # checked against interp_ref on the device's own planes, then handed to the oracle (check_base_power)
+        bp = self.p["power_grid_prop"]["base_power_props"]
+        self.table, self.interp, self.k = table, bp["mode"] == "interpolation", bp["interp_nb_agents"]
+        self.thermal = {k: np.broadcast_to(np.asarray(st0[k], dtype=np.float64), (self.R, self.N))[self.picks]
+                        for k in ("Ua", "Cm", "Ca", "Hm")}
+        self.fired = []          # driver steps on which the interpolator fired
 
     # ---- noise and state -------------------------------------------------------------------
     def _noise(self, step, epochs):
@@ -333,9 +346,49 @@ class OracleDriver:
 
         st = {k: (v[self.picks] if np.ndim(v) >= 1 and np.shape(v)[0] == self.R else v) for k, v in gpu_state.items()}
         st.update(self.static)
-        orc = NpOracle(self.env_prop, len(self.picks))
+        orc = NpOracle(self.env_prop, len(self.picks), table=self.table)
         orc.set_state(st)
         return orc
+
+    # ---- interpolated base power -------------------------------------------------------------
+    def interp_ids(self, step):
+        """``[picks, k]`` Philox ids of the sampled houses at Philox step ``step``; None when every house is read."""
+        from oracle import philox
+
+        if self.N <= self.k:
+            return None
+        return np.stack([philox.interp_choices(self.env.seed, self.env.rep_offset + r, step, self.k, self.N)
+                         for r in self.picks])
+
+    def check_base_power(self, got, step, what):
+        """The device's base power on the picked replicas against ``interp_ref.ref_base_power`` on the device's own
+        planes ``got`` (fp32: the bound of ``interp_ref``; fp64: 1e-12 relative)."""
+        import interp_ref
+
+        ids = self.interp_ids(step)
+        h = self.p["cluster_prop"]["house_prop"]
+        dflt = {"dUa": h["Ua"], "dCm": h["Cm"], "dCa": h["Ca"], "dHm": h["Hm"]}
+        for i, r in enumerate(self.picks):
+            house = {k: got[k][r] for k in ("t_air", "t_mass", "target", "cap")}
+            house.update({k: v[i] for k, v in self.thermal.items()})
+            want, tol = interp_ref.ref_base_power(self.table, house, dflt, np.arange(self.N) if ids is None else ids[i],
+                                                  got["od_temp"][r], got["epoch"][r], h["solar_gain"], self.N, self.k,
+                                                  self.precision == "f32")
+            err = abs(got["base_power"][r] - want)
+            assert err <= tol, f"{what}: replica {r}: base power {got['base_power'][r]!r} != {want!r} ({err:.3e} > {tol:.3e})"
+
+    def _use_device_base_power(self, orc, got, step, what):
+        """On a firing step the oracle takes the device's base power (checked first): the fp32 interpolation error is
+        then not carried through the signal (the ``regular_steps`` Heaviside), the observations and the metrics."""
+        checked = []
+
+        def fire(i, when, ids):
+            if not checked:
+                self.check_base_power(got, step, what)
+                checked.append(True)
+            return float(got["base_power"][self.picks[i]])
+
+        orc.interpolate_power = fire
 
     def _table(self):
         """The handle's own neighbour table; without one the oracle's ring table, or none at all when the rows carry no
@@ -360,6 +413,8 @@ class OracleDriver:
             bad = np.argwhere(got[k].astype(np.int64) != self.disc[k])
             assert bad.size == 0, f"{what}: {k} differs at (replica, house) {bad[:6].tolist()}"
         assert np.array_equal(got["epoch"].astype(np.int64), self.epoch), f"{what}: epoch"
+        if self.interp:   # one counter for the handle
+            assert np.all(got["t_since_interp"] == got["t_since_interp"][0]), f"{what}: t_since_interp"
         p_sum = (got["on"].astype(np.float64) * got["cap"] / self.cop).sum(axis=1)
         _close(got["power"], p_sum, 1e-6, 0.0, f"{what}: power (sum over houses)")
 
@@ -369,6 +424,8 @@ class OracleDriver:
         for k in ("on", "lockout", "sso"):
             assert np.array_equal(got[k][pk].astype(np.int64), s[k].astype(np.int64)), f"{what}: {k} (oracle)"
         assert np.array_equal(got["epoch"][pk], s["epoch"]), f"{what}: epoch (oracle)"
+        if self.interp:
+            assert np.array_equal(got["t_since_interp"][pk], s["t_since_interp"]), f"{what}: t_since_interp (oracle)"
         for k in ("od_temp", "signal", "base_power"):
             _close(got[k][pk], s[k], 1e-9, 0.0, f"{what}: {k}")
         _close(got["power"][pk], s["power"], 1e-6, 0.0, f"{what}: power")
@@ -420,14 +477,22 @@ class OracleDriver:
         if on_device and self.policy == "greedy_myopic":
             check_greedy_plane(self.env, acts, what)
         self._advance_discrete(acts)
+        if self.interp:
+            got = self.env.get_state()
+            if (got["t_since_interp"] == 0).any():
+                self.fired.append(self.n_steps)
         if self.free is not None:
+            if self.interp:
+                self._use_device_base_power(self.free, got, self.step_index, f"{what} (free-running)")
             self._advance_free_one(free_acts)
         if check:
             got, rew, obs = self._gpu()
             self._check_all_replicas(got, what)
             orc = self._oracle(before)
+            if self.interp:
+                self._use_device_base_power(orc, got, self.step_index, what)
             od, pe = self._noise(self.step_index, self.epoch[self.picks])
-            rew_ref = orc.step(acts[self.picks], od, pe)
+            rew_ref = orc.step(acts[self.picks], od, pe, self.interp_ids(self.step_index) if self.interp else None)
             self._check_picked(got, orc, rew, rew_ref, obs, True, what)
             self._check_step_metrics(before["signal"], m_before, orc.state, rew_ref, what)
         self.step_index += 1
@@ -476,7 +541,7 @@ class OracleDriver:
     def _advance_free_one(self, acts_picked):
         od, pe = self._noise(self.step_index, self.epoch[self.picks])
         signal_before = np.array(self.free.state["signal"], dtype=np.float64)
-        self.free_rew = self.free.step(acts_picked, od, pe)
+        self.free_rew = self.free.step(acts_picked, od, pe, self.interp_ids(self.step_index) if self.interp else None)
         s = self.free.state
         after = dict(d=s["t_air"] - s["target"], reward=self.free_rew, power=s["power"])
         tol = tolerances(self.precision, False)

@@ -12,6 +12,11 @@ step ran on, ``fused_info()`` the tile variant and the clusters per tile, ``laun
 * ``test_seeded_sweep_matches_oracle``: random (R, N, layout, modes) from a fixed list of seeds.
 * ``test_in_kernel_loop_matches_oracle``: ``run(T, tape, rotate=True)`` on the loop routes: one step kernel per
   schedule block, bit-identical to one launch per step, and free-running against the oracle.
+* ``test_route_interpolation_matches_oracle``: every route with the interpolated base power, fired every third step
+  (period 12 and 10 s: a multiple of the 4 s step and not) and on every step (period 3 s).  A firing step runs on
+  ``k_shard`` (the four-kernel path where k_shard is off), the next step back on the route, after regenerating the
+  schedule block the firing step ended.  The device's base power is checked against ``interp_ref`` at every firing,
+  the reset's included.
 
 Tolerances and the replicas compared are those of ``oracle_driver``.
 """
@@ -114,7 +119,7 @@ MATRIX["k_small"].append(dict(sig="perlin", nb="neighbours_2D", n=12, c=10))
 CASES = [pytest.param(route, i, id=f"{route}-{i}") for route in ROUTES for i in range(len(MATRIX[route]))]
 
 
-def _make(route, cell, monkeypatch, seed=21):
+def _make(route, cell, monkeypatch, seed=21, table=None):
     """The handle of one matrix cell, its properties and initial state; asserts the route it takes."""
     from marl_demandresponse_b200 import BatchedEnv
     from marl_demandresponse_b200.batched import synthetic_state
@@ -126,7 +131,7 @@ def _make(route, cell, monkeypatch, seed=21):
     for k, v in env_vars.items():
         monkeypatch.setenv(k, str(v))
     p = config(N, **cell)
-    env = BatchedEnv(p, R, precision=precision, obs_layout=layout, noise="philox", seed=seed, path=path)
+    env = BatchedEnv(p, R, precision=precision, obs_layout=layout, noise="philox", seed=seed, path=path, interp_table=table)
     info = env.sim.fused_info()
     print(route, cell, info)
     if "variant" in expect:
@@ -152,6 +157,58 @@ def test_route_matches_oracle(route, i, monkeypatch):
     launches += [drv.step(acts[t]) for t in range(1, T_STEPS)]
     # the first step generates the 64-step schedule block (two kernels), then one route's launches per step
     assert launches == [expect["launches"] + 2] + [expect["launches"]] * (T_STEPS - 1), launches
+    drv.check_metrics()
+    drv.check_free()
+
+
+INTERP_PERIODS = [12, 10, 3]
+INTERP_CASES = [pytest.param(route, period, id=f"{route}-interp{period}") for route in ROUTES for period in INTERP_PERIODS]
+
+
+def interp_cell(cell, period, k=100):
+    return {**cell, "power_grid_prop/base_power_props/mode": "interpolation",
+            "power_grid_prop/base_power_props/interp_update_period": period,
+            "power_grid_prop/base_power_props/interp_nb_agents": k}
+
+
+def fire_schedule(period, T, dt=4):
+    """Steps on which the interpolator fires after a reset that fired it (the counter starts at 0)."""
+    c, out = 0, []
+    for t in range(T):
+        c += dt
+        out.append(c >= period)
+        if c >= period:
+            c = 0
+    return out
+
+
+@pytest.mark.parametrize("route,period", INTERP_CASES)
+def test_route_interpolation_matches_oracle(route, period, monkeypatch):
+    """The first matrix cell of each route with the interpolated base power: re-anchored and free-running on the
+    oracle, the routes and launches of firing steps, of the steps after them and of the schedule regeneration."""
+    from oracle.config import synthetic_table
+
+    table = synthetic_table(7)
+    env, p, st, expect = _make(route, interp_cell(MATRIX[route][0], period), monkeypatch, table=table)
+    R, N = env.n_replicas, env.n_houses
+    drv = OracleDriver(env, p, st, table=table)
+    got = env.get_state()
+    assert np.all(got["t_since_interp"] == 0)            # the reset fired the interpolator
+    drv.check_base_power(got, 0, "reset")
+    drv.start_free()
+    T = 12
+    fires = fire_schedule(period, T)
+    fire_route = "four-kernel" if "DRSIM_NO_SHARD_KERNEL" in ROUTES[route][5] else "k_shard"
+    fire_launches = 4 if fire_route == "four-kernel" else 1
+    acts = (np.random.default_rng(200 + period).random((T, R, N)) < 0.5).astype(np.uint8)
+    valid = False   # the reset's refresh ended the schedule block
+    for t in range(T):
+        n = drv.step(acts[t])
+        want_route = fire_route if fires[t] else expect["route"]
+        want_n = (fire_launches if fires[t] else expect["launches"]) + (0 if valid else 2)
+        assert (env.sim.last_route, n) == (want_route, want_n), (t, fires[t], env.sim.last_route, n, want_route, want_n)
+        valid = not fires[t]
+    assert drv.fired == [t for t in range(T) if fires[t]], drv.fired
     drv.check_metrics()
     drv.check_free()
 
@@ -212,12 +269,22 @@ def test_seeded_sweep_matches_oracle(seed):
     cell = dict(pen=str(rng.choice(["individual_L2", "common_L2", "common_max_error", "mixture"])),
                 sig=str(rng.choice(["perlin", "sinusoidals", "regular_steps", "flat"])),
                 state=str(rng.choice(["none", "solar", "all"])), msg=str(rng.choice(["none", "th_hvac"])), nb=nb, c=c)
+    # the base-power mode from a stream of its own (the draws above are those of the constant-power sweep)
+    brng = np.random.default_rng(2000 + seed)
+    table = None
+    if brng.random() < 0.5:
+        from oracle.config import synthetic_table
+
+        table = synthetic_table(7)
+        cell = interp_cell(cell, int(brng.choice([3, 10, 12, 40])), int(brng.choice([1, 10, 100])))
     p = config(N, **cell)
-    env = BatchedEnv(p, R, precision=precision, obs_layout=layout, noise="philox", seed=seed)
+    env = BatchedEnv(p, R, precision=precision, obs_layout=layout, noise="philox", seed=seed, interp_table=table)
     print(seed, R, N, layout, precision, cell, env.sim.fused_info())
     st = synthetic_state(p, R, seed=seed)
     env.reset(copy.deepcopy(st))
-    drv = OracleDriver(env, p, st)
+    drv = OracleDriver(env, p, st, table=table)
+    if table is not None:
+        drv.check_base_power(env.get_state(), 0, "reset")
     T = 12
     acts = (rng.random((T, R, N)) < 0.5).astype(np.uint8)
     for t in range(T):
