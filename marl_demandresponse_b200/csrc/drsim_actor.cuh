@@ -1,20 +1,19 @@
 // drsim_actor.cuh -- MA-PPO actor on the observation rows, fused with the categorical draw
 // (SURVEY 8f-2; reference: agents/trainables/network.py:14-35 `Actor`, mappo.py:83-97 `select_actions`).
 //
-// The reference runs N batch-1 forwards of a [D -> h1 -> h2 -> 2] ReLU MLP per step on the CPU.  Here
-// one persistent CTA per SM takes 128 observation rows at a time:
-//
-//   A1 [128 x D]  (fp32 words, read as TF32)  x  W1^T  --tcgen05.mma-->  TMEM cols [0, N1)
-//   epilogue 1 (thread t owns row t = TMEM lane t): tcgen05.ld, + b1, ReLU  ->  A2 in shared memory
-//   A2 [128 x h1]                               x  W2^T  --tcgen05.mma-->  TMEM cols [N1, N1 + N2)
-//   epilogue 2: tcgen05.ld, + b2, ReLU, the 2-wide output layer on the CUDA cores, softmax,
-//               Philox uniform keyed (replica, house, step) -> action byte + probability of the draw
-//
-// Both GEMMs are issued by ONE thread per CTA (kind::tf32, cta_group::1, M = 128), accumulate in tensor
-// memory and signal completion through tcgen05.commit on an mbarrier.  Operands sit in shared memory in
-// the canonical no-swizzle K-major layout of the UMMA shared-memory descriptor: 8-row x 16-byte core
-// matrices, SBO = 128 B between 8-row groups, LBO = (rows / 8) * 128 B between 16-byte K chunks.  The
-// weights are converted once per CTA; only the 128 x D observation tile moves per iteration.
+// The reference runs N batch-1 forwards of a [D -> h1 -> h2 -> 2] ReLU MLP per step on the CPU.  Here a
+// persistent CTA takes 128 observation rows at a time (row t = TMEM lane t, UMMA M = 128); the hidden layers are
+// tcgen05 GEMMs issued by one thread per CTA (cta_group::1) into fp32 accumulators in tensor memory, and the
+// softmax and the Philox draw keyed (replica, house, step) -> action byte + probability of the draw follow in
+// the same kernel.  Three precisions:
+//   0 "tf32"    k_actor2: one TF32 pass per layer, the output layer a third GEMM;
+//   1 "tf32x3"  k_actor3<SplitTf32x3>: three TF32 passes per product on hi / lo halves (the default);
+//   2 "f16x3"   k_actor3<SplitF16x3>: three fp16 passes per product with per-neuron power-of-two weight scales.
+// A small pack kernel before each launch (k_actor_pack, k_actor_pack3x, k_actor_pack3h) converts the weights
+// once into the shared-memory image the actor kernel fetches; only the observation rows move per tile.
+// Operands sit in shared memory in the canonical no-swizzle K-major layout of the UMMA shared-memory
+// descriptor: 8-row x 16-byte core matrices, SBO = 128 B between 8-row groups, LBO = (rows / 8) * 128 B
+// between 16-byte K chunks.
 #pragma once
 
 #include <cuda_fp16.h>
@@ -25,13 +24,11 @@
 namespace drsim {
 
 constexpr int kActRows = 128;       // rows per tile == UMMA M == TMEM lanes
-constexpr int kActThreads = 128;    // one thread per row / TMEM lane
-constexpr int kActTmemCols = 256;   // power of two >= N1 + N2
 constexpr uint32_t PURPOSE_POLICY = 6;
 
 struct ActorArgs {
-  const void *obs;         // [rows][D] float, or __nv_bfloat16 (k_actor3x<PRE, __nv_bfloat16>)
-  const unsigned char *image;   // k_actor2: packed weight operands (k_actor_pack)
+  const void *obs;         // [rows][D] float, or __nv_bfloat16 (k_actor3<S, PRE, __nv_bfloat16>)
+  const unsigned char *image;   // packed weight operands (k_actor_pack, k_actor_pack3x, k_actor_pack3h)
   const float *w1, *b1;    // [h1][D], [h1]
   const float *w2, *b2;    // [h2][h1], [h2]
   const float *w3, *b3;    // [2][h2], [2]
@@ -40,14 +37,14 @@ struct ActorArgs {
   float *prob_on;          // [rows] or NULL: probability of action 1
   long long rows;          // R * Ns (padding slots included; they get action 0)
   int Ns, N, D, h1, h2;
-  int K1, N1, K2, N2, K3;  // padded: K multiple of 8 (UMMA_K of tf32), N multiple of 16 (K3: k_actor2's output layer)
-  int off_w1, off_w2, off_a1, off_a2, off_vec, off_bar, smem_bytes;
-  unsigned long long *dbg; // DRSIM_ACTOR_DBG: clock64 stamps [tile < 8][role][16] of CTA 0 (k_actor3x)
-  int off_w3, w_bytes;     // k_actor3x: the fp32 output layer in the image; size of one (hi or lo) weight block
+  int K1, N1, K2, N2, K3;  // padded: K multiple of UMMA_K (8 for tf32, 16 for f16), N multiple of 16 (K3: k_actor2's output layer)
+  int off_w1, off_w2, off_a1, off_a2, off_vec, off_bar, smem_bytes;   // off_a2, off_vec: k_actor2
+  unsigned long long *dbg; // DRSIM_ACTOR_DBG: clock64 stamps [tile < 8][role][16] of CTA 0 (k_actor3)
+  int off_w3, w_bytes;     // k_actor3: the fp32 output layer in the image; size of one (hi, d or lo) weight block
   unsigned long long seed;
   long long step, rep_offset;
-  int off_sc;              // k_actor3h: 2^-s of each layer-1 output column [N1] in the image
-  int *range_err;          // k_actor3h: mapped host flag, set when a live row's operand overflows fp16
+  int off_sc;              // k_actor3<SplitF16x3>: 2^-s of each layer-1 output column [N1] in the image
+  int *range_err;          // k_actor3<SplitF16x3>: mapped host flag, set when a live row's operand overflows fp16
 };
 
 // byte offset of element (row, k) of a K-major fp32 operand with `rows` rows in the canonical layout
@@ -89,21 +86,10 @@ DRSIM_D void umma_commit(uint64_t *bar) {
 // round-to-nearest (ties away from zero) TF32: the tensor core would otherwise truncate the 13 low mantissa bits.
 // Two integer instructions on the sign-magnitude bit pattern; `cvt.rna.tf32.f32` gives the same value for every
 // finite input but compiles to a six-instruction sequence with Inf / NaN handling on sm_100a, which made the
-// operand split of k_actor3x ALU-bound (activations and weights are finite).
+// operand split of k_actor3<SplitTf32x3> ALU-bound (activations and weights are finite).
 DRSIM_D float to_tf32(float x) { return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xffffe000u); }
 DRSIM_D void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 DRSIM_D void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-DRSIM_D void tmem_ld16(uint32_t taddr, float v[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
 // bounded wait on an mbarrier phase: a wedged tensor pipe must fail the launch, not hang the GPU
 DRSIM_D void mbar_wait_bounded(uint64_t *bar, uint32_t parity) {
   const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
@@ -124,7 +110,7 @@ DRSIM_D void mbar_wait_bounded(uint64_t *bar, uint32_t parity) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// k_actor2: the production variant.  Same network, but
+// k_actor2: the single-pass "tf32" precision:
 //   * two tiles in flight per CTA: 512 threads = two groups of 8 warps; group g owns tile slot g (its own
 //     observation buffers, TMEM columns, mbarrier and named barrier), so one slot runs its epilogue on the
 //     CUDA cores while the other's GEMM occupies the tensor core; the weights are shared;
@@ -412,9 +398,11 @@ __global__ void __launch_bounds__(kAct2Threads, 1) k_actor2(ActorArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// k_actor3x: the same network at fp32-grade accuracy on the same tensor cores ("3xTF32").
+// k_actor3<S, PRE, O>: the same network at fp32-grade accuracy on the same tensor cores, every product as three passes on
+// split operands.  S is the split: SplitTf32x3 ("3xTF32", precision 1, the default) or SplitF16x3 ("f16x3", precision 2,
+// below); the roles, the pipeline and the consumers are one code.
 //
-// A TF32 operand keeps 10 mantissa bits; splitting every operand into hi = tf32(x) and lo = tf32(x - hi) and
+// 3xTF32: a TF32 operand keeps 10 mantissa bits; splitting every operand into hi = tf32(x) and lo = tf32(x - hi) and
 // accumulating  A_hi W_hi + A_lo W_hi + A_hi W_lo  in the fp32 accumulator recovers ~21 bits per product (the
 // dropped A_lo W_lo term is 2^-22 relative): probabilities agree with a plain fp32 forward to ~1e-6 instead of
 // the 5e-3 of the single-pass kernel.
@@ -423,20 +411,20 @@ __global__ void __launch_bounds__(kAct2Threads, 1) k_actor2(ActorArgs a) {
 //   * producers (warps 0-7, two threads per row): the observation rows of the NEXT tile wait in registers; they
 //     are split into the hi / lo operands of layer 1 in shared memory (16-byte stores, canonical K-major layout),
 //     and after GEMM1 the accumulator R1 is turned into the layer-2 operand IN tensor memory: ReLU, hi in place,
-//     lo into a second column range L1.  This pass is pipelined with GEMM2 by 32-column chunks: a chunk's K steps
+//     lo into a second column range L1 (3xTF32).  This pass is pipelined with GEMM2 by 32-column chunks: a chunk's K steps
 //     are issued as soon as all rows have published it, so the tensor pipe idles for the first chunk only;
 //   * the MMA warp (warp 12, one thread): GEMM1 (shared x shared) and GEMM2 (A from tensor memory), three passes
 //     per K step, completion by tcgen05.commit on mbarriers;
 //   * consumers (warps 8-11, one thread per row): the layer-2 accumulator R2 is DOUBLE-buffered in tensor memory, so tile i's
 //     epilogue overlaps tile i+1's GEMMs: ReLU + the 2-wide output layer in plain fp32 FMAs straight from the
 //     tcgen05.ld registers (no third GEMM, no split, no write-back), softmax, Philox draw.
-// Tensor memory: R1 | L1 | R2[0] | R2[1] = 2 N1 + 2 N2 <= 512 columns.  Weight image (k_actor_pack3x):
+// 3xTF32 tensor memory: R1 | L1 | R2[0] | R2[1] = 2 N1 + 2 N2 <= 512 columns.  Weight image (k_actor_pack3x):
 // [w1_hi | w2_hi | w1_lo | w2_lo | w3 fp32 [2][N2] zero-padded, b3[2]], one TMA bulk copy per CTA.
+// The kernel is instantiated for the observation widths of S::kPre, so that the unrolled row handling carries no
+// predicated-off work.
 // ------------------------------------------------------------------------------------------------
 constexpr int kAct3Threads = 416;    // 8 producer warps + 4 consumer warps + the MMA warp (13 warps: 128 registers each)
 constexpr int kAct3MaxChunks = 5;    // 32-column chunks of the layer-2 operand (N1 <= 144)
-constexpr int kAct3PreChunks = 9;    // most 16-byte K chunks in HALF an observation row (K1 <= 72); the kernel is instantiated
-                                     // for 2 / 4 / 7 / 9 so that the unrolled row handling carries no predicated-off work
 
 DRSIM_D void pack_weights_split(unsigned char *dst_hi, unsigned char *dst_lo, const float *w, const float *b, int n_out, int n_in,
                                 int Np, int Kp, bool gen_one, int tid, int nthreads) {
@@ -491,369 +479,8 @@ DRSIM_D void tmem_wait_ld_dep(uint32_t r[16]) {
       a.dbg[(it * 3 + role) * 16 + (slot)] = (unsigned long long)clock64();                       \
   } while (0)
 
-// consumers of k_actor3h (warps 8-11, one thread per row): the consumer role of k_actor3x, statement for statement (kept
-// inline there so that its code stays as tuned) -- ReLU + the 2-wide output layer in plain fp32 FMAs straight from the
-// tcgen05.ld registers of the R2 slot, softmax, Philox draw
-DRSIM_D void act3_consumers(const ActorArgs &a, const unsigned char *smem, uint32_t R2, uint32_t lane_off, int n_my, int tid,
-                            int warp, uint64_t *bar2, uint64_t *r2_free, uint64_t *wbar) {
-  const int t = tid & 127, role = 1;
-  const float *w3 = reinterpret_cast<const float *>(smem + a.off_w3);   // [2][N2] zero-padded, then b3[2]
-  const int ng2 = (a.h2 + 15) >> 4;
-  if (n_my > 0) mbar_wait_bounded(wbar, 0);
-  for (int it = 0; it < n_my; ++it) {
-    const int s = it & 1;
-    const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-    const uint32_t src = R2 + (uint32_t)(s * a.N2) + lane_off;
-    float acc0 = w3[2 * a.N2], acc1 = w3[2 * a.N2 + 1];
-    ACT3_STAMP(0);
-    mbar_wait_bounded(bar2 + s, (uint32_t)((it >> 1) & 1));
-    tc_fence_after();
-    ACT3_STAMP(1);
-    // rounds of two 16-column granules; the next round's loads fly under this round's arithmetic, two accumulators
-    // per logit keep the FMA chains short
-    float acc2 = 0.f, acc3 = 0.f;
-    uint32_t r[2][2][16];
-    const int nrounds = (ng2 + 1) >> 1;
-    tmem_ld16_issue(src, r[0][0]);
-    if (1 < ng2) tmem_ld16_issue(src + 16u, r[0][1]);
-#pragma unroll
-    for (int rd = 0; rd < (kAct3MaxChunks + 1); ++rd) {
-      if (rd < nrounds) {
-        const int g = 2 * rd;
-        const bool two = g + 1 < ng2;
-        tmem_wait_ld_dep(r[rd & 1][0]);
-        if (two) tmem_wait_ld_dep(r[rd & 1][1]);
-        if (rd + 1 < nrounds) {
-          tmem_ld16_issue(src + (uint32_t)(16 * g + 32), r[(rd + 1) & 1][0]);
-          if (g + 3 < ng2) tmem_ld16_issue(src + (uint32_t)(16 * g + 48), r[(rd + 1) & 1][1]);
-        } else {                   // the slot's last loads have completed: GEMM2 of tile it + 2 may overwrite it
-          tc_fence_before();
-          mbar_arrive(r2_free + s);
-          ACT3_STAMP(2);
-        }
-        const float4 *wa = reinterpret_cast<const float4 *>(w3 + 16 * g), *wb = reinterpret_cast<const float4 *>(w3 + a.N2 + 16 * g);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float4 u = wa[q], v = wb[q];
-          const float x0 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 1]), 0.f),
-                      x2 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 3]), 0.f);
-          acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
-          acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
-        }
-        if (two) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float4 u = wa[4 + q], v = wb[4 + q];
-            const float x0 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 1]), 0.f),
-                        x2 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 3]), 0.f);
-            acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
-            acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
-          }
-        }
-      }
-    }
-    {
-      const float l0 = acc0 + acc2, l1 = acc1 + acc3;
-      const long long row = (long long)tile * kActRows + t;
-      if (row < a.rows) {
-        // replica / house of the row: 32-bit division whenever the row index allows it (the 64-bit one is ~100 instructions)
-        const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
-        const int n = (int)(row - rr * a.Ns);
-        uint8_t act = 0;
-        float p_draw = 0.f, p1 = 0.f;
-        if (n < a.N) {
-          const float m = fmaxf(l0, l1);                      // F.softmax(dim=1), network.py:34
-          const float e0 = expf(l0 - m), e1 = expf(l1 - m);
-          const float p0 = e0 / (e0 + e1);
-          p1 = e1 / (e0 + e1);
-          const U4 u = philox4x32_10(a.seed, (uint32_t)(a.rep_offset + rr), (uint32_t)n, (uint32_t)a.step, PURPOSE_POLICY);
-          const float uf = (float)(u.x >> 8) * 5.9604644775390625e-8f;   // 24 random bits: [0, 1) exactly
-          act = uf < p0 ? 0 : 1;
-          p_draw = act ? p1 : p0;
-        }
-        a.actions[row] = act;
-        if (a.prob) a.prob[row] = p_draw;
-        if (a.prob_on) a.prob_on[row] = p1;
-      }
-    }
-    ACT3_STAMP(3);
-  }
-}
-
-// O = element type of the observation rows.  bf16 rows are widened in the producers' load: a bf16 value is exact in
-// TF32, so its hi half is the value itself, its lo half zero, and the products equal those on the widened fp32 rows.
-template <int PRE, typename O = float>   // PRE: 16-byte K chunks per thread in the observation operand (>= K1 / 8)
-__global__ void __launch_bounds__(kAct3Threads, 1) k_actor3x(ActorArgs a) {
-  extern __shared__ __align__(1024) unsigned char smem[];
-  // mbarriers: 0 a1_ready (256) | 1 GEMM1 done | 2..6 a2_ready[chunk] (256) | 7, 8 GEMM2 done [slot] |
-  //            9, 10 R2 slot drained (128) | 11 weight image
-  uint64_t *s_bar = reinterpret_cast<uint64_t *>(smem + a.off_bar);
-  uint64_t *a1_ready = s_bar, *bar1 = s_bar + 1, *a2_ready = s_bar + 2, *bar2 = s_bar + 7, *r2_free = s_bar + 9, *wbar = s_bar + 11;
-  uint32_t *s_tmem = reinterpret_cast<uint32_t *>(s_bar + 12);
-  // the warp index through a shuffle: provably warp-uniform, so the role branches and the MMA warp's descriptor arithmetic
-  // stay on the uniform datapath (a divergent single-lane issuer costs ~100 cycles per tcgen05.mma: R2UR + an elect loop
-  // around every instruction, twice the 56 cycles the tensor pipe needs for it)
-  const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0), role = warp < 8 ? 0 : (warp < 12 ? 1 : 2);   // producer, consumer, MMA warp
-  const int t = tid & 127, part = (tid >> 7) & 1;                   // row of the tile (= TMEM lane), column half
-  const int n_tiles = (int)((a.rows + kActRows - 1) / kActRows);
-  const int n_my = blockIdx.x < n_tiles ? (n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-  unsigned char *s_a1h = smem + a.off_a1, *s_a1l = s_a1h + kActRows * a.K1 * 4;   // observation operand, hi and lo
-
-  if (tid == 0) {
-    mbar_init(a1_ready, 256);
-    mbar_init(bar1, 1);
-    for (int k = 0; k < kAct3MaxChunks; ++k) mbar_init(a2_ready + k, 256);
-    mbar_init(bar2, 1);
-    mbar_init(bar2 + 1, 1);
-    mbar_init(r2_free, 128);
-    mbar_init(r2_free + 1, 128);
-    mbar_init(wbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     (uint32_t)__cvta_generic_to_shared(s_tmem)),
-                 "r"((uint32_t)kAct2TmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  pdl_trigger();   // the env step behind us may become resident (it waits for our completion before it reads actions)
-  pdl_wait();      // the packed image, the observation rows; the action plane may still be read by the step before us
-  if (tid == 0) {  // the packed weight image (hi + lo + output layer): one TMA bulk copy per CTA
-    mbar_expect_tx(wbar, (uint32_t)a.off_a1);
-    bulk_load_g2s(smem, a.image, (uint32_t)a.off_a1, wbar);
-  }
-  const uint32_t tmem = *s_tmem;
-  const uint32_t R1 = tmem, L1 = tmem + (uint32_t)a.N1, R2 = tmem + (uint32_t)(2 * a.N1);   // R2 slot s at R2 + s * N2
-  const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;   // this warp's TMEM lane quadrant
-  const int ng = (a.K2 + 15) >> 4, nchunk = (ng + 1) >> 1;       // 16-column granules / 32-column chunks of the layer-2 operand
-
-  if (role == 0) {
-    // ---------------------------------------------------------------- producers
-    const int nch = a.K1 >> 2, c_lo = part ? nch / 2 : 0, c_hi = part ? nch : nch / 2;   // this thread's 16-byte K chunks
-    float pre[PRE * 4];
-    auto fetch = [&](int tile) {
-      const long long row = (long long)tile * kActRows + t;
-      const bool live = row < a.rows;
-      const O *g = static_cast<const O *>(a.obs) + (size_t)(live ? row : 0) * a.D;
-      if ((a.D & 1) == 0) {
-#pragma unroll
-        for (int j = 0; j < PRE * 2; ++j) {
-          const int k = c_lo * 4 + 2 * j;
-          float2 v = make_float2(0.f, 0.f);
-          if (live && k < c_hi * 4 && k < a.D) {
-            if constexpr (sizeof(O) == 2) v = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162 *>(g + k)));
-            else v = __ldg(reinterpret_cast<const float2 *>(g + k));
-          }
-          pre[2 * j] = v.x;
-          pre[2 * j + 1] = v.y;
-        }
-      } else {
-#pragma unroll
-        for (int j = 0; j < PRE * 4; ++j) {
-          const int k = c_lo * 4 + j;
-          pre[j] = (live && k < c_hi * 4 && k < a.D) ? (float)__ldg(g + k) : 0.f;
-        }
-      }
-    };
-    if (n_my > 0) fetch((int)blockIdx.x);
-    for (int it = 0; it < n_my; ++it) {
-      const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-      ACT3_STAMP(0);
-      // layer-1 operand: [obs | 1 | 0 ...] as hi + lo, one 16-byte store per K chunk (consecutive rows are contiguous:
-      // conflict-free).  The previous tile's GEMM1 has completed (bar1 was waited for below).
-#pragma unroll
-      for (int j = 0; j < PRE; ++j) {
-        const int c = c_lo + j;
-        if (c < c_hi) {
-          float v[4], h[4], l[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            v[i] = (4 * c + i == a.D) ? 1.f : pre[4 * j + i];
-            h[i] = to_tf32(v[i]);
-            l[i] = to_tf32(v[i] - h[i]);
-          }
-          const int off = c * (kActRows * 16) + t * 16;   // = umma_kmajor_off(kActRows, t, 4 c)
-          *reinterpret_cast<float4 *>(s_a1h + off) = make_float4(h[0], h[1], h[2], h[3]);
-          *reinterpret_cast<float4 *>(s_a1l + off) = make_float4(l[0], l[1], l[2], l[3]);
-        }
-      }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      mbar_arrive(a1_ready);
-      ACT3_STAMP(1);
-      if (it + 1 < n_my) fetch(tile + (int)gridDim.x);   // in flight during the rest of the round
-      ACT3_STAMP(2);
-      // layer-2 operand: A2 = relu(D1) as hi (in place) + lo, published chunk by chunk.  bar1 also covers GEMM2 of the
-      // previous tile (commit tracks everything issued before it): L1 is free to overwrite.
-      mbar_wait_bounded(bar1, (uint32_t)(it & 1));
-      tc_fence_after();
-      ACT3_STAMP(3);
-      uint32_t r[2][16];
-      const uint32_t src = R1 + lane_off;
-      if (part < ng) tmem_ld16_issue(src + (uint32_t)(16 * part), r[0]);
-#pragma unroll
-      for (int k = 0; k < kAct3MaxChunks; ++k) {
-        if (k < nchunk) {
-          const int g = 2 * k + part;                    // granule g of chunk k belongs to column half g & 1
-          if (g < ng) {
-            tmem_wait_ld_dep(r[k & 1]);
-            if (k + 1 < nchunk && g + 2 < ng)            // the next granule flies under this one
-              tmem_ld16_issue(src + (uint32_t)(16 * (g + 2)), r[(k + 1) & 1]);
-            uint32_t l[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-              const float x = fmaxf(__uint_as_float(r[k & 1][j]), 0.f);
-              const float hi = to_tf32(x);
-              r[k & 1][j] = __float_as_uint(hi);
-              l[j] = __float_as_uint(to_tf32(x - hi));
-            }
-            tmem_st16(R1 + lane_off + (uint32_t)(16 * g), r[k & 1]);
-            tmem_st16(L1 + lane_off + (uint32_t)(16 * g), l);
-            tmem_wait_st();
-          }
-          tc_fence_before();
-          mbar_arrive(a2_ready + k);
-          ACT3_STAMP(4 + k);
-        }
-      }
-    }
-  } else if (role == 2) {
-    // ---------------------------------------------------------------- MMA warp: one thread issues everything
-    if (n_my > 0 && elect_one_lane()) {
-      const uint32_t idesc1 = umma_instr_desc_tf32(kActRows, a.N1), idesc2 = umma_instr_desc_tf32(kActRows, a.N2);
-      const uint32_t w1h = (uint32_t)__cvta_generic_to_shared(smem + a.off_w1), w2h = (uint32_t)__cvta_generic_to_shared(smem + a.off_w2);
-      const uint32_t w1l = w1h + (uint32_t)a.w_bytes, w2l = w2h + (uint32_t)a.w_bytes;
-      const uint32_t a1h = (uint32_t)__cvta_generic_to_shared(s_a1h), a1l = (uint32_t)__cvta_generic_to_shared(s_a1l);
-      const uint32_t lbo_a = (kActRows / 8) * 128, lbo_w1 = (a.N1 / 8) * 128, lbo_w2 = (a.N2 / 8) * 128;
-      const int ks1 = a.K1 >> 3, ks2 = a.K2 >> 3;
-      mbar_wait_bounded(wbar, 0);   // the weight image has landed (async proxy -> tensor core: no proxy fence)
-      for (int it = 0; it < n_my; ++it) {
-        const int s = it & 1;
-        const uint32_t d2 = R2 + (uint32_t)(s * a.N2);
-        mbar_wait_bounded(a1_ready, (uint32_t)(it & 1));
-        tc_fence_after();
-        ACT3_STAMP(0);
-        for (int ks = 0; ks < ks1; ++ks) {      // layer 1: D1[128 x N1] = [obs | 1] . [W1 | b1]^T -- hi.hi, lo.hi, hi.lo
-          const uint64_t dah = umma_smem_desc(a1h + ks * 2 * lbo_a, lbo_a, 128), dal = umma_smem_desc(a1l + ks * 2 * lbo_a, lbo_a, 128);
-          const uint64_t dbh = umma_smem_desc(w1h + ks * 2 * lbo_w1, lbo_w1, 128), dbl = umma_smem_desc(w1l + ks * 2 * lbo_w1, lbo_w1, 128);
-          umma_tf32_ss(R1, dah, dbh, idesc1, ks > 0);
-          umma_tf32_ss(R1, dal, dbh, idesc1, 1);
-          umma_tf32_ss(R1, dah, dbl, idesc1, 1);
-        }
-        umma_commit(bar1);
-        ACT3_STAMP(1);
-        for (int k = 0; k < nchunk; ++k) {      // layer 2: D2[128 x N2] = A2 (tensor memory) . [W2 | b2]^T, chunk by chunk
-          mbar_wait_bounded(a2_ready + k, (uint32_t)(it & 1));
-          if (k == 0 && it >= 2) mbar_wait_bounded(r2_free + s, (uint32_t)(((it >> 1) & 1) ^ 1));   // tile it - 2 has left the slot
-          tc_fence_after();
-          ACT3_STAMP(2 + k);
-          const int ke = min(4 * k + 4, ks2);
-          for (int ks = 4 * k; ks < ke; ++ks) {
-            const uint64_t dbh = umma_smem_desc(w2h + ks * 2 * lbo_w2, lbo_w2, 128), dbl = umma_smem_desc(w2l + ks * 2 * lbo_w2, lbo_w2, 128);
-            umma_tf32_ts(d2, R1 + (uint32_t)(ks * 8), dbh, idesc2, ks > 0);
-            umma_tf32_ts(d2, L1 + (uint32_t)(ks * 8), dbh, idesc2, 1);
-            umma_tf32_ts(d2, R1 + (uint32_t)(ks * 8), dbl, idesc2, 1);
-          }
-        }
-        umma_commit(bar2 + s);
-        ACT3_STAMP(7);
-      }
-    }
-  } else {
-    // ---------------------------------------------------------------- consumers
-    const float *w3 = reinterpret_cast<const float *>(smem + a.off_w3);   // [2][N2] zero-padded, then b3[2]
-    const int ng2 = (a.h2 + 15) >> 4;
-    if (n_my > 0) mbar_wait_bounded(wbar, 0);
-    for (int it = 0; it < n_my; ++it) {
-      const int s = it & 1;
-      const int tile = (int)blockIdx.x + it * (int)gridDim.x;
-      const uint32_t src = R2 + (uint32_t)(s * a.N2) + lane_off;
-      float acc0 = w3[2 * a.N2], acc1 = w3[2 * a.N2 + 1];
-      ACT3_STAMP(0);
-      mbar_wait_bounded(bar2 + s, (uint32_t)((it >> 1) & 1));
-      tc_fence_after();
-      ACT3_STAMP(1);
-      // rounds of two 16-column granules; the next round's loads fly under this round's arithmetic, two accumulators
-      // per logit keep the FMA chains short
-      float acc2 = 0.f, acc3 = 0.f;
-      uint32_t r[2][2][16];
-      const int nrounds = (ng2 + 1) >> 1;
-      tmem_ld16_issue(src, r[0][0]);
-      if (1 < ng2) tmem_ld16_issue(src + 16u, r[0][1]);
-#pragma unroll
-      for (int rd = 0; rd < (kAct3MaxChunks + 1); ++rd) {
-        if (rd < nrounds) {
-          const int g = 2 * rd;
-          const bool two = g + 1 < ng2;
-          tmem_wait_ld_dep(r[rd & 1][0]);
-          if (two) tmem_wait_ld_dep(r[rd & 1][1]);
-          if (rd + 1 < nrounds) {
-            tmem_ld16_issue(src + (uint32_t)(16 * g + 32), r[(rd + 1) & 1][0]);
-            if (g + 3 < ng2) tmem_ld16_issue(src + (uint32_t)(16 * g + 48), r[(rd + 1) & 1][1]);
-          } else {                   // the slot's last loads have completed: GEMM2 of tile it + 2 may overwrite it
-            tc_fence_before();
-            mbar_arrive(r2_free + s);
-            ACT3_STAMP(2);
-          }
-          const float4 *wa = reinterpret_cast<const float4 *>(w3 + 16 * g), *wb = reinterpret_cast<const float4 *>(w3 + a.N2 + 16 * g);
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float4 u = wa[q], v = wb[q];
-            const float x0 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 1]), 0.f),
-                        x2 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 3]), 0.f);
-            acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
-            acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
-          }
-          if (two) {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const float4 u = wa[4 + q], v = wb[4 + q];
-              const float x0 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 1]), 0.f),
-                          x2 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 3]), 0.f);
-              acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
-              acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
-            }
-          }
-        }
-      }
-      {
-        const float l0 = acc0 + acc2, l1 = acc1 + acc3;
-        const long long row = (long long)tile * kActRows + t;
-        if (row < a.rows) {
-          // replica / house of the row: 32-bit division whenever the row index allows it (the 64-bit one is ~100 instructions)
-          const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
-          const int n = (int)(row - rr * a.Ns);
-          uint8_t act = 0;
-          float p_draw = 0.f, p1 = 0.f;
-          if (n < a.N) {
-            const float m = fmaxf(l0, l1);                      // F.softmax(dim=1), network.py:34
-            const float e0 = expf(l0 - m), e1 = expf(l1 - m);
-            const float p0 = e0 / (e0 + e1);
-            p1 = e1 / (e0 + e1);
-            const U4 u = philox4x32_10(a.seed, (uint32_t)(a.rep_offset + rr), (uint32_t)n, (uint32_t)a.step, PURPOSE_POLICY);
-            const float uf = (float)(u.x >> 8) * 5.9604644775390625e-8f;   // 24 random bits: [0, 1) exactly
-            act = uf < p0 ? 0 : 1;
-            p_draw = act ? p1 : p0;
-          }
-          a.actions[row] = act;
-          if (a.prob) a.prob[row] = p_draw;
-          if (a.prob_on) a.prob_on[row] = p1;
-        }
-      }
-      ACT3_STAMP(3);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*s_tmem), "r"((uint32_t)kAct2TmemCols) : "memory");
-}
-
 // ------------------------------------------------------------------------------------------------
-// k_actor3h: the "f16x3" precision -- k_actor3x's roles, pipeline and consumers, with all three passes of a product on fp16
+// SplitF16x3: the "f16x3" precision -- k_actor3's roles, pipeline and consumers, with all three passes of a product on fp16
 // halves (kind::f16, K = 16 per instruction instead of 8: C4's 100 x 100 actor issues 24 MMAs per tile instead of 45).
 //
 // Split, into ONE fp32 accumulator.  An fp16 value has 11 significant bits like TF32, so hi + lo carries 22 bits:
@@ -939,7 +566,7 @@ DRSIM_D float pack_row_f16x3(unsigned char *img, int w_bytes, int off, const flo
   return down;
 }
 
-// the image of k_actor3h, once per launch: one warp per output neuron of layers 1 and 2
+// the image of k_actor3<SplitF16x3>, once per launch: one warp per output neuron of layers 1 and 2
 __global__ void k_actor_pack3h(ActorArgs a, unsigned char *image) {
   pdl_trigger();
   const int lane = threadIdx.x & 31, wid = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), nw = (int)(gridDim.x * blockDim.x >> 5);
@@ -957,20 +584,108 @@ __global__ void k_actor_pack3h(ActorArgs a, unsigned char *image) {
   if (blockIdx.x == 0 && threadIdx.x < 2) w3[2 * a.N2 + threadIdx.x] = __ldg(a.b3 + threadIdx.x);
 }
 
-// PRE: 16-byte chunks (8 fp16 values) of the observation operand per producer thread, ceil(K1 / 16) with K1 = D + 1 rounded up
-// to 16; the instantiations 1 / 2 / 4 / 5 cover the observation widths of k_actor3x's 2 / 4 / 7 / 9.  O as for k_actor3x.
-template <int PRE, typename O = float>
-__global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
+// ------------------------------------------------------------------------------------------------
+// The operand split of k_actor3: everything in which precision 1 ("tf32x3") and precision 2 ("f16x3") differ.
+//   kEl          bytes of an operand element (a 16-byte chunk holds 16 / kEl values)
+//   kK           K of one MMA instruction
+//   kWBlocks     weight blocks in the image, w_bytes each: a K step multiplies A_hi by block 0, A_lo by block kWLo and
+//                A_hi by block kWHi
+//   kR1Sets      N1-wide column ranges in front of R2 in tensor memory
+//   kRangeCheck  fp16 range: padding slots enter as zero rows, layer 1's 2^-s sit in the image at off_sc, and the
+//                producers set a.range_err
+//   kPre         the PRE instantiations (16-byte K chunks of the observation operand per producer thread)
+// split_a1 writes 16 / kEl layer-1 values as one 16-byte chunk of A_hi and one of A_lo; split_a2 turns granule g of R1
+// (its 16 accumulator columns r, read from tensor-memory address col) into layer-2 A; mx collects the largest |A value|.
+// ------------------------------------------------------------------------------------------------
+struct SplitTf32x3 {   // fp32 as TF32 hi / lo; layer-2 A_lo in L1
+  static constexpr int kEl = 4, kK = 8, kWBlocks = 2, kWLo = 0, kWHi = 1, kR1Sets = 2;
+  static constexpr bool kRangeCheck = false;
+  static constexpr int kPre[4] = {2, 4, 7, 9};
+  static DRSIM_D uint32_t idesc(int N) { return umma_instr_desc_tf32(kActRows, N); }
+  static DRSIM_D void mma_ss(uint32_t d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t acc) { umma_tf32_ss(d, da, db, idesc, acc); }
+  static DRSIM_D void mma_ts(uint32_t d, uint32_t ta, uint64_t db, uint32_t idesc, uint32_t acc) { umma_tf32_ts(d, ta, db, idesc, acc); }
+  static DRSIM_D uint32_t a2_lo(int N1) { return (uint32_t)N1; }   // layer-2 A_lo, in columns from A_hi
+  static DRSIM_D void split_a1(const float (&v)[4], unsigned char *dh, unsigned char *dl, float &) {
+    float h[4], l[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      h[i] = to_tf32(v[i]);
+      l[i] = to_tf32(v[i] - h[i]);
+    }
+    *reinterpret_cast<float4 *>(dh) = make_float4(h[0], h[1], h[2], h[3]);
+    *reinterpret_cast<float4 *>(dl) = make_float4(l[0], l[1], l[2], l[3]);
+  }
+  // ReLU, hi in place, lo to L1
+  static DRSIM_D void split_a2(uint32_t (&r)[16], uint32_t col, int N1, const float *, float &) {
+    uint32_t l[16];
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+      const float x = fmaxf(__uint_as_float(r[j]), 0.f);
+      const float hi = to_tf32(x);
+      r[j] = __float_as_uint(hi);
+      l[j] = __float_as_uint(to_tf32(x - hi));
+    }
+    tmem_st16(col, r);
+    tmem_st16(col + (uint32_t)N1, l);
+  }
+};
+
+struct SplitF16x3 {    // fp16 hi / d / lo with per-neuron 2^s; layer-2 A as packed hi | lo pairs in place of R1
+  static constexpr int kEl = 2, kK = 16, kWBlocks = 3, kWLo = 1, kWHi = 2, kR1Sets = 1;
+  static constexpr bool kRangeCheck = true;
+  static constexpr int kPre[4] = {1, 2, 4, 5};
+  static DRSIM_D uint32_t idesc(int N) { return umma_instr_desc_f16(kActRows, N); }
+  static DRSIM_D void mma_ss(uint32_t d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t acc) { umma_f16_ss(d, da, db, idesc, acc); }
+  static DRSIM_D void mma_ts(uint32_t d, uint32_t ta, uint64_t db, uint32_t idesc, uint32_t acc) { umma_f16_ts(d, ta, db, idesc, acc); }
+  static DRSIM_D uint32_t a2_lo(int) { return 8u; }
+  static DRSIM_D void split_a1(const float (&v)[8], unsigned char *dh, unsigned char *dl, float &mx) {
+    uint32_t h[4], l[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      mx = fmaxf(mx, fmaxf(fabsf(v[2 * i]), fabsf(v[2 * i + 1])));
+      split_f16x2(v[2 * i], v[2 * i + 1], h[i], l[i]);
+    }
+    *reinterpret_cast<uint4 *>(dh) = make_uint4(h[0], h[1], h[2], h[3]);
+    *reinterpret_cast<uint4 *>(dl) = make_uint4(l[0], l[1], l[2], l[3]);
+  }
+  // ReLU(x 2^-s), s of each column from sc; packed hi pairs to [col, col + 8), lo pairs to [col + 8, col + 16)
+  static DRSIM_D void split_a2(uint32_t (&r)[16], uint32_t col, int, const float *sc, float &mx) {
+    const float4 *sc4 = reinterpret_cast<const float4 *>(sc);
+    uint32_t o[16];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const float4 u = sc4[q];
+      const float x0 = fmaxf(__uint_as_float(r[4 * q]) * u.x, 0.f), x1 = fmaxf(__uint_as_float(r[4 * q + 1]) * u.y, 0.f),
+                  x2 = fmaxf(__uint_as_float(r[4 * q + 2]) * u.z, 0.f), x3 = fmaxf(__uint_as_float(r[4 * q + 3]) * u.w, 0.f);
+      mx = fmaxf(mx, fmaxf(fmaxf(x0, x1), fmaxf(x2, x3)));
+      split_f16x2(x0, x1, o[2 * q], o[8 + 2 * q]);
+      split_f16x2(x2, x3, o[2 * q + 1], o[9 + 2 * q]);
+    }
+    tmem_st16(col, o);
+  }
+};
+
+// S: the split (SplitTf32x3, SplitF16x3).  PRE: 16-byte K chunks of the observation operand per producer thread, one of
+// S::kPre (>= K1 / S::kK).  O = element type of the observation rows.  bf16 rows are widened in the producers' load: a bf16
+// value is exact in TF32, so its hi half is the value itself, its lo half zero, and the products equal those on the widened
+// fp32 rows.
+template <class S, int PRE, typename O>
+__global__ void __launch_bounds__(kAct3Threads, 1) k_actor3(ActorArgs a) {
+  constexpr int kVec = 16 / S::kEl;   // operand values per 16-byte chunk
   extern __shared__ __align__(1024) unsigned char smem[];
-  // mbarriers as in k_actor3x
+  // mbarriers: 0 a1_ready (256) | 1 GEMM1 done | 2..6 a2_ready[chunk] (256) | 7, 8 GEMM2 done [slot] |
+  //            9, 10 R2 slot drained (128) | 11 weight image
   uint64_t *s_bar = reinterpret_cast<uint64_t *>(smem + a.off_bar);
   uint64_t *a1_ready = s_bar, *bar1 = s_bar + 1, *a2_ready = s_bar + 2, *bar2 = s_bar + 7, *r2_free = s_bar + 9, *wbar = s_bar + 11;
   uint32_t *s_tmem = reinterpret_cast<uint32_t *>(s_bar + 12);
-  const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0), role = warp < 8 ? 0 : (warp < 12 ? 1 : 2);
-  const int t = tid & 127, part = (tid >> 7) & 1;
+  // the warp index through a shuffle: provably warp-uniform, so the role branches and the MMA warp's descriptor arithmetic
+  // stay on the uniform datapath (a divergent single-lane issuer costs ~100 cycles per tcgen05.mma: R2UR + an elect loop
+  // around every instruction, twice the 56 cycles the tensor pipe needs for it)
+  const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0), role = warp < 8 ? 0 : (warp < 12 ? 1 : 2);   // producer, consumer, MMA warp
+  const int t = tid & 127, part = (tid >> 7) & 1;                   // row of the tile (= TMEM lane), column half
   const int n_tiles = (int)((a.rows + kActRows - 1) / kActRows);
   const int n_my = blockIdx.x < n_tiles ? (n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
-  unsigned char *s_a1h = smem + a.off_a1, *s_a1l = s_a1h + kActRows * a.K1 * 2;   // observation operand, hi and lo
+  unsigned char *s_a1h = smem + a.off_a1, *s_a1l = s_a1h + kActRows * a.K1 * S::kEl;   // observation operand, hi and lo
 
   if (tid == 0) {
     mbar_init(a1_ready, 256);
@@ -993,38 +708,40 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  pdl_trigger();
-  pdl_wait();
-  if (tid == 0) {
+  pdl_trigger();   // the env step behind us may become resident (it waits for our completion before it reads actions)
+  pdl_wait();      // the packed image, the observation rows; the action plane may still be read by the step before us
+  if (tid == 0) {  // the packed weight image (weight blocks + output layer): one TMA bulk copy per CTA
     mbar_expect_tx(wbar, (uint32_t)a.off_a1);
     bulk_load_g2s(smem, a.image, (uint32_t)a.off_a1, wbar);
   }
   const uint32_t tmem = *s_tmem;
-  const uint32_t R1 = tmem, R2 = tmem + (uint32_t)a.N1;             // R2 slot s at R2 + s * N2
-  const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
-  const int ng = a.K2 >> 4, nchunk = (ng + 1) >> 1;                  // 16-value granules / 32-column chunks of R1
+  const uint32_t R1 = tmem, R2 = tmem + (uint32_t)(S::kR1Sets * a.N1);   // R2 slot s at R2 + s * N2
+  const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;   // this warp's TMEM lane quadrant
+  const int ng = (a.K2 + 15) >> 4, nchunk = (ng + 1) >> 1;       // 16-column granules / 32-column chunks of R1
 
   if (role == 0) {
     // ---------------------------------------------------------------- producers
-    const int nch = a.K1 >> 3, c_lo = part ? nch / 2 : 0, c_hi = part ? nch : nch / 2;   // this thread's 16-byte K chunks
+    const int nch = (a.K1 * S::kEl) >> 4, c_lo = part ? nch / 2 : 0, c_hi = part ? nch : nch / 2;   // this thread's 16-byte K chunks
     const float *sc1 = reinterpret_cast<const float *>(smem + a.off_sc);
-    float pre[PRE * 8];
+    float pre[PRE * kVec];
     bool pre_live = false, bad = false;
     auto fetch = [&](int tile) {
       const long long row = (long long)tile * kActRows + t;
       bool live = row < a.rows;
-      if (live) {
-        const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
-        live = row - rr * a.Ns < a.N;
+      if constexpr (S::kRangeCheck) {
+        if (live) {
+          const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
+          live = row - rr * a.Ns < a.N;
+        }
+        pre_live = live;
       }
-      pre_live = live;
       const O *g = static_cast<const O *>(a.obs) + (size_t)(live ? row : 0) * a.D;
       if ((a.D & 1) == 0) {
 #pragma unroll
-        for (int j = 0; j < PRE * 4; ++j) {
-          const int k = c_lo * 8 + 2 * j;
+        for (int j = 0; j < PRE * kVec / 2; ++j) {
+          const int k = c_lo * kVec + 2 * j;
           float2 v = make_float2(0.f, 0.f);
-          if (live && k < c_hi * 8 && k < a.D) {
+          if (live && k < c_hi * kVec && k < a.D) {
             if constexpr (sizeof(O) == 2) v = __bfloat1622float2(__ldg(reinterpret_cast<const __nv_bfloat162 *>(g + k)));
             else v = __ldg(reinterpret_cast<const float2 *>(g + k));
           }
@@ -1033,9 +750,9 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
         }
       } else {
 #pragma unroll
-        for (int j = 0; j < PRE * 8; ++j) {
-          const int k = c_lo * 8 + j;
-          pre[j] = (live && k < c_hi * 8 && k < a.D) ? (float)__ldg(g + k) : 0.f;
+        for (int j = 0; j < PRE * kVec; ++j) {
+          const int k = c_lo * kVec + j;
+          pre[j] = (live && k < c_hi * kVec && k < a.D) ? (float)__ldg(g + k) : 0.f;
         }
       }
     };
@@ -1045,31 +762,26 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
       const bool live = pre_live;
       float mx = 0.f;   // largest |A value| of this row in this thread's columns
       ACT3_STAMP(0);
-      // layer-1 operand: [obs | 1 | 0 ...] as hi + lo, one 16-byte store per K chunk (8 values; conflict-free)
+      // layer-1 operand: [obs | 1 | 0 ...] as hi + lo, one 16-byte store per K chunk (consecutive rows are contiguous:
+      // conflict-free).  The previous tile's GEMM1 has completed (bar1 was waited for below).
 #pragma unroll
       for (int j = 0; j < PRE; ++j) {
         const int c = c_lo + j;
         if (c < c_hi) {
-          uint32_t h[4], l[4];
+          float v[kVec];
 #pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const float v0 = (8 * c + 2 * i == a.D) ? 1.f : pre[8 * j + 2 * i];
-            const float v1 = (8 * c + 2 * i + 1 == a.D) ? 1.f : pre[8 * j + 2 * i + 1];
-            mx = fmaxf(mx, fmaxf(fabsf(v0), fabsf(v1)));
-            split_f16x2(v0, v1, h[i], l[i]);
-          }
-          const int off = c * (kActRows * 16) + t * 16;
-          *reinterpret_cast<uint4 *>(s_a1h + off) = make_uint4(h[0], h[1], h[2], h[3]);
-          *reinterpret_cast<uint4 *>(s_a1l + off) = make_uint4(l[0], l[1], l[2], l[3]);
+          for (int i = 0; i < kVec; ++i) v[i] = (kVec * c + i == a.D) ? 1.f : pre[kVec * j + i];
+          const int off = c * (kActRows * 16) + t * 16;   // row t, 16-byte K chunk c of the canonical layout
+          S::split_a1(v, s_a1h + off, s_a1l + off, mx);
         }
       }
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       mbar_arrive(a1_ready);
       ACT3_STAMP(1);
-      if (it + 1 < n_my) fetch(tile + (int)gridDim.x);
+      if (it + 1 < n_my) fetch(tile + (int)gridDim.x);   // in flight during the rest of the round
       ACT3_STAMP(2);
-      // layer-2 operand: A2 = relu(D1 2^-s) as packed hi | lo pairs in place of each granule, published chunk by chunk.  bar1
-      // also covers GEMM2 of the previous tile, the last reader of R1.
+      // layer-2 operand from R1, published chunk by chunk.  bar1 also covers GEMM2 of the previous tile (commit tracks
+      // everything issued before it), the last reader of the layer-2 operand.
       mbar_wait_bounded(bar1, (uint32_t)(it & 1));
       tc_fence_after();
       ACT3_STAMP(3);
@@ -1079,22 +791,12 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
 #pragma unroll
       for (int k = 0; k < kAct3MaxChunks; ++k) {
         if (k < nchunk) {
-          const int g = 2 * k + part;
+          const int g = 2 * k + part;                    // granule g of chunk k belongs to column half g & 1
           if (g < ng) {
             tmem_wait_ld_dep(r[k & 1]);
-            if (k + 1 < nchunk && g + 2 < ng) tmem_ld16_issue(src + (uint32_t)(16 * (g + 2)), r[(k + 1) & 1]);
-            const float4 *sc = reinterpret_cast<const float4 *>(sc1 + 16 * g);
-            uint32_t o[16];
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              const float4 u = sc[q];
-              const float x0 = fmaxf(__uint_as_float(r[k & 1][4 * q]) * u.x, 0.f), x1 = fmaxf(__uint_as_float(r[k & 1][4 * q + 1]) * u.y, 0.f),
-                          x2 = fmaxf(__uint_as_float(r[k & 1][4 * q + 2]) * u.z, 0.f), x3 = fmaxf(__uint_as_float(r[k & 1][4 * q + 3]) * u.w, 0.f);
-              mx = fmaxf(mx, fmaxf(fmaxf(x0, x1), fmaxf(x2, x3)));
-              split_f16x2(x0, x1, o[2 * q], o[8 + 2 * q]);
-              split_f16x2(x2, x3, o[2 * q + 1], o[9 + 2 * q]);
-            }
-            tmem_st16(src + (uint32_t)(16 * g), o);
+            if (k + 1 < nchunk && g + 2 < ng)            // the next granule flies under this one
+              tmem_ld16_issue(src + (uint32_t)(16 * (g + 2)), r[(k + 1) & 1]);
+            S::split_a2(r[k & 1], src + (uint32_t)(16 * g), a.N1, sc1 + 16 * g, mx);
             tmem_wait_st();
           }
           tc_fence_before();
@@ -1102,45 +804,46 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
           ACT3_STAMP(4 + k);
         }
       }
-      bad |= live && mx >= kF16Overflow;
+      if constexpr (S::kRangeCheck) bad |= live && mx >= kF16Overflow;
     }
     if (bad) *reinterpret_cast<volatile int *>(a.range_err) = 1;
   } else if (role == 2) {
     // ---------------------------------------------------------------- MMA warp: one thread issues everything
     if (n_my > 0 && elect_one_lane()) {
-      const uint32_t idesc1 = umma_instr_desc_f16(kActRows, a.N1), idesc2 = umma_instr_desc_f16(kActRows, a.N2);
-      const uint32_t w1h = (uint32_t)__cvta_generic_to_shared(smem + a.off_w1), w2h = (uint32_t)__cvta_generic_to_shared(smem + a.off_w2);
-      const uint32_t wb = (uint32_t)a.w_bytes;   // W_hi, W_d, W_lo blocks
+      const uint32_t idesc1 = S::idesc(a.N1), idesc2 = S::idesc(a.N2);
+      const uint32_t w1 = (uint32_t)__cvta_generic_to_shared(smem + a.off_w1), w2 = (uint32_t)__cvta_generic_to_shared(smem + a.off_w2);
+      const uint32_t wlo = (uint32_t)(S::kWLo * a.w_bytes), whi = (uint32_t)(S::kWHi * a.w_bytes);   // weight blocks of passes 2, 3
       const uint32_t a1h = (uint32_t)__cvta_generic_to_shared(s_a1h), a1l = (uint32_t)__cvta_generic_to_shared(s_a1l);
+      const uint32_t a2l = S::a2_lo(a.N1);
       const uint32_t lbo_a = (kActRows / 8) * 128, lbo_w1 = (a.N1 / 8) * 128, lbo_w2 = (a.N2 / 8) * 128;
-      const int ks1 = a.K1 >> 4;
-      mbar_wait_bounded(wbar, 0);
+      const int ks1 = a.K1 / S::kK, ks2 = a.K2 / S::kK, kpc = 32 / S::kK;   // K steps of layer 1, of layer 2, per chunk
+      mbar_wait_bounded(wbar, 0);   // the weight image has landed (async proxy -> tensor core: no proxy fence)
       for (int it = 0; it < n_my; ++it) {
         const int s = it & 1;
         const uint32_t d2 = R2 + (uint32_t)(s * a.N2);
         mbar_wait_bounded(a1_ready, (uint32_t)(it & 1));
         tc_fence_after();
         ACT3_STAMP(0);
-        for (int ks = 0; ks < ks1; ++ks) {      // layer 1: hi.hi, lo.d, hi.lo
+        for (int ks = 0; ks < ks1; ++ks) {      // layer 1: D1[128 x N1] = [obs | 1] . [W1 | b1]^T
           const uint64_t dah = umma_smem_desc(a1h + ks * 2 * lbo_a, lbo_a, 128), dal = umma_smem_desc(a1l + ks * 2 * lbo_a, lbo_a, 128);
-          const uint32_t wk = w1h + ks * 2 * lbo_w1;
-          umma_f16_ss(R1, dah, umma_smem_desc(wk, lbo_w1, 128), idesc1, ks > 0);
-          umma_f16_ss(R1, dal, umma_smem_desc(wk + wb, lbo_w1, 128), idesc1, 1);
-          umma_f16_ss(R1, dah, umma_smem_desc(wk + 2 * wb, lbo_w1, 128), idesc1, 1);
+          const uint32_t wk = w1 + ks * 2 * lbo_w1;
+          S::mma_ss(R1, dah, umma_smem_desc(wk, lbo_w1, 128), idesc1, ks > 0);
+          S::mma_ss(R1, dal, umma_smem_desc(wk + wlo, lbo_w1, 128), idesc1, 1);
+          S::mma_ss(R1, dah, umma_smem_desc(wk + whi, lbo_w1, 128), idesc1, 1);
         }
         umma_commit(bar1);
         ACT3_STAMP(1);
-        for (int k = 0; k < nchunk; ++k) {      // layer 2: A2 from tensor memory, chunk by chunk
+        for (int k = 0; k < nchunk; ++k) {      // layer 2: D2[128 x N2] = A2 (tensor memory) . [W2 | b2]^T, chunk by chunk
           mbar_wait_bounded(a2_ready + k, (uint32_t)(it & 1));
-          if (k == 0 && it >= 2) mbar_wait_bounded(r2_free + s, (uint32_t)(((it >> 1) & 1) ^ 1));
+          if (k == 0 && it >= 2) mbar_wait_bounded(r2_free + s, (uint32_t)(((it >> 1) & 1) ^ 1));   // tile it - 2 has left the slot
           tc_fence_after();
           ACT3_STAMP(2 + k);
-          const int ge = min(2 * k + 2, ng);
-          for (int g = 2 * k; g < ge; ++g) {
-            const uint32_t wk = w2h + g * 2 * lbo_w2, ah = R1 + (uint32_t)(16 * g);
-            umma_f16_ts(d2, ah, umma_smem_desc(wk, lbo_w2, 128), idesc2, g > 0);
-            umma_f16_ts(d2, ah + 8u, umma_smem_desc(wk + wb, lbo_w2, 128), idesc2, 1);
-            umma_f16_ts(d2, ah, umma_smem_desc(wk + 2 * wb, lbo_w2, 128), idesc2, 1);
+          const int ke = min(kpc * k + kpc, ks2);
+          for (int ks = kpc * k; ks < ke; ++ks) {
+            const uint32_t wk = w2 + ks * 2 * lbo_w2, ah = R1 + (uint32_t)(ks * S::kK);
+            S::mma_ts(d2, ah, umma_smem_desc(wk, lbo_w2, 128), idesc2, ks > 0);
+            S::mma_ts(d2, ah + a2l, umma_smem_desc(wk + wlo, lbo_w2, 128), idesc2, 1);
+            S::mma_ts(d2, ah, umma_smem_desc(wk + whi, lbo_w2, 128), idesc2, 1);
           }
         }
         umma_commit(bar2 + s);
@@ -1148,7 +851,90 @@ __global__ void __launch_bounds__(kAct3Threads, 1) k_actor3h(ActorArgs a) {
       }
     }
   } else {
-    act3_consumers(a, smem, R2, lane_off, n_my, tid, warp, bar2, r2_free, wbar);
+    // ---------------------------------------------------------------- consumers
+    // one thread per row: ReLU + the 2-wide output layer in plain fp32 FMAs straight from the tcgen05.ld registers of the R2
+    // slot, softmax, Philox draw
+    const float *w3 = reinterpret_cast<const float *>(smem + a.off_w3);   // [2][N2] zero-padded, then b3[2]
+    const int ng2 = (a.h2 + 15) >> 4;
+    if (n_my > 0) mbar_wait_bounded(wbar, 0);
+    for (int it = 0; it < n_my; ++it) {
+      const int s = it & 1;
+      const int tile = (int)blockIdx.x + it * (int)gridDim.x;
+      const uint32_t src = R2 + (uint32_t)(s * a.N2) + lane_off;
+      float acc0 = w3[2 * a.N2], acc1 = w3[2 * a.N2 + 1];
+      ACT3_STAMP(0);
+      mbar_wait_bounded(bar2 + s, (uint32_t)((it >> 1) & 1));
+      tc_fence_after();
+      ACT3_STAMP(1);
+      // rounds of two 16-column granules; the next round's loads fly under this round's arithmetic, two accumulators
+      // per logit keep the FMA chains short
+      float acc2 = 0.f, acc3 = 0.f;
+      uint32_t r[2][2][16];
+      const int nrounds = (ng2 + 1) >> 1;
+      tmem_ld16_issue(src, r[0][0]);
+      if (1 < ng2) tmem_ld16_issue(src + 16u, r[0][1]);
+#pragma unroll
+      for (int rd = 0; rd < (kAct3MaxChunks + 1); ++rd) {
+        if (rd < nrounds) {
+          const int g = 2 * rd;
+          const bool two = g + 1 < ng2;
+          tmem_wait_ld_dep(r[rd & 1][0]);
+          if (two) tmem_wait_ld_dep(r[rd & 1][1]);
+          if (rd + 1 < nrounds) {
+            tmem_ld16_issue(src + (uint32_t)(16 * g + 32), r[(rd + 1) & 1][0]);
+            if (g + 3 < ng2) tmem_ld16_issue(src + (uint32_t)(16 * g + 48), r[(rd + 1) & 1][1]);
+          } else {                   // the slot's last loads have completed: GEMM2 of tile it + 2 may overwrite it
+            tc_fence_before();
+            mbar_arrive(r2_free + s);
+            ACT3_STAMP(2);
+          }
+          const float4 *wa = reinterpret_cast<const float4 *>(w3 + 16 * g), *wb = reinterpret_cast<const float4 *>(w3 + a.N2 + 16 * g);
+#pragma unroll
+          for (int q = 0; q < 4; ++q) {
+            const float4 u = wa[q], v = wb[q];
+            const float x0 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 1]), 0.f),
+                        x2 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][0][4 * q + 3]), 0.f);
+            acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
+            acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
+          }
+          if (two) {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              const float4 u = wa[4 + q], v = wb[4 + q];
+              const float x0 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q]), 0.f), x1 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 1]), 0.f),
+                          x2 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 2]), 0.f), x3 = fmaxf(__uint_as_float(r[rd & 1][1][4 * q + 3]), 0.f);
+              acc0 = fmaf(x0, u.x, acc0); acc2 = fmaf(x1, u.y, acc2); acc0 = fmaf(x2, u.z, acc0); acc2 = fmaf(x3, u.w, acc2);
+              acc1 = fmaf(x0, v.x, acc1); acc3 = fmaf(x1, v.y, acc3); acc1 = fmaf(x2, v.z, acc1); acc3 = fmaf(x3, v.w, acc3);
+            }
+          }
+        }
+      }
+      {
+        const float l0 = acc0 + acc2, l1 = acc1 + acc3;
+        const long long row = (long long)tile * kActRows + t;
+        if (row < a.rows) {
+          // replica / house of the row: 32-bit division whenever the row index allows it (the 64-bit one is ~100 instructions)
+          const long long rr = a.rows < (1ll << 31) ? (long long)((uint32_t)row / (uint32_t)a.Ns) : row / a.Ns;
+          const int n = (int)(row - rr * a.Ns);
+          uint8_t act = 0;
+          float p_draw = 0.f, p1 = 0.f;
+          if (n < a.N) {
+            const float m = fmaxf(l0, l1);                      // F.softmax(dim=1), network.py:34
+            const float e0 = expf(l0 - m), e1 = expf(l1 - m);
+            const float p0 = e0 / (e0 + e1);
+            p1 = e1 / (e0 + e1);
+            const U4 u = philox4x32_10(a.seed, (uint32_t)(a.rep_offset + rr), (uint32_t)n, (uint32_t)a.step, PURPOSE_POLICY);
+            const float uf = (float)(u.x >> 8) * 5.9604644775390625e-8f;   // 24 random bits: [0, 1) exactly
+            act = uf < p0 ? 0 : 1;
+            p_draw = act ? p1 : p0;
+          }
+          a.actions[row] = act;
+          if (a.prob) a.prob[row] = p_draw;
+          if (a.prob_on) a.prob_on[row] = p1;
+        }
+      }
+      ACT3_STAMP(3);
+    }
   }
   tc_fence_before();
   __syncthreads();

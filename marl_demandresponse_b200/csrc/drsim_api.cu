@@ -96,10 +96,10 @@ struct drsim_handle {
   unsigned char *h_snap = nullptr, *h_snap_dev = nullptr;
   size_t snap_bytes = 0, snap_obs_off = 0;
   bool snap_next = false, snap_fused = false;   // transient: the next small-cluster step writes the host snapshot itself
-  unsigned long long *actor_dbg = nullptr;   // DRSIM_ACTOR_DBG: phase stamps of CTA 0 of the last k_actor3x / k_actor3h launch
+  unsigned long long *actor_dbg = nullptr;   // DRSIM_ACTOR_DBG: phase stamps of CTA 0 of the last k_actor3 launch
   unsigned long long *shard_dbg = nullptr;   // DRSIM_SHARD_DBG: per-CTA time stamps of the last k_shard launch
   int *h_peer_err = nullptr, *h_peer_err_dev = nullptr;   // mapped: set by a kernel whose exchange wait timed out
-  int *h_actor_err = nullptr, *h_actor_err_dev = nullptr; // mapped: set by k_actor3h when an operand overflows fp16
+  int *h_actor_err = nullptr, *h_actor_err_dev = nullptr; // mapped: set by k_actor3<SplitF16x3> when an operand overflows fp16
   int pending_interp = 0;  // decision of drsim_step_begin, consumed by drsim_step_finish
   StepIn pending_in{};
   // pinned staging for drsim_step_host; h_env_dev = the same memory as the device sees it (mapped)
@@ -1927,7 +1927,18 @@ extern "C" int drsim_peer_status(drsim_t *h, void *stream) {
 static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t seed, const void *obs_in, uint8_t *actions_out,
                             float *prob_drawn, float *prob_on, void *stream);
 
-// the range flag of the f16x3 actor (k_actor3h), reported once and cleared
+using ActorKernel = void (*)(ActorArgs);
+
+// the k_actor3 instantiation for PRE = pre 16-byte K chunks per producer thread: the smallest of S::kPre that holds them
+template <class S, typename O>
+static ActorKernel act3_kernel(int pre) {
+  return pre <= S::kPre[0]   ? k_actor3<S, S::kPre[0], O>
+         : pre <= S::kPre[1] ? k_actor3<S, S::kPre[1], O>
+         : pre <= S::kPre[2] ? k_actor3<S, S::kPre[2], O>
+                             : k_actor3<S, S::kPre[3], O>;
+}
+
+// the range flag of the f16x3 actor (k_actor3<SplitF16x3>), reported once and cleared
 static int actor_range_error(drsim_t *h) {
   if (!h->h_actor_err || !*reinterpret_cast<volatile int *>(h->h_actor_err)) return 0;
   *reinterpret_cast<volatile int *>(h->h_actor_err) = 0;
@@ -1998,87 +2009,17 @@ static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t see
   a.Ns = p.Ns; a.N = p.N; a.D = p.obs_dim; a.h1 = net->h1; a.h2 = net->h2;
   int off = 0;
   auto take = [&](int b) { int o = off; off += (b + 127) / 128 * 128; return o; };
+  auto up = [](int x, int m) { return (x + m - 1) / m * m; };
   a.seed = seed; a.step = h->step; a.rep_offset = p.rep_offset;
   const int tiles = (int)((a.rows + kActRows - 1) / kActRows);
-  if (net->precision == 1) {
-    // 3xTF32: hi + lo operands, one CTA per SM, warp-specialised (see k_actor3x); the output layer runs in fp32 FMAs
-    a.K1 = (a.D + 1 + 7) / 8 * 8; a.N1 = (a.h1 + 1 + 15) / 16 * 16;
-    a.K2 = (a.h1 + 1 + 7) / 8 * 8; a.N2 = (a.h2 + 15) / 16 * 16;
-    a.K3 = a.N2;
-    if (2 * (a.N1 + a.N2) > 512)
-      return fail(DRSIM_E_ARG, "drsim_policy_step: h1 + h2 too wide for the split activations in tensor memory");
-    a.off_w1 = take(a.N1 * a.K1 * 4); a.off_w2 = take(a.N2 * a.K2 * 4);
-    a.w_bytes = off;                              // one (hi or lo) weight block
-    off = 2 * a.w_bytes;
-    a.off_w3 = take((2 * a.N2 + 2) * 4);          // output layer, plain fp32
-    a.off_vec = a.off_w3;
-    a.off_a1 = off;                               // = size of the packed image
-    take(2 * kActRows * a.K1 * 4);                // observation operand, hi and lo
-    a.off_a2 = off;                               // (no staging buffer: the next tile's rows wait in registers)
-    a.off_bar = take(128);
-    a.smem_bytes = off;
-    if (a.smem_bytes > 227 * 1024)
-      return fail(DRSIM_E_ARG, "drsim_policy_step: network / observation too wide for the 3xTF32 variant's shared memory "
-                               "(hi + lo weight halves); use precision = 0");
-    if (!h->actor_image) CU_TRY(cudaMalloc(&h->actor_image, 256 * 1024));
-    a.image = h->actor_image;
-    if (!h->actor_dbg && getenv("DRSIM_ACTOR_DBG")) {
-      CU_TRY(cudaMalloc(&h->actor_dbg, 8 * 3 * 16 * 8));
-      CU_TRY(cudaMemset(h->actor_dbg, 0, 8 * 3 * 16 * 8));
-    }
-    a.dbg = h->actor_dbg;
-    k_actor_pack3x<<<40, 512, 0, (cudaStream_t)stream>>>(a, h->actor_image);
-    const int pre = a.K1 / 8;                     // 16-byte K chunks per producer thread
-    auto kern = bf16 ? (pre <= 2   ? k_actor3x<2, __nv_bfloat16>
-                        : pre <= 4 ? k_actor3x<4, __nv_bfloat16>
-                        : pre <= 7 ? k_actor3x<7, __nv_bfloat16>
-                                   : k_actor3x<kAct3PreChunks, __nv_bfloat16>)
-                     : (pre <= 2 ? k_actor3x<2> : pre <= 4 ? k_actor3x<4> : pre <= 7 ? k_actor3x<7> : k_actor3x<kAct3PreChunks>);
-    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
-    launch_pdl(kern, std::min(tiles, h->sm_count), kAct3Threads, (size_t)a.smem_bytes, (cudaStream_t)stream, a);
-    h->launches++;
-  } else if (net->precision == 2) {
-    // f16x3: fp16 hi / d / lo operands with per-neuron power-of-two scales, k_actor3x's roles (see k_actor3h).  K is a multiple
-    // of 16 (UMMA_K of kind::f16).  The widest accepted shape (D = 64, h1 = h2 = 128) takes 222,592 bytes of shared memory and
-    // N1 + 2 N2 = 400 tensor-memory columns: no width within the limits above is refused.
-    if (!h->h_actor_err_dev) return fail(DRSIM_E_CUDA, "drsim_policy_step: f16x3 needs mapped host memory for its range flag");
-    a.K1 = (a.D + 1 + 15) / 16 * 16; a.N1 = (a.h1 + 1 + 15) / 16 * 16;
-    a.K2 = a.N1; a.N2 = (a.h2 + 15) / 16 * 16;
-    a.K3 = a.N2;
-    a.off_w1 = take(a.N1 * a.K1 * 2); a.off_w2 = take(a.N2 * a.K2 * 2);
-    a.w_bytes = off;                              // one (hi, d or lo) weight block
-    off = 3 * a.w_bytes;
-    a.off_sc = take(a.N1 * 4);                    // 2^-s of the layer-1 columns
-    a.off_w3 = take((2 * a.N2 + 2) * 4);          // output layer, fp32, carrying the layer-2 2^-s
-    a.off_vec = a.off_w3;
-    a.off_a1 = off;                               // = size of the packed image
-    take(2 * kActRows * a.K1 * 2);                // observation operand, hi and lo
-    a.off_a2 = off;
-    a.off_bar = take(128);
-    a.smem_bytes = off;
-    a.range_err = h->h_actor_err_dev;
-    if (!h->actor_image) CU_TRY(cudaMalloc(&h->actor_image, 256 * 1024));
-    a.image = h->actor_image;
-    if (!h->actor_dbg && getenv("DRSIM_ACTOR_DBG")) {
-      CU_TRY(cudaMalloc(&h->actor_dbg, 8 * 3 * 16 * 8));
-      CU_TRY(cudaMemset(h->actor_dbg, 0, 8 * 3 * 16 * 8));
-    }
-    a.dbg = h->actor_dbg;
-    k_actor_pack3h<<<(a.N1 + a.N2 + 15) / 16, 512, 0, (cudaStream_t)stream>>>(a, h->actor_image);
-    const int pre = a.K1 / 16;                    // 16-byte chunks (8 fp16 values) per producer thread
-    auto kern = bf16 ? (pre <= 1   ? k_actor3h<1, __nv_bfloat16>
-                        : pre <= 2 ? k_actor3h<2, __nv_bfloat16>
-                        : pre <= 4 ? k_actor3h<4, __nv_bfloat16>
-                                   : k_actor3h<5, __nv_bfloat16>)
-                     : (pre <= 1 ? k_actor3h<1> : pre <= 2 ? k_actor3h<2> : pre <= 4 ? k_actor3h<4> : k_actor3h<5>);
-    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
-    launch_pdl(kern, std::min(tiles, h->sm_count), kAct3Threads, (size_t)a.smem_bytes, (cudaStream_t)stream, a);
-    h->launches++;
-  } else {
+  const cudaStream_t st = (cudaStream_t)stream;
+  ActorKernel kern = k_actor2;
+  int grid = std::min((tiles + 1) / 2, h->sm_count), threads = kAct2Threads;
+  if (net->precision == 0) {
     // one spare K column per layer carries the bias (constant-one column in A), one spare output row regenerates the one
-    a.K1 = (a.D + 1 + 7) / 8 * 8; a.N1 = (a.h1 + 1 + 15) / 16 * 16;
-    a.K2 = (a.h1 + 1 + 7) / 8 * 8; a.N2 = (a.h2 + 1 + 15) / 16 * 16;
-    a.K3 = (a.h2 + 1 + 7) / 8 * 8;
+    a.K1 = up(a.D + 1, 8); a.N1 = up(a.h1 + 1, 16);
+    a.K2 = up(a.h1 + 1, 8); a.N2 = up(a.h2 + 1, 16);
+    a.K3 = up(a.h2 + 1, 8);
     if (a.N1 + a.N2 + kActN3 > 256)
       return fail(DRSIM_E_ARG, "drsim_policy_step: h1 + h2 too wide for two tile slots in tensor memory (N1 + N2 + 16 <= 256 "
                                "columns, N1 = h1 + 1 and N2 = h2 + 1 each rounded up to 16)");
@@ -2089,14 +2030,52 @@ static int policy_step_impl(drsim_t *h, const drsim_actor_net *net, uint64_t see
     a.off_bar = take(128);
     a.smem_bytes = off;
     if (a.smem_bytes > 227 * 1024) return fail(DRSIM_E_ARG, "drsim_policy_step: network / observation too wide for shared memory");
-    if (!h->actor_image) CU_TRY(cudaMalloc(&h->actor_image, 256 * 1024));
-    a.image = h->actor_image;
-    k_actor_pack<<<40, 512, 0, (cudaStream_t)stream>>>(a, h->actor_image);
-    CU_TRY(cudaFuncSetAttribute(k_actor2, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
-    launch_pdl(k_actor2, std::min((tiles + 1) / 2, h->sm_count), kAct2Threads, (size_t)a.smem_bytes, (cudaStream_t)stream, a);
-    h->launches++;
+  } else {
+    // k_actor3<S>: split operands (S = SplitTf32x3 for precision 1, SplitF16x3 for 2), one CTA per SM, warp-specialised; the
+    // output layer runs in fp32 FMAs.  The widest f16x3 shape (D = 64, h1 = h2 = 128) takes 222,592 bytes of shared memory and
+    // N1 + 2 N2 = 400 tensor-memory columns: no f16x3 width within the limits above is refused.
+    auto layout = [&](auto split) -> int {
+      using S = decltype(split);
+      if (S::kRangeCheck && !h->h_actor_err_dev)
+        return fail(DRSIM_E_CUDA, "drsim_policy_step: f16x3 needs mapped host memory for its range flag");
+      a.K1 = up(a.D + 1, S::kK); a.N1 = up(a.h1 + 1, 16);
+      a.K2 = up(a.h1 + 1, S::kK); a.N2 = up(a.h2, 16);
+      if (S::kR1Sets * a.N1 + 2 * a.N2 > 512)
+        return fail(DRSIM_E_ARG, "drsim_policy_step: h1 + h2 too wide for the split activations in tensor memory");
+      a.off_w1 = take(a.N1 * a.K1 * S::kEl); a.off_w2 = take(a.N2 * a.K2 * S::kEl);
+      a.w_bytes = off;                              // one weight block
+      off = S::kWBlocks * a.w_bytes;
+      if (S::kRangeCheck) a.off_sc = take(a.N1 * 4);   // 2^-s of the layer-1 columns
+      a.off_w3 = take((2 * a.N2 + 2) * 4);          // output layer, fp32 (f16x3: carrying the layer-2 2^-s)
+      a.off_a1 = off;                               // = size of the packed image
+      take(2 * kActRows * a.K1 * S::kEl);           // observation operand, hi and lo (the next tile's rows wait in registers)
+      a.off_bar = take(128);
+      a.smem_bytes = off;
+      if (a.smem_bytes > 227 * 1024)
+        return fail(DRSIM_E_ARG, "drsim_policy_step: network / observation too wide for the 3xTF32 variant's shared memory "
+                                 "(hi + lo weight halves); use precision = 0");
+      const int pre = a.K1 / S::kK;                 // 16-byte K chunks per producer thread
+      kern = bf16 ? act3_kernel<S, __nv_bfloat16>(pre) : act3_kernel<S, float>(pre);
+      return 0;
+    };
+    if (int rc = net->precision == 1 ? layout(SplitTf32x3{}) : layout(SplitF16x3{})) return rc;
+    a.range_err = h->h_actor_err_dev;
+    grid = std::min(tiles, h->sm_count);
+    threads = kAct3Threads;
+    if (!h->actor_dbg && getenv("DRSIM_ACTOR_DBG")) {
+      CU_TRY(cudaMalloc(&h->actor_dbg, 8 * 3 * 16 * 8));
+      CU_TRY(cudaMemset(h->actor_dbg, 0, 8 * 3 * 16 * 8));
+    }
+    a.dbg = h->actor_dbg;
   }
-  h->launches++;
+  if (!h->actor_image) CU_TRY(cudaMalloc(&h->actor_image, 256 * 1024));
+  a.image = h->actor_image;
+  if (net->precision == 0) k_actor_pack<<<40, 512, 0, st>>>(a, h->actor_image);
+  else if (net->precision == 1) k_actor_pack3x<<<40, 512, 0, st>>>(a, h->actor_image);
+  else k_actor_pack3h<<<(a.N1 + a.N2 + 15) / 16, 512, 0, st>>>(a, h->actor_image);
+  CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, a.smem_bytes));
+  launch_pdl(kern, grid, threads, (size_t)a.smem_bytes, st, a);
+  h->launches += 2;   // pack + actor
   CU_TRY(cudaGetLastError());
   return 0;
 }
@@ -2128,7 +2107,7 @@ extern "C" int drsim_debug_tile_phases(unsigned long long *host_out, int max_cta
 }
 
 // diagnostics, not part of the documented ABI: clock64 stamps [tile < 8][producer, consumer, MMA warp][16] of CTA 0 of the
-// last k_actor3x / k_actor3h launch (DRSIM_ACTOR_DBG=1)
+// last k_actor3 launch (DRSIM_ACTOR_DBG=1)
 extern "C" int drsim_debug_actor_times(drsim_t *h, unsigned long long *host_out) {
   if (!h || !h->actor_dbg || !host_out) return 0;
   cudaMemcpy(host_out, h->actor_dbg, 8 * 3 * 16 * 8, cudaMemcpyDeviceToHost);

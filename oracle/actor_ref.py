@@ -9,7 +9,7 @@ probability of action 1 per row and a per-row bound on ``|p_kernel - p_ref|``.
 column); after each ReLU the activation is rounded to TF32 in tensor memory; the output layer is a TF32 GEMM too;
 softmax with ``__expf`` and ``p1 = 1 - p0``.
 
-``k_actor3x`` ("tf32x3"): every GEMM operand is split as ``hi = tf32(x)``, ``lo = tf32(x - hi)`` and the products are
+``k_actor3<SplitTf32x3>`` ("tf32x3"): every GEMM operand is split as ``hi = tf32(x)``, ``lo = tf32(x - hi)`` and the products are
 accumulated as ``A_hi W_hi + A_lo W_hi + A_hi W_lo`` (layers 1 and 2, bias again in the GEMM); ReLU on fp32 activations;
 the output layer in fp32 FMAs on plain fp32 ``w3``, ``b3``; softmax with ``expf`` and ``p1 = e1 / (e0 + e1)``.
 
@@ -94,7 +94,7 @@ def _dot(a, ra, w, b, n_terms):
 
 
 def _dot3x(a, ra, w, b):
-    """Layer of ``k_actor3x``: ``A_hi W_hi + A_lo W_hi + A_hi W_lo`` with the bias as the K column of a constant one."""
+    """Layer of ``k_actor3<SplitTf32x3>``: ``A_hi W_hi + A_lo W_hi + A_hi W_lo`` with the bias as the K column of a constant one."""
     a_hi, a_lo = split(a)
     w_hi, w_lo = split(w)
     b_hi, b_lo = split(b)
@@ -171,7 +171,7 @@ def forward32(rows, w1, b1, w2, b2, w3, b3):
 
 
 def fp32_grade_tolerance(rows, *net):
-    """What ``k_actor3x`` promises beyond the operand-exact bound: fp32-grade probabilities, within
+    """What ``k_actor3<SplitTf32x3>`` promises beyond the operand-exact bound: fp32-grade probabilities, within
     ``2e-6 + 2 max |p_fp32 - p_fp64|`` of the plain fp64 forward on the same rows (the rule of the torch comparison in
     test_gpu_batched).  The first-principles bound of ``forward`` charges every accumulation its worst case and is too
     wide to tell three TF32 passes from one; this tolerance is not, since a single pass is ~2^-11 off per product."""
@@ -211,7 +211,7 @@ def sample_net(rng, d: int, h1: int, h2: int, out_scale: float = 1.0):
 
 
 def emulate_split_product(a, w):
-    """``a * w`` the way ``k_actor3x`` forms one product from fp32 operands (hi.hi + lo.hi + hi.lo, exact products),
+    """``a * w`` the way ``k_actor3<SplitTf32x3>`` forms one product from fp32 operands (hi.hi + lo.hi + hi.lo, exact products),
     in fp64: for the reference's own tests."""
     a_hi, a_lo = split(np.asarray(a, dtype=np.float32))
     w_hi, w_lo = split(np.asarray(w, dtype=np.float32))

@@ -1,5 +1,5 @@
-"""Per-role phase time lines of k_actor3x ("tf32x3") or k_actor3h ("f16x3") (CTA 0, first 8 tiles), from the clock64
-stamps of DRSIM_ACTOR_DBG=1.  Both kernels stamp the same phases; k_actor3h's chunks are 32 columns of R1 as well.
+"""Per-role phase time lines of k_actor3 ("tf32x3" or "f16x3") (CTA 0, first 8 tiles), from the clock64
+stamps of DRSIM_ACTOR_DBG=1.  Both precisions stamp the same phases; a chunk is 32 columns of R1 in both.
 
     DRSIM_ACTOR_DBG=1 python profiles/tools/actor_phases.py [c3|c4] [tf32x3|f16x3]
 """

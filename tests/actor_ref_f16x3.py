@@ -1,4 +1,4 @@
-"""Operand-exact reference of the "f16x3" actor (``k_actor3h`` of ``csrc/drsim_actor.cuh``) -- test infrastructure, in the
+"""Operand-exact reference of the "f16x3" actor (``k_actor3<SplitF16x3>`` of ``csrc/drsim_actor.cuh``) -- test infrastructure, in the
 manner of ``oracle/actor_ref.py`` (whose ``KERNELS`` / ``forward`` cover "tf32" and "tf32x3"; the rules below extend its
 radius rules to the fp16 split).
 
@@ -10,7 +10,7 @@ The kernel, operand for operand (layers 1 and 2; ``[a | 1]`` and ``[W | b]`` are
   ``A_lo = fp16((x - A_hi) 2^11)`` (fp16: round to nearest even, subnormals, overflow to infinity from 65520 on);
 * ``D' = A_hi W_hi + A_lo W_d + A_hi W_lo`` accumulated in fp32; layer 1: ``a1 = relu(D' 2^-s)`` (producers); layer 2:
   ``relu(D')`` times ``fp32(w3 2^-s)`` (consumers) -- the same fp32 product as ``relu(D' 2^-s) w3``;
-* output layer in fp32 FMAs, softmax with ``expf``, ``p1 = e1 / (e0 + e1)`` (as ``k_actor3x``);
+* output layer in fp32 FMAs, softmax with ``expf``, ``p1 = e1 / (e0 + e1)`` (as ``k_actor3<SplitTf32x3>``);
 * range: a live row whose observation elements or hidden activations reach ``|x| >= 65520`` sets the handle's flag.
 
 Radius rules beyond ``oracle/actor_ref.py``: with ``u = 2^-11`` and normal fp16 halves, ``x = A_hi + A_lo u + e_a`` with
@@ -72,7 +72,7 @@ def split_weights(w_aug):
 
 
 def _layer(a, ra, w, b):
-    """One tensor-core layer of ``k_actor3h``: value (unscaled, before ReLU) and radius.  ``a`` fp64 ``[M, K]`` with
+    """One tensor-core layer of ``k_actor3<SplitF16x3>``: value (unscaled, before ReLU) and radius.  ``a`` fp64 ``[M, K]`` with
     radius ``ra``; ``w``, ``b`` fp32."""
     w_aug = np.concatenate([np.asarray(w, np.float32), np.asarray(b, np.float32)[:, None]], axis=1)
     w_hi, w_d, w_lo, s = split_weights(w_aug)

@@ -68,7 +68,7 @@ def _trunc(x):
 
 def _emulate(rows, net, kernel, rnd=ar.tf32, passes=("hh", "lh", "hl")):
     """The kernel in NumPy fp32 (BLAS accumulation order, ``rnd`` for every TF32 rounding); ``passes``: the split
-    products ``k_actor3x`` accumulates (hi.hi, lo.hi, hi.lo)."""
+    products ``k_actor3<SplitTf32x3>`` accumulates (hi.hi, lo.hi, hi.lo)."""
     w1, b1, w2, b2, w3, b3 = net
     if kernel == "tf32":
         a = rnd(rows)

@@ -1,4 +1,4 @@
-"""The tcgen05 actor kernels (``k_actor2`` = "tf32", ``k_actor3x<PRE, O>`` = "tf32x3") against the operand-exact
+"""The tcgen05 actor kernels (``k_actor2`` = "tf32", ``k_actor3<SplitTf32x3, PRE, O>`` = "tf32x3") against the operand-exact
 reference ``oracle.actor_ref``: every row's ``prob_on`` must lie within the reference's first-principles error bound.
 
 The rows are synthetic (``actor_ref.sample_rows``: four decades of magnitudes, exact zeros, values on TF32 ties, a few
@@ -7,7 +7,7 @@ step.  The handle has stepped a few times first (the draw is keyed by a step ind
 non-zero global index and the seed uses both key words of the Philox draw.  Padding slots (house >= N) hold huge finite
 values: they must still get action 0 and probability 0, and leave every other row bit-identical.
 
-Covered: every ``k_actor3x`` instantiation (PRE = 2, 4, 7, 9) with fp32 and bf16 rows of even and odd width, and
+Covered: every ``k_actor3<SplitTf32x3>`` instantiation (PRE = 2, 4, 7, 9) with fp32 and bf16 rows of even and odd width, and
 ``k_actor2`` on the fp32 rows; hidden widths from 1 to 128 up to each kernel's tensor- and shared-memory limits; row
 counts below one tile, one row into a tile, and many tiles per CTA; all output-pointer combinations; the refusals."""
 import ctypes as C
@@ -40,7 +40,7 @@ def _comm(c, **over):
 
 
 WIDTHS = {
-    10: ("tarmac", {}),                                          # k_actor3x<2>
+    10: ("tarmac", {}),                                          # k_actor3<SplitTf32x3, 2>
     11: ("tarmac", _SOLAR),
     22: ("hand_engineered", _comm(3)),                           # <4>
     23: ("hand_engineered", _comm(3, **_SOLAR)),
@@ -227,7 +227,7 @@ def test_network_widths(d, h1, h2, kernel):
     tmem, smem, ok = actor_layout(d, h1, h2, kernel)
     assert ok
     if (h1, h2) in ((128, 95), (127, 111), (111, 127), (128, 112), (127, 128)):
-        assert tmem == 512        # k_actor2: both 256-column slots full; k_actor3x: R1 | L1 | R2[0] | R2[1] fill 512
+        assert tmem == 512        # k_actor2: both 256-column slots full; k_actor3 (tf32x3): R1 | L1 | R2[0] | R2[1] fill 512
     if (d, h1, h2) == (47, 120, 127):
         assert SMEM_MAX - 2048 < smem <= SMEM_MAX
     env = _env(d, 99, 13)
@@ -239,7 +239,7 @@ def test_network_widths(d, h1, h2, kernel):
 @pytest.mark.parametrize("dtype,kernels", [("float32", ("tf32x3", "tf32")), ("bfloat16", ("tf32x3",))])
 @pytest.mark.parametrize("r,n", [(3, 37), (9, 99), (1600, 99)])
 def test_row_counts(r, n, dtype, kernels):
-    # 120 rows; 900 = 7 * 128 + 4; 160000 rows = 1250 tiles: each of 148 CTAs takes about 8.4 tiles (k_actor3x: both
+    # 120 rows; 900 = 7 * 128 + 4; 160000 rows = 1250 tiles: each of 148 CTAs takes about 8.4 tiles (k_actor3: both
     # R2 slots recycled four times) or 4.2 per tile slot (k_actor2)
     env = _env(11, n, r, dtype)
     _case(env, 11, 100, 100, kernels, seed=r, what=f"R={r} N={n} {dtype}", padding_check=True)

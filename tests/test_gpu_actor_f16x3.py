@@ -1,4 +1,4 @@
-"""The "f16x3" actor (``k_actor3h<PRE, O>``: three passes on fp16 halves with per-neuron power-of-two weight scales)
+"""The "f16x3" actor (``k_actor3<SplitF16x3, PRE, O>``: three passes on fp16 halves with per-neuron power-of-two weight scales)
 against its operand-exact reference ``actor_ref_f16x3``: every compared row's ``prob_on`` lies within the
 first-principles bound AND within the fp32-grade tolerance of the plain fp64 forward, and the max |dp| against that
 forward is printed next to the 3xTF32 actor's on the same rows.
